@@ -235,6 +235,26 @@ ME_RANGE = 64          # --SearchRange=64
 ME_MARGIN = 80         # TComPicYuv margin: CTU + 16 (TComPicYuv.cpp:83-84)
 
 
+DUMP_BUDGET_BYTES = 60 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: write each output of the timed path's last step as out_dir/<name>.npy, exact in float64 (float32 for
+    16-bit outputs).  `arrays` maps name -> (device tensor, numpy dtype the tensor's bits hold).  An array larger than its share
+    of DUMP_BUDGET_BYTES is reduced to a fixed sample: the sorted, de-duplicated flat indices drawn by default_rng(0), the same
+    for every run of the same arguments, so that two builds can be compared output for output."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    cap = DUMP_BUDGET_BYTES // (8 * len(arrays))
+    for name, (t, dtype) in arrays.items():
+        flat = t.reshape(-1)
+        if flat.numel() > cap:
+            idx = np.unique(np.random.default_rng(0).integers(0, flat.numel(), cap))
+            flat = flat[torch.from_numpy(idx).to(flat.device)]
+        a = flat.cpu().numpy().view(dtype)
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32 if a.itemsize <= 2 else np.float64))
+
+
 def inter_pus(W, H):
     """the square 2Nx2N PUs of every CU at depths 0..3 that lies inside the picture (85 per whole CTU): (x, y, size)"""
     pus = []
@@ -439,6 +459,10 @@ def run_ours(args, rank, world, local_rank):
     barrier()
     launches = eng.launch_count - l0
     dev_ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"rmd_cost": (d_cost, np.uint32), "obf": (d_obf, np.int16), "outlier": (d_outl, np.int16),
+                                         "ctu_src_had": (d_had, np.int32), **{f"num_obf{d}": (t, np.int32) for d, t in enumerate(d_num)},
+                                         **{f"n_outlier{d}": (t, np.int32) for d, t in enumerate(d_sum)}})
     rmd_ms, n_timed = eng.rmd_kernel_time_ms(min(args.steps, 64))
 
     # ---- end to end through the host-buffer ABI -------------------------------------------------------
@@ -657,6 +681,10 @@ def run_inter(args, rank, world, local_rank):
     barrier()
     launches = eng.launch_count - l0
     dev_ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"rmd_cost": (d_cost, np.uint32), "obf": (d_obf, np.int16), "outlier": (d_outl, np.int16),
+                                         "ctu_src_had": (d_had, np.int32), **{f"me_sad_ref{k}": (d_sad[k], np.uint32) for k in range(NR)},
+                                         **{f"me_subpel_ref{k}": (d_sub[k], np.uint32) for k in range(NR)}})
     me_ms = float(np.mean([a.elapsed_time(b) for a, b in me_ev]))
 
     # ---- end to end: host planes up, every table down ---------------------------------------------------
@@ -759,7 +787,14 @@ def main():
                          "early decisions would skip (cucd_set_decision_switches; switches as a real 416x240 encode held them: Skip2Nx2N on at every depth, "
                          "TerminateCU on at depths 0-2)")
     ap.add_argument("--e2e-instances", type=int, default=2, help="encoder instances (handles + host threads) per GPU in the e2e measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (rank 0's device-resident outputs) as DIR/<name>.npy, "
+                         "float32/float64, at most 60 MiB in all (larger arrays as a fixed seeded sample)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     cfg = CONFIGS[args.config]
     custom = any(v is not None for v in (args.width, args.height, args.bit_depth))
     args.width, args.height = args.width or cfg["width"], args.height or cfg["height"]

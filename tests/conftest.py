@@ -27,11 +27,9 @@ def emul():
 
 @pytest.fixture(scope="session")
 def hmref():
+    """the reference's compiled functions (oracle/_ref/libhmref.so), or None where they were not built"""
     import _util
-    lib = _util.load_hmref()
-    if lib is None:
-        pytest.skip("oracle/_ref/libhmref.so not built (needs /root/reference)")
-    return lib
+    return _util.load_hmref()
 
 
 @pytest.fixture(scope="session")
