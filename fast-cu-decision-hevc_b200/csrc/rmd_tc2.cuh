@@ -168,7 +168,8 @@ struct Cfg {
   // buffers, which are first written after the prologue
   static constexpr int TILE_OFF = B1_OFF;
   static constexpr int TILE_PITCH = 68;                          // 17 words: a column walk touches 32 different banks
-  static constexpr int TILE_TOP = 64 * TILE_PITCH;               // row y = -1, x = -1 .. 127
+  static constexpr int TILE_X0 = 4;                              // tile[y][x] = t[y * TILE_PITCH + TILE_X0 + x], x = -1 .. 63
+  static constexpr int TILE_TOP = 64 * TILE_PITCH;               // row y = -1: top[x] = t[TILE_TOP + TILE_X0 + x], x = -1 .. 127
   static constexpr int TILE_BYTES = al16(TILE_TOP + 136);
   static_assert(CTUS * TILE_BYTES <= kGroups * 2 * B1_BYTES + kGroups * 8192, "tiles must fit the aliased operand buffers");
 };
@@ -183,6 +184,14 @@ template <int LOG2N> CUCD_HD int arr_k0_off(int grp, int slot, int o, int filt) 
   return grp * C::GROUP_BYTES + 16 + slot * C::PU_BYTES + (filt * 2 + o) * C::AS8 + C::N;
 }
 CUCD_HD int rec_off(int ctu, int o, int pu) { return ((ctu * 2 + o) * 256 + pu) * 16; }
+// the cost of element i (= pu * 35 + mode) of the CTA's CTU c in the accumulators at ACC_OFF: uint16 for N = 4, uint32 otherwise
+template <int LOG2N> struct CostRead {
+  const uint32_t* acc;
+  CUCD_HD uint32_t operator()(int c, int i) const {
+    const int e = c * Cfg<LOG2N>::PUS * kNumModes + i;
+    return LOG2N == 2 ? (uint32_t)reinterpret_cast<const uint16_t*>(acc)[e] : acc[e];
+  }
+};
 
 // ---------------------------------------------------------------------------------------------
 // which tile a thread (= MMA row = TMEM lane) owns
@@ -381,31 +390,58 @@ CUCD_HD void dc_region4(const unsigned char* rec, uint32_t* p) {
 // ---------------------------------------------------------------------------------------------
 // prologue: reference arrays of one CTU straight from the reconstruction plane (frame / replay mode)
 // ---------------------------------------------------------------------------------------------
-// Phase 1: the CTU's 64x64 reconstruction block, the row above it (x = -1 .. 127) and the column left of it as
-// bytes in shared memory.  tile[y][x] = t[y * PITCH + 4 + x], y = 0..63, x = -1..63;  top[x] = t[TOP + 4 + x].
-// Samples outside the picture are not touched (never consumed: availability masks them).
+// 8 samples = one 128-bit load (g++ builds the emulators without the CUDA headers, so no uint4), and half of it
+struct alignas(16) Vec16 { uint32_t x, y, z, w; };
+struct alignas(8) Vec8 { uint32_t x, y; };
+
+// Phase 1 (frame / replay mode): the CTU's 64x64 reconstruction block, the row above it (x = -1 .. 127) and the column left of it, split
+// into the global loads (tile_load), issued for all the CTA's CTUs before anything waits, and the shared-memory stores (tile_store).
+// A thread of the CTA's 256 holds two 8-sample chunks of the block, thread t < 64 the left neighbour of row t, thread t < 129 the
+// above neighbour x = t - 1.  Samples outside the picture are not stored (never consumed: availability masks them).
+// Shared with tc3 (uint16 tiles); the frame kernels' set-up is rmd_tc_frame.cuh setup_loads.
+constexpr int kTileThreads = 256;
+struct TileLoad { Vec16 v[2]; int left, top; };
+CUCD_HD void tile_load(int tid, const int16_t* rec, int recStride, int W, int H, int ctuX, int ctuY, TileLoad& t) {
+#pragma unroll
+  for (int it = 0; it < 2; it++) {
+    const int idx = tid + it * kTileThreads, y = idx >> 3, x = (idx & 7) * 8;
+    t.v[it] = Vec16{0u, 0u, 0u, 0u};
+    if (ctuY + y < H && ctuX + x < W) t.v[it] = *reinterpret_cast<const Vec16*>(rec + (size_t)(ctuY + y) * recStride + ctuX + x);
+  }
+  t.left = 0; t.top = 0;
+  if (ctuX > 0 && tid < 64 && ctuY + tid < H) t.left = rec[(size_t)(ctuY + tid) * recStride + ctuX - 1];
+  const int gx = ctuX - 1 + tid;
+  if (ctuY > 0 && tid < 129 && gx >= 0 && gx < W) t.top = rec[(size_t)(ctuY - 1) * recStride + gx];
+}
+// tile[y][x] = dst[y * TILE_PITCH + TILE_X0 + x], top[x] = dst[TILE_TOP + TILE_X0 + x]: bytes (the low byte of each sample, tc2) or
+// the samples themselves (uint16, tc3)
+template <template <int> class Cfg, int LOG2N, class T>
+CUCD_HD void tile_store(int tid, int W, int H, int ctuX, int ctuY, const TileLoad& t, T* dst) {
+  typedef Cfg<LOG2N> C;
+#pragma unroll
+  for (int it = 0; it < 2; it++) {
+    const int idx = tid + it * kTileThreads, y = idx >> 3, x = (idx & 7) * 8;
+    if (ctuY + y >= H || ctuX + x >= W) continue;
+    const Vec16& v = t.v[it];
+    if (sizeof(T) == 1) {
+      uint32_t* d = reinterpret_cast<uint32_t*>(dst + y * C::TILE_PITCH + C::TILE_X0 + x);
+      d[0] = bperm(v.x, v.y, 0x6420); d[1] = bperm(v.z, v.w, 0x6420);
+    } else {
+      Vec8* d = reinterpret_cast<Vec8*>(dst + y * C::TILE_PITCH + C::TILE_X0 + x);      // rows are 8-byte aligned
+      d[0] = Vec8{v.x, v.y}; d[1] = Vec8{v.z, v.w};
+    }
+  }
+  if (ctuX > 0 && tid < 64 && ctuY + tid < H) dst[tid * C::TILE_PITCH + C::TILE_X0 - 1] = (T)t.left;
+  const int gx = ctuX - 1 + tid;
+  if (ctuY > 0 && tid < 129 && gx >= 0 && gx < W) dst[C::TILE_TOP + C::TILE_X0 - 1 + tid] = (T)t.top;
+}
+// phase 1 of one CTU in one call, thread ids tid, tid + nthreads, ... of the 256 (the CPU replay's form)
 template <int LOG2N>
 CUCD_HD void stage_tile(int tid, int nthreads, const int16_t* rec, int recStride, int W, int H, int ctuX, int ctuY, unsigned char* t) {
-  typedef Cfg<LOG2N> C;
-  for (int idx = tid; idx < 64 * 8; idx += nthreads) {
-    const int y = idx >> 3, x = (idx & 7) * 8;
-    if (ctuY + y >= H || ctuX + x >= W) continue;                  // W, H are multiples of 8
-    const int16_t* src = rec + (size_t)(ctuY + y) * recStride + ctuX + x;
-    uint32_t w0, w1;
-#if defined(__CUDA_ARCH__)
-    const uint4 v = *reinterpret_cast<const uint4*>(src);
-    w0 = __byte_perm(v.x, v.y, 0x6420); w1 = __byte_perm(v.z, v.w, 0x6420);
-#else
-    w0 = 0; w1 = 0;
-    for (int i = 0; i < 4; i++) { w0 |= (uint32_t)(src[i] & 0xff) << (8 * i); w1 |= (uint32_t)(src[4 + i] & 0xff) << (8 * i); }
-#endif
-    uint32_t* d = reinterpret_cast<uint32_t*>(t + y * C::TILE_PITCH + 4 + x);
-    d[0] = w0; d[1] = w1;
-  }
-  if (ctuX > 0) for (int y = tid; y < 64; y += nthreads) if (ctuY + y < H) t[y * C::TILE_PITCH + 3] = (unsigned char)rec[(size_t)(ctuY + y) * recStride + ctuX - 1];
-  if (ctuY > 0) for (int x = tid; x < 129; x += nthreads) {
-    const int gx = ctuX - 1 + x;
-    if (gx >= 0 && gx < W) t[C::TILE_TOP + 3 + x] = (unsigned char)rec[(size_t)(ctuY - 1) * recStride + gx];
+  for (int k = tid; k < kTileThreads; k += nthreads) {
+    TileLoad l;
+    tile_load(k, rec, recStride, W, H, ctuX, ctuY, l);
+    tile_store<Cfg, LOG2N>(k, W, H, ctuX, ctuY, l, t);
   }
 }
 
@@ -453,8 +489,8 @@ CUCD_HD void build_unfiltered(int tid, int ctu, int W, int H, int ctuX, int ctuY
   int px, py; demorton(p, px, py);
   const int x0 = px * N, y0 = py * N;
   const PuAvail a = pu_avail<LOG2N>(ctuX + x0, ctuY + y0, W, H);
-  const unsigned char* rowT = y0 == 0 ? t + C::TILE_TOP + 4 + x0 - 1 : t + (y0 - 1) * C::TILE_PITCH + 4 + x0 - 1;   // rowT[k] = T[k]
-  const unsigned char* colL = t + (y0 - 1) * C::TILE_PITCH + 4 + x0 - 1;                                            // colL[k * PITCH] = L[k], k >= 1
+  const unsigned char* rowT = y0 == 0 ? t + C::TILE_TOP + C::TILE_X0 + x0 - 1 : t + (y0 - 1) * C::TILE_PITCH + C::TILE_X0 + x0 - 1;   // rowT[k] = T[k]
+  const unsigned char* colL = t + (y0 - 1) * C::TILE_PITCH + C::TILE_X0 + x0 - 1;                                                    // colL[k * PITCH] = L[k], k >= 1
   const int firstAvail = a.lenL > 0 ? colL[a.lenL * C::TILE_PITCH] : (a.availC ? rowT[0] : (a.lenT > 0 ? rowT[1] : 128));
   const int cval = a.availC ? rowT[0] : (a.lenL > 0 ? colL[C::TILE_PITCH] : firstAvail);
   const int tailT = a.lenT > 0 ? rowT[a.lenT] : cval;

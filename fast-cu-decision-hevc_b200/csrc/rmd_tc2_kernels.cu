@@ -9,10 +9,12 @@
 //     epilogue 1: tcgen05.ld.pack::16b + 16 PRMT -> 64 predicted bytes -> TMEM (A2)
 //     MMA 2: D2 = source tile (shared memory, static) x -(H8 (x) H8) + A2 x (H8 (x) H8)      Hadamard of the residual
 //     epilogue 2: sum |D2|, HM rounding
-// See rmd_tc2.cuh for the arithmetic and the reference citations; planar and DC are predicted on the ALU.
+// See rmd_tc2.cuh for the arithmetic and the reference citations; planar and DC are predicted on the ALU.  The frame-mode set-up
+// loads, PU states and copy-out are shared with rmd_tc3_kernels.cu (rmd_tc_frame.cuh), the tcgen05 wrappers live in satd_tc.cuh.
 // Replaces, per PU, the reference loop TEncSearch.cpp:2327-2361.
 #include <cuda_runtime.h>
 #include "rmd_tc2.cuh"
+#include "rmd_tc_frame.cuh"
 #include "satd_tc.cuh"
 #include "kernels.h"
 
@@ -22,6 +24,7 @@ extern __shared__ __align__(128) unsigned char smem2[];
 
 using namespace tc;
 using namespace tc2;
+using namespace tcf;
 
 // CUCD_TC2_TIMING (profiles/ubench/tc2_timing.cu only): per-CTA clock64 stamps of thread 0 at phase boundaries
 #ifdef CUCD_TC2_TIMING
@@ -53,49 +56,6 @@ struct Tc2Args {
   const uint8_t* tabWin; const uint8_t* tabN4; const int8_t* had;
 };
 
-__device__ __forceinline__ uint32_t make_idesc_i8x(int M, int N, int aSigned, int bSigned) {
-  uint32_t d = 0;
-  d |= 2u << 4;                                   // D = S32
-  d |= (uint32_t)(aSigned ? 1 : 0) << 7;
-  d |= (uint32_t)(bSigned ? 1 : 0) << 10;
-  d |= (uint32_t)(N >> 3) << 17;
-  d |= (uint32_t)(M >> 4) << 24;
-  return d;
-}
-// A operand in TMEM (lane = row, 4 K-bytes per 32-bit column), B through a shared-memory descriptor
-__device__ __forceinline__ void mma_i8_ts(uint32_t tmemD, uint32_t tmemA, uint64_t descB, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::i8 [%0], [%1], %2, %3, {%5, %5, %5, %5}, p;\n\t}\n"
-      :: "r"(tmemD), "r"(tmemA), "l"(descB), "r"(idesc), "r"(accumulate), "r"(0u) : "memory");
-}
-__device__ __forceinline__ void tmem_st8(uint32_t addr, const uint32_t* v) {
-  asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};\n"
-      :: "r"(addr), "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]) : "memory");
-}
-__device__ __forceinline__ void tmem_st16(uint32_t addr, const uint32_t* v) {
-  asm volatile("tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16};\n"
-      :: "r"(addr), "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]), "r"(v[8]), "r"(v[9]),
-         "r"(v[10]), "r"(v[11]), "r"(v[12]), "r"(v[13]), "r"(v[14]), "r"(v[15]) : "memory");
-}
-__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;\n" ::: "memory"); }
-// 32 accumulator columns -> 16 registers: (col 2j & 0xffff) | (col 2j+1 << 16)
-__device__ __forceinline__ void tmem_ld16_pack(uint32_t addr, uint32_t* v) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.pack::16b.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];\n"
-      : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]),
-        "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-      : "r"(addr) : "memory");
-}
-__device__ __forceinline__ void tmem_ld32(uint32_t addr, uint32_t* v) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];\n"
-      : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]),
-        "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]), "=r"(v[16]), "=r"(v[17]), "=r"(v[18]), "=r"(v[19]),
-        "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]), "=r"(v[24]), "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]),
-        "=r"(v[30]), "=r"(v[31])
-      : "r"(addr) : "memory");
-}
 // A CTA = 256 worker threads (the rows) + one MMA-issuing warp per row group.  The workers only ARRIVE on mbarriers when their
 // operands are in place; the issuing warp waits for the 128 arrivals, issues the tcgen05.mma and the bulk copy of the next weights
 // and commits.  (With the issue inside worker warp 0 that warp ran ~490 cycles behind the other three in every round - the
@@ -103,59 +63,10 @@ __device__ __forceinline__ void tmem_ld32(uint32_t addr, uint32_t* v) {
 constexpr int kIssuerThreads = 32 * kGroups;
 constexpr int kCtaThreads = kThreads + kIssuerThreads;
 __device__ __forceinline__ void worker_bar() { asm volatile("bar.sync 1, 256;\n" ::: "memory"); }     // the 256 workers only
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* mbar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;\n" :: "r"(smem_u32(mbar)), "r"(bytes) : "memory");
-}
-// global -> shared bulk copy (TMA engine, 1-D); completes `bytes` on the mbarrier
-__device__ __forceinline__ void bulk_g2s(void* dstSmem, const void* srcGlobal, uint32_t bytes, uint64_t* mbar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];\n"
-               :: "r"(smem_u32(dstSmem)), "l"(srcGlobal), "r"(bytes), "r"(smem_u32(mbar)) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* mbar) { asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];\n" :: "r"(smem_u32(mbar)) : "memory"); }
-// one lane of a converged warp
-__device__ __forceinline__ bool elect_one() {
-  uint32_t pred;
-  asm volatile("{\n\t.reg .pred p;\n\telect.sync _|p, 0xffffffff;\n\tselp.u32 %0, 1, 0, p;\n\t}\n" : "=r"(pred));
-  return pred != 0;
-}
-
-// Phase 1 of the prologue (rmd_tc2.cuh stage_tile) split into its global loads and its shared-memory stores, so that the
-// loads of ALL the CTA's CTUs (and the rows' source tiles, tc2_body) are in flight together: the prologue used to pay four
-// dependent global-memory round trips per CTU, ~4.5 k cycles each CTU, with the CTA's TMEM idle.
-struct TileLoad { uint4 v[2]; int left, top; };
-template <int LOG2N>
-__device__ __forceinline__ void tile_load(int tid, const int16_t* rec, int recStride, int W, int H, int ctuX, int ctuY, TileLoad& t) {
-#pragma unroll
-  for (int it = 0; it < 2; it++) {
-    const int idx = tid + it * kThreads, y = idx >> 3, x = (idx & 7) * 8;
-    t.v[it] = make_uint4(0u, 0u, 0u, 0u);
-    if (ctuY + y < H && ctuX + x < W) t.v[it] = *reinterpret_cast<const uint4*>(rec + (size_t)(ctuY + y) * recStride + ctuX + x);
-  }
-  t.left = 0; t.top = 0;
-  if (ctuX > 0 && tid < 64 && ctuY + tid < H) t.left = rec[(size_t)(ctuY + tid) * recStride + ctuX - 1];
-  const int gx = ctuX - 1 + tid;
-  if (ctuY > 0 && tid < 129 && gx >= 0 && gx < W) t.top = rec[(size_t)(ctuY - 1) * recStride + gx];
-}
-template <int LOG2N>
-__device__ __forceinline__ void tile_store(int tid, int W, int H, int ctuX, int ctuY, const TileLoad& t, unsigned char* dst) {
-  typedef Cfg<LOG2N> C;
-#pragma unroll
-  for (int it = 0; it < 2; it++) {
-    const int idx = tid + it * kThreads, y = idx >> 3, x = (idx & 7) * 8;
-    if (ctuY + y >= H || ctuX + x >= W) continue;
-    uint32_t* d = reinterpret_cast<uint32_t*>(dst + y * C::TILE_PITCH + 4 + x);
-    d[0] = __byte_perm(t.v[it].x, t.v[it].y, 0x6420); d[1] = __byte_perm(t.v[it].z, t.v[it].w, 0x6420);
-  }
-  if (ctuX > 0 && tid < 64 && ctuY + tid < H) dst[tid * C::TILE_PITCH + 3] = (unsigned char)t.left;
-  const int gx = ctuX - 1 + tid;
-  if (ctuY > 0 && tid < 129 && gx >= 0 && gx < W) dst[C::TILE_TOP + 3 + tid] = (unsigned char)t.top;
-}
-
 // ---- prologue: reference arrays of the CTA's CTUs (rmd_tc2.cuh phases 1-3) --------------------------------
 template <int LOG2N, bool FRAME>
 __device__ __forceinline__ void tc2_prologue(const Tc2Args& a, const int unit, const TileLoad* tl, const int* ctuX, const int* ctuY) {
   typedef Cfg<LOG2N> C;
-  constexpr int N = C::N;
   unsigned char* smem = smem2;
   const int tid = threadIdx.x;
   const FrameSource& fs = a.fs;
@@ -186,19 +97,15 @@ __device__ __forceinline__ void tc2_prologue(const Tc2Args& a, const int unit, c
     const int cg = unit * C::CTUS + c;
     uint8_t* valid = smem + C::VALID_OFF + c * 256;
     if (ctuX[c] < 0) {
-      for (int p = tid; p < C::PUS; p += kThreads) valid[p] = 0;
+      for (int p = tid; p < C::PUS; p += kThreads) valid[p] = kPuOutside;
       continue;
     }
-    const uint8_t* need = fs.needed ? fs.needed + ((size_t)cg * kPusPerCtu + pu_offset_of_depth(6 - LOG2N)) : nullptr;
-    for (int p = tid; p < C::PUS; p += kThreads) {
-      int px, py; demorton(p, px, py);
-      const bool inside = (ctuX[c] + (px + 1) * N <= fs.W) && (ctuY[c] + (py + 1) * N <= fs.H);
-      valid[p] = !inside ? kPuOutside : ((need && !need[p]) ? kPuPruned : kPuEvaluate);
-    }
+    const uint8_t* need = ctu_needed<LOG2N>(fs, cg);
+    for (int p = tid; p < C::PUS; p += kThreads) valid[p] = pu_state<LOG2N>(fs, need, ctuX[c], ctuY[c], p);
   }
 #pragma unroll
   for (int c = 0; c < C::CTUS; c++)
-    if (ctuX[c] >= 0) tile_store<LOG2N>(tid, fs.W, fs.H, ctuX[c], ctuY[c], tl[c], smem + C::TILE_OFF + c * C::TILE_BYTES);
+    if (ctuX[c] >= 0) tile_store<Cfg, LOG2N>(tid, fs.W, fs.H, ctuX[c], ctuY[c], tl[c], smem + C::TILE_OFF + c * C::TILE_BYTES);
   worker_bar();
   TC2_STAMP(51);
 #pragma unroll
@@ -220,21 +127,9 @@ __device__ __forceinline__ void tc2_prologue(const Tc2Args& a, const int unit, c
 //     wait MMA1(i) | epilogue 1 -> A2, projected refs of round i+1 | issue MMA2(i) | stage B1/A1 of round i+1 |
 //     wait MMA2(i) | issue MMA1(i+1) | epilogue 2 of round i (costs)
 // TMEM per row group: D1 = columns [0, 64) (A2 aliases its first 16 once they have been read), D2 = [64, 128).
-// first sample of the row's source tile in frame mode (tile origin inside the CTU from the row map)
-template <int LOG2N>
-__device__ __forceinline__ const int16_t* frame_src_ptr(const FrameSource& fs, const Row& r, int cg, int& tileX, int& tileY) {
-  constexpr int N = Cfg<LOG2N>::N;
-  const int pic = cg / fs.ctusPerPic, ctu = cg - pic * fs.ctusPerPic;
-  int px, py; demorton(r.pu, px, py);
-  if (LOG2N == 2) { px *= 8; py *= 8; }
-  else { px = px * N + (r.o ? r.v0 : r.u0); py = py * N + (r.o ? r.u0 : r.v0); }
-  tileX = (ctu % fs.ctusPerRow) * 64 + px; tileY = (ctu / fs.ctusPerRow) * 64 + py;
-  return fs.org + (size_t)pic * fs.orgPicStride + (size_t)tileY * fs.orgStride + tileX;
-}
-
 // `pre`: the eight rows of the source tile of pass 0, loaded by tc2_body before the prologue (frame mode), or nullptr
 template <int LOG2N, bool FRAME>
-__device__ __forceinline__ void tc2_pass(const Tc2Args& a, const int unit, const int pass, const uint32_t tmemBase, uint32_t& ph1, uint32_t& ph2, const uint4* pre) {
+__device__ __forceinline__ void tc2_pass(const Tc2Args& a, const int unit, const int pass, const uint32_t tmemBase, uint32_t& ph1, uint32_t& ph2, const Vec16* pre) {
   typedef Cfg<LOG2N> C;
   constexpr int N = C::N, SEG = RowSeg<LOG2N>::value;
   unsigned char* smem = smem2;
@@ -487,7 +382,7 @@ __device__ __forceinline__ void tc2_issue_pass(const Tc2Args& a, const int pass,
   uint64_t* barT = bars + 4 * kGroups + g;
   const uint32_t uD1 = tmemBase + g * 128, uA2 = uD1, uD2 = uD1 + 64;
   unsigned char* sB1 = smem + C::B1_OFF + g * 2 * C::B1_BYTES;
-  const uint32_t idescPred = make_idesc_i8x(128, 64, 0, 0), idescHad = make_idesc_i8x(128, 64, 0, 1);
+  const uint32_t idescPred = make_idesc_i8(128, 64, 0, 0), idescHad = make_idesc_i8(128, 64, 0, 1);
   const uint64_t dHad = make_desc(smem_u32(smem + C::HAD_OFF), 1024, 128), dHadNeg = make_desc(smem_u32(smem + C::HAD_OFF + 4096), 1024, 128);
   const uint64_t dAorg = make_desc(smem_u32(smem + C::AORG_OFF + g * 8192), 2048, 128);
   const uint64_t dB1 = make_desc(smem_u32(sB1), 1024, 128), dA1 = make_desc(smem_u32(smem + C::A1_OFF + g * 8192), 2048, 128);
@@ -554,46 +449,24 @@ __device__ __noinline__ void tc2_body(const Tc2Args& a, const int unit) {
   unsigned char* smem = smem2;
   const int tid = threadIdx.x, warp = tid >> 5;
   const bool worker = tid < kThreads;               // threads 256.. are the MMA-issuing warps (tc2_issue_pass)
+  uint32_t* acc = reinterpret_cast<uint32_t*>(smem + C::ACC_OFF);
   if (FRAME && a.fs.needed) {
     // fork-aware mode: a CTA none of whose PUs has to be evaluated writes the table codes and leaves
-    const FrameSource& fs = a.fs;
-    int any = 0;
-    if (worker) for (int i = tid; i < C::CTUS * C::PUS; i += kThreads) {
-      const int c = i / C::PUS, p = i - c * C::PUS, cg = unit * C::CTUS + c;
-      if (cg >= a.totalCtus) continue;
-      const int pic = cg / fs.ctusPerPic, ctu = cg - pic * fs.ctusPerPic;
-      int px, py; demorton(p, px, py);
-      const bool inside = ((ctu % fs.ctusPerRow) * 64 + (px + 1) * C::N <= fs.W) && ((ctu / fs.ctusPerRow) * 64 + (py + 1) * C::N <= fs.H);
-      const uint8_t st = !inside ? kPuOutside : (fs.needed[(size_t)cg * kPusPerCtu + pu_offset_of_depth(6 - LOG2N) + p] ? kPuEvaluate : kPuPruned);
-      smem[C::VALID_OFF + c * 256 + p] = st;
-      any |= st == kPuEvaluate;
-    }
+    const int any = worker ? fork_states<Cfg, LOG2N>(a.fs, unit, a.totalCtus, smem + C::VALID_OFF, tid, kThreads) : 0;
     if (!__syncthreads_or(any)) {
-      if (!worker) return;
-      for (int c = 0; c < C::CTUS; c++) {
-        const int cgc = unit * C::CTUS + c;
-        if (cgc >= a.totalCtus) break;
-        const uint8_t* valid = smem + C::VALID_OFF + c * 256;
-        auto val = [&](int i) -> uint32_t { return valid[i / kNumModes] == kPuPruned ? kCostPruned : kCostOutside; };
-        if (fs.out) {
-          uint32_t* o = fs.out + ((size_t)cgc * kPusPerCtu + pu_offset_of_depth(6 - LOG2N)) * kNumModes;
-          for (int i = tid; i < C::PUS * kNumModes; i += kThreads) o[i] = val(i);
-        }
-        if (fs.outPacked) store_packed_depth<LOG2N>(fs.outPacked + (size_t)cgc * kPackedCtuBytes, tid, kThreads, val);
-      }
+      if (worker) copy_out<Cfg, LOG2N>(a.fs, unit, a.totalCtus, smem + C::VALID_OFF, false, CostRead<LOG2N>{acc}, tid, kThreads);
       return;
     }
     if (worker) worker_bar();
   }
   uint32_t* tmemSlot = reinterpret_cast<uint32_t*>(smem + C::BAR_OFF + 96);
-  uint32_t* acc = reinterpret_cast<uint32_t*>(smem + C::ACC_OFF);
   if (tid == 0) {
     for (int i = 0; i < 5 * kGroups; i++)           // MMA done x2 (1 arrival: the commit), operands ready x2 (128 rows), weights landed (1 + bytes)
       mbar_init(reinterpret_cast<uint64_t*>(smem + C::BAR_OFF) + i, (i >= 2 * kGroups && i < 4 * kGroups) ? 128 : 1);
     asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
   }
   uint32_t ph1 = 0, ph2 = 0;
-  uint4 pre[8];
+  Vec16 pre[8];
   if (worker) {
   TC2_STAMP(0);
   if (warp == 0) tmem_alloc(tmemSlot, 256);
@@ -604,31 +477,7 @@ __device__ __noinline__ void tc2_body(const Tc2Args& a, const int unit) {
   const uint4 hadN = reinterpret_cast<const uint4*>(a.had + (LOG2N == 2 ? 8192 : 0))[tid + 256];  // -H
   int ctuX[C::CTUS], ctuY[C::CTUS];
   TileLoad tl[C::CTUS];
-  if (FRAME) {
-#pragma unroll
-    for (int c = 0; c < C::CTUS; c++) {
-      const int cg = unit * C::CTUS + c;
-      ctuX[c] = -1; ctuY[c] = -1;
-      if (cg >= a.totalCtus) continue;                           // CTA-uniform
-      const int pic = cg / a.fs.ctusPerPic, ctu = cg - pic * a.fs.ctusPerPic;
-      ctuX[c] = (ctu % a.fs.ctusPerRow) * 64; ctuY[c] = (ctu / a.fs.ctusPerRow) * 64;
-      tile_load<LOG2N>(tid, a.fs.rec + (size_t)pic * a.fs.recPicStride, a.fs.recStride, a.fs.W, a.fs.H, ctuX[c], ctuY[c], tl[c]);
-    }
-  }
-  if (FRAME) {
-    const Row r0 = row_map<LOG2N>(tid, 0);
-    const int cg0 = unit * C::CTUS + r0.ctu;
-#pragma unroll
-    for (int y = 0; y < 8; y++) pre[y] = make_uint4(0u, 0u, 0u, 0u);
-    if (cg0 < a.totalCtus) {
-      int tx, ty;
-      const int16_t* src = frame_src_ptr<LOG2N>(a.fs, r0, cg0, tx, ty);
-      if (tx + 8 <= a.fs.W && ty + 8 <= a.fs.H) {
-#pragma unroll
-        for (int y = 0; y < 8; y++) pre[y] = *reinterpret_cast<const uint4*>(src + (size_t)y * a.fs.orgStride);
-      }
-    }
-  }
+  if (FRAME) setup_loads<Cfg, LOG2N>(a.fs, unit, a.totalCtus, tid, ctuX, ctuY, tl, pre);
   TC2_STAMP(59);
   if (LOG2N >= 4) for (int i = tid; i < C::CTUS * C::PUS * kNumModes; i += kThreads) acc[i] = 0;   // accumulated with atomics
   reinterpret_cast<int*>(smem + C::DC_OFF)[tid] = 0;          // CTUS * 64 <= 256 sums
@@ -660,48 +509,21 @@ __device__ __noinline__ void tc2_body(const Tc2Args& a, const int unit) {
   tc_fence_before();
   // the common case - every PU of the CTA evaluated - copies the accumulators without a per-element state look-up
   bool mine = true;
-  if (FRAME && worker) for (int i = tid; i < C::CTUS * 256; i += kThreads) mine = mine && ((i & 255) >= C::PUS || smem[C::VALID_OFF + i] == kPuEvaluate);
+  if (FRAME && worker) mine = all_evaluated<Cfg, LOG2N>(smem + C::VALID_OFF, tid, kThreads);
   const bool allEval = __syncthreads_and(mine) && unit * C::CTUS + C::CTUS <= a.totalCtus;
   if (!worker) return;
-  const FrameSource& fs = a.fs;
   if (!FRAME) {
     // batch mode: row outIndex of the caller's [nPU][35] table per PU
     const BatchSource& bs = a.bs;
     for (int i = tid; i < C::CTUS * C::PUS * kNumModes; i += kThreads) {
       const int pl = i / kNumModes, m = i - pl * kNumModes, idx = unit * C::CTUS * C::PUS + pl;
       if (idx >= bs.count) continue;
-      const uint32_t v = LOG2N == 2 ? (uint32_t)reinterpret_cast<const uint16_t*>(acc)[i] : acc[i];
-      bs.out[(size_t)bs.pus[idx].outIndex * kNumModes + m] = v;
+      bs.out[(size_t)bs.pus[idx].outIndex * kNumModes + m] = CostRead<LOG2N>{acc}(0, i);
     }
     if (warp == 0) tmem_dealloc(tmemBase, 256);
     return;
   }
-  for (int c = 0; c < C::CTUS; c++) {
-    const int cgc = unit * C::CTUS + c;
-    if (cgc >= a.totalCtus) break;
-    const uint8_t* valid = smem + C::VALID_OFF + c * 256;
-    const uint16_t* a16 = reinterpret_cast<const uint16_t*>(acc) + c * C::PUS * kNumModes;
-    const uint32_t* a32 = acc + c * C::PUS * kNumModes;
-    auto val = [&](int i) -> uint32_t {
-      const uint8_t v = valid[i / kNumModes];
-      return v == kPuEvaluate ? (LOG2N == 2 ? (uint32_t)a16[i] : a32[i]) : (v == kPuPruned ? kCostPruned : kCostOutside);
-    };
-    auto valAll = [&](int i) -> uint32_t { return LOG2N == 2 ? (uint32_t)a16[i] : a32[i]; };
-    if (fs.out) {
-      uint32_t* o = fs.out + ((size_t)cgc * kPusPerCtu + pu_offset_of_depth(6 - LOG2N)) * kNumModes;
-      if (allEval) {
-#pragma unroll 4
-        for (int i = tid; i < C::PUS * kNumModes; i += kThreads) o[i] = valAll(i);
-      } else {
-#pragma unroll 4
-        for (int i = tid; i < C::PUS * kNumModes; i += kThreads) o[i] = val(i);
-      }
-    }
-    if (fs.outPacked) {
-      if (allEval) store_packed_depth<LOG2N>(fs.outPacked + (size_t)cgc * kPackedCtuBytes, tid, kThreads, valAll);
-      else store_packed_depth<LOG2N>(fs.outPacked + (size_t)cgc * kPackedCtuBytes, tid, kThreads, val);
-    }
-  }
+  copy_out<Cfg, LOG2N>(a.fs, unit, a.totalCtus, smem + C::VALID_OFF, allEval, CostRead<LOG2N>{acc}, tid, kThreads);
   if (warp == 0) tmem_dealloc(tmemBase, 256);
   TC2_STAMP(3);
 #ifdef CUCD_TC2_TIMING
@@ -709,19 +531,17 @@ __device__ __noinline__ void tc2_body(const Tc2Args& a, const int unit) {
 #endif
 }
 
-// blocks of one launch: depth-major (as rmd_frame_kernel); a depth has ceil(totalCtus / CTUS) units
+// blocks of one launch: depth-major (rmd_tc_frame.cuh frame_block)
 __global__ void __launch_bounds__(kCtaThreads, 2)
 rmd_frame_tc2_kernel(const __grid_constant__ Tc2Args a) {
-  const int u2 = (a.totalCtus + 1) >> 1, u4 = (a.totalCtus + 3) >> 2;
-  int b = blockIdx.x;
-  if (b < u4) { tc2_body<6, true>(a, b); return; }
-  b -= u4;
-  if (b < u4) { tc2_body<5, true>(a, b); return; }
-  b -= u4;
-  if (b < u2) { tc2_body<4, true>(a, b); return; }
-  b -= u2;
-  if (b < u2) { tc2_body<3, true>(a, b); return; }
-  tc2_body<2, true>(a, b - u2);
+  const FrameBlock fb = frame_block(a.totalCtus, blockIdx.x);
+  switch (fb.log2n) {
+    case 6: tc2_body<6, true>(a, fb.unit); break;
+    case 5: tc2_body<5, true>(a, fb.unit); break;
+    case 4: tc2_body<4, true>(a, fb.unit); break;
+    case 3: tc2_body<3, true>(a, fb.unit); break;
+    default: tc2_body<2, true>(a, fb.unit);
+  }
 }
 
 // batch (S2) mode: one launch per PU size
@@ -775,8 +595,7 @@ cudaError_t launch_rmd_frames_tc2(const FrameSource& fs, int nPics, int strong, 
   if (total <= 0) return cudaSuccess;
   Tc2Args a;
   a.fs = fs; a.bs = BatchSource{}; a.strong = strong; a.totalCtus = total; a.tabWin = tabWin; a.tabN4 = tabN4; a.had = hadamard;
-  const int u2 = (total + 1) >> 1, u4 = (total + 3) >> 2;
-  rmd_frame_tc2_kernel<<<2 * u4 + 3 * u2, kCtaThreads, kSmemBytes, st>>>(a);
+  rmd_frame_tc2_kernel<<<frame_blocks(total), kCtaThreads, kSmemBytes, st>>>(a);
   if (launches) *launches += 1;
   return cudaGetLastError();
 }

@@ -144,8 +144,9 @@ struct Cfg {
   // 16-bit copy of the reconstruction around each CTU while the reference arrays are built.  N >= 8: aliases the window and
   // source operands (first written after the prologue); N = 4: only the source operand (the records are built into A1).
   static constexpr int TILE_OFF = LOG2N == 2 ? AORG_OFF : A1_OFF;
-  static constexpr int TILE_PITCH = 68;                            // elements; tile[y][x] = t[y * PITCH + 8 + x], x = -1 .. 63
-  static constexpr int TILE_TOP = 64 * TILE_PITCH;                 // row y = -1: top[x] = t[TOP + 8 + x], x = -1 .. 127
+  static constexpr int TILE_PITCH = 68;                            // elements
+  static constexpr int TILE_X0 = 8;                                // tile[y][x] = t[y * TILE_PITCH + TILE_X0 + x], x = -1 .. 63
+  static constexpr int TILE_TOP = 64 * TILE_PITCH;                 // row y = -1: top[x] = t[TILE_TOP + TILE_X0 + x], x = -1 .. 127
   static constexpr int TILE_BYTES = al16(2 * (TILE_TOP + 8 + 128));
   static_assert(CTUS * TILE_BYTES <= BAR_OFF - TILE_OFF, "tiles must fit the aliased operand buffers");
   static_assert(TOTAL <= 113 * 1024, "two CTAs per SM");
@@ -167,6 +168,15 @@ CUCD_HD int rec_slot_off(int ctu, int o, int pu4, int s) {
   const int row = o * 64 + (pu4 >> 2), q = pu4 & 3;
   return Cfg<2>::A1_OFF + ctu * Cfg<2>::A1_BYTES + (2 * q + (s >> 3)) * 2048 + row_chunk(row) + (s & 7) * 2;
 }
+// the cost of element i (= pu * 35 + mode) of the CTA's CTU c in the accumulators at ACC_OFF: final uint16 costs for N <= 8,
+// uint32 sums >> (bitDepth - 8) otherwise
+template <int LOG2N> struct CostRead {
+  const uint32_t* acc; int shift;
+  CUCD_HD uint32_t operator()(int c, int i) const {
+    const int e = c * Cfg<LOG2N>::PUS * kNumModes + i;
+    return LOG2N <= 3 ? (uint32_t)reinterpret_cast<const uint16_t*>(acc)[e] : acc[e] >> shift;
+  }
+};
 CUCD_HD int ld_s16(const unsigned char* p) { return (int)(*reinterpret_cast<const uint16_t*>(p) & 0x3ffu); }   // sample of a stored 1024 + s
 
 // ---------------------------------------------------------------------------------------------
@@ -331,21 +341,15 @@ CUCD_HD void dc_region16(Rec rec, uint32_t* p) {
 }
 
 // ---------------------------------------------------------------------------------------------
-// prologue: reference arrays of one CTU straight from the reconstruction plane (frame / replay mode), as tc2
+// prologue: reference arrays of one CTU straight from the reconstruction plane (frame / replay mode), as tc2; phase 1 is
+// tc2::tile_load / tile_store with 16-bit samples
 // ---------------------------------------------------------------------------------------------
-struct alignas(8) Word2 { uint32_t x, y; };   // four samples
 template <int LOG2N>
 CUCD_HD void stage_tile16(int tid, int nthreads, const int16_t* rec, int recStride, int W, int H, int ctuX, int ctuY, uint16_t* t) {
-  typedef Cfg<LOG2N> C;
-  for (int idx = tid; idx < 64 * 16; idx += nthreads) {
-    const int y = idx >> 4, x = (idx & 15) * 4;
-    if (ctuY + y >= H || ctuX + x >= W) continue;                  // W, H are multiples of 8
-    *reinterpret_cast<Word2*>(t + y * C::TILE_PITCH + 8 + x) = *reinterpret_cast<const Word2*>(rec + (size_t)(ctuY + y) * recStride + ctuX + x);
-  }
-  if (ctuX > 0) for (int y = tid; y < 64; y += nthreads) if (ctuY + y < H) t[y * C::TILE_PITCH + 7] = (uint16_t)rec[(size_t)(ctuY + y) * recStride + ctuX - 1];
-  if (ctuY > 0) for (int x = tid; x < 129; x += nthreads) {
-    const int gx = ctuX - 1 + x;
-    if (gx >= 0 && gx < W) t[C::TILE_TOP + 7 + x] = (uint16_t)rec[(size_t)(ctuY - 1) * recStride + gx];
+  for (int k = tid; k < tc2::kTileThreads; k += nthreads) {
+    tc2::TileLoad l;
+    tc2::tile_load(k, rec, recStride, W, H, ctuX, ctuY, l);
+    tc2::tile_store<Cfg, LOG2N>(k, W, H, ctuX, ctuY, l, t);
   }
 }
 template <int LOG2N>
@@ -369,8 +373,8 @@ CUCD_HD void build_unfiltered16(int tid, int ctu, int W, int H, int ctuX, int ct
   int px, py; demorton(p, px, py);
   const int x0 = px * N, y0 = py * N;
   const PuAvail a = pu_avail<LOG2N>(ctuX + x0, ctuY + y0, W, H);
-  const uint16_t* rowT = y0 == 0 ? t + C::TILE_TOP + 8 + x0 - 1 : t + (y0 - 1) * P + 8 + x0 - 1;   // rowT[k] = T[k]
-  const uint16_t* colL = t + (y0 - 1) * P + 8 + x0 - 1;                                            // colL[k * P] = L[k], k >= 1
+  const uint16_t* rowT = y0 == 0 ? t + C::TILE_TOP + C::TILE_X0 + x0 - 1 : t + (y0 - 1) * P + C::TILE_X0 + x0 - 1;   // rowT[k] = T[k]
+  const uint16_t* colL = t + (y0 - 1) * P + C::TILE_X0 + x0 - 1;                                                    // colL[k * P] = L[k], k >= 1
   const int firstAvail = a.lenL > 0 ? colL[a.lenL * P] : (a.availC ? rowT[0] : (a.lenT > 0 ? rowT[1] : (1 << (bitDepth - 1))));
   const int cval = a.availC ? rowT[0] : (a.lenL > 0 ? colL[P] : firstAvail);
   const int tailT = a.lenT > 0 ? rowT[a.lenT] : cval;

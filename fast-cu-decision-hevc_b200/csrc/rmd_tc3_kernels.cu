@@ -13,10 +13,13 @@
 // MMA 1 weights are fetched by one elected lane with a bulk copy that completes on an mbarrier (no registers, no LDG/STS per
 // thread), N = 4 runs four N = 16, K = 16 products per MMA against one 512-byte table, and every operand byte the tensor
 // core can see is a finite number (the stores are zeroed first: 0 x NaN would poison an accumulator).
+// The frame-mode set-up loads, PU states and copy-out are those of rmd_tc2_kernels.cu (rmd_tc_frame.cuh), the tcgen05 wrappers
+// live in satd_tc.cuh.
 // Replaces, per PU, the reference loop TEncSearch.cpp:2327-2361 for internal bit depths 9 and 10 (8 also works and is tested).
 #include <cuda_runtime.h>
 #include <cuda_fp16.h>
 #include "rmd_tc3.cuh"
+#include "rmd_tc_frame.cuh"
 #include "satd_tc.cuh"
 #include "kernels.h"
 
@@ -26,6 +29,7 @@ extern __shared__ __align__(128) unsigned char smem3[];
 
 using namespace tc;
 using namespace tc3;
+using namespace tcf;
 
 namespace {
 
@@ -35,94 +39,10 @@ struct Tc3Args {
   const uint8_t* tabWin; const uint8_t* tabN4; const uint8_t* had;
 };
 
-// kind::f16 instruction descriptor: D f32, A and B f16 K-major, M x N; aNeg negates the A operand
-__device__ __forceinline__ uint32_t make_idesc_f16(int M, int N, int aNeg) {
-  uint32_t d = 0;
-  d |= 1u << 4;                                   // D = F32
-  d |= (uint32_t)(aNeg ? 1 : 0) << 13;
-  d |= (uint32_t)(N >> 3) << 17;
-  d |= (uint32_t)(M >> 4) << 24;
-  return d;
-}
-__device__ __forceinline__ void mma_f16_ss(uint32_t tmemD, uint64_t descA, uint64_t descB, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}\n"
-      :: "r"(tmemD), "l"(descA), "l"(descB), "r"(idesc), "r"(accumulate) : "memory");
-}
-// A operand in TMEM (lane = row, two K elements per 32-bit column)
-__device__ __forceinline__ void mma_f16_ts(uint32_t tmemD, uint32_t tmemA, uint64_t descB, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}\n"
-      :: "r"(tmemD), "r"(tmemA), "l"(descB), "r"(idesc), "r"(accumulate) : "memory");
-}
-__device__ __forceinline__ void tmem_st32(uint32_t addr, const uint32_t* v) {
-  asm volatile(
-      "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31,%32};\n"
-      :: "r"(addr), "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]), "r"(v[8]), "r"(v[9]), "r"(v[10]),
-         "r"(v[11]), "r"(v[12]), "r"(v[13]), "r"(v[14]), "r"(v[15]), "r"(v[16]), "r"(v[17]), "r"(v[18]), "r"(v[19]), "r"(v[20]), "r"(v[21]),
-         "r"(v[22]), "r"(v[23]), "r"(v[24]), "r"(v[25]), "r"(v[26]), "r"(v[27]), "r"(v[28]), "r"(v[29]), "r"(v[30]), "r"(v[31]) : "memory");
-}
-__device__ __forceinline__ void tmem_st_wait3() { asm volatile("tcgen05.wait::st.sync.aligned;\n" ::: "memory"); }
-// 32 accumulator columns -> 16 registers: (col 2j & 0xffff) | (col 2j+1 << 16)
-__device__ __forceinline__ void tmem_ld16_pack3(uint32_t addr, uint32_t* v) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.pack::16b.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];\n"
-      : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]),
-        "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-      : "r"(addr) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive3(uint64_t* mbar) { asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];\n" :: "r"(smem_u32(mbar)) : "memory"); }
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* mbar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;\n" :: "r"(smem_u32(mbar)), "r"(bytes) : "memory");
-}
-// global -> shared bulk copy (TMA engine, 1-D); completes `bytes` on the mbarrier
-__device__ __forceinline__ void bulk_g2s(void* dstSmem, const void* srcGlobal, uint32_t bytes, uint64_t* mbar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];\n"
-               :: "r"(smem_u32(dstSmem)), "l"(srcGlobal), "r"(bytes), "r"(smem_u32(mbar)) : "memory");
-}
-__device__ __forceinline__ bool elect_one3() {
-  uint32_t pred;
-  asm volatile("{\n\t.reg .pred p;\n\telect.sync _|p, 0xffffffff;\n\tselp.u32 %0, 1, 0, p;\n\t}\n" : "=r"(pred));
-  return pred != 0;
-}
-
-// Phase 1 of the prologue (rmd_tc3.cuh stage_tile16) split into its global loads and its shared-memory stores, so that the
-// loads of all the CTA's CTUs, the Hadamard operand and the rows' source tiles share one memory round trip (tc3_body).
-struct TileLoad { uint4 v[2]; int left, top; };
-__device__ __forceinline__ void tile_load(int tid, const int16_t* rec, int recStride, int W, int H, int ctuX, int ctuY, TileLoad& t) {
-#pragma unroll
-  for (int it = 0; it < 2; it++) {
-    const int idx = tid + it * kThreads, y = idx >> 3, x = (idx & 7) * 8;
-    t.v[it] = make_uint4(0u, 0u, 0u, 0u);
-    if (ctuY + y < H && ctuX + x < W) t.v[it] = *reinterpret_cast<const uint4*>(rec + (size_t)(ctuY + y) * recStride + ctuX + x);
-  }
-  t.left = 0; t.top = 0;
-  if (ctuX > 0 && tid < 64 && ctuY + tid < H) t.left = rec[(size_t)(ctuY + tid) * recStride + ctuX - 1];
-  const int gx = ctuX - 1 + tid;
-  if (ctuY > 0 && tid < 129 && gx >= 0 && gx < W) t.top = rec[(size_t)(ctuY - 1) * recStride + gx];
-}
-template <int LOG2N>
-__device__ __forceinline__ void tile_store(int tid, int W, int H, int ctuX, int ctuY, const TileLoad& t, uint16_t* dst) {
-  typedef Cfg<LOG2N> C;
-#pragma unroll
-  for (int it = 0; it < 2; it++) {
-    const int idx = tid + it * kThreads, y = idx >> 3, x = (idx & 7) * 8;
-    if (ctuY + y >= H || ctuX + x >= W) continue;
-    uint2* d = reinterpret_cast<uint2*>(dst + y * C::TILE_PITCH + 8 + x);      // rows are 8-byte aligned (pitch 136 B)
-    d[0] = make_uint2(t.v[it].x, t.v[it].y); d[1] = make_uint2(t.v[it].z, t.v[it].w);
-  }
-  if (ctuX > 0 && tid < 64 && ctuY + tid < H) dst[tid * C::TILE_PITCH + 7] = (uint16_t)t.left;
-  const int gx = ctuX - 1 + tid;
-  if (ctuY > 0 && tid < 129 && gx >= 0 && gx < W) dst[C::TILE_TOP + 7 + tid] = (uint16_t)t.top;
-}
-
 // ---- prologue: reference arrays of the CTA's CTUs (rmd_tc3.cuh phases 1-3) --------------------------------
 template <int LOG2N>
 __device__ __forceinline__ void tc3_prologue(const Tc3Args& a, const int unit, const TileLoad* tl, const int* ctuX, const int* ctuY) {
   typedef Cfg<LOG2N> C;
-  constexpr int N = C::N;
   unsigned char* smem = smem3;
   const int tid = threadIdx.x;
   const FrameSource& fs = a.fs;
@@ -131,16 +51,12 @@ __device__ __forceinline__ void tc3_prologue(const Tc3Args& a, const int unit, c
     const int cg = unit * C::CTUS + c;
     uint8_t* valid = smem + C::VALID_OFF + c * 256;
     if (ctuX[c] < 0) {                                         // CTA-uniform
-      for (int p = tid; p < C::PUS; p += kThreads) valid[p] = 0;
+      for (int p = tid; p < C::PUS; p += kThreads) valid[p] = kPuOutside;
       continue;
     }
-    const uint8_t* need = fs.needed ? fs.needed + ((size_t)cg * kPusPerCtu + pu_offset_of_depth(6 - LOG2N)) : nullptr;
-    for (int p = tid; p < C::PUS; p += kThreads) {
-      int px, py; demorton(p, px, py);
-      const bool inside = (ctuX[c] + (px + 1) * N <= fs.W) && (ctuY[c] + (py + 1) * N <= fs.H);
-      valid[p] = !inside ? kPuOutside : ((need && !need[p]) ? kPuPruned : kPuEvaluate);
-    }
-    tile_store<LOG2N>(tid, fs.W, fs.H, ctuX[c], ctuY[c], tl[c], reinterpret_cast<uint16_t*>(smem + C::TILE_OFF + c * C::TILE_BYTES));
+    const uint8_t* need = ctu_needed<LOG2N>(fs, cg);
+    for (int p = tid; p < C::PUS; p += kThreads) valid[p] = pu_state<LOG2N>(fs, need, ctuX[c], ctuY[c], p);
+    tile_store<Cfg, LOG2N>(tid, fs.W, fs.H, ctuX[c], ctuY[c], tl[c], reinterpret_cast<uint16_t*>(smem + C::TILE_OFF + c * C::TILE_BYTES));
   }
   __syncthreads();
 #pragma unroll
@@ -157,22 +73,10 @@ __device__ __forceinline__ void tc3_prologue(const Tc3Args& a, const int unit, c
 
 // ---- the mode rounds of one pass (pipeline of rmd_tc2_kernels.cu tc2_pass) ------------------------------------------
 // TMEM per row group: D1 = columns [0, 64) (A2 aliases its first 32 once they have been read), D2 = [64, 128).
-// first sample of the row's source tile (tile origin inside the CTU from the row map)
-template <int LOG2N>
-__device__ __forceinline__ const int16_t* frame_src_ptr(const FrameSource& fs, const Row& r, int cg, int& tileX, int& tileY) {
-  constexpr int N = Cfg<LOG2N>::N;
-  const int pic = cg / fs.ctusPerPic, ctu = cg - pic * fs.ctusPerPic;
-  int px, py; demorton(r.pu, px, py);
-  if (LOG2N == 2) { px *= 8; py *= 8; }
-  else { px = px * N + (r.o ? r.v0 : r.u0); py = py * N + (r.o ? r.u0 : r.v0); }
-  tileX = (ctu % fs.ctusPerRow) * 64 + px; tileY = (ctu / fs.ctusPerRow) * 64 + py;
-  return fs.org + (size_t)pic * fs.orgPicStride + (size_t)tileY * fs.orgStride + tileX;
-}
-
 // `pre`: the eight rows of the source tile of pass 0, loaded by tc3_body before the prologue
 template <int LOG2N>
 __device__ __forceinline__ void tc3_pass(const Tc3Args& a, const int unit, const int pass, const uint32_t tmemBase, uint32_t& ph1, uint32_t& ph2,
-                                         uint32_t& phA, uint32_t& phB, uint32_t& phT, const uint4* pre) {
+                                         uint32_t& phA, uint32_t& phB, uint32_t& phT, const Vec16* pre) {
   typedef Cfg<LOG2N> C;
   constexpr int N = C::N, SEG = RowSeg<LOG2N>::value;
   unsigned char* smem = smem3;
@@ -245,15 +149,15 @@ __device__ __forceinline__ void tc3_pass(const Tc3Args& a, const int unit, const
 
   // -(source) x H + A2 (already stored to TMEM by every thread) x H -> D2
   auto arrive_mma2 = [&]() {
-    tmem_st_wait3();
+    tmem_st_wait();
     tc_fence_before();
-    mbar_arrive3(arrA);
+    mbar_arrive(arrA);
   };
   auto fire_mma2 = [&]() {
     if (issuer) {
       mbar_wait(uarrA, phA);
       tc_fence_after();
-      if (elect_one3()) {
+      if (elect_one()) {
         // A2 holds the residual pred - src itself (exact in fp16: |.| <= 1023): one product, no source operand
         if (LOG2N == 2) {
 #pragma unroll
@@ -274,12 +178,12 @@ __device__ __forceinline__ void tc3_pass(const Tc3Args& a, const int unit, const
   auto issue_mma1 = [&]() {
     fence_async_smem();
     tc_fence_before();
-    mbar_arrive3(arrB);
+    mbar_arrive(arrB);
     if (issuer) {
       mbar_wait(uarrB, phB);
       mbar_wait(ubarT, phT);
       tc_fence_after();
-      if (elect_one3()) {
+      if (elect_one()) {
         if (LOG2N == 2) {
 #pragma unroll
           for (int q = 0; q < 4; q++) mma_f16_ss(uD1 + 16 * q, dA1 + q * kStepA, dB1, idescPred, 0u);
@@ -297,7 +201,7 @@ __device__ __forceinline__ void tc3_pass(const Tc3Args& a, const int unit, const
   // weights of round `am`: one bulk copy per row group.  The buffer is free: the MMA 1 that read it has completed.
   auto fetch_weights = [&](int am, int angle) {
     if (issuer) {
-      if (elect_one3()) {
+      if (elect_one()) {
         const uint8_t* src = LOG2N == 2 ? a.tabN4 + (am + 8) * kN4Table16
                                         : a.tabWin + ((am + 8) * 4 + (group_frac0<LOG2N>(grpU, pass, angle) >> 3)) * kWinTable16;
         mbar_expect_tx(ubarT, C::B1_BYTES);
@@ -413,8 +317,8 @@ __device__ __forceinline__ void tc3_pass(const Tc3Args& a, const int unit, const
     // epilogue 1: the low 16 bits of every accumulator hold 32768 + 32 * pred + remainder
     {
       uint32_t v[32];
-      tmem_ld16_pack3(tD1 + laneOff, v);
-      tmem_ld16_pack3(tD1 + laneOff + 32, v + 16);
+      tmem_ld16_pack(tD1 + laneOff, v);
+      tmem_ld16_pack(tD1 + laneOff + 32, v + 16);
       tmem_ld_wait();
 #pragma unroll
       for (int i = 0; i < 32; i++) p[i] = pack_pred16(v[i]);
@@ -446,39 +350,17 @@ __device__ __noinline__ void tc3_body(const Tc3Args& a, const int unit) {
   unsigned char* smem = smem3;
   const int tid = threadIdx.x, warp = tid >> 5;
   const int shift = a.bitDepth - 8;
+  uint32_t* acc = reinterpret_cast<uint32_t*>(smem + C::ACC_OFF);
   if (a.fs.needed) {
     // fork-aware mode: a CTA none of whose PUs has to be evaluated writes the table codes and leaves
-    const FrameSource& fs = a.fs;
-    int any = 0;
-    for (int i = tid; i < C::CTUS * C::PUS; i += kThreads) {
-      const int c = i / C::PUS, p = i - c * C::PUS, cg = unit * C::CTUS + c;
-      if (cg >= a.totalCtus) continue;
-      const int pic = cg / fs.ctusPerPic, ctu = cg - pic * fs.ctusPerPic;
-      int px, py; demorton(p, px, py);
-      const bool inside = ((ctu % fs.ctusPerRow) * 64 + (px + 1) * C::N <= fs.W) && ((ctu / fs.ctusPerRow) * 64 + (py + 1) * C::N <= fs.H);
-      const uint8_t st = !inside ? kPuOutside : (fs.needed[(size_t)cg * kPusPerCtu + pu_offset_of_depth(6 - LOG2N) + p] ? kPuEvaluate : kPuPruned);
-      smem[C::VALID_OFF + c * 256 + p] = st;
-      any |= st == kPuEvaluate;
-    }
-    if (!__syncthreads_or(any)) {
-      for (int c = 0; c < C::CTUS; c++) {
-        const int cgc = unit * C::CTUS + c;
-        if (cgc >= a.totalCtus) break;
-        const uint8_t* valid = smem + C::VALID_OFF + c * 256;
-        auto val = [&](int i) -> uint32_t { return valid[i / kNumModes] == kPuPruned ? kCostPruned : kCostOutside; };
-        if (fs.out) {
-          uint32_t* o = fs.out + ((size_t)cgc * kPusPerCtu + pu_offset_of_depth(6 - LOG2N)) * kNumModes;
-          for (int i = tid; i < C::PUS * kNumModes; i += kThreads) o[i] = val(i);
-        }
-        if (fs.outPacked) store_packed_depth<LOG2N>(fs.outPacked + (size_t)cgc * kPackedCtuBytes, tid, kThreads, val);
-      }
+    if (!__syncthreads_or(fork_states<Cfg, LOG2N>(a.fs, unit, a.totalCtus, smem + C::VALID_OFF, tid, kThreads))) {
+      copy_out<Cfg, LOG2N>(a.fs, unit, a.totalCtus, smem + C::VALID_OFF, false, CostRead<LOG2N>{acc, shift}, tid, kThreads);
       return;
     }
     __syncthreads();
   }
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + C::BAR_OFF);
   uint32_t* tmemSlot = reinterpret_cast<uint32_t*>(smem + C::BAR_OFF + 96);
-  uint32_t* acc = reinterpret_cast<uint32_t*>(smem + C::ACC_OFF);
   if (tid == 0) {
     for (int i = 0; i < 5 * kGroups; i++) mbar_init(bars + i, (i >= 2 * kGroups && i < 4 * kGroups) ? 128 : 1);   // MMA done x2, operands ready x2, weights landed
     asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
@@ -495,30 +377,8 @@ __device__ __noinline__ void tc3_body(const Tc3Args& a, const int unit) {
   }
   int ctuX[C::CTUS], ctuY[C::CTUS];
   TileLoad tl[C::CTUS];
-#pragma unroll
-  for (int c = 0; c < C::CTUS; c++) {
-    const int cg = unit * C::CTUS + c;
-    ctuX[c] = -1; ctuY[c] = -1;
-    if (cg >= a.totalCtus) continue;                           // CTA-uniform
-    const int pic = cg / a.fs.ctusPerPic, ctu = cg - pic * a.fs.ctusPerPic;
-    ctuX[c] = (ctu % a.fs.ctusPerRow) * 64; ctuY[c] = (ctu / a.fs.ctusPerRow) * 64;
-    tile_load(tid, a.fs.rec + (size_t)pic * a.fs.recPicStride, a.fs.recStride, a.fs.W, a.fs.H, ctuX[c], ctuY[c], tl[c]);
-  }
-  uint4 pre[8];
-  {
-    const Row r0 = row_map<LOG2N>(tid, 0);
-    const int cg0 = unit * C::CTUS + r0.ctu;
-#pragma unroll
-    for (int y = 0; y < 8; y++) pre[y] = make_uint4(0u, 0u, 0u, 0u);
-    if (cg0 < a.totalCtus) {
-      int tx, ty;
-      const int16_t* src = frame_src_ptr<LOG2N>(a.fs, r0, cg0, tx, ty);
-      if (tx + 8 <= a.fs.W && ty + 8 <= a.fs.H) {
-#pragma unroll
-        for (int y = 0; y < 8; y++) pre[y] = *reinterpret_cast<const uint4*>(src + (size_t)y * a.fs.orgStride);
-      }
-    }
-  }
+  Vec16 pre[8];
+  setup_loads<Cfg, LOG2N>(a.fs, unit, a.totalCtus, tid, ctuX, ctuY, tl, pre);
   // every byte a window, a record or an accumulator update may touch starts as zero (finite operands; sums for N >= 16)
   {
     const uint4 z = make_uint4(0u, 0u, 0u, 0u);
@@ -548,52 +408,22 @@ __device__ __noinline__ void tc3_body(const Tc3Args& a, const int unit) {
   // ---- costs leave the SM ------------------------------------------------------------------------------------
   tc_fence_before();
   // the common case - every PU of the CTA evaluated - copies the accumulators without a per-element state look-up
-  bool mine = true;
-  for (int i = tid; i < C::CTUS * 256; i += kThreads) mine = mine && ((i & 255) >= C::PUS || smem[C::VALID_OFF + i] == kPuEvaluate);
-  const bool allEval = __syncthreads_and(mine) && unit * C::CTUS + C::CTUS <= a.totalCtus;
-  const FrameSource& fs = a.fs;
-  for (int c = 0; c < C::CTUS; c++) {
-    const int cgc = unit * C::CTUS + c;
-    if (cgc >= a.totalCtus) break;
-    const uint8_t* valid = smem + C::VALID_OFF + c * 256;
-    const uint16_t* a16 = reinterpret_cast<const uint16_t*>(acc) + c * C::PUS * kNumModes;
-    const uint32_t* a32 = acc + c * C::PUS * kNumModes;
-    auto val = [&](int i) -> uint32_t {
-      const uint8_t v = valid[i / kNumModes];
-      return v == kPuEvaluate ? (LOG2N <= 3 ? (uint32_t)a16[i] : (a32[i] >> shift)) : (v == kPuPruned ? kCostPruned : kCostOutside);
-    };
-    auto valAll = [&](int i) -> uint32_t { return LOG2N <= 3 ? (uint32_t)a16[i] : (a32[i] >> shift); };
-    if (fs.out) {
-      uint32_t* o = fs.out + ((size_t)cgc * kPusPerCtu + pu_offset_of_depth(6 - LOG2N)) * kNumModes;
-      if (allEval) {
-#pragma unroll 4
-        for (int i = tid; i < C::PUS * kNumModes; i += kThreads) o[i] = valAll(i);
-      } else {
-#pragma unroll 4
-        for (int i = tid; i < C::PUS * kNumModes; i += kThreads) o[i] = val(i);
-      }
-    }
-    if (fs.outPacked) {
-      if (allEval) store_packed_depth<LOG2N>(fs.outPacked + (size_t)cgc * kPackedCtuBytes, tid, kThreads, valAll);
-      else store_packed_depth<LOG2N>(fs.outPacked + (size_t)cgc * kPackedCtuBytes, tid, kThreads, val);
-    }
-  }
+  const bool allEval = __syncthreads_and(all_evaluated<Cfg, LOG2N>(smem + C::VALID_OFF, tid, kThreads)) && unit * C::CTUS + C::CTUS <= a.totalCtus;
+  copy_out<Cfg, LOG2N>(a.fs, unit, a.totalCtus, smem + C::VALID_OFF, allEval, CostRead<LOG2N>{acc, shift}, tid, kThreads);
   if (warp == 0) tmem_dealloc(tmemBase, 256);
 }
 
-// blocks of one launch: depth-major (as rmd_frame_tc2_kernel); a depth has ceil(totalCtus / CTUS) units
+// blocks of one launch: depth-major (rmd_tc_frame.cuh frame_block)
 __global__ void __launch_bounds__(kThreads, 2)
 rmd_frame_tc3_kernel(const __grid_constant__ Tc3Args a) {
-  const int u2 = (a.totalCtus + 1) >> 1, u4 = (a.totalCtus + 3) >> 2;
-  int b = blockIdx.x;
-  if (b < u4) { tc3_body<6>(a, b); return; }
-  b -= u4;
-  if (b < u4) { tc3_body<5>(a, b); return; }
-  b -= u4;
-  if (b < u2) { tc3_body<4>(a, b); return; }
-  b -= u2;
-  if (b < u2) { tc3_body<3>(a, b); return; }
-  tc3_body<2>(a, b - u2);
+  const FrameBlock fb = frame_block(a.totalCtus, blockIdx.x);
+  switch (fb.log2n) {
+    case 6: tc3_body<6>(a, fb.unit); break;
+    case 5: tc3_body<5>(a, fb.unit); break;
+    case 4: tc3_body<4>(a, fb.unit); break;
+    case 3: tc3_body<3>(a, fb.unit); break;
+    default: tc3_body<2>(a, fb.unit);
+  }
 }
 
 }  // namespace
@@ -610,8 +440,7 @@ cudaError_t launch_rmd_frames_tc3(const FrameSource& fs, int nPics, int bitDepth
   if (total <= 0) return cudaSuccess;
   Tc3Args a;
   a.fs = fs; a.strong = strong; a.totalCtus = total; a.bitDepth = bitDepth; a.tabWin = tabWin16; a.tabN4 = tabN416; a.had = hadamard16;
-  const int u2 = (total + 1) >> 1, u4 = (total + 3) >> 2;
-  rmd_frame_tc3_kernel<<<2 * u4 + 3 * u2, kThreads, kSmemBytes, st>>>(a);
+  rmd_frame_tc3_kernel<<<frame_blocks(total), kThreads, kSmemBytes, st>>>(a);
   if (launches) *launches += 1;
   return cudaGetLastError();
 }

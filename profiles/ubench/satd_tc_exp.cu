@@ -31,7 +31,7 @@ satd_tc_exp_kernel(const uint8_t* __restrict__ org, const uint8_t* __restrict__ 
   __syncthreads();
   tc_fence_after();
   const uint32_t tmemBase = tmemSlot;
-  const uint32_t idesc = make_idesc_i8(128, 64, 0);
+  const uint32_t idesc = make_idesc_i8(128, 64, 0, 1);
   const uint64_t dAO = make_desc(smem_u32(sAO), 2048, 128), dAP = make_desc(smem_u32(sAP), 2048, 128);
   const uint64_t dBp = make_desc(smem_u32(sBpos), 1024, 128), dBn = make_desc(smem_u32(sBneg), 1024, 128);
   uint32_t parity = 0;

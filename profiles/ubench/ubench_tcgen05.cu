@@ -9,17 +9,6 @@
 #include "satd_tc.cuh"
 using namespace cucd::tc;
 
-__device__ __forceinline__ void tmem_st16(uint32_t addr, const uint32_t* v) {
-  asm volatile("tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16};\n"
-      :: "r"(addr), "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]), "r"(v[8]), "r"(v[9]),
-         "r"(v[10]), "r"(v[11]), "r"(v[12]), "r"(v[13]), "r"(v[14]), "r"(v[15]) : "memory");
-  asm volatile("tcgen05.wait::st.sync.aligned;\n" ::: "memory");
-}
-__device__ __forceinline__ void tmem_ld16_pack(uint32_t addr, uint32_t* v) {
-  asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.pack::16b.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];\n"
-      : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]),
-        "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]) : "r"(addr) : "memory");
-}
 #define LD32_ASM(PACK) \
   asm volatile("tcgen05.ld.sync.aligned.32x32b.x32" PACK ".b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];\n" \
       : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]), \
@@ -40,6 +29,7 @@ __global__ void k_pack(uint32_t* out) {
   for (int h = 0; h < 2; h++) {
     for (int c = 0; c < 16; c++) v[c] = (uint32_t)(0x100 * (h * 16 + c) + lane) | ((uint32_t)(0xA000 + h * 16 + c) << 16);
     tmem_st16(base + h * 16, v);
+    tmem_st_wait();
   }
   tc_fence_before(); __syncthreads(); tc_fence_after();
   tmem_ld16_pack(base, v); tmem_ld_wait();
@@ -111,12 +101,6 @@ __global__ void k_mma(const uint8_t* A /*128x32 row-major*/, const uint8_t* B /*
 
 
 // ---- E: A operand in TMEM (one row per lane, K bytes packed 4 per 32-bit column) ---------------------
-__device__ __forceinline__ void mma_i8_ts(uint32_t tmemD, uint32_t tmemA, uint64_t descB, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::i8 [%0], [%1], %2, %3, {%5, %5, %5, %5}, p;\n\t}\n"
-      :: "r"(tmemD), "r"(tmemA), "l"(descB), "r"(idesc), "r"(accumulate), "r"(0u) : "memory");
-}
 __global__ void k_mma_ts(const uint8_t* A /*128x64 row-major*/, const uint8_t* B /*64x64 row-major*/, uint32_t* D /*128x64*/) {
   extern __shared__ __align__(128) unsigned char sm[];
   unsigned char* sB = sm;
@@ -131,6 +115,7 @@ __global__ void k_mma_ts(const uint8_t* A /*128x64 row-major*/, const uint8_t* B
   uint32_t v[16];
   for (int c = 0; c < 16; c++) v[c] = reinterpret_cast<const uint32_t*>(A + tid * 64)[c];
   tmem_st16(tmem + lane0 + 64, v);                 // A at columns 64..79, D at 0..63
+  tmem_st_wait();
   tc_fence_before(); __syncthreads(); tc_fence_after();
   if (tid == 0) {
     const uint64_t dB = make_desc(smem_u32(sB), 1024, 128);

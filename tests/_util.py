@@ -62,7 +62,7 @@ def load_emul():
     so = os.path.join(d, "librmd_emul.so")
     csrc = os.path.join(ROOT, PKG, "csrc")
     cpps = [os.path.join(d, "rmd_emul.cpp"), os.path.join(d, "rmd_tc2_emul.cpp"), os.path.join(d, "rmd_tc3_emul.cpp"), os.path.join(d, "me_emul.cpp")]
-    srcs = cpps + [os.path.join(csrc, f) for f in ("rmd_core.cuh", "rmd_chunk.cuh", "rmd_tc2.cuh", "rmd_tc3.cuh", "feature_core.cuh", "me_core.cuh")]
+    srcs = cpps + [os.path.join(csrc, f) for f in ("rmd_core.cuh", "rmd_chunk.cuh", "rmd_tc2.cuh", "rmd_tc3.cuh", "rmd_tc_frame.cuh", "feature_core.cuh", "me_core.cuh")]
     if not _newer(so, srcs):
         subprocess.run(["g++", "-std=c++17", "-O2", "-fPIC", "-shared", "-Wno-unknown-pragmas", "-I" + csrc, "-o", so] + cpps,
                        check=True, capture_output=True)

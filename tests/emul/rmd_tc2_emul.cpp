@@ -1,8 +1,9 @@
 // rmd_tc2_emul.cpp - CPU replay of the tensor-core RMD frame kernel (TEST HARNESS, not a product path).
 //
 // Compiles csrc/rmd_tc2.cuh (the kernel's __host__ __device__ logic: weight tables, row map, window
-// gather, byte packing, planar/DC, border conversion) with g++ and replays one CTA of rmd_tc2_kernels.cu
-// phase by phase for all 512 thread ids.  The two tcgen05 products are replaced by exact integer matmuls
+// gather, byte packing, planar/DC, border conversion) and csrc/rmd_tc_frame.cuh (block decode, PU states, set-up
+// loads, tile staging, copy-out) with g++ and replays one CTA of rmd_tc2_kernels.cu phase by phase for all 256
+// worker thread ids.  The two tcgen05 products are replaced by exact integer matmuls
 // that read their operands through the same UMMA shared-memory layout / TMEM row layout the kernel uses,
 // and tcgen05.ld.pack::16b by its measured behaviour (profiles/ubench).  Built only by tests/.
 #include <cstdint>
@@ -10,9 +11,11 @@
 #include <type_traits>
 #include <vector>
 #include "rmd_tc2.cuh"
+#include "rmd_tc_frame.cuh"
 
 using namespace cucd;
 using namespace cucd::tc2;
+using namespace cucd::tcf;
 
 namespace {
 
@@ -59,8 +62,14 @@ void emul_cta(const FrameSource& fs, int strong, int totalCtus, int unit, const 
   std::vector<unsigned char> smemStore(C::TOTAL + 256, 0xA5);
   unsigned char* smem = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(smemStore.data()) + 127) & ~uintptr_t(127));
   uint32_t* acc = reinterpret_cast<uint32_t*>(smem + C::ACC_OFF);
+  uint8_t* valid = smem + C::VALID_OFF;
+  if (!bs && fs.needed && !fork_states<Cfg, LOG2N>(fs, unit, totalCtus, valid, 0, 1)) {   // fork-aware early exit (tc2_body)
+    copy_out<Cfg, LOG2N>(fs, unit, totalCtus, valid, false, CostRead<LOG2N>{acc}, 0, 1);
+    return;
+  }
   if (LOG2N >= 4) for (int i = 0; i < C::CTUS * C::PUS * kNumModes; i++) acc[i] = 0;
   for (int i = 0; i < C::CTUS * 64; i++) reinterpret_cast<int*>(smem + C::DC_OFF)[i] = 0;
+  std::vector<Vec16> pre(kThreads * 8);            // frame mode: the rows' source tiles of pass 0 (setup_loads)
   // ---- prologue (tc2_prologue) ----
   if (bs) {
     constexpr int TPP = 256 / C::PUS;
@@ -77,17 +86,15 @@ void emul_cta(const FrameSource& fs, int strong, int totalCtus, int unit, const 
       if ((unit * C::CTUS + c) * C::PUS < bs->count) for (int tid = 0; tid < kThreads; tid++) build_filtered<LOG2N>(tid, c, strong, smem);
   } else {
   int ctuXs[C::CTUS], ctuYs[C::CTUS];
+  TileLoad tl[C::CTUS];                            // (phase 1 is replayed below by stage_tile)
+  for (int tid = 0; tid < kThreads; tid++) setup_loads<Cfg, LOG2N>(fs, unit, totalCtus, tid, ctuXs, ctuYs, tl, &pre[tid * 8]);
   for (int c = 0; c < C::CTUS; c++) {
-    const int cg = unit * C::CTUS + c;
-    uint8_t* valid = smem + C::VALID_OFF + c * 256;
-    ctuXs[c] = ctuYs[c] = -1;
-    if (cg >= totalCtus) { for (int p = 0; p < G::PUS; p++) valid[p] = 0; continue; }
-    const int pic = cg / fs.ctusPerPic, ctu = cg - pic * fs.ctusPerPic;
-    const int ctuX = ctuXs[c] = (ctu % fs.ctusPerRow) * 64, ctuY = ctuYs[c] = (ctu / fs.ctusPerRow) * 64;
-    const int16_t* recPic = fs.rec + (size_t)pic * fs.recPicStride;
-    for (int p = 0; p < G::PUS; p++) { int px, py; demorton(p, px, py); valid[p] = ((ctuX + (px + 1) * N <= fs.W) && (ctuY + (py + 1) * N <= fs.H)) ? 1 : 0; }
-    for (int tid = 0; tid < kThreads; tid++) stage_tile<LOG2N>(tid, kThreads, recPic, fs.recStride, fs.W, fs.H, ctuX, ctuY, smem + C::TILE_OFF + c * C::TILE_BYTES);
+    if (ctuXs[c] < 0) { for (int p = 0; p < G::PUS; p++) valid[c * 256 + p] = kPuOutside; continue; }
+    const uint8_t* need = ctu_needed<LOG2N>(fs, unit * C::CTUS + c);
+    for (int p = 0; p < G::PUS; p++) valid[c * 256 + p] = pu_state<LOG2N>(fs, need, ctuXs[c], ctuYs[c], p);
   }
+  for (int c = 0; c < C::CTUS; c++)          // phase 1: every thread id's tile_load + tile_store
+    if (ctuXs[c] >= 0) stage_tile<LOG2N>(0, 1, fs.rec + (size_t)ctu_pos(fs, unit * C::CTUS + c).pic * fs.recPicStride, fs.recStride, fs.W, fs.H, ctuXs[c], ctuYs[c], smem + C::TILE_OFF + c * C::TILE_BYTES);
   for (int c = 0; c < C::CTUS; c++)
     if (ctuXs[c] >= 0) for (int tid = 0; tid < kThreads; tid++) build_unfiltered<LOG2N>(tid, c, fs.W, fs.H, ctuXs[c], ctuYs[c], smem + C::TILE_OFF + c * C::TILE_BYTES, smem);
   for (int c = 0; c < C::CTUS; c++)
@@ -103,18 +110,18 @@ void emul_cta(const FrameSource& fs, int strong, int totalCtus, int unit, const 
     for (int tid = 0; tid < kThreads; tid++) {
       const Row r = rows[tid] = row_map<LOG2N>(tid, pass);
       const int cg = unit * C::CTUS + r.ctu;
-      ok[tid] = smem[C::VALID_OFF + r.ctu * 256 + (log2n == 2 ? 4 * r.pu : r.pu)] != 0;
+      ok[tid] = valid[r.ctu * 256 + (log2n == 2 ? 4 * r.pu : r.pu)] == kPuEvaluate;
       uint32_t* p = &P[tid * 16];
       if (ok[tid]) {
         uint32_t raw[16];
         auto pack4 = [](const int16_t* q) { uint32_t w = 0; for (int i = 0; i < 4; i++) w |= (uint32_t)(q[i] & 0xff) << (8 * i); return w; };
         if (!bs) {
-          const int pic = cg / fs.ctusPerPic, ctu = cg - pic * fs.ctusPerPic;
-          int px, py; demorton(r.pu, px, py);
-          if (log2n == 2) { px *= 8; py *= 8; }
-          else { px = px * N + (r.o ? r.v0 : r.u0); py = py * N + (r.o ? r.u0 : r.v0); }
-          const int16_t* src = fs.org + (size_t)pic * fs.orgPicStride + (size_t)((ctu / fs.ctusPerRow) * 64 + py) * fs.orgStride + (ctu % fs.ctusPerRow) * 64 + px;
-          for (int y = 0; y < 8; y++) for (int h = 0; h < 2; h++) raw[2 * y + h] = pack4(src + (size_t)y * fs.orgStride + 4 * h);
+          int tx, ty;
+          const int16_t* src = frame_src_ptr<LOG2N>(fs, r, cg, tx, ty);
+          for (int y = 0; y < 8; y++) {
+            const Vec16 v = pass == 0 ? pre[tid * 8 + y] : *reinterpret_cast<const Vec16*>(src + (size_t)y * fs.orgStride);
+            raw[2 * y] = bperm(v.x, v.y, 0x6420); raw[2 * y + 1] = bperm(v.z, v.w, 0x6420);
+          }
         } else {
           const int first = cg * C::PUS;
           if (log2n == 2) {
@@ -212,35 +219,33 @@ void emul_cta(const FrameSource& fs, int strong, int totalCtus, int unit, const 
     for (int i = 0; i < C::CTUS * C::PUS * kNumModes; i++) {
       const int pl = i / kNumModes, m = i - pl * kNumModes, idx = unit * C::CTUS * C::PUS + pl;
       if (idx >= bs->count) continue;
-      bs->out[(size_t)bs->pus[idx].outIndex * kNumModes + m] = LOG2N == 2 ? (uint32_t)reinterpret_cast<const uint16_t*>(acc)[i] : acc[i];
+      bs->out[(size_t)bs->pus[idx].outIndex * kNumModes + m] = CostRead<LOG2N>{acc}(0, i);
     }
     return;
   }
-  for (int c = 0; c < C::CTUS; c++) {
-    const int cgc = unit * C::CTUS + c;
-    if (cgc >= totalCtus) break;
-    const uint8_t* valid = smem + C::VALID_OFF + c * 256;
-    uint32_t* o = fs.out + ((size_t)cgc * kPusPerCtu + pu_offset_of_depth(6 - log2n)) * kNumModes;
-    for (int i = 0; i < C::PUS * kNumModes; i++) {
-      const bool v = valid[i / kNumModes] != 0;
-      if (LOG2N == 2) o[i] = v ? (uint32_t)reinterpret_cast<const uint16_t*>(acc)[c * C::PUS * kNumModes + i] : 0xffffffffu;
-      else o[i] = v ? acc[c * C::PUS * kNumModes + i] : 0xffffffffu;
-    }
-  }
+  copy_out<Cfg, LOG2N>(fs, unit, totalCtus, valid, all_evaluated<Cfg, LOG2N>(valid, 0, 1) && unit * C::CTUS + C::CTUS <= totalCtus, CostRead<LOG2N>{acc}, 0, 1);
 }
 
 }  // namespace
 
 extern "C" {
 
-// 8-bit frame (replay) mode over ALL CTUs of one picture, as rmd_frame_tc2_kernel writes it
-int emul_rmd_frame_tc2(int strong, const int16_t* org, int orgStride, const int16_t* rec, int recStride, int W, int H, uint32_t* out) {
+// 8-bit frame (replay) mode over ALL CTUs of one picture, as rmd_frame_tc2_kernel writes it; needed: [ctu][341] fork-aware mask or null
+int emul_rmd_frame_tc2(int strong, const int16_t* org, int orgStride, const int16_t* rec, int recStride, int W, int H, uint32_t* out, const uint8_t* needed) {
   FrameSource fs;
   fs.org = org; fs.rec = rec; fs.orgPicStride = 0; fs.recPicStride = 0; fs.orgStride = orgStride; fs.recStride = recStride;
-  fs.W = W; fs.H = H; fs.ctusPerRow = (W + 63) / 64; fs.ctusPerPic = fs.ctusPerRow * ((H + 63) / 64); fs.out = out; fs.outPacked = nullptr;
-  const int total = fs.ctusPerPic, u2 = (total + 1) >> 1, u4 = (total + 3) >> 2;
-  for (int u = 0; u < u4; u++) { emul_cta<6>(fs, strong, total, u); emul_cta<5>(fs, strong, total, u); }
-  for (int u = 0; u < u2; u++) { emul_cta<4>(fs, strong, total, u); emul_cta<3>(fs, strong, total, u); emul_cta<2>(fs, strong, total, u); }
+  fs.W = W; fs.H = H; fs.ctusPerRow = (W + 63) / 64; fs.ctusPerPic = fs.ctusPerRow * ((H + 63) / 64); fs.out = out; fs.outPacked = nullptr; fs.needed = needed;
+  const int total = fs.ctusPerPic;
+  for (int b = 0; b < frame_blocks(total); b++) {
+    const FrameBlock fb = frame_block(total, b);
+    switch (fb.log2n) {
+      case 6: emul_cta<6>(fs, strong, total, fb.unit); break;
+      case 5: emul_cta<5>(fs, strong, total, fb.unit); break;
+      case 4: emul_cta<4>(fs, strong, total, fb.unit); break;
+      case 3: emul_cta<3>(fs, strong, total, fb.unit); break;
+      default: emul_cta<2>(fs, strong, total, fb.unit);
+    }
+  }
   return 0;
 }
 // batch (S2) mode: `count` PUs of ONE size, tightly packed org blocks and borders, out[count][35]

@@ -1,7 +1,8 @@
 // rmd_tc3_emul.cpp - CPU replay of the half-precision tensor-core RMD frame kernel (TEST HARNESS, not a product path).
 //
 // Compiles csrc/rmd_tc3.cuh (the kernel's __host__ __device__ logic: fp16 weight tables, shared-memory layout, window
-// gather, record layout of the N = 4 path, planar / DC, border construction) with g++ and replays one CTA of
+// gather, record layout of the N = 4 path, planar / DC, border construction) and csrc/rmd_tc_frame.cuh (block decode, PU
+// states, set-up loads, tile staging, copy-out) with g++ and replays one CTA of
 // rmd_tc3_kernels.cu phase by phase for all 256 thread ids.  The tcgen05 kind::f16 products are replaced by products of the
 // decoded half-precision operands read through the same UMMA shared-memory layout, accumulated in double and rounded to
 // fp32 once (every intermediate is an integer below 2^24, so any accumulation order gives this value), and
@@ -11,9 +12,11 @@
 #include <cstring>
 #include <vector>
 #include "rmd_tc3.cuh"
+#include "rmd_tc_frame.cuh"
 
 using namespace cucd;
 using namespace cucd::tc3;
+using namespace cucd::tcf;
 
 namespace {
 
@@ -47,23 +50,27 @@ void emul_cta3(const FrameSource& fs, int strong, int bitDepth, int totalCtus, i
   unsigned char* smem = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(smemStore.data()) + 127) & ~uintptr_t(127));
   uint32_t* acc = reinterpret_cast<uint32_t*>(smem + C::ACC_OFF);
   uint16_t* acc16 = reinterpret_cast<uint16_t*>(acc);
+  uint8_t* valid = smem + C::VALID_OFF;
+  if (fs.needed && !fork_states<Cfg, LOG2N>(fs, unit, totalCtus, valid, 0, 1)) {   // fork-aware early exit (tc3_body)
+    copy_out<Cfg, LOG2N>(fs, unit, totalCtus, valid, false, CostRead<LOG2N>{acc, shift}, 0, 1);
+    return;
+  }
   // ---- tc3_body set-up ----
   std::memcpy(smem + C::HAD_OFF, tb.had.data() + (log2n == 2 ? 8192 : 0), C::HAD_BYTES);
   std::memset(smem + C::STORE_OFF, 0, C::TOTAL - C::STORE_OFF);
   if (log2n == 2) std::memset(smem + C::A1_OFF, 0, kGroups * C::A1_BYTES);
   for (int i = 0; i < 256; i++) reinterpret_cast<int*>(smem + C::DC_OFF)[i] = 0;
-  // ---- tc3_prologue ----
   int ctuXs[C::CTUS], ctuYs[C::CTUS];
+  TileLoad tl[C::CTUS];                                                // (phase 1 is replayed below by stage_tile16)
+  std::vector<Vec16> pre(kThreads * 8);                                // the rows' source tiles of pass 0
+  for (int tid = 0; tid < kThreads; tid++) setup_loads<Cfg, LOG2N>(fs, unit, totalCtus, tid, ctuXs, ctuYs, tl, &pre[tid * 8]);
+  // ---- tc3_prologue ----
   for (int c = 0; c < C::CTUS; c++) {
-    const int cg = unit * C::CTUS + c;
-    uint8_t* valid = smem + C::VALID_OFF + c * 256;
-    ctuXs[c] = ctuYs[c] = -1;
-    if (cg >= totalCtus) { for (int p = 0; p < C::PUS; p++) valid[p] = 0; continue; }
-    const int pic = cg / fs.ctusPerPic, ctu = cg - pic * fs.ctusPerPic;
-    const int ctuX = ctuXs[c] = (ctu % fs.ctusPerRow) * 64, ctuY = ctuYs[c] = (ctu / fs.ctusPerRow) * 64;
-    for (int p = 0; p < C::PUS; p++) { int px, py; demorton(p, px, py); valid[p] = ((ctuX + (px + 1) * N <= fs.W) && (ctuY + (py + 1) * N <= fs.H)) ? 1 : 0; }
-    for (int tid = 0; tid < kThreads; tid++)
-      stage_tile16<LOG2N>(tid, kThreads, fs.rec + (size_t)pic * fs.recPicStride, fs.recStride, fs.W, fs.H, ctuX, ctuY, reinterpret_cast<uint16_t*>(smem + C::TILE_OFF + c * C::TILE_BYTES));
+    if (ctuXs[c] < 0) { for (int p = 0; p < C::PUS; p++) valid[c * 256 + p] = kPuOutside; continue; }
+    const uint8_t* need = ctu_needed<LOG2N>(fs, unit * C::CTUS + c);
+    for (int p = 0; p < C::PUS; p++) valid[c * 256 + p] = pu_state<LOG2N>(fs, need, ctuXs[c], ctuYs[c], p);
+    stage_tile16<LOG2N>(0, 1, fs.rec + (size_t)ctu_pos(fs, unit * C::CTUS + c).pic * fs.recPicStride, fs.recStride, fs.W, fs.H, ctuXs[c], ctuYs[c],
+                        reinterpret_cast<uint16_t*>(smem + C::TILE_OFF + c * C::TILE_BYTES));   // phase 1: every thread id's tile_load + tile_store
   }
   for (int c = 0; c < C::CTUS; c++)
     if (ctuXs[c] >= 0)
@@ -85,17 +92,16 @@ void emul_cta3(const FrameSource& fs, int strong, int bitDepth, int totalCtus, i
       const int grp = tid >> 7, rowTid = tid & 127;
       const Row r = rows[tid] = row_map<LOG2N>(tid, pass);
       const int cg = unit * C::CTUS + r.ctu;
-      ok[tid] = smem[C::VALID_OFF + r.ctu * 256 + (log2n == 2 ? 4 * r.pu : r.pu)] == kPuEvaluate;
+      ok[tid] = valid[r.ctu * 256 + (log2n == 2 ? 4 * r.pu : r.pu)] == kPuEvaluate;
       uint32_t* p = &P[tid * 32];
       if (ok[tid]) {
         uint32_t raw[32];
-        const int pic = cg / fs.ctusPerPic, ctu = cg - pic * fs.ctusPerPic;
-        int px, py; demorton(r.pu, px, py);
-        if (log2n == 2) { px *= 8; py *= 8; }
-        else { px = px * N + (r.o ? r.v0 : r.u0); py = py * N + (r.o ? r.u0 : r.v0); }
-        const int16_t* src = fs.org + (size_t)pic * fs.orgPicStride + (size_t)((ctu / fs.ctusPerRow) * 64 + py) * fs.orgStride + (ctu % fs.ctusPerRow) * 64 + px;
-        for (int y = 0; y < 8; y++)
-          for (int h = 0; h < 4; h++) raw[4 * y + h] = (uint32_t)(uint16_t)src[(size_t)y * fs.orgStride + 2 * h] | ((uint32_t)(uint16_t)src[(size_t)y * fs.orgStride + 2 * h + 1] << 16);
+        int tx, ty;
+        const int16_t* src = frame_src_ptr<LOG2N>(fs, r, cg, tx, ty);
+        for (int y = 0; y < 8; y++) {
+          const Vec16 v = pass == 0 ? pre[tid * 8 + y] : *reinterpret_cast<const Vec16*>(src + (size_t)y * fs.orgStride);
+          raw[4 * y] = v.x; raw[4 * y + 1] = v.y; raw[4 * y + 2] = v.z; raw[4 * y + 3] = v.w;
+        }
         if (log2n == 2) region_to_quadrants16(raw, p, r.o != 0);
         else if (r.o) tile_transpose16(raw, p);
         else std::memcpy(p, raw, sizeof(raw));
@@ -209,31 +215,32 @@ void emul_cta3(const FrameSource& fs, int strong, int bitDepth, int totalCtus, i
       cost_out(am, true);
     }
   }
-  for (int c = 0; c < C::CTUS; c++) {
-    const int cgc = unit * C::CTUS + c;
-    if (cgc >= totalCtus) break;
-    const uint8_t* valid = smem + C::VALID_OFF + c * 256;
-    uint32_t* o = fs.out + ((size_t)cgc * kPusPerCtu + pu_offset_of_depth(6 - log2n)) * kNumModes;
-    for (int i = 0; i < C::PUS * kNumModes; i++) {
-      const bool v = valid[i / kNumModes] != 0;
-      if (LOG2N <= 3) o[i] = v ? (uint32_t)acc16[c * C::PUS * kNumModes + i] : 0xffffffffu;
-      else o[i] = v ? (acc[c * C::PUS * kNumModes + i] >> shift) : 0xffffffffu;
-    }
-  }
+  copy_out<Cfg, LOG2N>(fs, unit, totalCtus, valid, all_evaluated<Cfg, LOG2N>(valid, 0, 1) && unit * C::CTUS + C::CTUS <= totalCtus,
+                       CostRead<LOG2N>{acc, shift}, 0, 1);
 }
 
 }  // namespace
 
 extern "C" {
 
-// frame (replay) mode over ALL CTUs of one picture, as rmd_frame_tc3_kernel writes it (bit depth 8..10)
-int emul_rmd_frame_tc3(int bitDepth, int strong, const int16_t* org, int orgStride, const int16_t* rec, int recStride, int W, int H, uint32_t* out) {
+// frame (replay) mode over ALL CTUs of one picture, as rmd_frame_tc3_kernel writes it (bit depth 8..10); needed: [ctu][341]
+// fork-aware mask or null
+int emul_rmd_frame_tc3(int bitDepth, int strong, const int16_t* org, int orgStride, const int16_t* rec, int recStride, int W, int H, uint32_t* out,
+                       const uint8_t* needed) {
   FrameSource fs;
   fs.org = org; fs.rec = rec; fs.orgPicStride = 0; fs.recPicStride = 0; fs.orgStride = orgStride; fs.recStride = recStride;
-  fs.W = W; fs.H = H; fs.ctusPerRow = (W + 63) / 64; fs.ctusPerPic = fs.ctusPerRow * ((H + 63) / 64); fs.out = out; fs.outPacked = nullptr; fs.needed = nullptr;
-  const int total = fs.ctusPerPic, u2 = (total + 1) >> 1, u4 = (total + 3) >> 2;
-  for (int u = 0; u < u4; u++) { emul_cta3<6>(fs, strong, bitDepth, total, u); emul_cta3<5>(fs, strong, bitDepth, total, u); }
-  for (int u = 0; u < u2; u++) { emul_cta3<4>(fs, strong, bitDepth, total, u); emul_cta3<3>(fs, strong, bitDepth, total, u); emul_cta3<2>(fs, strong, bitDepth, total, u); }
+  fs.W = W; fs.H = H; fs.ctusPerRow = (W + 63) / 64; fs.ctusPerPic = fs.ctusPerRow * ((H + 63) / 64); fs.out = out; fs.outPacked = nullptr; fs.needed = needed;
+  const int total = fs.ctusPerPic;
+  for (int b = 0; b < frame_blocks(total); b++) {
+    const FrameBlock fb = frame_block(total, b);
+    switch (fb.log2n) {
+      case 6: emul_cta3<6>(fs, strong, bitDepth, total, fb.unit); break;
+      case 5: emul_cta3<5>(fs, strong, bitDepth, total, fb.unit); break;
+      case 4: emul_cta3<4>(fs, strong, bitDepth, total, fb.unit); break;
+      case 3: emul_cta3<3>(fs, strong, bitDepth, total, fb.unit); break;
+      default: emul_cta3<2>(fs, strong, bitDepth, total, fb.unit);
+    }
+  }
   return 0;
 }
 int emul_tc3_smem_bytes() { return kSmemBytes; }

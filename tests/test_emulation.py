@@ -4,7 +4,7 @@ arithmetic be checked where there is no GPU; the -m gpu tests check the real ker
 import numpy as np
 import pytest
 
-from _util import P, golden, i16p, i32p, u32p, oracle_outlier_frame, oracle_rmd_frame, pseudo_recon, textured_plane
+from _util import P, golden, i16p, i32p, u8p, u32p, oracle_outlier_frame, oracle_rmd_frame, pseudo_recon, textured_plane
 
 
 @pytest.mark.parametrize("clip", ["ai8", "ai10"])
@@ -42,7 +42,7 @@ def test_tensor_core_frame_kernel_code_vs_oracle(emul, oracle, W, H, seed):
     rec[:, : W // 2] = (np.arange(H)[:, None] // 3 + np.arange(W // 2)[None, :] // 5 + 40).astype(np.int16)
     want = oracle_rmd_frame(oracle, org, rec, 8)
     got = np.zeros_like(want)
-    emul.emul_rmd_frame_tc2(1, P(org, i16p), W, P(rec, i16p), W, W, H, P(got, u32p))
+    emul.emul_rmd_frame_tc2(1, P(org, i16p), W, P(rec, i16p), W, W, H, P(got, u32p), None)
     assert np.array_equal(got, want)
 
 
@@ -58,7 +58,7 @@ def test_half_precision_tensor_core_frame_kernel_code_vs_oracle(emul, oracle, bd
     orgp = np.zeros((H, S), np.int16); orgp[:, :W] = org
     recp = np.zeros((H, S), np.int16); recp[:, :W] = rec
     got = np.zeros_like(want)
-    emul.emul_rmd_frame_tc3(bd, 1, P(orgp, i16p), S, P(recp, i16p), S, W, H, P(got, u32p))
+    emul.emul_rmd_frame_tc3(bd, 1, P(orgp, i16p), S, P(recp, i16p), S, W, H, P(got, u32p), None)
     assert np.array_equal(got, want)
 
 
@@ -73,8 +73,29 @@ def test_half_precision_tensor_core_frame_kernel_code_extreme_values(emul, oracl
         org = np.ascontiguousarray(org.astype(np.int16)); rec = np.ascontiguousarray(rec.astype(np.int16))
         want = oracle_rmd_frame(oracle, org, rec, 10)
         got = np.zeros_like(want)
-        emul.emul_rmd_frame_tc3(10, 1, P(org, i16p), W, P(rec, i16p), W, W, H, P(got, u32p))
+        emul.emul_rmd_frame_tc3(10, 1, P(org, i16p), W, P(rec, i16p), W, W, H, P(got, u32p), None)
         assert np.array_equal(got, want)
+
+
+@pytest.mark.parametrize("bd,W,H", [(8, 200, 136), (10, 136, 72)])
+def test_tensor_core_frame_kernel_code_fork_aware_mask(emul, oracle, bd, W, H):
+    """fork-aware mode of rmd_tc2 / rmd_tc3: a random `needed` mask, every 32x32 PU pruned (each of those CTAs takes the early exit);
+    the table is the oracle's with CUCD_COST_PRUNED for a pruned PU and CUCD_COST_NOT_INSIDE outside the picture"""
+    org = textured_plane(W, H, bd, seed=6)
+    rec = pseudo_recon(org, bd)
+    full = oracle_rmd_frame(oracle, org, rec, bd)
+    need = (np.random.default_rng(bd).random(full.shape[:2]) < 0.5).astype(np.uint8)
+    need[:, 1:5] = 0
+    need[:, 85:] = np.repeat(need[:, 85::4], 4, axis=1)               # 4x4 PUs: NxN of an 8x8 CU is pruned as a whole
+    inside = full[:, :, 0] != 0xFFFFFFFF
+    want = np.where(((need == 0) & inside)[:, :, None], np.uint32(0xFFFFFFFE), full)
+    got = np.zeros_like(full)
+    if bd == 8:
+        emul.emul_rmd_frame_tc2(1, P(org, i16p), W, P(rec, i16p), W, W, H, P(got, u32p), P(need, u8p))
+    else:
+        emul.emul_rmd_frame_tc3(bd, 1, P(org, i16p), W, P(rec, i16p), W, W, H, P(got, u32p), P(need, u8p))
+    assert (~inside).any() and (inside & (need == 0)).any() and (inside & (need == 1)).any()
+    assert np.array_equal(got, want)
 
 
 @pytest.mark.parametrize("n", [4, 8, 16, 32, 64])
@@ -99,7 +120,7 @@ def test_tensor_core_frame_kernel_code_extreme_values(emul, oracle):
         org = np.ascontiguousarray(org.astype(np.int16)); rec = np.ascontiguousarray(rec.astype(np.int16))
         want = oracle_rmd_frame(oracle, org, rec, 8)
         got = np.zeros_like(want)
-        emul.emul_rmd_frame_tc2(1, P(org, i16p), W, P(rec, i16p), W, W, H, P(got, u32p))
+        emul.emul_rmd_frame_tc2(1, P(org, i16p), W, P(rec, i16p), W, W, H, P(got, u32p), None)
         assert np.array_equal(got, want)
 
 
