@@ -69,8 +69,17 @@ FeaturePlanes make_feature_planes(const cucd_handle* h, const int16_t* org, long
 }
 
 cudaError_t launch_rmd_auto(cucd_handle* h, const FrameSource& fs, int nPics, cudaStream_t st) {
-  if (h->useTensor == 1 && h->cfg.bit_depth == 8)     // kind::i8: samples are bytes
-    return launch_rmd_frames_tc2(fs, nPics, h->cfg.strong_intra_smoothing, h->dTc2Tables.p, h->dTc2Tables.p + tc2::kWinTableBytes, h->dHadamard.p, st, &h->launches);
+  if (h->useTensor == 1 && h->cfg.bit_depth == 8) {   // kind::i8: samples are bytes
+    // one scratch per handle: sized for max_pictures at creation (cucd_dev_rmd_frames may ask for more); a launch on another stream
+    // than the previous one waits until that one has read it
+    cudaError_t e = h->dTc2Prep.reserve(rmd_tc2_prep_bytes(nPics * h->ctusPerPic));
+    if (e == cudaSuccess) e = cudaStreamWaitEvent(st, h->evTc2Prep, 0);
+    if (e == cudaSuccess)
+      e = launch_rmd_frames_tc2(fs, nPics, h->cfg.strong_intra_smoothing, h->dTc2Tables.p, h->dTc2Tables.p + tc2::kWinTableBytes, h->dHadamard.p,
+                                h->dTc2Prep.p, st, &h->launches);
+    if (e == cudaSuccess) e = cudaEventRecord(h->evTc2Prep, st);
+    return e;
+  }
   if (h->useTensor >= 1)      // 9/10-bit content (or path 2: any bit depth): half-precision operands, fp32 accumulators (exact integers)
     return launch_rmd_frames_tc3(fs, nPics, h->cfg.bit_depth, h->cfg.strong_intra_smoothing, h->dTc3Tables.p, h->dTc3Tables.p + tc3::kWinTableBytes16,
                                  h->dTc3Tables.p + tc3::kWinTableBytes16 + tc3::kN4TableBytes16, st, &h->launches);
@@ -172,6 +181,8 @@ int cucd_create(const cucd_config* cfg, cucd_handle** out) {
     ok = ok && cudaEventCreateWithFlags(&h->evUpG[i], cudaEventDisableTiming) == cudaSuccess && cudaEventCreateWithFlags(&h->evRmdG[i], cudaEventDisableTiming) == cudaSuccess;
   ok = ok && cudaEventCreate(&h->evK0) == cudaSuccess && cudaEventCreate(&h->evK1) == cudaSuccess;
   ok = ok && cudaEventCreateWithFlags(&h->evMask, cudaEventDisableTiming) == cudaSuccess;
+  ok = ok && cudaEventCreateWithFlags(&h->evTc2Prep, cudaEventDisableTiming) == cudaSuccess;
+  if (cfg->bit_depth == 8) ok = ok && h->dTc2Prep.reserve(rmd_tc2_prep_bytes((int)P * h->ctusPerPic)) == cudaSuccess;
   ok = ok && cudaEventCreateWithFlags(&h->evDevUp, cudaEventDisableTiming) == cudaSuccess && cudaEventCreateWithFlags(&h->evDevDone, cudaEventDisableTiming) == cudaSuccess;
   for (int i = 0; i < cucd_handle::kTimeRing; i++) ok = ok && cudaEventCreate(&h->evRmd0[i]) == cudaSuccess && cudaEventCreate(&h->evRmd1[i]) == cudaSuccess;
   for (FrameSlot& s : h->slots) {
@@ -225,7 +236,8 @@ int cucd_destroy(cucd_handle* h) {
     if (s.evJoin) cudaEventDestroy(s.evJoin);
   }
   for (int d = 0; d < 4; d++) { h->dNum[d].release(); h->dSum[d].release(); }
-  h->dCtuHad.release(); h->dHadamard.release(); h->dTc2Tables.release();
+  h->dCtuHad.release(); h->dHadamard.release(); h->dTc2Tables.release(); h->dTc2Prep.release();
+  if (h->evTc2Prep) cudaEventDestroy(h->evTc2Prep);
   h->bOut.release(); h->bStage.release(); h->hStage.release(); h->hStageOut.release(); h->hScratch.release();
   for (auto& r : h->refs) r.buf.release();
   h->dCur.release(); h->dRefPtr.release(); h->dRefStride.release();

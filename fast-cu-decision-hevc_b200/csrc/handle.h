@@ -140,6 +140,8 @@ struct cucd_handle {
   cucd::DevBuf<int8_t> dHadamard;                 // +-(H8 x H8), +-(blockdiag H4 x H4) operands of the tensor-core SATD
   cucd::DevBuf<uint8_t> dTc3Tables;               // half-precision weight / Hadamard operands of the 9/10-bit tensor-core path (rmd_tc3.cuh)
   cucd::DevBuf<uint8_t> dTc2Tables;               // interpolation-weight operands of the tensor-core prediction (rmd_tc2.cuh)
+  cucd::DevBuf<uint8_t> dTc2Prep;                 // 8-bit content: the border pre-pass's reference arrays, rmd_tc2_prep_bytes per launch
+  cudaEvent_t evTc2Prep = nullptr;                // after the last launch that read dTc2Prep: a launch on another stream waits for it
   int useTensor = 0;                              // cucd_set_rmd_path: 1 = predictions + Hadamard on tcgen05, 0 = integer ALU
   cucd::DevBuf<int32_t> dNum[4], dSum[4], dCtuHad;
   size_t cuCount[4] = {0, 0, 0, 0};

@@ -16,9 +16,16 @@ cudaError_t configure_rmd_kernels();
 cudaError_t configure_rmd_tc2_kernels();
 // +-(H8 (x) H8), +-(blockdiag H4 (x) H4) as s8 UMMA operands, 16 KB: B operand of the tensor-core SATD
 cudaError_t launch_hadamard_operands(int8_t* dst, cudaStream_t st);
-// predictions AND Hadamard on tcgen05 (rmd_tc2_kernels.cu); tabWin / tabN4 = tc2::fill_win_tables / fill_n4_tables uploaded by the caller
+// predictions AND Hadamard on tcgen05 (rmd_tc2_kernels.cu); tabWin / tabN4 = tc2::fill_win_tables / fill_n4_tables uploaded by the caller.
+// Two launches on st: the border pre-pass writes the reference arrays of every CTU and depth to `prep` (rmd_tc2_prep_bytes(nPics *
+// fs.ctusPerPic) bytes of device scratch, which must not be in use by another launch), then the RMD kernel reads them.
 cudaError_t launch_rmd_frames_tc2(const FrameSource& fs, int nPics, int strong, const uint8_t* tabWin, const uint8_t* tabN4, const int8_t* hadamard,
-                                  cudaStream_t st, int* launches);
+                                  uint8_t* prep, cudaStream_t st, int* launches);
+size_t rmd_tc2_prep_bytes(int nCtus);
+// the two launches one at a time (profiles/ubench)
+cudaError_t launch_rmd_border_prep(const FrameSource& fs, int nPics, int strong, uint8_t* prep, cudaStream_t st, int* launches);
+cudaError_t launch_rmd_frame_tc2(const FrameSource& fs, int nPics, int strong, const uint8_t* tabWin, const uint8_t* tabN4, const int8_t* hadamard,
+                                 const uint8_t* prep, cudaStream_t st, int* launches);
 int rmd_tc2_smem_bytes();
 // the same on tcgen05 kind::f16 for 9/10-bit content (rmd_tc3_kernels.cu); tables = tc3::fill_win_tables16 / fill_n4_tables16 / fill_had_tables16
 cudaError_t configure_rmd_tc3_kernels();

@@ -146,7 +146,9 @@ struct Cfg {
   static constexpr int NARR = HAS_FILT ? 4 : 2;
   static constexpr int AS8 = (3 * N + 21 + 3) & ~3;
   static constexpr int PU_RAW = NARR * AS8;
-  static constexpr int PU_BYTES = PU_RAW + (((PU_RAW >> 2) & 1) ? 0 : 4);   // odd number of words: lanes of different PUs hit different banks
+  // odd number of words: lanes of different PUs hit different banks.  N = 64: a warp reads one PU, and the 432 bytes of a CTU's slot stay a
+  // 16-byte multiple, as its bulk copy needs (border pre-pass, rmd_tc_frame.cuh)
+  static constexpr int PU_BYTES = LOG2N == 6 ? PU_RAW : PU_RAW + (((PU_RAW >> 2) & 1) ? 0 : 4);
   static constexpr int SLOTS = LOG2N == 3 ? 64 : CTUS * PUS;     // PUs seen by one row group
   static constexpr int GROUP_BYTES = LOG2N == 2 ? 0 : al16(16 + SLOTS * PU_BYTES);
   static constexpr int STORE_BYTES = LOG2N == 2 ? CTUS * 256 * 2 * 16 : kGroups * GROUP_BYTES;   // N = 4: shared 16-byte records [ctu][o][pu]
@@ -164,7 +166,8 @@ struct Cfg {
   static constexpr int STORE_OFF = DC_OFF + CTUS * 64 * 4;
   static constexpr int ACC_OFF = STORE_OFF + al16(STORE_BYTES);
   static constexpr int TOTAL = ACC_OFF + al16(CTUS * PUS * kNumModes * ACC_ELEM);
-  // u8 copy of the reconstruction around each CTU while the reference arrays are built; aliases the MMA 1 operand
+  // u8 copy of the reconstruction around each CTU while the reference arrays are built (frame mode): the border pre-pass holds one
+  // per CTA; the CPU replay of the in-kernel prologue (tests/emul/rmd_tc2_emul.cpp) stages them at TILE_OFF, in the MMA 1 operand
   // buffers, which are first written after the prologue
   static constexpr int TILE_OFF = B1_OFF;
   static constexpr int TILE_PITCH = 68;                          // 17 words: a column walk touches 32 different banks
@@ -184,6 +187,41 @@ template <int LOG2N> CUCD_HD int arr_k0_off(int grp, int slot, int o, int filt) 
   return grp * C::GROUP_BYTES + 16 + slot * C::PU_BYTES + (filt * 2 + o) * C::AS8 + C::N;
 }
 CUCD_HD int rec_off(int ctu, int o, int pu) { return ((ctu * 2 + o) * 256 + pu) * 16; }
+
+// Frame mode: the border pre-pass (rmd_border_prep_kernel) builds the reference arrays of every CTU at every depth once, as an
+// IMAGE per (CTU, depth): the bytes the prologue of the CTU's CTA would write into one row-group copy of the store - N = 4: the
+// records [o][pu], N = 8: the slots of the CTU's row group, N >= 16: the CTU's PUS consecutive slots - then its DC sums (N >= 8).
+// Both parts are 16-byte multiples; the RMD CTA places them with cp.async.bulk.  The images of a CTU are consecutive, depth 0 (N = 64)
+// first: kPrepCtuBytes per CTU.
+template <int LOG2N>
+struct PrepSize {
+  typedef Cfg<LOG2N> C;
+  static constexpr int STORE = LOG2N == 2 ? 2 * 256 * 16 : C::PUS * C::PU_BYTES;
+  static constexpr int DC = LOG2N == 2 ? 0 : C::al16(C::PUS * 4);
+  static constexpr int BYTES = STORE + DC;
+  static_assert(STORE % 16 == 0, "a bulk copy moves 16-byte multiples");
+};
+constexpr int kPrepCtuBytes = PrepSize<2>::BYTES + PrepSize<3>::BYTES + PrepSize<4>::BYTES + PrepSize<5>::BYTES + PrepSize<6>::BYTES;
+template <int LOG2N> CUCD_HD constexpr int prep_off() {
+  return (LOG2N < 6 ? PrepSize<6>::BYTES : 0) + (LOG2N < 5 ? PrepSize<5>::BYTES : 0) + (LOG2N < 4 ? PrepSize<4>::BYTES : 0) + (LOG2N < 3 ? PrepSize<3>::BYTES : 0);
+}
+// where the store image of the CTA's CTU c lands in row group grp's copy of the store (N <= 8: one copy, grp unused)
+template <int LOG2N> CUCD_HD int prep_store_off(int grp, int c) {
+  typedef Cfg<LOG2N> C;
+  return LOG2N == 2 ? rec_off(c, 0, 0) : (LOG2N == 3 ? c * C::GROUP_BYTES + 16 : grp * C::GROUP_BYTES + 16 + c * C::PUS * C::PU_BYTES);
+}
+// The bulk copies that place the image of the CTA's CTU c: one per row-group copy of the store (N >= 16: two) and the DC sums.
+// Copy i: `bytes` bytes from offset `src` of the image to offset `dst` of the CTA's shared memory.
+struct PrepCopy { int dst, src, bytes; };
+template <int LOG2N> CUCD_HD constexpr int prep_copies() { return LOG2N == 2 ? 1 : (LOG2N == 3 ? 2 : 3); }
+template <int LOG2N> CUCD_HD PrepCopy prep_copy(int c, int i) {
+  typedef Cfg<LOG2N> C;
+  typedef PrepSize<LOG2N> S;
+  if (LOG2N >= 3 && i == prep_copies<LOG2N>() - 1) return PrepCopy{C::DC_OFF + c * 256, S::STORE, S::DC};
+  return PrepCopy{C::STORE_OFF + prep_store_off<LOG2N>(i, c), 0, S::STORE};
+}
+// bytes of the copies of one CTU (what the CTA's mbarrier expects per CTU)
+template <int LOG2N> CUCD_HD constexpr int prep_copy_bytes() { return (prep_copies<LOG2N>() - (LOG2N >= 3 ? 1 : 0)) * PrepSize<LOG2N>::STORE + PrepSize<LOG2N>::DC; }
 // the cost of element i (= pu * 35 + mode) of the CTA's CTU c in the accumulators at ACC_OFF: uint16 for N = 4, uint32 otherwise
 template <int LOG2N> struct CostRead {
   const uint32_t* acc;
@@ -479,13 +517,19 @@ CUCD_HD void put_ref(unsigned char* store, int ctu, int p, int o, int k, int v) 
 }
 // 256 / PUS threads share a PU; each produces 4N / (256 / PUS) consecutive samples of the sequence T[1..2N], L[1..2N]
 // (N = 4: one thread per PU, 16 samples) and the first of them the corner.
+// The `_at` builders write through `prol`, the CTA's shared memory from VALID_OFF on (PU states, DC sums, store: offsets ProlOff), so
+// that the border pre-pass can run them on a staging area of that layout (rmd_tc_frame.cuh prep_phase); build_unfiltered /
+// build_filtered take the CTA's shared memory itself.
+template <int LOG2N> struct ProlOff {
+  static constexpr int DC = Cfg<LOG2N>::DC_OFF - Cfg<LOG2N>::VALID_OFF, STORE = Cfg<LOG2N>::STORE_OFF - Cfg<LOG2N>::VALID_OFF;
+};
 template <int LOG2N>
-CUCD_HD void build_unfiltered(int tid, int ctu, int W, int H, int ctuX, int ctuY, const unsigned char* t, unsigned char* smem) {
+CUCD_HD void build_unfiltered_at(int tid, int ctu, int W, int H, int ctuX, int ctuY, const unsigned char* t, unsigned char* prol) {
   typedef Cfg<LOG2N> C;
   constexpr int N = C::N, TPP = 256 / C::PUS, SPT = 4 * N / TPP;
-  unsigned char* store = smem + C::STORE_OFF;
+  unsigned char* store = prol + ProlOff<LOG2N>::STORE;
   const int p = tid / TPP, sub = tid % TPP;
-  if (!smem[C::VALID_OFF + ctu * 256 + p]) return;
+  if (!prol[ctu * 256 + p]) return;
   int px, py; demorton(p, px, py);
   const int x0 = px * N, y0 = py * N;
   const PuAvail a = pu_avail<LOG2N>(ctuX + x0, ctuY + y0, W, H);
@@ -532,13 +576,17 @@ CUCD_HD void build_unfiltered(int tid, int ctu, int W, int H, int ctuX, int ctuY
     put_ref<LOG2N>(store, ctu, p, o, k, vals[e]);
   }
   if (LOG2N >= 3) {
-    int* dst = reinterpret_cast<int*>(smem + C::DC_OFF) + ctu * 64 + p;
+    int* dst = reinterpret_cast<int*>(prol + ProlOff<LOG2N>::DC) + ctu * 64 + p;
 #if defined(__CUDA_ARCH__)
     if (dcSum) atomicAdd(dst, dcSum);
 #else
     *dst += dcSum;
 #endif
   }
+}
+template <int LOG2N>
+CUCD_HD void build_unfiltered(int tid, int ctu, int W, int H, int ctuX, int ctuY, const unsigned char* t, unsigned char* smem) {
+  build_unfiltered_at<LOG2N>(tid, ctu, W, H, ctuX, ctuY, t, smem + Cfg<LOG2N>::VALID_OFF);
 }
 // Batch (S2) mode: the caller supplies the unfiltered border of every PU as the linear 4N+1 array of
 // include/cucudecide.h ([0..2N-1] left column bottom -> top, [2N] corner, [2N+1..4N] above row); substitution has
@@ -579,13 +627,13 @@ CUCD_HD void build_unfiltered_batch(int tid, int ctu, const int16_t* b /*border 
 
 // Phase 3: smoothed arrays (TComPattern.cpp:185-283) from the unfiltered ones, same thread -> sample map
 template <int LOG2N>
-CUCD_HD void build_filtered(int tid, int ctu, int strongEnabled, unsigned char* smem) {
+CUCD_HD void build_filtered_at(int tid, int ctu, int strongEnabled, unsigned char* prol) {
   typedef Cfg<LOG2N> C;
   if (!C::HAS_FILT) return;
   constexpr int N = C::N, TPP = 256 / C::PUS, SPT = 4 * N / TPP;
-  unsigned char* store = smem + C::STORE_OFF;
+  unsigned char* store = prol + ProlOff<LOG2N>::STORE;
   const int p = tid / TPP, sub = tid % TPP;
-  if (!smem[C::VALID_OFF + ctu * 256 + p]) return;
+  if (!prol[ctu * 256 + p]) return;
   const int slot = pu_slot2<LOG2N>(ctu, p);
   const int g0 = LOG2N == 3 ? ctu : 0;
   const unsigned char* T = store + arr_k0_off<LOG2N>(g0, slot, 0, 0);
@@ -618,6 +666,9 @@ CUCD_HD void build_filtered(int tid, int ctu, int strongEnabled, unsigned char* 
     put(o, k, vals[e]);
   }
 }
+
+template <int LOG2N>
+CUCD_HD void build_filtered(int tid, int ctu, int strongEnabled, unsigned char* smem) { build_filtered_at<LOG2N>(tid, ctu, strongEnabled, smem + Cfg<LOG2N>::VALID_OFF); }
 
 // projected samples of a negative-angle round, by the 128 threads of row group `grp` for its private arrays:
 // store[main][-j] = store[side][(128 + j*inv) >> 8] (TComPrediction.cpp:300-322).  128 / (2 * SLOTS) threads share one

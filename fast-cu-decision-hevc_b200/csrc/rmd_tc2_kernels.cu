@@ -11,8 +11,11 @@
 //     epilogue 2: sum |D2|, HM rounding
 // See rmd_tc2.cuh for the arithmetic and the reference citations; planar and DC are predicted on the ALU.  The frame-mode set-up
 // loads, PU states and copy-out are shared with rmd_tc3_kernels.cu (rmd_tc_frame.cuh), the tcgen05 wrappers live in satd_tc.cuh.
+// In frame mode the reference arrays come from rmd_border_prep_kernel, launched first on the same stream: one CTA per CTU builds
+// them for all five depths, and an RMD CTA bulk-copies its CTUs' images into shared memory while its workers load their source tiles.
 // Replaces, per PU, the reference loop TEncSearch.cpp:2327-2361.
 #include <cuda_runtime.h>
+#include <type_traits>
 #include "rmd_tc2.cuh"
 #include "rmd_tc_frame.cuh"
 #include "satd_tc.cuh"
@@ -54,6 +57,7 @@ struct Tc2Args {
   BatchSource bs;             // batch (S2) mode: a unit is 4096 / N^2 caller-described PUs of one size ("virtual CTU")
   int strong, totalCtus;      // totalCtus = number of units
   const uint8_t* tabWin; const uint8_t* tabN4; const int8_t* had;
+  const uint8_t* prep;        // frame mode: the images of rmd_border_prep_kernel, kPrepCtuBytes per CTU
 };
 
 // A CTA = 256 worker threads (the rows) + one MMA-issuing warp per row group.  The workers only ARRIVE on mbarriers when their
@@ -63,9 +67,11 @@ struct Tc2Args {
 constexpr int kIssuerThreads = 32 * kGroups;
 constexpr int kCtaThreads = kThreads + kIssuerThreads;
 __device__ __forceinline__ void worker_bar() { asm volatile("bar.sync 1, 256;\n" ::: "memory"); }     // the 256 workers only
-// ---- prologue: reference arrays of the CTA's CTUs (rmd_tc2.cuh phases 1-3) --------------------------------
+// ---- prologue: reference arrays of the CTA's CTUs ------------------------------------------------------------
+// Batch mode builds them here (rmd_tc2.cuh phases 2-3).  Frame mode only writes the PU states: the arrays are the border pre-pass's
+// images, which tc2_prep_copies has set on their way.
 template <int LOG2N, bool FRAME>
-__device__ __forceinline__ void tc2_prologue(const Tc2Args& a, const int unit, const TileLoad* tl, const int* ctuX, const int* ctuY) {
+__device__ __forceinline__ void tc2_prologue(const Tc2Args& a, const int unit, const int* ctuX, const int* ctuY) {
   typedef Cfg<LOG2N> C;
   unsigned char* smem = smem2;
   const int tid = threadIdx.x;
@@ -103,21 +109,26 @@ __device__ __forceinline__ void tc2_prologue(const Tc2Args& a, const int unit, c
     const uint8_t* need = ctu_needed<LOG2N>(fs, cg);
     for (int p = tid; p < C::PUS; p += kThreads) valid[p] = pu_state<LOG2N>(fs, need, ctuX[c], ctuY[c], p);
   }
+}
+
+// ---- frame mode: one lane of the first MMA-issuing warp bulk-copies the images of the CTA's CTUs into the store and the DC sums ----
+// It initialises the barrier it signals on itself, so the copies start as the CTA does; the workers wait for them after the CTA-wide
+// barrier that ends the set-up.
+template <int LOG2N>
+__device__ __forceinline__ void tc2_prep_copies(const Tc2Args& a, const int unit, uint64_t* bar) {
+  typedef Cfg<LOG2N> C;
+  if (!elect_one()) return;
+  mbar_init(bar, 1);
+  asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
+  const int n = min(C::CTUS, a.totalCtus - unit * C::CTUS);
+  mbar_expect_tx(bar, n * prep_copy_bytes<LOG2N>());
+  for (int c = 0; c < n; c++) {
+    const uint8_t* img = a.prep + (size_t)(unit * C::CTUS + c) * kPrepCtuBytes + prep_off<LOG2N>();
 #pragma unroll
-  for (int c = 0; c < C::CTUS; c++)
-    if (ctuX[c] >= 0) tile_store<Cfg, LOG2N>(tid, fs.W, fs.H, ctuX[c], ctuY[c], tl[c], smem + C::TILE_OFF + c * C::TILE_BYTES);
-  worker_bar();
-  TC2_STAMP(51);
-#pragma unroll
-  for (int c = 0; c < C::CTUS; c++)
-    if (ctuX[c] >= 0) build_unfiltered<LOG2N>(tid, c, fs.W, fs.H, ctuX[c], ctuY[c], smem + C::TILE_OFF + c * C::TILE_BYTES, smem);
-  TC2_STAMP(52);
-  if (C::HAS_FILT) {
-    worker_bar();
-    TC2_STAMP(53);
-#pragma unroll
-    for (int c = 0; c < C::CTUS; c++)
-      if (ctuX[c] >= 0) build_filtered<LOG2N>(tid, c, a.strong, smem);
+    for (int i = 0; i < prep_copies<LOG2N>(); i++) {
+      const PrepCopy pc = prep_copy<LOG2N>(c, i);
+      bulk_g2s(smem2 + pc.dst, img + pc.src, pc.bytes, bar);
+    }
   }
 }
 
@@ -459,6 +470,8 @@ __device__ __noinline__ void tc2_body(const Tc2Args& a, const int unit) {
     }
     if (worker) worker_bar();
   }
+  uint64_t* prepBar = reinterpret_cast<uint64_t*>(smem + C::BAR_OFF) + 5 * kGroups;
+  if (FRAME && warp == kThreads / 32) tc2_prep_copies<LOG2N>(a, unit, prepBar);
   uint32_t* tmemSlot = reinterpret_cast<uint32_t*>(smem + C::BAR_OFF + 96);
   if (tid == 0) {
     for (int i = 0; i < 5 * kGroups; i++)           // MMA done x2 (1 arrival: the commit), operands ready x2 (128 rows), weights landed (1 + bytes)
@@ -471,22 +484,21 @@ __device__ __noinline__ void tc2_body(const Tc2Args& a, const int unit) {
   TC2_STAMP(0);
   if (warp == 0) tmem_alloc(tmemSlot, 256);
   TC2_STAMP(58);
-  // Every global load of the set-up is issued here, before anything waits: the Hadamard operands, the reconstruction
-  // neighbourhoods of the CTA's CTUs (tile_load) and the rows' source tiles of pass 0 share ONE memory round trip.
+  // Every global load of the set-up is issued here, before anything waits: the Hadamard operands and the rows' source tiles of
+  // pass 0 (frame mode) share ONE memory round trip, and the bulk copies of the reference arrays are in flight beside them.
   const uint4 hadP = reinterpret_cast<const uint4*>(a.had + (LOG2N == 2 ? 8192 : 0))[tid];        // +H
   const uint4 hadN = reinterpret_cast<const uint4*>(a.had + (LOG2N == 2 ? 8192 : 0))[tid + 256];  // -H
   int ctuX[C::CTUS], ctuY[C::CTUS];
-  TileLoad tl[C::CTUS];
-  if (FRAME) setup_loads<Cfg, LOG2N>(a.fs, unit, a.totalCtus, tid, ctuX, ctuY, tl, pre);
+  if (FRAME) setup_loads<Cfg, LOG2N>(a.fs, unit, a.totalCtus, tid, ctuX, ctuY, nullptr, pre);
   TC2_STAMP(59);
   if (LOG2N >= 4) for (int i = tid; i < C::CTUS * C::PUS * kNumModes; i += kThreads) acc[i] = 0;   // accumulated with atomics
-  reinterpret_cast<int*>(smem + C::DC_OFF)[tid] = 0;          // CTUS * 64 <= 256 sums
+  if (!FRAME) reinterpret_cast<int*>(smem + C::DC_OFF)[tid] = 0;   // CTUS * 64 <= 256 sums (frame mode: copied in)
   reinterpret_cast<uint4*>(smem + C::HAD_OFF)[tid] = hadP;
   TC2_STAMP(60);
   reinterpret_cast<uint4*>(smem + C::HAD_OFF)[tid + 256] = hadN;
   worker_bar();
   TC2_STAMP(50);
-  tc2_prologue<LOG2N, FRAME>(a, unit, tl, ctuX, ctuY);
+  tc2_prologue<LOG2N, FRAME>(a, unit, ctuX, ctuY);
   TC2_STAMP(54);
   tc_fence_before();
   fence_async_smem();
@@ -494,6 +506,8 @@ __device__ __noinline__ void tc2_body(const Tc2Args& a, const int unit) {
   __syncthreads();                                  // barriers initialised, TMEM allocated, operands of the set-up visible: workers and issuers
   tc_fence_after();
   const uint32_t tmemBase = *tmemSlot;
+  TC2_STAMP(55);
+  if (FRAME && worker) mbar_wait(prepBar, 0);       // the reference arrays and DC sums are in the store
   TC2_STAMP(1);
   if (worker) {
 #pragma unroll 1
@@ -544,6 +558,36 @@ rmd_frame_tc2_kernel(const __grid_constant__ Tc2Args a) {
   }
 }
 
+// Border pre-pass of a frame launch: one CTA per CTU writes the CTU's images of all five depths (rmd_tc_frame.cuh prep_phase).
+// Reading the reconstruction neighbourhood once per CTU instead of once per CTU and depth, with the builders on a kernel that keeps
+// eight CTAs per SM (32 registers), takes them off the tensor-core CTAs, whose TMEM sits idle while their prologue runs.
+__global__ void __launch_bounds__(kTileThreads, 8)
+rmd_border_prep_kernel(const __grid_constant__ FrameSource fs, int strong, uint8_t* img) {
+  __shared__ __align__(16) unsigned char tile[Cfg<2>::TILE_BYTES];
+  __shared__ __align__(16) unsigned char stage[kPrepStageBytes];
+  const int cg = blockIdx.x, tid = threadIdx.x;
+  const CtuPos pos = ctu_pos(fs, cg);
+  {
+    TileLoad tl;
+    tile_load(tid, fs.rec + (size_t)pos.pic * fs.recPicStride, fs.recStride, fs.W, fs.H, pos.x, pos.y, tl);
+    tile_store<Cfg, 2>(tid, fs.W, fs.H, pos.x, pos.y, tl, tile);
+  }
+  auto depth = [&](auto tag) {
+    constexpr int L = decltype(tag)::value;
+    if (!__syncthreads_or(prep_phase<L>(0, fs, strong, cg, pos, tile, tid, stage, img))) return;
+#pragma unroll
+    for (int ph = 1; ph < kPrepPhases; ph++) {
+      prep_phase<L>(ph, fs, strong, cg, pos, tile, tid, stage, img);
+      __syncthreads();
+    }
+  };
+  depth(std::integral_constant<int, 6>());
+  depth(std::integral_constant<int, 5>());
+  depth(std::integral_constant<int, 4>());
+  depth(std::integral_constant<int, 3>());
+  depth(std::integral_constant<int, 2>());
+}
+
 // batch (S2) mode: one launch per PU size
 template <int LOG2N>
 __global__ void __launch_bounds__(kCtaThreads, 2)
@@ -576,6 +620,7 @@ cudaError_t launch_rmd_batch_tc2(int log2n, const BatchSource& bs, int strong, c
   const int n = 1 << log2n, pus = 4096 / (n * n);
   Tc2Args a;
   a.fs = FrameSource{}; a.bs = bs; a.strong = strong; a.totalCtus = (bs.count + pus - 1) / pus; a.tabWin = tabWin; a.tabN4 = tabN4; a.had = hadamard;
+  a.prep = nullptr;
   cudaError_t e;
   switch (log2n) {
     case 2: e = launch_batch_tc2<2>(a, a.totalCtus, st); break;
@@ -589,15 +634,32 @@ cudaError_t launch_rmd_batch_tc2(int log2n, const BatchSource& bs, int strong, c
   return e;
 }
 
-cudaError_t launch_rmd_frames_tc2(const FrameSource& fs, int nPics, int strong, const uint8_t* tabWin, const uint8_t* tabN4, const int8_t* hadamard,
-                                  cudaStream_t st, int* launches) {
+size_t rmd_tc2_prep_bytes(int nCtus) { return (size_t)nCtus * kPrepCtuBytes; }
+
+cudaError_t launch_rmd_border_prep(const FrameSource& fs, int nPics, int strong, uint8_t* prep, cudaStream_t st, int* launches) {
+  const int total = nPics * fs.ctusPerPic;
+  if (total <= 0) return cudaSuccess;
+  rmd_border_prep_kernel<<<total, kTileThreads, 0, st>>>(fs, strong, prep);
+  if (launches) *launches += 1;
+  return cudaGetLastError();
+}
+
+cudaError_t launch_rmd_frame_tc2(const FrameSource& fs, int nPics, int strong, const uint8_t* tabWin, const uint8_t* tabN4, const int8_t* hadamard,
+                                 const uint8_t* prep, cudaStream_t st, int* launches) {
   const int total = nPics * fs.ctusPerPic;
   if (total <= 0) return cudaSuccess;
   Tc2Args a;
-  a.fs = fs; a.bs = BatchSource{}; a.strong = strong; a.totalCtus = total; a.tabWin = tabWin; a.tabN4 = tabN4; a.had = hadamard;
+  a.fs = fs; a.bs = BatchSource{}; a.strong = strong; a.totalCtus = total; a.tabWin = tabWin; a.tabN4 = tabN4; a.had = hadamard; a.prep = prep;
   rmd_frame_tc2_kernel<<<frame_blocks(total), kCtaThreads, kSmemBytes, st>>>(a);
   if (launches) *launches += 1;
   return cudaGetLastError();
+}
+
+cudaError_t launch_rmd_frames_tc2(const FrameSource& fs, int nPics, int strong, const uint8_t* tabWin, const uint8_t* tabN4, const int8_t* hadamard,
+                                  uint8_t* prep, cudaStream_t st, int* launches) {
+  cudaError_t e = launch_rmd_border_prep(fs, nPics, strong, prep, st, launches);
+  if (e == cudaSuccess) e = launch_rmd_frame_tc2(fs, nPics, strong, tabWin, tabN4, hadamard, prep, st, launches);
+  return e;
 }
 
 }  // namespace cucd

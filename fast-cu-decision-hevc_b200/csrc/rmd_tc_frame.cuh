@@ -1,6 +1,7 @@
 // rmd_tc_frame.cuh - frame-mode pieces shared by the two tensor-core RMD kernels (rmd_tc2_kernels.cu: 8-bit content,
 // rmd_tc3_kernels.cu: 9/10-bit content) and by their CPU replays (tests/emul): block decode, CTU origins, PU states, the set-up
-// loads of the reconstruction neighbourhoods and source tiles, and the copy-out of the cost tables.  Phase 1 of the prologue
+// loads of the reconstruction neighbourhoods and source tiles, the border pre-pass of the 8-bit kernel, and the copy-out of the cost
+// tables.  Phase 1 of the prologue
 // (TileLoad / tile_load / tile_store) is in rmd_tc2.cuh beside the border builders that read its tiles.
 //
 // Everything is `__host__ __device__` and holds no barrier: a function is driven per thread by (tid, nthreads), the kernel bodies
@@ -88,8 +89,9 @@ CUCD_HD int fork_states(const FrameSource& fs, int unit, int totalCtus, uint8_t*
   return any;
 }
 
-// The set-up loads of a CTA: the origins of the unit's CTUs (-1 past the last CTU) and thread tid's part of their reconstruction
-// neighbourhoods, and `pre`, the eight rows of the source tile of the thread's row in pass 0 (zero unless the tile is inside the picture).
+// The set-up loads of a CTA: the origins of the unit's CTUs (-1 past the last CTU), thread tid's part of their reconstruction
+// neighbourhoods (tl; null for tc2, whose border pre-pass has read them), and `pre`, the eight rows of the source tile of the thread's
+// row in pass 0 (zero unless the tile is inside the picture).
 template <template <int> class Cfg, int LOG2N>
 CUCD_HD void setup_loads(const FrameSource& fs, int unit, int totalCtus, int tid, int* ctuX, int* ctuY, TileLoad* tl, Vec16* pre) {
   typedef Cfg<LOG2N> C;
@@ -100,7 +102,7 @@ CUCD_HD void setup_loads(const FrameSource& fs, int unit, int totalCtus, int tid
     if (cg >= totalCtus) continue;                           // CTA-uniform
     const CtuPos p = ctu_pos(fs, cg);
     ctuX[c] = p.x; ctuY[c] = p.y;
-    tile_load(tid, fs.rec + (size_t)p.pic * fs.recPicStride, fs.recStride, fs.W, fs.H, p.x, p.y, tl[c]);
+    if (tl) tile_load(tid, fs.rec + (size_t)p.pic * fs.recPicStride, fs.recStride, fs.W, fs.H, p.x, p.y, tl[c]);
   }
   const Row r0 = row_map<LOG2N>(tid, 0);
   const int cg0 = unit * C::CTUS + r0.ctu;
@@ -114,6 +116,58 @@ CUCD_HD void setup_loads(const FrameSource& fs, int unit, int totalCtus, int tid
       for (int y = 0; y < 8; y++) pre[y] = *reinterpret_cast<const Vec16*>(src + (size_t)y * fs.orgStride);
     }
   }
+}
+
+// ---------------------------------------------------------------------------------------------
+// border pre-pass of the 8-bit kernel (rmd_border_prep_kernel): one CTA of kTileThreads threads per CTU writes the CTU's images
+// (rmd_tc2.cuh PrepSize) of all five depths
+// ---------------------------------------------------------------------------------------------
+// It stages the reconstruction neighbourhood once (tile_load / tile_store) and then, per depth, runs the prologue's own builders for
+// CTU 0 of a CTA of that depth, on a staging area laid out as the RMD CTA's shared memory from VALID_OFF on (rmd_tc2.cuh ProlOff): the PU
+// states, the DC sums and the part of the store that CTU 0 touches (N >= 16: both row-group copies, of which the image is the first).
+template <int LOG2N>
+struct PrepStage {
+  typedef tc2::Cfg<LOG2N> C;
+  static constexpr int STORE_END = LOG2N == 2 ? 2 * 256 * 16 : (LOG2N == 3 ? 16 : C::GROUP_BYTES + 16) + C::PUS * C::PU_BYTES;
+  static constexpr int BYTES = tc2::ProlOff<LOG2N>::STORE + STORE_END;
+  static_assert(BYTES % 16 == 0, "the staging is cleared 16 bytes at a time");
+};
+constexpr int kPrepStageBytes = tc2::cmax(tc2::cmax(tc2::cmax(PrepStage<2>::BYTES, PrepStage<3>::BYTES), tc2::cmax(PrepStage<4>::BYTES, PrepStage<5>::BYTES)),
+                                          PrepStage<6>::BYTES);
+constexpr int kPrepPhases = 4;      // the kernel syncs its threads after each phase
+// Phase `phase` of depth LOG2N for thread tid of CTU cg (origin pos; `tile`: its staged neighbourhood).  img: the pre-pass output,
+// kPrepCtuBytes per CTU of the launch.
+//   0: clear the staging (so that the bytes no builder writes are the same in every image) and write the PU states of CTU 0; returns
+//      whether this thread found a PU to evaluate.  Where no thread did (outside the picture, or pruned in fork-aware mode) the
+//      kernel skips phases 1-3: no RMD row consumes that image.
+//   1: build_unfiltered   2: build_filtered   3: the image leaves for img
+template <int LOG2N>
+CUCD_HD int prep_phase(int phase, const FrameSource& fs, int strong, int cg, const CtuPos& pos, const unsigned char* tile, int tid, unsigned char* stage,
+                        unsigned char* img) {
+  typedef tc2::Cfg<LOG2N> C;
+  typedef tc2::PrepSize<LOG2N> S;
+  typedef tc2::ProlOff<LOG2N> O;
+  constexpr int nthreads = tc2::kTileThreads;
+  int any = 0;
+  if (phase == 0) {
+    Vec16* s = reinterpret_cast<Vec16*>(stage + O::DC);
+    for (int i = tid; i < (PrepStage<LOG2N>::BYTES - O::DC) / 16; i += nthreads) s[i] = Vec16{0u, 0u, 0u, 0u};
+    const uint8_t* need = ctu_needed<LOG2N>(fs, cg);
+    for (int p = tid; p < C::PUS; p += nthreads) {
+      stage[p] = pu_state<LOG2N>(fs, need, pos.x, pos.y, p);
+      any |= stage[p] == kPuEvaluate;
+    }
+  } else if (phase == 1) {
+    tc2::build_unfiltered_at<LOG2N>(tid, 0, fs.W, fs.H, pos.x, pos.y, tile, stage);
+  } else if (phase == 2) {
+    tc2::build_filtered_at<LOG2N>(tid, 0, strong, stage);
+  } else {
+    const Vec16* st = reinterpret_cast<const Vec16*>(stage + O::STORE + tc2::prep_store_off<LOG2N>(0, 0));
+    const Vec16* dc = reinterpret_cast<const Vec16*>(stage + O::DC);
+    Vec16* d = reinterpret_cast<Vec16*>(img + (size_t)cg * tc2::kPrepCtuBytes + tc2::prep_off<LOG2N>());
+    for (int i = tid; i < S::BYTES / 16; i += nthreads) d[i] = i < S::STORE / 16 ? st[i] : dc[i - S::STORE / 16];
+  }
+  return any;
 }
 
 // ---------------------------------------------------------------------------------------------

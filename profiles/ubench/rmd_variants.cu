@@ -3,8 +3,11 @@
 //   nvcc -std=c++17 -O3 -gencode arch=compute_100a,code=sm_100a -DKERNEL=2 [-DCUCD_V_...=..] -I../../fast-cu-decision-hevc_b200/csrc rmd_variants.cu -o v_xxx
 // KERNEL=2: rmd_frame_tc2_kernel (8-bit content, kind::i8); KERNEL=3: rmd_frame_tc3_kernel (10-bit content, kind::f16).
 // Prints the mean launch time and a checksum of the cost tables (variants of one kernel must print the same checksum).
+// KERNEL=2 takes a third argument: full (default: border pre-pass + RMD kernel, as the library launches them), rmd (the RMD kernel
+// alone, on images the pre-pass wrote once before the timing: what a free pre-pass would give) or prep (the pre-pass alone).
 #include <cstdio>
 #include <cstdlib>
+#include <cstring>
 #include <vector>
 #ifndef KERNEL
 #define KERNEL 2
@@ -59,7 +62,16 @@ int main(int argc, char** argv) {
     CK(cudaMemcpy(dHad, had.data(), had.size(), cudaMemcpyHostToDevice));
   }
   CK(configure_rmd_tc2_kernels());
-  auto launch = [&]() { return launch_rmd_frames_tc2(fs, P, 1, dTab, dTab + tc2::kWinTableBytes, dHad, 0, nullptr); };
+  uint8_t* dPrep;
+  CK(cudaMalloc(&dPrep, rmd_tc2_prep_bytes(total)));
+  CK(cudaMemset(dOut, 0, (size_t)total * 341 * 35 * 4));
+  const char* mode = argc > 3 ? argv[3] : "full";
+  CK(launch_rmd_border_prep(fs, P, 1, dPrep, 0, nullptr));
+  auto launch = [&]() {
+    if (!strcmp(mode, "prep")) return launch_rmd_border_prep(fs, P, 1, dPrep, 0, nullptr);
+    if (!strcmp(mode, "rmd")) return launch_rmd_frame_tc2(fs, P, 1, dTab, dTab + tc2::kWinTableBytes, dHad, dPrep, 0, nullptr);
+    return launch_rmd_frames_tc2(fs, P, 1, dTab, dTab + tc2::kWinTableBytes, dHad, dPrep, 0, nullptr);
+  };
 #else
   uint8_t* dTab;
   std::vector<uint8_t> tab(tc3::kWinTableBytes16 + tc3::kN4TableBytes16 + tc3::kHadBytes16);
@@ -79,6 +91,6 @@ int main(int argc, char** argv) {
   CK(cudaMemcpy(out.data(), dOut, out.size() * 4, cudaMemcpyDeviceToHost));
   unsigned long long sum = 0;
   for (size_t i = 0; i < out.size(); i++) sum = sum * 1000003ull + out[i];
-  printf("%s: %.4f ms per %d-picture launch (%d CTUs, %.3f M CTU/s), checksum %016llx\n", argv[0], ms, P, total, total / ms / 1e3, sum);
+  printf("%s%s%s: %.4f ms per %d-picture launch (%d CTUs, %.3f M CTU/s), checksum %016llx\n", argv[0], KERNEL == 2 ? " " : "", KERNEL == 2 ? (argc > 3 ? argv[3] : "full") : "", ms, P, total, total / ms / 1e3, sum);
   return 0;
 }

@@ -17,7 +17,7 @@ int main() {
   srand(1); for (auto& v : h) v = rand() & 255;
   int16_t *dOrg, *dRec; uint32_t* dOut; int8_t* dHad; uint8_t* dTab; long long* dDbg;
   CK(cudaMalloc(&dOrg, h.size() * 2)); CK(cudaMalloc(&dRec, h.size() * 2)); CK(cudaMalloc(&dOut, (size_t)total * 341 * 35 * 4));
-  CK(cudaMalloc(&dHad, 16384)); CK(cudaMalloc(&dTab, tc2::kWinTableBytes + tc2::kN4TableBytes));
+  CK(cudaMalloc(&dHad, 16384)); uint8_t* dPrep; CK(cudaMalloc(&dPrep, rmd_tc2_prep_bytes(total))); CK(cudaMalloc(&dTab, tc2::kWinTableBytes + tc2::kN4TableBytes));
   CK(cudaMemcpy(dOrg, h.data(), h.size() * 2, cudaMemcpyHostToDevice)); CK(cudaMemcpy(dRec, h.data(), h.size() * 2, cudaMemcpyHostToDevice));
   std::vector<uint8_t> tab(tc2::kWinTableBytes + tc2::kN4TableBytes);
   tc2::fill_win_tables(tab.data()); tc2::fill_n4_tables(tab.data() + tc2::kWinTableBytes);
@@ -42,7 +42,7 @@ int main() {
   FrameSource fs; fs.org = dOrg; fs.rec = dRec; fs.orgPicStride = (long long)pitch * H; fs.recPicStride = fs.orgPicStride; fs.orgStride = pitch; fs.recStride = pitch;
   fs.W = W; fs.H = H; fs.ctusPerRow = ctusPerRow; fs.ctusPerPic = ctusPerPic; fs.out = dOut; fs.outPacked = nullptr; fs.needed = nullptr;
   CK(configure_rmd_tc2_kernels());
-  for (int it = 0; it < 2; it++) CK(launch_rmd_frames_tc2(fs, P, 1, dTab, dTab + tc2::kWinTableBytes, dHad, 0, nullptr));
+  for (int it = 0; it < 2; it++) CK(launch_rmd_frames_tc2(fs, P, 1, dTab, dTab + tc2::kWinTableBytes, dHad, dPrep, 0, nullptr));
   CK(cudaDeviceSynchronize());
   std::vector<long long> d((size_t)blocks * 64); CK(cudaMemcpy(d.data(), dDbg, d.size() * 8, cudaMemcpyDeviceToHost));
   // N = 8 blocks: indices [2*u4 + u2, 2*u4 + 2*u2)

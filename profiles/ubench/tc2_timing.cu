@@ -15,7 +15,7 @@ int main(int argc, char** argv) {
   srand(1); for (auto& v : h) v = rand() & 255;
   int16_t *dOrg, *dRec; uint32_t* dOut; int8_t* dHad; uint8_t* dTab; long long* dDbg;
   CK(cudaMalloc(&dOrg, h.size() * 2)); CK(cudaMalloc(&dRec, h.size() * 2)); CK(cudaMalloc(&dOut, (size_t)total * 341 * 35 * 4));
-  CK(cudaMalloc(&dHad, 16384)); CK(cudaMalloc(&dTab, tc2::kWinTableBytes + tc2::kN4TableBytes));
+  CK(cudaMalloc(&dHad, 16384)); uint8_t* dPrep; CK(cudaMalloc(&dPrep, rmd_tc2_prep_bytes(total))); CK(cudaMalloc(&dTab, tc2::kWinTableBytes + tc2::kN4TableBytes));
   CK(cudaMemcpy(dOrg, h.data(), h.size() * 2, cudaMemcpyHostToDevice)); CK(cudaMemcpy(dRec, h.data(), h.size() * 2, cudaMemcpyHostToDevice));
   std::vector<uint8_t> tab(tc2::kWinTableBytes + tc2::kN4TableBytes);
   tc2::fill_win_tables(tab.data()); tc2::fill_n4_tables(tab.data() + tc2::kWinTableBytes);
@@ -43,7 +43,7 @@ int main(int argc, char** argv) {
   cudaEvent_t e0, e1; cudaEventCreate(&e0); cudaEventCreate(&e1);
   for (int it = 0; it < 3; it++) {
     cudaEventRecord(e0);
-    CK(launch_rmd_frames_tc2(fs, P, 1, dTab, dTab + tc2::kWinTableBytes, dHad, 0, nullptr));
+    CK(launch_rmd_frames_tc2(fs, P, 1, dTab, dTab + tc2::kWinTableBytes, dHad, dPrep, 0, nullptr));
     cudaEventRecord(e1); CK(cudaDeviceSynchronize());
     float ms; cudaEventElapsedTime(&ms, e0, e1); printf("launch %d: %.3f ms (%d CTUs, %.2f M CTU/s)\n", it, ms, total, total / ms / 1e3);
   }
@@ -65,13 +65,13 @@ int main(int argc, char** argv) {
       for (int b = 0; b < blocks; b++) {
         const long long* t = &d[(size_t)b * 64];
         if (t[4] != l) continue;
-        g[0] += t[50] - t[0]; g[1] += t[51] - t[50]; g[2] += t[52] - t[51]; g[3] += (t[53] ? t[53] - t[52] : 0); g[4] += t[54] - (t[53] ? t[53] : t[52]); g[5] += t[1] - t[54];
+        g[0] += t[50] - t[0]; g[1] += t[54] - t[50]; g[2] += t[55] - t[54]; g[3] += t[1] - t[55];
         g[6] += t[56] - t[1]; g[7] += t[57] - t[56];
       }
       { double h[4] = {0}; for (int b = 0; b < blocks; b++) { const long long* t = &d[(size_t)b * 64]; if (t[4] != l) continue; h[0] += t[58] - t[0]; h[1] += t[59] - t[58]; h[2] += t[60] - t[59]; h[3] += t[50] - t[60]; }
         printf("      first phase: tmem alloc %5.0f | issue loads %5.0f | zero + first load lands %5.0f | second table store + sync %5.0f\n", h[0] / n, h[1] / n, h[2] / n, h[3] / n); }
-      printf("      prologue: alloc+tables+zero+sync %5.0f | tile staging+sync %5.0f | unfiltered %5.0f | sync %5.0f | filtered %5.0f | fences+sync %5.0f || pass set-up: source tile %5.0f | operands+planar/DC %5.0f\n",
-             g[0] / n, g[1] / n, g[2] / n, g[3] / n, g[4] / n, g[5] / n, g[6] / n, g[7] / n);
+      printf("      prologue: alloc+tables+zero+sync %5.0f | PU states %5.0f | fences+CTA barrier %5.0f | wait for the border copies %5.0f || pass set-up: source tile %5.0f | operands+planar/DC %5.0f\n",
+             g[0] / n, g[1] / n, g[2] / n, g[3] / n, g[6] / n, g[7] / n);
     }
     for (int base = 30; base <= 40; base += 10) {
       double seg[8] = {0};
