@@ -62,7 +62,7 @@ def load_emul():
     so = os.path.join(d, "librmd_emul.so")
     csrc = os.path.join(ROOT, PKG, "csrc")
     cpps = [os.path.join(d, "rmd_emul.cpp"), os.path.join(d, "rmd_tc2_emul.cpp"), os.path.join(d, "rmd_tc3_emul.cpp"), os.path.join(d, "me_emul.cpp")]
-    srcs = cpps + [os.path.join(csrc, f) for f in ("rmd_core.cuh", "rmd_chunk.cuh", "rmd_tc2.cuh", "rmd_tc3.cuh", "rmd_tc_frame.cuh", "feature_core.cuh", "me_core.cuh")]
+    srcs = cpps + [os.path.join(d, "tc2_prep_replay.h")] + [os.path.join(csrc, f) for f in ("rmd_core.cuh", "rmd_chunk.cuh", "rmd_tc2.cuh", "rmd_tc3.cuh", "rmd_tc_frame.cuh", "feature_core.cuh", "me_core.cuh")]
     if not _newer(so, srcs):
         subprocess.run(["g++", "-std=c++17", "-O2", "-fPIC", "-shared", "-Wno-unknown-pragmas", "-I" + csrc, "-o", so] + cpps,
                        check=True, capture_output=True)
@@ -233,3 +233,90 @@ def oracle_prune_mask(lib, obf, W, H, skip, term):
     need = np.zeros((((W + 63) // 64) * ((H + 63) // 64), 341), np.uint8)
     lib.oracle_prune_mask(C.c_void_p(obf.ctypes.data), W, H, C.c_void_p(skip.ctypes.data), C.c_void_p(term.ctypes.data), C.c_void_p(need.ctypes.data))
     return need
+
+
+# ---------------------------------------------------------------------------------------------------
+# picture geometries of the frame paths
+# ---------------------------------------------------------------------------------------------------
+# The frame kernels build their borders in closed form (rmd_tc2.cuh pu_avail): the below-left and above-right runs are cut by the
+# picture edge, so they depend on W % 64 and H % 64.  Every residue 8 .. 56 occurs in both dimensions of a picture wider / taller than
+# one CTU; pictures narrower, shorter and smaller than one CTU, and odd CTU counts (CTAs of 2 and 4 CTUs straddle pictures of a
+# multi-picture launch), are in the list too.  Most sizes are 2 x 2 CTUs or fewer, so that the CPU replays stay cheap.
+EDGE_SIZES = [(72, 120), (80, 112), (88, 104), (96, 96), (104, 88), (112, 80), (120, 72),
+              (8, 8), (24, 136), (136, 40), (40, 24)]
+
+
+def edge_content(W, H, bd, seed):
+    """source and reconstruction for the geometry sweeps.  The source is textured.  The reconstruction is a gentle ramp everywhere but
+    its lower right quadrant, which is textured and holds full-range noise in its own lower right quarter: the ramp covers the whole
+    border of the 32x32 PUs along the top and the left, cut runs at the picture edge included, so the strong filter fires there"""
+    org = textured_plane(W, H, bd, seed=seed)
+    rec = pseudo_recon(org, bd, seed=seed + 1)
+    ramp = ((np.arange(H)[:, None] // 8 + np.arange(W)[None, :] // 6 + 40) << (bd - 8)).astype(np.int16)
+    y0, x0 = H // 2 // 8 * 8, W // 2 // 8 * 8
+    keep = np.zeros((H, W), bool)
+    keep[y0:, x0:] = True
+    rec = np.where(keep, rec, ramp)
+    y1, x1 = (H + y0) // 2, (W + x0) // 2
+    rec[y1:, x1:] = np.random.default_rng(seed + 2).integers(0, 1 << bd, (H - y1, W - x1))
+    return np.ascontiguousarray(org), np.ascontiguousarray(rec.astype(np.int16))
+
+
+def strong_filter_pus(oracle, org, rec, bd):
+    """the 32x32 PUs whose oracle costs differ between strong smoothing on and off, as (x0, y0, left units, above units): the number of
+    available 4-sample units of the left column with its below-left run and of the above row with its above-right run (16 each at most)"""
+    H, W = org.shape
+    diff = (oracle_rmd_frame(oracle, org, rec, bd, 1) != oracle_rmd_frame(oracle, org, rec, bd, 0)).any(axis=2)
+    out = []
+    for y0 in range(0, H - 31, 32):
+        for x0 in range(0, W - 31, 32):
+            if diff[(y0 // 64) * ((W + 63) // 64) + x0 // 64, pu_table_index(x0, y0, 32)]:
+                flags = np.zeros(33, np.uint8)
+                oracle.oracle_neighbour_flags(x0, y0, 32, W, H, P(flags, u8p))
+                out.append((x0, y0, int(flags[:16].sum()), int(flags[17:].sum())))
+    return out
+
+
+def threshold_recon(W, H, bd, seed):
+    """a ramp with noise of +-(1 << (bd - 6)) (+-4 at 8 bit, +-16 at 10 bit): the strong-smoothing deviations of its 32x32 PUs fall
+    around the threshold 1 << (bd - 5)"""
+    a = 1 << (bd - 6)
+    ramp = ((np.arange(H)[:, None] + np.arange(W)[None, :]) // 4 + 60) << (bd - 8)
+    noise = np.random.default_rng(seed).integers(-a, a + 1, (H, W))
+    return np.ascontiguousarray(np.clip(ramp + noise, 0, (1 << bd) - 1).astype(np.int16))
+
+
+def strong_deviations(lib, rec, bd):
+    """(|bl + tl - 2 L[N]|, |tl + tr - 2 T[N]|) of the unfiltered border (oracle_neighbour_flags + oracle_fill_border) of every 32x32 PU
+    inside the picture: the two values the strong-smoothing decision compares with 1 << (bd - 5)"""
+    H, W = rec.shape
+    rec = np.ascontiguousarray(rec, np.int16)
+    n = 32
+    out = []
+    for y0 in range(0, H - n + 1, n):
+        for x0 in range(0, W - n + 1, n):
+            flags = np.zeros(n + 1, np.uint8)                 # 2N / 4 units on each side and the corner
+            lib.oracle_neighbour_flags(x0, y0, n, W, H, P(flags, u8p))
+            b = np.zeros(4 * n + 1, np.int16)
+            lib.oracle_fill_border(bd, n, C.c_void_p(rec.ctypes.data + 2 * (y0 * W + x0)), W, P(flags, u8p), P(b, i16p))
+            b = b.astype(np.int64)
+            out.append((abs(b[0] + b[2 * n] - 2 * b[n]), abs(b[2 * n] + b[4 * n] - 2 * b[3 * n])))
+    return out
+
+
+THRESHOLD_PICTURES = {8: (192, 128, 0), 10: (192, 128, 48)}     # bit depth: W, H, seed of threshold_recon
+
+
+def threshold_picture(oracle, bd):
+    """source and reconstruction whose 32x32 borders put both strong-smoothing deviations, on the left and on the above side, at
+    1 << (bd - 5) and one below it; asserted here, so that a change of content cannot silently drop the case"""
+    W, H, seed = THRESHOLD_PICTURES[bd]
+    rec = threshold_recon(W, H, bd, seed)
+    thr = 1 << (bd - 5)
+    dev = strong_deviations(oracle, rec, bd)
+    for side in (0, 1):
+        vals = {d[side] for d in dev}
+        assert thr - 1 in vals and thr in vals, (bd, side)
+    assert any(max(d) == thr for d in dev)            # the decision fails only by reaching the threshold
+    assert any(max(d) == thr - 1 for d in dev)        # the decision holds one below it
+    return textured_plane(W, H, bd, seed=seed + 5), rec

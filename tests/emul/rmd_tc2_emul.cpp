@@ -6,12 +6,17 @@
 // worker thread ids.  The two tcgen05 products are replaced by exact integer matmuls
 // that read their operands through the same UMMA shared-memory layout / TMEM row layout the kernel uses,
 // and tcgen05.ld.pack::16b by its measured behaviour (profiles/ubench).  Built only by tests/.
+//
+// Frame mode builds the CTA's reference arrays in one of two ways: with the in-CTA prologue the kernel ran before its border pre-pass
+// existed (tile_store + build_unfiltered + build_filtered, emul_rmd_frame_tc2), or as the GPU does now, from the images of the replayed
+// pre-pass (tests/emul/tc2_prep_replay.h) placed by the CTA's bulk copies (emul_rmd_frames_tc2_prep).
 #include <cstdint>
 #include <cstring>
 #include <type_traits>
 #include <vector>
 #include "rmd_tc2.cuh"
 #include "rmd_tc_frame.cuh"
+#include "tc2_prep_replay.h"
 
 using namespace cucd;
 using namespace cucd::tc2;
@@ -52,9 +57,10 @@ void mma(const uint32_t* aWords, int aStride, int K, const void* b, bool bSigned
     }
 }
 
-// bs == nullptr: frame (replay) mode; otherwise batch (S2) mode over the PUs of one size described by *bs
+// bs == nullptr: frame (replay) mode; otherwise batch (S2) mode over the PUs of one size described by *bs.  Frame mode with img: the store
+// and the DC sums come from the pre-pass images img (kPrepCtuBytes per CTU of the launch), as rmd_frame_tc2_kernel takes them
 template <int LOG2N>
-void emul_cta(const FrameSource& fs, int strong, int totalCtus, int unit, const BatchSource* bs = nullptr) {
+void emul_cta(const FrameSource& fs, int strong, int totalCtus, int unit, const BatchSource* bs = nullptr, const uint8_t* img = nullptr) {
   typedef Geo<LOG2N> G;
   typedef Cfg<LOG2N> C;
   constexpr int N = G::N, log2n = LOG2N;
@@ -68,7 +74,7 @@ void emul_cta(const FrameSource& fs, int strong, int totalCtus, int unit, const 
     return;
   }
   if (LOG2N >= 4) for (int i = 0; i < C::CTUS * C::PUS * kNumModes; i++) acc[i] = 0;
-  for (int i = 0; i < C::CTUS * 64; i++) reinterpret_cast<int*>(smem + C::DC_OFF)[i] = 0;
+  if (!img) for (int i = 0; i < C::CTUS * 64; i++) reinterpret_cast<int*>(smem + C::DC_OFF)[i] = 0;   // image mode: copied in
   std::vector<Vec16> pre(kThreads * 8);            // frame mode: the rows' source tiles of pass 0 (setup_loads)
   // ---- prologue (tc2_prologue) ----
   if (bs) {
@@ -87,18 +93,22 @@ void emul_cta(const FrameSource& fs, int strong, int totalCtus, int unit, const 
   } else {
   int ctuXs[C::CTUS], ctuYs[C::CTUS];
   TileLoad tl[C::CTUS];                            // (phase 1 is replayed below by stage_tile)
-  for (int tid = 0; tid < kThreads; tid++) setup_loads<Cfg, LOG2N>(fs, unit, totalCtus, tid, ctuXs, ctuYs, tl, &pre[tid * 8]);
+  for (int tid = 0; tid < kThreads; tid++) setup_loads<Cfg, LOG2N>(fs, unit, totalCtus, tid, ctuXs, ctuYs, img ? nullptr : tl, &pre[tid * 8]);
   for (int c = 0; c < C::CTUS; c++) {
     if (ctuXs[c] < 0) { for (int p = 0; p < G::PUS; p++) valid[c * 256 + p] = kPuOutside; continue; }
     const uint8_t* need = ctu_needed<LOG2N>(fs, unit * C::CTUS + c);
     for (int p = 0; p < G::PUS; p++) valid[c * 256 + p] = pu_state<LOG2N>(fs, need, ctuXs[c], ctuYs[c], p);
   }
+  if (img) {
+    tc2replay::place_images<LOG2N>(img, unit, totalCtus, smem);
+  } else {
   for (int c = 0; c < C::CTUS; c++)          // phase 1: every thread id's tile_load + tile_store
     if (ctuXs[c] >= 0) stage_tile<LOG2N>(0, 1, fs.rec + (size_t)ctu_pos(fs, unit * C::CTUS + c).pic * fs.recPicStride, fs.recStride, fs.W, fs.H, ctuXs[c], ctuYs[c], smem + C::TILE_OFF + c * C::TILE_BYTES);
   for (int c = 0; c < C::CTUS; c++)
     if (ctuXs[c] >= 0) for (int tid = 0; tid < kThreads; tid++) build_unfiltered<LOG2N>(tid, c, fs.W, fs.H, ctuXs[c], ctuYs[c], smem + C::TILE_OFF + c * C::TILE_BYTES, smem);
   for (int c = 0; c < C::CTUS; c++)
     if (ctuXs[c] >= 0) for (int tid = 0; tid < kThreads; tid++) build_filtered<LOG2N>(tid, c, strong, smem);
+  }
   }
   std::memset(smem + C::TILE_OFF, 0x5A, C::CTUS * C::TILE_BYTES);   // the tiles alias the operand buffers: gone after the prologue
   unsigned char* store = smem + C::STORE_OFF;
@@ -246,6 +256,42 @@ int emul_rmd_frame_tc2(int strong, const int16_t* org, int orgStride, const int1
       default: emul_cta<2>(fs, strong, total, fb.unit);
     }
   }
+  return 0;
+}
+// The frame path the GPU runs: the border pre-pass over nPics pictures (picture p at org + p * orgPicStride, rec + p * recPicStride)
+// into an image buffer that holds `poison` everywhere before it runs (what an earlier launch left in the scratch), then every CTA of the
+// launch on the images.  needed: [ctu][341] fork-aware mask of the launch or null; out: [nPics * ctusPerPic][341][35]
+int emul_rmd_frames_tc2_prep(int strong, int nPics, const int16_t* org, long long orgPicStride, int orgStride, const int16_t* rec, long long recPicStride,
+                             int recStride, int W, int H, uint32_t* out, const uint8_t* needed, int poison) {
+  FrameSource fs;
+  fs.org = org; fs.rec = rec; fs.orgPicStride = orgPicStride; fs.recPicStride = recPicStride; fs.orgStride = orgStride; fs.recStride = recStride;
+  fs.W = W; fs.H = H; fs.ctusPerRow = (W + 63) / 64; fs.ctusPerPic = fs.ctusPerRow * ((H + 63) / 64); fs.out = out; fs.outPacked = nullptr; fs.needed = needed;
+  const int total = nPics * fs.ctusPerPic;
+  const std::vector<uint8_t> img = tc2replay::emul_prep(fs, strong, total, (uint8_t)poison);
+  for (int b = 0; b < frame_blocks(total); b++) {
+    const FrameBlock fb = frame_block(total, b);
+    switch (fb.log2n) {
+      case 6: emul_cta<6>(fs, strong, total, fb.unit, nullptr, img.data()); break;
+      case 5: emul_cta<5>(fs, strong, total, fb.unit, nullptr, img.data()); break;
+      case 4: emul_cta<4>(fs, strong, total, fb.unit, nullptr, img.data()); break;
+      case 3: emul_cta<3>(fs, strong, total, fb.unit, nullptr, img.data()); break;
+      default: emul_cta<2>(fs, strong, total, fb.unit, nullptr, img.data());
+    }
+  }
+  return 0;
+}
+// tc2::pu_avail of the PU of size 1 << log2n at (x0, y0): out = {lenL, lenT, availC}
+int emul_pu_avail(int log2n, int x0, int y0, int W, int H, int* out) {
+  PuAvail a;
+  switch (log2n) {
+    case 2: a = pu_avail<2>(x0, y0, W, H); break;
+    case 3: a = pu_avail<3>(x0, y0, W, H); break;
+    case 4: a = pu_avail<4>(x0, y0, W, H); break;
+    case 5: a = pu_avail<5>(x0, y0, W, H); break;
+    case 6: a = pu_avail<6>(x0, y0, W, H); break;
+    default: return -1;
+  }
+  out[0] = a.lenL; out[1] = a.lenT; out[2] = a.availC;
   return 0;
 }
 // batch (S2) mode: `count` PUs of ONE size, tightly packed org blocks and borders, out[count][35]

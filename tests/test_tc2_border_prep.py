@@ -35,7 +35,7 @@ def _rec(W, H, seed):
 def test_prepass_images_match_in_kernel_prologue(prep, strong, W, H, seed):
     rec = _rec(W, H, seed)
     compared = C.c_longlong(0)
-    bad = prep.emul_tc2_prep_check(strong, P(rec, i16p), W, W, H, C.byref(compared))
+    bad = prep.emul_tc2_prep_check(strong, 1, P(rec, i16p), C.c_longlong(0), W, W, H, None, C.byref(compared))
     assert compared.value > 0
     assert bad == 0
 
