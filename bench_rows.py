@@ -13,6 +13,7 @@ each on a 1080p-sized workload, and prints ONE JSON line per row:
            bounded sample, on `cores` host threads
 Rows: s2 (cucd_intra_rmd_batch), f1 (cucd_queue_*: K concurrent instances), s3 (cucd_me_sad_surface), f3 (cucd_me_subpel_cost),
 a12 (cucd_tmv_features), a13 (cucd_aq_activity), f2 (cucd_intra_tu_code / _forward / _recon).  Usage: python bench_rows.py [--iters 5] > gpurun_out/rows.jsonl
+Last row: f5 (cucd_me_mc_cost, motion compensation + distortion of inter candidates; row_f5 runs it on its own).
 """
 import argparse
 import ctypes as C
@@ -252,6 +253,82 @@ def main():
         emit(name, "TU/s", n_tu, k_s, w_s, algo, cpu, {"luma_samples_per_call": int(samples)}, p_s=p_s,
              h2d=int(o.nbytes + b.nbytes + n_tu * 16 + (samples * 4 if stage == 2 else 0)), d2h=int(out_bytes))
     eng.close()
+    row_f5(cucd, a.iters, T)
+
+
+def gpu_identity():
+    """name and power limit of the card the row ran on, read in the same run as the measurement"""
+    import subprocess
+    try:
+        r = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"], capture_output=True, text=True, timeout=30)
+        return r.stdout.strip().splitlines()[0]
+    except (OSError, IndexError, subprocess.SubprocessError):
+        return "unknown"
+
+
+def row_f5(cucd, iters=5, threads=8):
+    """f5: motion compensation + distortion of inter candidates (cucd_me_mc_cost) on a 1920x1080 10-bit picture with two references.
+    Batched: every whole 32x32, 16x16 and 8x8 PU carries five merge-like candidates (quarter-pel MVs within +-64 samples; a third uni
+    L0, a third uni L1, a third bi; Hadamard), one call for the picture.  Latency: one request of one 16x16 bi candidate, what an
+    encoder pays per call when it sends a PU at a time."""
+    bd, pad = 10, 80
+    org = _util.textured_plane(W, H, bd, seed=51)
+    refs = [np.pad(_util.pseudo_recon(_util.textured_plane(W, H, bd, seed=51, t=k + 1), bd), pad, mode="edge") for k in range(2)]
+    rng = np.random.default_rng(5)
+    eng = cucd.Engine(W, H, bit_depth=bd)
+    eng.set_cur_picture(org)
+    for k, r in enumerate(refs):
+        eng.set_ref_picture(k, r, pad, pad)
+    descs = []
+    for n in (32, 16, 8):
+        for y in range(0, H - n + 1, n):
+            for x in range(0, W - n + 1, n):
+                for c in range(5):
+                    mv = [int(v) for v in rng.integers(-256, 257, 4)]
+                    kind = (len(descs)) % 3
+                    ref = ((0, -1), (-1, 1), (0, 1))[kind]
+                    descs.append(dict(x=x, y=y, w=n, h=n, ref_idx=ref, mvx=(mv[0], mv[1]), mvy=(mv[2], mv[3]), use_hadamard=1))
+    arr, n_c, samples = cucd.Engine.mc_descs(descs)
+    dist = np.zeros(n_c, np.uint32)
+    pred = np.zeros(samples, np.int16)
+    k_s, w_s, p_s = timed(lambda: eng.me_mc_cost_raw(arr, n_c, dist), eng, iters, pin=(dist,))
+    kp_s, wp_s, _ = timed(lambda: eng.me_mc_cost_raw(arr, n_c, dist, pred), eng, iters, pin=(dist, pred))
+    n_lists = sum(2 if d["ref_idx"][0] >= 0 and d["ref_idx"][1] >= 0 else 1 for d in descs)
+    algo = sum(d["w"] * d["h"] * 2 + 4 + 44 for d in descs) + sum((d["w"] + 7) * (d["h"] + 7) * 2 for d in descs for r in d["ref_idx"] if r >= 0)
+    # CPU: the oracle on host threads, every 97th candidate
+    import mc_util
+    mco = mc_util.load_mc_oracle()
+    samp = descs[::97]
+    Wp = W + 2 * pad
+
+    def work(i):
+        d = samp[i]
+        blk = np.ascontiguousarray(org[d["y"]:d["y"] + d["h"], d["x"]:d["x"] + d["w"]])
+        a = [(C.c_void_p(refs[r].ctypes.data + 2 * ((d["y"] + (d["mvy"][l] >> 2) + pad) * Wp + d["x"] + (d["mvx"][l] >> 2) + pad)), d["mvx"][l] & 3, d["mvy"][l] & 3)
+             for l, r in enumerate(d["ref_idx"]) if r >= 0]
+        b = a[1] if len(a) == 2 else (None, 0, 0)
+        mco.oracle_mc_cost(bd, P(blk, i16p), d["w"], len(a), a[0][0], Wp, a[0][1], a[0][2], b[0], Wp, b[1], b[2], d["w"], d["h"], 1, None)
+    sec = cpu_parallel(work, len(samp), threads)
+    # single-candidate latency: wall clock of one call, median over many
+    one = [dict(x=960, y=528, w=16, h=16, ref_idx=(0, 1), mvx=(37, -90), mvy=(-13, 58), use_hadamard=1)]
+    one_arr, _, _ = cucd.Engine.mc_descs(one)
+    one_dist = np.zeros(1, np.uint32)
+    for _ in range(50):
+        eng.me_mc_cost_raw(one_arr, 1, one_dist)
+    lat = []
+    for _ in range(2000):
+        t0 = time.perf_counter()
+        eng.me_mc_cost_raw(one_arr, 1, one_dist)
+        lat.append(time.perf_counter() - t0)
+    eng.close()
+    emit("f5_me_mc_cost", "candidate/s", n_c, k_s, w_s, algo,
+         {"value": len(samp) / sec, "unit": "candidate/s", "cores": threads, "kind": "port",
+          "sample": f"every 97th candidate ({len(samp)}) through tests/mc_oracle.c in {sec:.2f} s"},
+         {"gpu": gpu_identity(), "bit_depth": bd, "pus": n_c // 5, "candidates_per_call": n_c, "lists_per_call": n_lists,
+          "with_pred": {"kernel_ms": kp_s * 1e3, "e2e_ms": wp_s * 1e3, "d2h_bytes": int(dist.nbytes + pred.nbytes)},
+          "single_candidate_latency_us": {"median": float(np.median(lat)) * 1e6, "p10": float(np.percentile(lat, 10)) * 1e6,
+                                          "p90": float(np.percentile(lat, 90)) * 1e6, "calls": len(lat), "candidate": "16x16 bi, Hadamard"}},
+         p_s=p_s, h2d=int(n_c * 44), d2h=int(dist.nbytes))
 
 
 if __name__ == "__main__":

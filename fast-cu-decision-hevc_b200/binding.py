@@ -91,6 +91,11 @@ class _SubpelDesc(C.Structure):
     _fields_ = [(n, C.c_int) for n in ("x", "y", "w", "h", "ref_idx", "mvx", "mvy", "use_hadamard")]
 
 
+class _McDesc(C.Structure):
+    _fields_ = [("x", C.c_int), ("y", C.c_int), ("w", C.c_int), ("h", C.c_int), ("ref_idx", C.c_int * 2), ("mvx", C.c_int * 2), ("mvy", C.c_int * 2),
+                ("use_hadamard", C.c_int)]
+
+
 class _TuDesc(C.Structure):
     _fields_ = [("log2_size", C.c_uint8), ("mode", C.c_uint8), ("qp", C.c_int8), ("flags", C.c_uint8)]
 
@@ -149,6 +154,7 @@ def load_library():
     lib.cucd_me_subpel_cost.argtypes = [C.c_void_p, C.c_int, C.POINTER(_SubpelDesc), C.c_void_p]
     lib.cucd_me_sad_surface_src.argtypes = [C.c_void_p, C.c_int, C.POINTER(_MeDesc), C.c_void_p, C.c_void_p]
     lib.cucd_me_subpel_cost_src.argtypes = [C.c_void_p, C.c_int, C.POINTER(_SubpelDesc), C.c_void_p, C.c_void_p]
+    lib.cucd_me_mc_cost.argtypes = [C.c_void_p, C.c_int, C.POINTER(_McDesc), C.c_void_p, C.c_void_p]
     lib.cucd_intra_tu_forward.argtypes = [C.c_void_p, C.c_int, C.POINTER(_TuDesc), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.cucd_intra_tu_recon.argtypes = [C.c_void_p, C.c_int, C.POINTER(_TuDesc), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.cucd_intra_tu_code.argtypes = [C.c_void_p, C.c_int, C.POINTER(_TuDesc), C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
@@ -464,6 +470,42 @@ class Engine:
             assert src.size == sum(int(d["w"]) * int(d["h"]) for d in descs)
             self._check(self.lib.cucd_me_subpel_cost_src(self.h, n, arr, src.ctypes.data, out.ctypes.data), "cucd_me_subpel_cost_src")
         return out
+
+    @staticmethod
+    def mc_descs(descs):
+        """list of dicts(x,y,w,h,ref_idx=(r0,r1),mvx=(..),mvy=(..),use_hadamard) -> (ctypes array, n, prediction samples)"""
+        arr = (_McDesc * max(len(descs), 1))()
+        samples = 0
+        for i, d in enumerate(descs):
+            for k in ("x", "y", "w", "h", "use_hadamard"):
+                setattr(arr[i], k, int(d[k]))
+            for k in ("ref_idx", "mvx", "mvy"):
+                a, b = d[k]
+                getattr(arr[i], k)[0] = int(a)
+                getattr(arr[i], k)[1] = int(b)
+            samples += int(d["w"]) * int(d["h"])
+        return arr, len(descs), samples
+
+    def me_mc_cost_raw(self, arr, n, dist, pred=None):
+        """cucd_me_mc_cost with a prebuilt descriptor array; dist: uint32 host array of n, pred: int16 host array or None"""
+        self._check(self.lib.cucd_me_mc_cost(self.h, n, arr, dist.ctypes.data, None if pred is None else pred.ctypes.data), "cucd_me_mc_cost")
+
+    def me_mc_cost(self, descs, want_pred=False):
+        """Motion compensation + distortion of inter candidates (cucd_me_mc_cost).  descs: list of dicts(x, y, w, h, ref_idx=(r0, r1),
+        mvx=(mx0, mx1), mvy=(my0, my1), use_hadamard); ref_idx -1 = list unused, MVs in quarter pels.  Returns dist, (n,) uint32, and
+        with want_pred=True also the list of (h, w) int16 predictions: (dist, preds)."""
+        arr, n, samples = self.mc_descs(descs)
+        dist = np.zeros(n, np.uint32)
+        pred = np.zeros(max(samples, 1), np.int16) if want_pred else None
+        self.me_mc_cost_raw(arr, n, dist, pred)
+        if not want_pred:
+            return dist
+        res, off = [], 0
+        for d in descs:
+            w, h = int(d["w"]), int(d["h"])
+            res.append(pred[off:off + w * h].reshape(h, w))
+            off += w * h
+        return dist, res
 
     # ---- intra luma TU coding (xIntraCodingTUBlock) ------------------------------------------------
     @staticmethod

@@ -602,6 +602,60 @@ int cucd_dev_me_subpel_cost(cucd_handle* h, void* stream, int nPU, const cucd_su
 }
 
 // ------------------------------------------------------------------------------------------------
+// Motion compensation and distortion of inter candidates (uni- and bi-predictive), me_core.cuh me_mc_*
+// ------------------------------------------------------------------------------------------------
+int cucd_me_mc_cost(cucd_handle* h, int nPU, const cucd_mc_desc* desc, uint32_t* dist, int16_t* pred) {
+  if (!h || nPU < 0 || (nPU > 0 && (!desc || !dist))) return fail(h, CUCD_ERR_INVALID, "cucd_me_mc_cost: bad argument");
+  if (nPU == 0) return CUCD_OK;
+  LOCK(h);
+  if (!h->curSet) return fail(h, CUCD_ERR_INVALID, "cucd_me_mc_cost: cucd_set_cur_picture not called");
+  CK(cudaSetDevice(h->cfg.device));
+  const int W = h->cfg.width, H = h->cfg.height;
+  // pinned scratch: [sorted jobs | CTA starts]; the jobs in caller order are built in a host vector first
+  std::vector<McJob> jobs(nPU);
+  long long predOff = 0;
+  for (int i = 0; i < nPU; i++) {
+    const cucd_mc_desc& d = desc[i];
+    if (d.w < 4 || d.h < 4 || d.w > 64 || d.h > 64 || (d.w & 3) || (d.h & 3) || d.x < 0 || d.y < 0 || d.x + d.w > W || d.y + d.h > H)
+      return fail(h, CUCD_ERR_INVALID, "cucd_me_mc_cost: bad PU (w, h multiples of 4 in 4..64, inside the picture)");
+    int nl = 0, slot[2], mvx[2], mvy[2], stride[2], mX[2], mY[2];
+    for (int l = 0; l < 2; l++) {
+      if (d.ref_idx[l] < 0) continue;
+      if (d.ref_idx[l] >= (int)h->refs.size() || !h->refs[d.ref_idx[l]].set) return fail(h, CUCD_ERR_INVALID, "cucd_me_mc_cost: reference picture not set");
+      const RefPlane& r = h->refs[d.ref_idx[l]];
+      const int ix = d.x + (d.mvx[l] >> 2), iy = d.y + (d.mvy[l] >> 2);
+      if (ix - 3 < -r.marginX || iy - 3 < -r.marginY || ix + d.w + 3 > W - 1 + r.marginX || iy + d.h + 3 > H - 1 + r.marginY)
+        return fail(h, CUCD_ERR_INVALID, "cucd_me_mc_cost: the interpolation support leaves the padded reference picture");
+      slot[nl] = d.ref_idx[l]; mvx[nl] = d.mvx[l]; mvy[nl] = d.mvy[l]; stride[nl] = r.stride; mX[nl] = r.marginX; mY[nl] = r.marginY; nl++;
+    }
+    if (nl == 0) return fail(h, CUCD_ERR_INVALID, "cucd_me_mc_cost: a candidate uses neither list (ref_idx both < 0)");
+    jobs[i] = me_mc_job(d.y * h->curStride + d.x, d.x, d.y, d.w, d.h, nl, slot, mvx, mvy, stride, mX, mY, d.use_hadamard, i, predOff);
+    predOff += (long long)d.w * d.h;
+  }
+  const size_t jobBytes = up16((size_t)nPU * sizeof(McJob)), ctaBytes = up16((size_t)(nPU + 1) * sizeof(int32_t));
+  CK(h->hScratch.reserve(jobBytes + ctaBytes));
+  McJob* sorted = reinterpret_cast<McJob*>(h->hScratch.p);
+  int32_t* ctaFirst = reinterpret_cast<int32_t*>(h->hScratch.p + jobBytes);
+  const int nCta = me_mc_plan(nPU, jobs.data(), sorted, ctaFirst);
+  if (sync_ref_table(h) != CUCD_OK) return CUCD_ERR_CUDA;
+  BatchIo io(h);
+  const int iAll = io.add_in(h->hScratch.p, jobBytes + ctaBytes, true);
+  const int oDist = io.add_out(dist, (size_t)nPU * sizeof(uint32_t));
+  const int oPred = io.add_out(pred, (size_t)predOff * sizeof(int16_t));
+  if (io.reserve() != CUCD_OK || io.upload(h->sMain) != CUCD_OK) return CUCD_ERR_CUDA;
+  MePlanes mp;
+  mp.cur = h->dCur.p; mp.curStride = h->curStride; mp.ref = h->dRefPtr.p; mp.refStride = h->dRefStride.p; mp.bitDepth = h->cfg.bit_depth;
+  const uint8_t* dAll = io.din<uint8_t>(iAll);
+  if (!io.direct) CK(cudaEventRecord(h->evK0, h->sMain));
+  CK(launch_me_mc(mp, reinterpret_cast<const McJob*>(dAll), reinterpret_cast<const int32_t*>(dAll + jobBytes), nCta, io.dout<uint32_t>(oDist),
+                  pred ? io.dout<int16_t>(oPred) : nullptr, h->sMain, &h->launches));
+  if (!io.direct) { CK(cudaEventRecord(h->evK1, h->sMain)); h->kTimed = true; } else h->kTimed = false;
+  if (io.download(h->sMain) != CUCD_OK) return CUCD_ERR_CUDA;
+  flush_launches(h);
+  return CUCD_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
 // Intra luma TU coding (xIntraCodingTUBlock): forward half, reconstruction half, or the whole chain with the plain quantiser
 // ------------------------------------------------------------------------------------------------
 static int tu_batch(cucd_handle* h, const char* who, int stage, int flags, int nTU, const cucd_tu_desc* desc, const int16_t* org, const int16_t* border,

@@ -116,6 +116,10 @@ struct SubpelJob {
 };
 // out[job][49]: distortion at quarter-pel offsets (dy+3)*7 + (dx+3), dx, dy = -3..3 around the integer mv
 cudaError_t launch_me_subpel(const MePlanes& mp, const SubpelJob* jobs, int nJobs, uint32_t* out, cudaStream_t st, int* launches);
+// motion compensation + distortion of inter candidates (me_core.cuh, McJob): CTA b takes jobs[ctaFirst[b] .. ctaFirst[b + 1]);
+// dist[outIndex] per candidate, pred (may be null) the w x h predictions at predOff
+struct McJob;
+cudaError_t launch_me_mc(const MePlanes& mp, const McJob* jobs, const int32_t* ctaFirst, int nCta, uint32_t* dist, int16_t* pred, cudaStream_t st, int* launches);
 cudaError_t launch_me_sad(const MePlanes& mp, const MeJob* jobs, int nJobs, const int32_t* tileJob, const int32_t* tileIdx, int nTilesDy, int nTilesO,
                           uint32_t* out, cudaStream_t st, int* launches);
 

@@ -327,14 +327,15 @@ CUCD_HD void me_smem_add(int* where, int what) {       // shared-memory atomic i
 #endif
 }
 // distortion of the nP predicted blocks: xGetHADs (8x8 tiles when both sizes are multiples of 8, else 4x4) or xGetSAD, one thread per
-// tile / per sample
-CUCD_HD void subpel_small_dist(int tid, const SubpelGeo& g, int nP, int useHadamard, const int16_t* sCur, const int16_t* sPred, int* sSum) {
+// tile / per sample.  curPlane: 0 = one source block for every prediction (the 49 positions of one PU), wh = block pl has its own
+// source block at sCur + pl * wh (the candidates of me_mc_kernel)
+CUCD_HD void subpel_small_dist(int tid, const SubpelGeo& g, int nP, int useHadamard, const int16_t* sCur, const int16_t* sPred, int* sSum, int curPlane = 0) {
   if (useHadamard) {
     const bool tile8 = !(g.w & 7) && !(g.h & 7);
     const int T = tile8 ? 8 : 4, tilesX = g.w / T, nTiles = tilesX * (g.h / T);
     for (int task = tid; task < nP * nTiles; task += 256) {
       const int pl = task / nTiles, tile = task - pl * nTiles, ty = tile / tilesX, tx = tile - ty * tilesX;
-      const int16_t* a = sCur + ty * T * g.w + tx * T;
+      const int16_t* a = sCur + pl * curPlane + ty * T * g.w + tx * T;
       const int16_t* b = sPred + pl * g.wh + ty * T * g.w + tx * T;
       uint32_t cost;
       if (tile8) {
@@ -357,9 +358,152 @@ CUCD_HD void subpel_small_dist(int tid, const SubpelGeo& g, int nP, int useHadam
   } else {
     for (int i = tid; i < nP * g.wh; i += 256) {
       const int pl = (int)me_mulhi((uint32_t)i, g.invWh);
-      const int d = iabs32((int)sCur[i - pl * g.wh] - (int)sPred[i]);
+      const int d = iabs32((int)sCur[i - pl * g.wh + pl * curPlane] - (int)sPred[i]);
       if (d) me_smem_add(&sSum[pl], d);
     }
+  }
+}
+
+// =============================================================================================================================
+// Motion compensation and distortion of inter candidates (cucd_me_mc_cost): TComPrediction::motionCompensation for luma
+// (xPredInterUni / xPredInterBi -> xPredInterBlk, TComPrediction.cpp:496-620; TComInterpolationFilter.cpp:57-290 filter /
+// filterCopy; TComYuv::addAvg, TComYuv.cpp:260-310) followed by the DistFunc of xGetInterPredictionError (TEncSearch.cpp:2905-2926,
+// iSubShift = 0).  A candidate is one PU at one quarter-pel motion of one list (uni) or two lists (bi).  The host sorts the
+// candidates into classes of equal shape, list count and distortion; a CTA takes up to me_mc_per_cta() candidates of one class, so
+// that every phase maps a flat index onto (candidate, list, row, column) with multiply-high divisions and small PUs share a CTA.
+//   stage  the source blocks and, per candidate and list, the (w + 7) x (h + 7) reference window whose origin is (-3, -3) from the
+//          integer part of the MV
+//   hor    rows -> 14-bit intermediates (filterHor, isFirst, !isLast; filterCopy isFirst for a zero fraction), h + 7 rows per list
+//   ver    columns.  Uni: filterVer (!isFirst, isLast) with rounding and clipping, as subpel_small_ver.  Bi: filterVer (!isFirst,
+//          !isLast) - sum >> 6, a plain copy at fraction 0 - per list, then addAvg: clip((p0 + p1 + 2^(14-bd) + 16384) >> (15-bd)).
+//          The predictions overwrite the dead windows.
+//   dist   subpel_small_dist on the candidates' own source blocks
+// =============================================================================================================================
+constexpr int kMcCurCap = 4096;           // source blocks (and predictions) of a CTA, int16
+constexpr int kMcWinCap = 10240;          // reference windows: sum over candidates and lists of (w + 7) (h + 7), >= 2 * 71 * 71
+constexpr int kMcTmpCap = 9216;           // row intermediates: sum of (h + 7) w, >= 2 * 71 * 64
+constexpr int kMcMaxCand = 64;            // candidates of a CTA
+CUCD_HD int me_mc_per_cta(int w, int h, int nl) {
+  int k = kMcCurCap / (w * h);
+  const int kw = kMcWinCap / (nl * (w + 7) * (h + 7)), kt = kMcTmpCap / (nl * (h + 7) * w);
+  k = k < kw ? k : kw; k = k < kt ? k : kt;
+  return k < kMcMaxCand ? k : kMcMaxCand;
+}
+// CTAs hold candidates of one class: shape, list count and distortion function
+inline int me_mc_class(int w, int h, int nl, int had) { return (((((w >> 2) - 1) * 16 + (h >> 2) - 1) * 2 + nl - 1) * 2) + (had ? 1 : 0); }
+constexpr int kMcClasses = 16 * 16 * 4;
+
+struct McJob {
+  int32_t curOff;      // PU origin inside the current picture plane
+  int32_t refOff[2];   // per list: the window origin (-3, -3 from the integer MV position) inside the padded plane of refSlot
+  int16_t refSlot[2];
+  int8_t fx[2], fy[2]; // per list: quarter-pel fractions
+  int16_t w, h;
+  int8_t nl, had;      // lists used (1 uni, 2 bi; list 1 of a uni L1 candidate sits in entry 0); xGetHADs / xGetSAD
+  int16_t pad;
+  int32_t outIndex;    // candidate index in the caller's order (dist)
+  int64_t predOff;     // offset of its w x h prediction block in the caller's pred array
+};
+// host: the job of a candidate whose nl used lists (compacted: entry 0, then entry 1) have reference slot, quarter-pel MV and padded
+// plane stride / margins slot[l], mvx[l], mvy[l], stride[l], mX[l], mY[l]
+inline McJob me_mc_job(int curOff, int x, int y, int w, int h, int nl, const int* slot, const int* mvx, const int* mvy, const int* stride, const int* mX,
+                       const int* mY, int had, int outIndex, long long predOff) {
+  McJob j;
+  j.curOff = curOff;
+  for (int l = 0; l < 2; l++) {
+    const int u = l < nl ? l : 0;
+    j.refOff[l] = (y + (mvy[u] >> 2) - 3 + mY[u]) * stride[u] + x + (mvx[u] >> 2) - 3 + mX[u];
+    j.refSlot[l] = (int16_t)slot[u]; j.fx[l] = (int8_t)(mvx[u] & 3); j.fy[l] = (int8_t)(mvy[u] & 3);
+  }
+  j.w = (int16_t)w; j.h = (int16_t)h; j.nl = (int8_t)nl; j.had = (int8_t)(had ? 1 : 0); j.pad = 0;
+  j.outIndex = outIndex; j.predOff = predOff;
+  return j;
+}
+// host: the jobs sorted by class into `sorted`, every class cut into CTAs of me_mc_per_cta candidates; CTA b takes
+// sorted[ctaFirst[b] .. ctaFirst[b + 1]).  ctaFirst has room for n + 1 entries; returns the number of CTAs.
+inline int me_mc_plan(int n, const McJob* jobs, McJob* sorted, int32_t* ctaFirst) {
+  int start[kMcClasses + 1] = {0};
+  for (int i = 0; i < n; i++) start[me_mc_class(jobs[i].w, jobs[i].h, jobs[i].nl, jobs[i].had) + 1]++;
+  for (int c = 0; c < kMcClasses; c++) start[c + 1] += start[c];
+  // stable scatter: start[c] advances to the end of class c
+  for (int i = 0; i < n; i++) sorted[start[me_mc_class(jobs[i].w, jobs[i].h, jobs[i].nl, jobs[i].had)]++] = jobs[i];
+  int nCta = 0;
+  for (int b = 0; b < n;) {
+    const McJob& j = sorted[b];
+    const int c = me_mc_class(j.w, j.h, j.nl, j.had), per = me_mc_per_cta(j.w, j.h, j.nl), e = start[c];
+    for (; b < e; b += per) ctaFirst[nCta++] = b;
+    b = e;
+  }
+  ctaFirst[nCta] = n;
+  return nCta;
+}
+struct McGeo {
+  int w, h, bd, head, nl, n, wh, pw /* w + 7 */, win /* (w + 7)(h + 7) */, tmp /* (h + 7) w */;
+  uint32_t invW, invPw, invWh, invWin, invTmp;
+};
+CUCD_HD McGeo me_mc_geo(int w, int h, int nl, int n, int bd) {
+  McGeo g;
+  g.w = w; g.h = h; g.bd = bd; g.head = 14 - bd; g.nl = nl; g.n = n; g.wh = w * h; g.pw = w + 7; g.win = (w + 7) * (h + 7); g.tmp = (h + 7) * w;
+  g.invW = me_inv((uint32_t)w); g.invPw = me_inv((uint32_t)g.pw); g.invWh = me_inv((uint32_t)g.wh); g.invWin = me_inv((uint32_t)g.win); g.invTmp = me_inv((uint32_t)g.tmp);
+  return g;
+}
+// every index below is < 10240 and every divisor <= 5041: i * d < 2^32, so the multiply-high divisions are exact
+CUCD_HD void me_mc_stage(int tid, const McGeo& g, const McJob* jobs, const int16_t* cur, int curStride, const int16_t* const* ref, const int32_t* refStride,
+                         int16_t* sCur, int16_t* sWin) {
+  for (int i = tid; i < g.n * g.wh; i += 256) {
+    const int k = (int)me_mulhi((uint32_t)i, g.invWh), rem = i - k * g.wh;
+    const int y = (int)me_mulhi((uint32_t)rem, g.invW), x = rem - y * g.w;
+    sCur[i] = cur[jobs[k].curOff + (long long)y * curStride + x];
+  }
+  for (int i = tid; i < g.n * g.nl * g.win; i += 256) {
+    const int kl = (int)me_mulhi((uint32_t)i, g.invWin), rem = i - kl * g.win;
+    const int y = (int)me_mulhi((uint32_t)rem, g.invPw), x = rem - y * g.pw;
+    const McJob& j = jobs[kl >> (g.nl - 1)];
+    const int l = kl & (g.nl - 1), slot = j.refSlot[l];
+    sWin[i] = ref[slot][j.refOff[l] + (long long)y * refStride[slot] + x];
+  }
+}
+// rows of every window -> sTmp[kl][r][c], r = 0 .. h + 6 (filterHor, isFirst, !isLast; filterCopy isFirst at fx = 0)
+CUCD_HD void me_mc_hor(int tid, const McGeo& g, const McJob* jobs, const int16_t* sWin, int16_t* sTmp) {
+  for (int i = tid; i < g.n * g.nl * g.tmp; i += 256) {
+    const int kl = (int)me_mulhi((uint32_t)i, g.invTmp), rem = i - kl * g.tmp;
+    const int r = (int)me_mulhi((uint32_t)rem, g.invW), c = rem - r * g.w;
+    const int fx = jobs[kl >> (g.nl - 1)].fx[kl & (g.nl - 1)];
+    const int16_t* s = &sWin[kl * g.win + r * g.pw + c + 3];
+    sTmp[i] = (int16_t)(fx == 0 ? (s[0] << g.head) - 8192 : (luma_filter8(s, 1, fx) - (8192 << (6 - g.head))) >> (6 - g.head));
+  }
+}
+// columns -> the clipped prediction sPred[k][r][c] (and pred[predOff + r w + c] when pred is not null).
+// Bi: HM reaches the 14-bit intermediate of a list through four branches of xPredInterBlk (TComPrediction.cpp:560-600): filterCopy
+// (isFirst, !isLast) for fx = fy = 0, filterHor (isFirst, !isLast) for fy = 0, filterVer (isFirst, !isLast) on the reference for
+// fx = 0, and filterHor (isFirst, !isLast) + filterVer (!isFirst, !isLast) otherwise.  The two-stage form below equals all four:
+// the first three are it with a plain-copy second stage or (fx = 0, fy != 0) with taps summing to 64 over s << head - 8192, where
+// (sum c (s << head) - 8192 * 64) >> 6 == (sum c s - (8192 << (6 - head))) >> (6 - head) because 2^head divides both numerator
+// and divisor.  Intermediates stay in int16: |stage 1| <= 14 330, |stage 2| <= 25 072 at 10 bits; the sums are int32.
+CUCD_HD void me_mc_ver(int tid, const McGeo& g, const McJob* jobs, const int16_t* sTmp, int16_t* sPred, int16_t* pred) {
+  const int maxVal = (1 << g.bd) - 1;
+  for (int i = tid; i < g.n * g.wh; i += 256) {
+    const int k = (int)me_mulhi((uint32_t)i, g.invWh), rem = i - k * g.wh;
+    const int r = (int)me_mulhi((uint32_t)rem, g.invW), c = rem - r * g.w;
+    const McJob& j = jobs[k];
+    int v;
+    if (g.nl == 1) {
+      const int16_t* s = &sTmp[k * g.tmp + (r + 3) * g.w + c];
+      const int fy = j.fy[0];
+      v = fy == 0 ? (s[0] + 8192 + (1 << (g.head - 1))) >> g.head : (luma_filter8(s, g.w, fy) + (1 << (5 + g.head)) + (8192 << 6)) >> (6 + g.head);
+    } else {
+      int p[2];
+#pragma unroll
+      for (int l = 0; l < 2; l++) {
+        const int16_t* s = &sTmp[(2 * k + l) * g.tmp + (r + 3) * g.w + c];
+        const int fy = j.fy[l];
+        p[l] = fy == 0 ? s[0] : luma_filter8(s, g.w, fy) >> 6;
+      }
+      v = (p[0] + p[1] + (1 << g.head) + 16384) >> (g.head + 1);
+    }
+    v = v < 0 ? 0 : (v > maxVal ? maxVal : v);
+    sPred[i] = (int16_t)v;
+    if (pred) pred[j.predOff + rem] = (int16_t)v;
   }
 }
 

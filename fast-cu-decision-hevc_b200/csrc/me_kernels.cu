@@ -361,6 +361,38 @@ me_subpel_small_kernel(const MePlanes mp, const SubpelJob* __restrict__ jobs, ui
   }
 }
 
+// Motion compensation + distortion of inter candidates (me_core.cuh, me_mc_*): a CTA takes the candidates jobs[ctaFirst[b] ..
+// ctaFirst[b + 1]) of one class; the predictions reuse the shared memory of the dead reference windows.
+__global__ void __launch_bounds__(256)
+me_mc_kernel(const MePlanes mp, const McJob* __restrict__ jobs, const int32_t* __restrict__ ctaFirst, uint32_t* __restrict__ dist, int16_t* __restrict__ pred) {
+  __shared__ __align__(16) int16_t sCur[kMcCurCap];
+  __shared__ __align__(16) int16_t sWin[kMcWinCap];
+  __shared__ __align__(16) int16_t sTmp[kMcTmpCap];
+  __shared__ int sSum[kMcMaxCand];
+  const int tid = threadIdx.x;
+  const int first = ctaFirst[blockIdx.x];
+  const McJob* J = jobs + first;
+  const McGeo g = me_mc_geo(J[0].w, J[0].h, J[0].nl, ctaFirst[blockIdx.x + 1] - first, mp.bitDepth);
+  const int had = J[0].had;
+  if (tid < g.n) sSum[tid] = 0;
+  me_mc_stage(tid, g, J, mp.cur, mp.curStride, mp.ref, mp.refStride, sCur, sWin);
+  __syncthreads();
+  me_mc_hor(tid, g, J, sWin, sTmp);
+  __syncthreads();
+  me_mc_ver(tid, g, J, sTmp, sWin, pred);
+  __syncthreads();
+  subpel_small_dist(tid, subpel_geo(g.w, g.h, g.bd), g.n, had, sCur, sWin, sSum, g.wh);
+  __syncthreads();
+  if (tid < g.n) dist[J[tid].outIndex] = (uint32_t)sSum[tid] >> (g.bd - 8);
+}
+
+cudaError_t launch_me_mc(const MePlanes& mp, const McJob* jobs, const int32_t* ctaFirst, int nCta, uint32_t* dist, int16_t* pred, cudaStream_t st, int* launches) {
+  if (nCta <= 0) return cudaSuccess;
+  me_mc_kernel<<<nCta, 256, 0, st>>>(mp, jobs, ctaFirst, dist, pred);
+  if (launches) *launches += 1;
+  return cudaGetLastError();
+}
+
 cudaError_t launch_me_subpel(const MePlanes& mp, const SubpelJob* jobs, int nJobs, uint32_t* out, cudaStream_t st, int* launches) {
   if (nJobs <= 0) return cudaSuccess;
   me_subpel_kernel<<<dim3(nJobs, 7), 256, 0, st>>>(mp, jobs, out);

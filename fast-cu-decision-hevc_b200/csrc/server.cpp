@@ -4,7 +4,7 @@
 // segment this program creates, post their requests and sleep.  The server loop polls the slots:
 //   - S2 requests (rough mode decision of a few PUs with caller-supplied borders - what TEncSearch.cpp:2327-2361 can offer at a
 //     time) of ALL instances are gathered for a short batching window and run as ONE cucd_intra_rmd_batch per bit depth;
-//   - S1 / S3 / sub-pel requests depend on their instance's pictures and run on that instance's handle, in arrival order.
+//   - S1 / S3 / sub-pel / inter-candidate requests depend on their instance's pictures and run on that instance's handle, in arrival order.
 // Only the C ABI of include/cucudecide.h is used: the server is an ordinary client of the library.
 //
 //   cucd_server --name /cucd_xyz --clients N [--window-us 20] [--device 0]      prints one JSON line of statistics on exit
@@ -162,6 +162,22 @@ int main(int argc, char** argv) {
           reply(s, rc, rc == CUCD_OK ? nullptr : cucd_last_error(k.h));
           break;
         }
+        case CUCD_IPC_MC: {
+          // the reply must fit what the client reserved: dist, then (args[0]) the predictions
+          const size_t nC = (size_t)(s.n > 0 ? s.n : 0), distBytes = (nC * 4 + 15) & ~(size_t)15;
+          const cucd_mc_desc* desc = reinterpret_cast<const cucd_mc_desc*>(in);
+          size_t need = distBytes;
+          if (nC * sizeof(cucd_mc_desc) <= s.in_bytes && s.args[0])
+            for (size_t i = 0; i < nC; i++) need += (size_t)(desc[i].w > 0 ? desc[i].w : 0) * (size_t)(desc[i].h > 0 ? desc[i].h : 0) * 2;
+          if (nC * sizeof(cucd_mc_desc) > s.in_bytes || need > s.out_bytes || s.out_off + s.out_bytes > hdr->arena_bytes) {
+            reply(s, CUCD_ERR_INVALID, "cucd_me_mc_cost: request and reply sizes disagree");
+            break;
+          }
+          int16_t* pred = s.args[0] ? reinterpret_cast<int16_t*>(out + distBytes) : nullptr;
+          const int rc = k.h ? cucd_me_mc_cost(k.h, s.n, desc, reinterpret_cast<uint32_t*>(out), pred) : CUCD_ERR_INVALID;
+          reply(s, rc, rc == CUCD_OK ? nullptr : cucd_last_error(k.h));
+          break;
+        }
         default:
           reply(s, CUCD_ERR_INVALID, "unknown request");
       }
@@ -223,10 +239,10 @@ int main(int argc, char** argv) {
   if (segPinned) cudaHostUnregister(mem);
   printf("{\"clients\": %d, \"closed\": %d, \"seconds\": %.3f, \"rmd_requests\": %lld, \"rmd_pus\": %lld, \"rmd_batches\": %lld, \"pus_per_batch\": %.1f, "
          "\"requests_per_batch\": %.2f, \"max_batch_pus\": %lld, \"rmd_busy_seconds\": %.3f, \"frames\": %lld, \"me_surfaces\": %lld, \"subpel\": %lld, "
-         "\"set_ref\": %lld, \"window_us\": %.1f, \"segment_pinned\": %s}\n",
+         "\"mc\": %lld, \"set_ref\": %lld, \"window_us\": %.1f, \"segment_pinned\": %s}\n",
          nSeen, nClosed, (now_us() - t0) * 1e-6, rmdReqs, rmdPus, rmdBatches, rmdBatches ? (double)rmdPus / rmdBatches : 0.0,
          rmdBatches ? (double)rmdReqs / rmdBatches : 0.0, maxBatchPus, rmdBusyUs * 1e-6, nReq[CUCD_IPC_FRAME], nReq[CUCD_IPC_ME_SURFACE], nReq[CUCD_IPC_SUBPEL],
-         nReq[CUCD_IPC_SET_REF], windowUs, segPinned ? "true" : "false");
+         nReq[CUCD_IPC_MC], nReq[CUCD_IPC_SET_REF], windowUs, segPinned ? "true" : "false");
   munmap(mem, total);
   shm_unlink(name.c_str());
   return 0;

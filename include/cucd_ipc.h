@@ -8,8 +8,9 @@
  * owns the device and the handles; every encoder instance maps the same POSIX shared-memory segment, posts its request into its
  * own slot + arena and sleeps on a futex; the server turns everything that is pending into one batch per request kind.
  *   S2  (cucd_intra_rmd_batch)   stateless: requests of ALL instances with the same bit depth are coalesced into one batch
- *   S1  (cuCUDecide_frame), S3 (cucd_set_cur/ref_picture, cucd_me_sad_surface), sub-pel (cucd_me_subpel_cost): served on the
- *        instance's own handle inside the server (they depend on that instance's pictures), in arrival order
+ *   S1  (cuCUDecide_frame), S3 (cucd_set_cur/ref_picture, cucd_me_sad_surface), sub-pel (cucd_me_subpel_cost), inter candidates
+ *        (cucd_me_mc_cost): served on the instance's own handle inside the server (they depend on that instance's pictures), in
+ *        arrival order.  A server that predates an op answers it with CUCD_ERR_INVALID, "unknown request".
  * The client side below is header-only C++ (what the reference's shim includes); the entry points mirror the C ABI of
  * include/cucudecide.h one to one, so an integration switches between in-process and server mode without other changes.
  */
@@ -35,7 +36,8 @@
 #define CUCD_IPC_MAX_CLIENTS 64
 #define CUCD_IPC_ARENA_BYTES ((size_t)96 << 20)      /* request + reply payload of one instance (a padded 2160p plane is 34 MB) */
 
-enum cucd_ipc_op { CUCD_IPC_OPEN = 1, CUCD_IPC_CLOSE, CUCD_IPC_FRAME, CUCD_IPC_RMD, CUCD_IPC_SET_CUR, CUCD_IPC_SET_REF, CUCD_IPC_ME_SURFACE, CUCD_IPC_SUBPEL };
+enum cucd_ipc_op { CUCD_IPC_OPEN = 1, CUCD_IPC_CLOSE, CUCD_IPC_FRAME, CUCD_IPC_RMD, CUCD_IPC_SET_CUR, CUCD_IPC_SET_REF, CUCD_IPC_ME_SURFACE, CUCD_IPC_SUBPEL,
+                   CUCD_IPC_MC };
 enum cucd_ipc_state { CUCD_IPC_FREE = 0, CUCD_IPC_IDLE = 1, CUCD_IPC_READY = 2, CUCD_IPC_DONE = 3, CUCD_IPC_CLOSED = 4 };
 
 struct alignas(128) cucd_ipc_slot {
@@ -152,6 +154,24 @@ struct cucd_ipc_client {
     memcpy(arena, desc, (size_t)nPU * sizeof(cucd_subpel_desc));
     const int rc = call(CUCD_IPC_SUBPEL, nPU, (size_t)nPU * sizeof(cucd_subpel_desc), (size_t)nPU * CUCD_SUBPEL_POINTS * 4);
     if (rc == CUCD_OK) memcpy(cost, reply(), (size_t)nPU * CUCD_SUBPEL_POINTS * 4);
+    return rc;
+  }
+  /* cucd_me_mc_cost: reply = [dist | pad | pred]; pred may be NULL (args[0] tells the server) */
+  int me_mc_cost(int nPU, const cucd_mc_desc* desc, uint32_t* dist, int16_t* pred) {
+    if (nPU < 0 || (nPU > 0 && (!desc || !dist))) { snprintf(err, sizeof err, "me_mc_cost: bad argument"); return CUCD_ERR_INVALID; }
+    size_t samples = 0;
+    for (int i = 0; i < nPU; i++) samples += (size_t)(desc[i].w > 0 ? desc[i].w : 0) * (size_t)(desc[i].h > 0 ? desc[i].h : 0);
+    const size_t inBytes = (size_t)nPU * sizeof(cucd_mc_desc), distBytes = ((size_t)nPU * 4 + 15) & ~(size_t)15;
+    const size_t outBytes = distBytes + (pred ? samples * 2 : 0);
+    if (((inBytes + 255) & ~(size_t)255) + outBytes > hdr->arena_bytes) {
+      snprintf(err, sizeof err, "me_mc_cost: %d candidates need %llu bytes, more than the %llu-byte arena", nPU,
+               (unsigned long long)(((inBytes + 255) & ~(size_t)255) + outBytes), (unsigned long long)hdr->arena_bytes);
+      return CUCD_ERR_NOMEM;
+    }
+    memcpy(arena, desc, inBytes);
+    s->args[0] = pred ? 1 : 0;
+    const int rc = call(CUCD_IPC_MC, nPU, inBytes, outBytes);
+    if (rc == CUCD_OK) { memcpy(dist, reply(), (size_t)nPU * 4); if (pred) memcpy(pred, reply() + distBytes, samples * 2); }
     return rc;
   }
 };

@@ -222,6 +222,26 @@ typedef struct {
 int cucd_me_subpel_cost(cucd_handle* h, int nPU, const cucd_subpel_desc* desc, uint32_t* cost);
 
 /* ------------------------------------------------------------------------------------------------
+ * Motion compensation and distortion of inter candidates.  Replaces xGetInterPredictionError (TEncSearch.cpp:2905-2926: the
+ * merge candidates of xMergeEstimation) and xGetTemplateCost (AMVP) for luma: candidate i is one PU at one quarter-pel motion
+ * of list 0, list 1 or both.  pred receives TComPrediction::motionCompensation's luma prediction (xPredInterUni, or
+ * xPredInterBi: two 14-bit list predictions averaged by TComYuv::addAvg before the clip) and dist[i] the DistFunc of that
+ * prediction against the source block of cucd_set_cur_picture: xGetHADs (8x8 tiles when w and h are multiples of 8, else 4x4)
+ * or xGetSAD with iSubShift = 0, both >> (bitDepth - 8).  The candidates of a PU's merge list go in one call.  Weighted
+ * prediction is not covered (callers with WP slices keep their own path).  References are the slots of cucd_set_ref_picture;
+ * the 8-tap support of every used list must stay inside the padded plane:
+ *   x + (mvx >> 2) - 3 >= -marginX, x + (mvx >> 2) + w + 3 <= W - 1 + marginX, and the same vertically.
+ * pred (may be NULL) holds the clipped w x h blocks back to back, row-major, in candidate order.  nPU == 0 is a no-op.
+ * ---------------------------------------------------------------------------------------------- */
+typedef struct {
+  int x, y, w, h;            /* PU position and size in luma samples; w, h multiples of 4, 4..64 (every HEVC PU shape, AMP included) */
+  int ref_idx[2];            /* cucd_set_ref_picture slot of the L0 / L1 prediction; -1 = list unused; at least one >= 0 */
+  int mvx[2], mvy[2];        /* quarter-pel MV per list (TComMv units), already clipped by the caller as xPredInterUni does (TComDataCU::clipMv) */
+  int use_hadamard;          /* m_pcEncCfg->getUseHADME() && !transquant bypass: xGetHADs, else xGetSAD */
+} cucd_mc_desc;
+int cucd_me_mc_cost(cucd_handle* h, int nPU, const cucd_mc_desc* desc, uint32_t* dist, int16_t* pred);
+
+/* ------------------------------------------------------------------------------------------------
  * The same two searches for a caller-supplied source block ("pattern key") instead of the block of the current picture:
  * what the bi-predictive refinement of xMotionEstimation needs (if (bBi), TEncSearch.cpp:3787-3797, 3826-3849: the key is
  * m_cYuvPredTemp = 2 * org - prediction of the other list, TComYuv::removeHighFreq, so its samples may be negative or exceed
@@ -348,7 +368,8 @@ int cucd_set_rmd_path(cucd_handle* h, int path);
  * the number of calls averaged, or a negative status; *avg_ms = mean duration of one launch. */
 int cucd_rmd_kernel_time(cucd_handle* h, int nCalls, float* avg_ms);
 /* Device time between the first and the last kernel of the most recent batch call on this handle (cucd_intra_rmd_batch,
- * cucd_me_sad_surface, cucd_intra_tu_*, cucd_tmv_features, cucd_aq_activity): CUDA events on the library's stream, host<->device
+ * cucd_me_sad_surface, cucd_me_subpel_cost, cucd_me_mc_cost, cucd_intra_tu_*, cucd_tmv_features, cucd_aq_activity): CUDA events on
+ * the library's stream, host<->device
  * copies outside.  What bench_rows.py reports as the kernel-only figure of those paths. */
 int cucd_last_kernel_time(cucd_handle* h, float* ms);
 /* the host-side fit that sits between the two passes (TEncSlice.cpp:291-392): hist = 16*4096 counts
