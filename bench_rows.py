@@ -13,7 +13,8 @@ each on a 1080p-sized workload, and prints ONE JSON line per row:
            bounded sample, on `cores` host threads
 Rows: s2 (cucd_intra_rmd_batch), f1 (cucd_queue_*: K concurrent instances), s3 (cucd_me_sad_surface), f3 (cucd_me_subpel_cost),
 a12 (cucd_tmv_features), a13 (cucd_aq_activity), f2 (cucd_intra_tu_code / _forward / _recon).  Usage: python bench_rows.py [--iters 5] > gpurun_out/rows.jsonl
-Last row: f5 (cucd_me_mc_cost, motion compensation + distortion of inter candidates; row_f5 runs it on its own).
+Last rows: f5 (cucd_me_mc_cost, motion compensation + distortion of inter candidates; row_f5 runs it on its own) and f6
+(cucd_inter_tu_forward / _code / _recon, the TUs of inter residual quadtrees; row_f6).  --only f5 / f6 runs one of them alone.
 """
 import argparse
 import ctypes as C
@@ -91,8 +92,12 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--iters", type=int, default=5)
     ap.add_argument("--cpu-threads", type=int, default=min(16, os.cpu_count() or 1))
+    ap.add_argument("--only", choices=["f5", "f6"], default=None, help="run one of the last rows alone")
     a = ap.parse_args()
     cucd = importlib.import_module("fast-cu-decision-hevc_b200")
+    if a.only:
+        (row_f5 if a.only == "f5" else row_f6)(cucd, a.iters, a.cpu_threads)
+        return
     oracle = _util.load_oracle()
     ref = _util.load_hmref()
     T = a.cpu_threads
@@ -254,6 +259,7 @@ def main():
              h2d=int(o.nbytes + b.nbytes + n_tu * 16 + (samples * 4 if stage == 2 else 0)), d2h=int(out_bytes))
     eng.close()
     row_f5(cucd, a.iters, T)
+    row_f6(cucd, a.iters, T)
 
 
 def gpu_identity():
@@ -329,6 +335,59 @@ def row_f5(cucd, iters=5, threads=8):
           "single_candidate_latency_us": {"median": float(np.median(lat)) * 1e6, "p10": float(np.percentile(lat, 10)) * 1e6,
                                           "p90": float(np.percentile(lat, 90)) * 1e6, "calls": len(lat), "candidate": "16x16 bi, Hadamard"}},
          p_s=p_s, h2d=int(n_c * 44), d2h=int(dist.nbytes))
+
+
+def row_f6(cucd, iters=5, threads=8):
+    """f6: inter TU coding (cucd_inter_tu_forward / _code / _recon) on the residual of one 1920x1080 8-bit picture: the source minus a
+    copy shifted by (3, 2) samples, tiled at every luma RQT level 32/16/8/4 (whole TUs) and, for each 4:2:0 chroma plane (the source
+    sub-sampled at two phases, minus its shifted copy), at 16/8/4; QP 32 (chroma 31), sign hiding; one call for the picture."""
+    bd = 8
+    org = _util.textured_plane(W, H, bd, seed=61).astype(np.int32)
+    planes = [(org - np.roll(org, (2, 3), axis=(0, 1)), (32, 16, 8, 4), 32, 0)]
+    for ph in (0, 1):
+        c = org[ph::2, ph::2]
+        planes.append((c - np.roll(c, (1, 2), axis=(0, 1)), (16, 8, 4), 31, 1))
+    tus, blocks = [], []
+    for plane, sizes, qp, chroma in planes:
+        for n in sizes:
+            ph, pw = plane.shape[0] // n * n, plane.shape[1] // n * n
+            b = plane[:ph, :pw].reshape(ph // n, n, pw // n, n).transpose(0, 2, 1, 3).reshape(-1, n * n)
+            tus += [(int(np.log2(n)), qp, 0, chroma)] * b.shape[0]
+            blocks.append(b.ravel())
+    resi = np.concatenate(blocks).astype(np.int16)
+    n_tu, samples = len(tus), int(resi.size)
+    _, arr, total = cucd.Engine._inter_tu_descs(tus)
+    assert total == samples
+    coef = np.zeros(samples, np.int32); rresi = np.zeros(samples, np.int16)
+    dist = np.zeros(n_tu, np.uint32); dz = np.zeros(n_tu, np.uint32); asum = np.zeros(n_tu, np.int32)
+    pins = (resi, coef, rresi, dist, dz, asum)
+    eng = cucd.Engine(W, H, bit_depth=bd)
+    import inter_tu_util
+    ito = inter_tu_util.load_inter_tu_oracle()
+    offs = np.cumsum([0] + [1 << (2 * t[0]) for t in tus])
+    gpu = gpu_identity()
+    rows = (("f6_inter_tu_forward", 0, samples * 4 + n_tu * 4, samples * 2),
+            ("f6_inter_tu_code", 1, samples * 6 + n_tu * 12, samples * 2),
+            ("f6_inter_tu_recon", 2, samples * 2 + n_tu * 4, samples * 6))
+    for name, stage, out_bytes, in_bytes in rows:
+        k_s, w_s, p_s = timed(lambda: eng.inter_tu_raw(stage, arr, n_tu, resi, coef, rresi=None if stage == 0 else rresi,
+                                                       dist=None if stage == 0 else dist, dist_zero=None if stage == 2 else dz,
+                                                       abs_sum=asum if stage == 1 else None), eng, iters, pin=pins)
+        cpu = None
+        if stage == 1:
+            samp = list(range(0, n_tu, 53))
+
+            def work(i):
+                j = samp[i]; t = tus[j]
+                inter_tu_util.oracle_inter_tu(ito, bd, 1 << t[0], t[1], t[2], t[3], 1, 1, resi[offs[j]:offs[j + 1]])
+            sec = cpu_parallel(work, len(samp), threads)
+            cpu = {"value": len(samp) / sec, "unit": "TU/s", "cores": threads, "kind": "port",
+                   "sample": f"every 53rd TU ({len(samp)}, same size mix) through tests/inter_tu_oracle.c in {sec:.2f} s"}
+        emit(name, "TU/s", n_tu, k_s, w_s, in_bytes + out_bytes, cpu,
+             {"gpu": gpu, "bit_depth": bd, "samples_per_call": samples, "tus_per_call": n_tu, "luma_tus": sum(1 for t in tus if not t[3]),
+              "qp": "32 luma / 31 chroma", "sign_hiding": True},
+             p_s=p_s, h2d=int(in_bytes + n_tu * 16), d2h=int(out_bytes))
+    eng.close()
 
 
 if __name__ == "__main__":

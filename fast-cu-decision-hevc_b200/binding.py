@@ -159,6 +159,10 @@ def load_library():
     lib.cucd_intra_tu_recon.argtypes = [C.c_void_p, C.c_int, C.POINTER(_TuDesc), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.cucd_intra_tu_code.argtypes = [C.c_void_p, C.c_int, C.POINTER(_TuDesc), C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
                                        C.c_void_p, C.c_void_p]
+    lib.cucd_inter_tu_forward.argtypes = [C.c_void_p, C.c_int, C.POINTER(_TuDesc), C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.cucd_inter_tu_recon.argtypes = [C.c_void_p, C.c_int, C.POINTER(_TuDesc), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.cucd_inter_tu_code.argtypes = [C.c_void_p, C.c_int, C.POINTER(_TuDesc), C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                                       C.c_void_p, C.c_void_p]
     lib.cucd_tmv_features.argtypes = [C.c_void_p, C.c_int, C.POINTER(_CuDesc), C.c_void_p]
     lib.cucd_aq_activity.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_void_p), C.c_void_p]
     lib.cucd_dev_rmd_frames.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_longlong, C.c_int, C.c_void_p,
@@ -384,6 +388,19 @@ class Engine:
             rc = self.lib.cucd_intra_tu_recon(self.h, n, arr, org.ctypes.data, border.ctypes.data, coef_or_level.ctypes.data, pix.ctypes.data, dist.ctypes.data)
         self._check(rc, "cucd_intra_tu_*")
 
+    def inter_tu_raw(self, stage, arr, n, resi, coef_or_level, rresi=None, dist=None, dist_zero=None, abs_sum=None, flags=TU_SIGN_HIDING):
+        """stage 0: cucd_inter_tu_forward (coef out), 1: cucd_inter_tu_code, 2: cucd_inter_tu_recon (level in) on prebuilt descriptors;
+        outputs are caller-owned numpy arrays, None where the call allows NULL"""
+        ptr = lambda a: None if a is None else a.ctypes.data
+        if stage == 0:
+            rc = self.lib.cucd_inter_tu_forward(self.h, n, arr, resi.ctypes.data, coef_or_level.ctypes.data, ptr(dist_zero))
+        elif stage == 1:
+            rc = self.lib.cucd_inter_tu_code(self.h, n, arr, resi.ctypes.data, int(flags), coef_or_level.ctypes.data, ptr(rresi), ptr(dist),
+                                             ptr(dist_zero), ptr(abs_sum))
+        else:
+            rc = self.lib.cucd_inter_tu_recon(self.h, n, arr, resi.ctypes.data, coef_or_level.ctypes.data, ptr(rresi), ptr(dist))
+        self._check(rc, "cucd_inter_tu_*")
+
     # ---- S3 ---------------------------------------------------------------------------------------
     def set_ref_picture(self, ref_idx, padded, margin_x, margin_y):
         """padded: (H+2my, W+2mx) int16 plane including the replicated margins."""
@@ -552,6 +569,45 @@ class Engine:
         self._check(self.lib.cucd_intra_tu_code(self.h, len(tus), arr, org.ctypes.data, border.ctypes.data, int(flags), level.ctypes.data,
                                                 reco.ctypes.data, dist.ctypes.data, abs_sum.ctypes.data), "cucd_intra_tu_code")
         return level, reco, dist, abs_sum
+
+    # ---- inter TU coding (xEstimateResidualQT): the TUs of inter residual quadtrees ------------------------------------
+    @staticmethod
+    def _inter_tu_descs(tus):
+        """tus: iterable of (log2_size, qp, transform_skip[, chroma]); the mode of every descriptor is 0"""
+        tus = [(t[0], 0) + tuple(t[1:]) for t in tus]
+        return Engine._tu_descs(tus)
+
+    def inter_tu_forward(self, tus, resi):
+        """resi: the residual blocks org - pred, N*N int16 per TU back to back.  Returns (coef int32 flat, dist_zero uint32 per TU)."""
+        tus, arr, total = self._inter_tu_descs(tus)
+        resi = np.ascontiguousarray(resi, np.int16).ravel()
+        assert resi.size == total
+        coef = np.zeros(total, np.int32)
+        dist_zero = np.zeros(len(tus), np.uint32)
+        self.inter_tu_raw(0, arr, len(tus), resi, coef, dist_zero=dist_zero)
+        return coef, dist_zero
+
+    def inter_tu_recon(self, tus, resi, level):
+        """levels chosen by the caller (RDOQ).  Returns (rresi int16 flat, dist uint32 per TU)."""
+        tus, arr, total = self._inter_tu_descs(tus)
+        resi = np.ascontiguousarray(resi, np.int16).ravel()
+        level = np.ascontiguousarray(level, np.int32).ravel()
+        assert resi.size == total and level.size == total
+        rresi = np.zeros(total, np.int16)
+        dist = np.zeros(len(tus), np.uint32)
+        self.inter_tu_raw(2, arr, len(tus), resi, level, rresi=rresi, dist=dist)
+        return rresi, dist
+
+    def inter_tu_code(self, tus, resi, sign_hiding=True):
+        """Whole chain with the plain quantiser.  Returns (level int32 flat, rresi int16 flat, dist uint32, dist_zero uint32, abs_sum int32)."""
+        tus, arr, total = self._inter_tu_descs(tus)
+        resi = np.ascontiguousarray(resi, np.int16).ravel()
+        assert resi.size == total
+        level = np.zeros(total, np.int32); rresi = np.zeros(total, np.int16)
+        dist = np.zeros(len(tus), np.uint32); dist_zero = np.zeros(len(tus), np.uint32); abs_sum = np.zeros(len(tus), np.int32)
+        self.inter_tu_raw(1, arr, len(tus), resi, level, rresi=rresi, dist=dist, dist_zero=dist_zero, abs_sum=abs_sum,
+                          flags=TU_SIGN_HIDING if sign_hiding else 0)
+        return level, rresi, dist, dist_zero, abs_sum
 
     def tmv_features(self, cus):
         """cus: iterable of (x, y, log2_size) of the picture given to set_cur_picture. Returns (nCU, 5, 26) float64

@@ -656,12 +656,17 @@ int cucd_me_mc_cost(cucd_handle* h, int nPU, const cucd_mc_desc* desc, uint32_t*
 }
 
 // ------------------------------------------------------------------------------------------------
-// Intra luma TU coding (xIntraCodingTUBlock): forward half, reconstruction half, or the whole chain with the plain quantiser
+// TU coding: intra TUs (xIntraCodingTUBlock) and the TUs of inter residual quadtrees (xEstimateResidualQT): forward half,
+// reconstruction half, or the whole chain with the plain quantiser.  Inter calls (`inter`) pass the residual blocks as `org`,
+// no border, and may ask for the SSE of the residual alone (`distZero`).
 // ------------------------------------------------------------------------------------------------
 static int tu_batch(cucd_handle* h, const char* who, int stage, int flags, int nTU, const cucd_tu_desc* desc, const int16_t* org, const int16_t* border,
-                    int32_t* coefOut, const int32_t* levelIn, int16_t* pixOut, uint32_t* dist, int32_t* absSum) {
-  if (!h || nTU < 0 || (nTU > 0 && (!desc || !org || !border))) return fail(h, CUCD_ERR_INVALID, std::string(who) + ": bad argument");
+                    int32_t* coefOut, const int32_t* levelIn, int16_t* pixOut, uint32_t* dist, int32_t* absSum, bool inter = false,
+                    uint32_t* distZero = nullptr) {
+  if (!h || nTU < 0 || (nTU > 0 && (!desc || !org || (!inter && !border)))) return fail(h, CUCD_ERR_INVALID, std::string(who) + ": bad argument");
   if (nTU == 0) return CUCD_OK;
+  if (inter && (flags & ~CUCD_TU_SIGN_HIDING))
+    return fail(h, CUCD_ERR_INVALID, std::string(who) + ": flags may only hold CUCD_TU_SIGN_HIDING (an inter CU never lies in an I slice)");
   LOCK(h);
   CK(cudaSetDevice(h->cfg.device));
   // pass 1: validate, count per size class
@@ -670,6 +675,8 @@ static int tu_batch(cucd_handle* h, const char* who, int stage, int flags, int n
     const cucd_tu_desc& d = desc[i];
     if (d.log2_size < 2 || d.log2_size > 5) return fail(h, CUCD_ERR_INVALID, std::string(who) + ": log2_size must be 2..5");
     if (d.mode > 34 || d.qp < 0 || d.qp > 51) return fail(h, CUCD_ERR_INVALID, std::string(who) + ": mode must be 0..34 and qp 0..51");
+    if (inter && d.mode != 0) return fail(h, CUCD_ERR_INVALID, std::string(who) + ": mode must be 0 (inter blocks are not predicted here)");
+    if (inter && (d.flags & ~(CUCD_TU_TRANSFORM_SKIP | CUCD_TU_CHROMA))) return fail(h, CUCD_ERR_INVALID, std::string(who) + ": unknown descriptor flags");
     if ((d.flags & CUCD_TU_TRANSFORM_SKIP) && d.log2_size != 2) return fail(h, CUCD_ERR_UNSUPPORTED, std::string(who) + ": transform skip is a 4x4 tool (log2MaxTransformSkipSize = 2)");
     count[d.log2_size]++;
   }
@@ -691,7 +698,7 @@ static int tu_batch(cucd_handle* h, const char* who, int stage, int flags, int n
   }
   BatchIo io(h);
   const int iOrg = io.add_in(org, orgOff * 2);
-  const int iBrd = io.add_in(border, borderOff * 2);
+  const int iBrd = inter ? -1 : io.add_in(border, borderOff * 2);
   const int iJobs = io.add_in(jobs, (size_t)nTU * sizeof(TuJob), true);
   const int iLev = stage == 2 ? io.add_in(levelIn, orgOff * sizeof(int32_t)) : -1;
   io.inBytes += 256;
@@ -700,19 +707,21 @@ static int tu_batch(cucd_handle* h, const char* who, int stage, int flags, int n
   const int oPix = (pixOut || stage != 0) ? (pixOut ? io.add_out(pixOut, orgOff * sizeof(int16_t)) : io.add_scratch_out(orgOff * sizeof(int16_t))) : -1;
   const int oDist = dist ? io.add_out(dist, (size_t)nTU * sizeof(uint32_t)) : io.add_scratch_out((size_t)nTU * sizeof(uint32_t));
   const int oAbs = absSum ? io.add_out(absSum, (size_t)nTU * sizeof(int32_t)) : io.add_scratch_out((size_t)nTU * sizeof(int32_t));
+  const int oZero = distZero ? io.add_out(distZero, (size_t)nTU * sizeof(uint32_t)) : -1;
   if (io.reserve() != CUCD_OK || io.upload(h->sMain) != CUCD_OK) return CUCD_ERR_CUDA;
   CK(cudaEventRecord(h->evK0, h->sMain));
   for (int l = 5; l >= 2; l--) {
     if (!count[l]) continue;
     TuBatch tb;
-    tb.org = io.din<int16_t>(iOrg); tb.border = io.din<int16_t>(iBrd); tb.jobs = io.din<TuJob>(iJobs) + first[l]; tb.count = count[l];
+    tb.org = io.din<int16_t>(iOrg); tb.border = inter ? nullptr : io.din<int16_t>(iBrd); tb.jobs = io.din<TuJob>(iJobs) + first[l]; tb.count = count[l];
+    tb.inter = inter ? 1 : 0; tb.distZero = oZero >= 0 ? io.dout<uint32_t>(oZero) : nullptr;
     tb.stage = stage; tb.bitDepth = h->cfg.bit_depth; tb.strong = h->cfg.strong_intra_smoothing;
     tb.intraSlice = (flags & CUCD_TU_INTRA_SLICE) ? 1 : 0; tb.signHiding = (flags & CUCD_TU_SIGN_HIDING) ? 1 : 0;
     tb.coef = stage == 2 ? io.din<int32_t>(iLev) : io.dout<int32_t>(oCoef);
     tb.pred = (stage == 0 && pixOut) ? io.dout<int16_t>(oPix) : nullptr;
     tb.reco = oPix >= 0 ? io.dout<int16_t>(oPix) : nullptr;
     tb.dist = io.dout<uint32_t>(oDist); tb.absSum = io.dout<int32_t>(oAbs);
-    CK(launch_intra_tu(l, tb, h->sMain, &h->launches));
+    CK(launch_tu(l, tb, h->sMain, &h->launches));
   }
   CK(cudaEventRecord(h->evK1, h->sMain)); h->kTimed = true;
   if (io.download(h->sMain) != CUCD_OK) return CUCD_ERR_CUDA;
@@ -733,6 +742,19 @@ int cucd_intra_tu_code(cucd_handle* h, int nTU, const cucd_tu_desc* desc, const 
                        int32_t* level, int16_t* reco, uint32_t* dist, int32_t* abs_sum) {
   if (nTU > 0 && (!level || !reco || !dist)) return fail(h, CUCD_ERR_INVALID, "cucd_intra_tu_code: NULL level / reco / dist");
   return tu_batch(h, "cucd_intra_tu_code", 1, flags, nTU, desc, org, border, level, nullptr, reco, dist, abs_sum);
+}
+int cucd_inter_tu_forward(cucd_handle* h, int nTU, const cucd_tu_desc* desc, const int16_t* resi, int32_t* coef, uint32_t* dist_zero) {
+  if (nTU > 0 && !coef) return fail(h, CUCD_ERR_INVALID, "cucd_inter_tu_forward: coef is NULL");
+  return tu_batch(h, "cucd_inter_tu_forward", 0, 0, nTU, desc, resi, nullptr, coef, nullptr, nullptr, nullptr, nullptr, true, dist_zero);
+}
+int cucd_inter_tu_recon(cucd_handle* h, int nTU, const cucd_tu_desc* desc, const int16_t* resi, const int32_t* level, int16_t* rresi, uint32_t* dist) {
+  if (nTU > 0 && (!level || !dist)) return fail(h, CUCD_ERR_INVALID, "cucd_inter_tu_recon: NULL level / dist");
+  return tu_batch(h, "cucd_inter_tu_recon", 2, 0, nTU, desc, resi, nullptr, nullptr, level, rresi, dist, nullptr, true, nullptr);
+}
+int cucd_inter_tu_code(cucd_handle* h, int nTU, const cucd_tu_desc* desc, const int16_t* resi, int flags, int32_t* level, int16_t* rresi,
+                       uint32_t* dist, uint32_t* dist_zero, int32_t* abs_sum) {
+  if (nTU > 0 && (!level || !rresi || !dist)) return fail(h, CUCD_ERR_INVALID, "cucd_inter_tu_code: NULL level / rresi / dist");
+  return tu_batch(h, "cucd_inter_tu_code", 1, flags, nTU, desc, resi, nullptr, level, nullptr, rresi, dist, abs_sum, true, dist_zero);
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -73,23 +73,25 @@ cudaError_t launch_tmv_features(const int16_t* org, int stride, const TmvCu* cus
 struct AqLayers { int count, total; int part[4]; int off[5]; };   // layer d: units of part[d] samples, results at out[off[d]..off[d+1])
 cudaError_t launch_aq_activity(const int16_t* org, int stride, int W, int H, const AqLayers& layers, double* out, cudaStream_t st, int* launches);
 
-// ---- intra luma TU coding chain (tu_kernels.cu) -------------------------------------------------
+// ---- TU coding chain: intra TUs, and the TUs of inter residual quadtrees (tu_kernels.cu) ----------------
 struct TuJob {
-  int32_t orgOff;      // sample offset of the TU's source block (and of its coef / level / pred / reco blocks)
-  int32_t borderOff;   // sample offset of its 4N+1 border
+  int32_t orgOff;      // sample offset of the TU's source (inter: residual) block and of its coef / level / pred / reco blocks
+  int32_t borderOff;   // sample offset of its 4N+1 border (intra)
   int32_t outIndex;    // TU index in the caller's order (dist / absSum)
-  uint8_t mode, ts;    // intra mode 0..34; bit 0 transform skip, bit 1 chroma block (cucd_tu_desc.flags)
+  uint8_t mode, ts;    // intra mode 0..34 (inter: 0); bit 0 transform skip, bit 1 chroma block (cucd_tu_desc.flags)
   int8_t qp; uint8_t pad;
 };
 struct TuBatch {
-  const int16_t* org; const int16_t* border; const TuJob* jobs; int count;
+  const int16_t* org; const int16_t* border; const TuJob* jobs; int count;   // inter: org = the residual blocks, no border
   int stage;           // 0 forward only (coef, pred out), 1 whole chain with the plain quantiser, 2 reconstruction from given levels
   int bitDepth, strong, intraSlice, signHiding;
   int32_t* coef;       // stage 0: transform output; stage 1: levels out; stage 2: levels in
   int16_t* pred;       // stage 0 (may be null)
-  int16_t* reco; uint32_t* dist; int32_t* absSum;   // stages 1, 2
+  int16_t* reco; uint32_t* dist; int32_t* absSum;   // stages 1, 2; inter: reco = the inverse-transformed residual
+  int inter;           // 1: tu_kernel<LG, true> (xEstimateResidualQT), 0: the intra chain
+  uint32_t* distZero;  // inter, every stage (may be null): SSE of the residual alone
 };
-cudaError_t launch_intra_tu(int log2n, const TuBatch& tb, cudaStream_t st, int* launches);
+cudaError_t launch_tu(int log2n, const TuBatch& tb, cudaStream_t st, int* launches);
 
 // ---- integer-ME SAD surfaces (me_kernels.cu) ---------------------------------------------------
 struct MeJob {

@@ -4,6 +4,10 @@
 //   plain quantiser xQuant + signBitHidingHDQ (:991-1240, flat scaling lists; RDOQ is CABAC-coupled and stays on the host)
 //   -> invTransformNxN: xDeQuant (:1242-1352) + xITrMxN / xITransformSkip (:927-985, 1980-2031)
 //   -> reconstruction with clipping (:1360-1381) -> SSE getDistPart / xGetSSE* (TComRdCost.cpp:433-455, 970-1315).
+// The INTER instantiation is the same chain for the TUs of an inter residual quadtree (TEncSearch::xEstimateResidualQT): the
+// residual org - pred comes from the caller (no border, no prediction), the DCT runs at every size (TComTU::useDST is intra-only),
+// sign hiding uses the diagonal scan, and the back end returns the inverse-transformed residual with its SSE against the
+// residual (getDistPart(rresi, resi)) and the SSE of the residual alone (the CBF-0 distortion, nonCoeffDist), both in uint32.
 //
 // One CTA of 256 threads codes a chunk of TUs of ONE size: 1 TU of 32x32 (4 samples per thread) or 16x16, 4 of 8x8, 16 of 4x4
 // (one sample per thread).  Everything of a TU lives in shared memory; the partial butterflies of the reference are exact
@@ -12,6 +16,7 @@
 // accesses of the second stage are bank-conflict free.  Traffic per TU: N*N*2 + (4N+1)*2 bytes in, N*N*(4+2) + 8 bytes out -
 // a streaming kernel whose arithmetic (4 N-term dot products per sample) stays far below the HBM time for N <= 32.
 #include <cuda_runtime.h>
+#include <type_traits>
 #include "kernels.h"
 
 namespace cucd {
@@ -119,9 +124,9 @@ __device__ __forceinline__ void tu_matvec(const uint32_t (&in)[N / 2], const uin
   }
 }
 
-template <int LG>
+template <int LG, bool INTER>
 __global__ void __launch_bounds__(256)
-intra_tu_kernel(const TuBatch tb) {
+tu_kernel(const TuBatch tb) {
   constexpr int N = 1 << LG, NN = N * N, P = N + 1;
   constexpr int TPT = NN < 256 ? NN : 256;       // threads per TU
   constexpr int TUS = 256 / TPT;                 // TUs per CTA
@@ -138,6 +143,9 @@ intra_tu_kernel(const TuBatch tb) {
   __shared__ int32_t sB[TUS][N * P];                         // transform output / residual, row-padded
   __shared__ int32_t sLevel[TUS][NN], sDelta[TUS][NN];
   __shared__ int sAbs[TUS], sDist[TUS], sCgNz[TUS][CGS];
+  __shared__ uint32_t sZero[TUS];                            // INTER: SSE of the residual alone
+  using Acc = std::conditional_t<INTER, uint32_t, int>;      // INTER sums wrap as HM's Distortion (UInt) does
+  constexpr int SEG = TPT < 32 ? TPT : 32;                   // 4x4 TUs: two per warp, sums reduced inside the TU's 16 lanes
 
   const int tid = threadIdx.x, grp = tid / TPT, t = tid % TPT;
   const int tuIdx = blockIdx.x * TUS + grp;
@@ -145,7 +153,7 @@ intra_tu_kernel(const TuBatch tb) {
   const TuJob job = live ? tb.jobs[tuIdx] : TuJob{0, 0, 0, 0, 0, 0, 0};
   const int bd = tb.bitDepth, mode = job.mode, ts = job.ts & 1;
   const bool luma = !(job.ts & 2);
-  const bool dst = N == 4 && luma;                           // TComTU::useDST: intra luma 4x4
+  const bool dst = !INTER && N == 4 && luma;                 // TComTU::useDST: intra luma 4x4
   const int row = t & (N - 1), kg = t >> LG;                 // transform-stage role of this thread
 
   for (int i = tid; i < NN; i += 256) {                      // rows of the 32-point matrix, sub-sampled (TComRom.cpp:356-460)
@@ -155,15 +163,15 @@ intra_tu_kernel(const TuBatch tb) {
     const int8_t v = k == 0 ? (int8_t)64 : (a <= 32 ? kDctC[a] : (int8_t)-kDctC[64 - a]);
     sMF[k * N + x] = v; sMI[x * N + k] = v;
   }
-  if (N == 4 && tid < 16) { sDF[tid] = kDst4[tid]; sDI[(tid & 3) * 4 + (tid >> 2)] = kDst4[tid]; }
-  if (live) {
+  if (!INTER && N == 4 && tid < 16) { sDF[tid] = kDst4[tid]; sDI[(tid & 3) * 4 + (tid >> 2)] = kDst4[tid]; }
+  if (!INTER && live) {
     const int16_t* bsrc = tb.border + job.borderOff;
     for (int i = t; i < 4 * N + 1; i += TPT) sUnf[grp][i] = bsrc[i];
   }
-  if (t == 0) { sAbs[grp] = 0; sDist[grp] = 0; }
+  if (t == 0) { sAbs[grp] = 0; sDist[grp] = 0; if (INTER) sZero[grp] = 0; }
   __syncthreads();
   // ---- reference smoothing (TComPattern.cpp:185-283) ----------------------------------------------------------------
-  {
+  if constexpr (!INTER) {
     const int16_t* b = sUnf[grp];
     bool strong = false;
     if (N == 32 && tb.strong) {
@@ -180,13 +188,29 @@ intra_tu_kernel(const TuBatch tb) {
       } else v = (b[i - 1] + 2 * b[i] + b[i + 1] + 2) >> 2;
       sFil[grp][i] = (int16_t)v;
     }
+    __syncthreads();
   }
-  __syncthreads();
   // ---- prediction, residual (int16, row-major: the input rows of the first transform stage) ----------------------------------
-  const int16_t* org = tb.org + job.orgOff;
+  const int16_t* org = tb.org + job.orgOff;                  // INTER: the caller's residual blocks
   int16_t* in16 = reinterpret_cast<int16_t*>(sIn[grp]);
   int16_t* mid16 = reinterpret_cast<int16_t*>(sMid[grp]);
-  {
+  if constexpr (INTER) {
+    // the residual goes straight into the first stage's rows, a copy into sPred for the SSE after sIn is overwritten; its SSE
+    // against zero is nonCoeffDist
+    const int sh = (bd - 8) << 1;
+    uint32_t zero = 0;
+#pragma unroll
+    for (int e = 0; e < IPT; e++) {
+      const int o = t + e * TPT, r = o >> LG, c = o & (N - 1);
+      const int v = live ? org[o] : 0;
+      sPred[grp][o] = (int16_t)v;
+      in16[r * 2 * PW + c] = (int16_t)v;
+      zero += (uint32_t)((v * v) >> sh);
+    }
+#pragma unroll
+    for (int m = SEG / 2; m > 0; m >>= 1) zero += __shfl_xor_sync(0xffffffffu, zero, m);
+    if ((t & (SEG - 1)) == 0 && zero) atomicAdd(&sZero[grp], zero);
+  } else {
     const int16_t* b = (luma && tu_use_filtered(LG, mode)) ? sFil[grp] : sUnf[grp];      // chroma of 4:2:0: never smoothed
     int dc = 0;
     if (mode == 1) { int s = 0; for (int i = 0; i < N; i++) s += b[2 * N + 1 + i] + b[2 * N - 1 - i]; dc = (s + N) / (2 * N); }
@@ -234,6 +258,7 @@ intra_tu_kernel(const TuBatch tb) {
       if (live) {
 #pragma unroll
         for (int e = 0; e < IPT; e++) { const int o = t + e * TPT; tb.coef[job.orgOff + o] = sB[grp][(o >> LG) * P + (o & (N - 1))]; }
+        if (INTER && t == 0 && tb.distZero) tb.distZero[job.outIndex] = sZero[grp];
       }
       return;
     }
@@ -258,7 +283,7 @@ intra_tu_kernel(const TuBatch tb) {
     __syncthreads();
     // ---- sign-bit hiding (signBitHidingHDQ): one thread per 4x4 coefficient group ---------------------------------------
     if (tb.signHiding) {
-      const int scanIdx = N > (luma ? 8 : 4) ? 0 : (abs(mode - 26) <= 4 ? 1 : (abs(mode - 10) <= 4 ? 2 : 0));       // TComDataCU.cpp:3356-3410
+      const int scanIdx = INTER || N > (luma ? 8 : 4) ? 0 : (abs(mode - 26) <= 4 ? 1 : (abs(mode - 10) <= 4 ? 2 : 0));   // TComDataCU.cpp:3356-3410
       constexpr int LGG = LG - 2, G = 1 << LGG;
       int gpos = 0;
       if (t < CGS) {
@@ -355,43 +380,48 @@ intra_tu_kernel(const TuBatch tb) {
     }
   }
   __syncthreads();
-  // ---- reconstruction, SSE, outputs ---------------------------------------------------------------------------------------------------
+  // ---- reconstruction (INTER: the residual rresi, Pel-clipped above), SSE, outputs ------------------------------------------------------
   {
     const int sh = (bd - 8) << 1;
-    int sse = 0;
+    Acc sse = 0;
 #pragma unroll
     for (int e = 0; e < IPT; e++) {
       const int o = t + e * TPT;
       const int resi = coded ? sB[grp][(o >> LG) * P + (o & (N - 1))] : 0;
-      const int rec = clip3i(0, (1 << bd) - 1, sPred[grp][o] + resi);
+      const int rec = INTER ? resi : clip3i(0, (1 << bd) - 1, sPred[grp][o] + resi);
       if (live) {
-        const int d = rec - org[o];
-        sse += (d * d) >> sh;
+        const int d = INTER ? sPred[grp][o] - rec : rec - org[o];   // |d| <= 2^bd - 1 + 2^15: d * d fits int
+        sse += (Acc)((d * d) >> sh);
         tb.reco[job.orgOff + o] = (int16_t)rec;
         if (tb.stage == 1) tb.coef[job.orgOff + o] = coded ? sLevel[grp][o] : 0;
       }
     }
-    constexpr int SEG = TPT < 32 ? TPT : 32;               // 4x4 TUs: two per warp, reduce inside the TU's 16 lanes
 #pragma unroll
     for (int m = SEG / 2; m > 0; m >>= 1) sse += __shfl_xor_sync(0xffffffffu, sse, m);
-    if ((t & (SEG - 1)) == 0 && sse) atomicAdd(&sDist[grp], sse);
+    if ((t & (SEG - 1)) == 0 && sse) atomicAdd(reinterpret_cast<Acc*>(&sDist[grp]), sse);
   }
   __syncthreads();
   if (live && t == 0) {
     tb.dist[job.outIndex] = (uint32_t)sDist[grp];
     if (tb.absSum) tb.absSum[job.outIndex] = sAbs[grp];
+    if (INTER && tb.distZero) tb.distZero[job.outIndex] = sZero[grp];
   }
 }
 
-cudaError_t launch_intra_tu(int log2n, const TuBatch& tb, cudaStream_t st, int* launches) {
-  if (tb.count <= 0) return cudaSuccess;
+template <bool INTER>
+static void launch_tu_size(int log2n, const TuBatch& tb, cudaStream_t st) {
   switch (log2n) {
-    case 2: intra_tu_kernel<2><<<(tb.count + 15) / 16, 256, 0, st>>>(tb); break;
-    case 3: intra_tu_kernel<3><<<(tb.count + 3) / 4, 256, 0, st>>>(tb); break;
-    case 4: intra_tu_kernel<4><<<tb.count, 256, 0, st>>>(tb); break;
-    case 5: intra_tu_kernel<5><<<tb.count, 256, 0, st>>>(tb); break;
-    default: return cudaErrorInvalidValue;
+    case 2: tu_kernel<2, INTER><<<(tb.count + 15) / 16, 256, 0, st>>>(tb); break;
+    case 3: tu_kernel<3, INTER><<<(tb.count + 3) / 4, 256, 0, st>>>(tb); break;
+    case 4: tu_kernel<4, INTER><<<tb.count, 256, 0, st>>>(tb); break;
+    case 5: tu_kernel<5, INTER><<<tb.count, 256, 0, st>>>(tb); break;
   }
+}
+
+cudaError_t launch_tu(int log2n, const TuBatch& tb, cudaStream_t st, int* launches) {
+  if (tb.count <= 0) return cudaSuccess;
+  if (log2n < 2 || log2n > 5) return cudaErrorInvalidValue;
+  if (tb.inter) launch_tu_size<true>(log2n, tb, st); else launch_tu_size<false>(log2n, tb, st);
   if (launches) *launches += 1;
   return cudaGetLastError();
 }

@@ -295,6 +295,42 @@ int cucd_intra_tu_code(cucd_handle* h, int nTU, const cucd_tu_desc* desc, const 
                        int32_t* level, int16_t* reco, uint32_t* dist, int32_t* abs_sum);
 
 /* ------------------------------------------------------------------------------------------------
+ * Inter TU coding: the arithmetic of TEncSearch::xEstimateResidualQT (TEncSearch.cpp, called by
+ * encodeResAndCalcRdInterCU for every inter candidate) for the TUs of inter residual quadtrees.  An inter residual does not depend on the
+ * reconstruction of the TU before it, so every TU of every RQT depth of a CU, luma and chroma, and the TUs of all merge
+ * candidates of a PU can go in one call.  resi holds the residual blocks org - pred (cut by the caller from pcResi; chroma from
+ * the caller's own chroma motion compensation), N*N per TU back to back in descriptor order; coef / level / rresi use the same
+ * layout, dist / dist_zero / abs_sum hold one value per TU.  Descriptors as above with mode = 0; flags CUCD_TU_TRANSFORM_SKIP
+ * (4x4 only) and / or CUCD_TU_CHROMA.
+ * Precondition: |resi| <= 2^bit_depth - 1, which the difference of two in-range planes satisfies (the forward stages keep
+ * int16 intermediates, exact only in that range).
+ * Differences from the intra chain: the DCT at every size (TComTU::useDST is intra-only), the diagonal scan for sign hiding
+ * (getCoefScanIdx of a non-intra CU, TComDataCU.cpp:3356-3410), the rounding offset 85/512 of xQuant (an inter CU never lies in
+ * an I slice, so the call's flags accept CUCD_TU_SIGN_HIDING only), and the back end: the residual is returned, not a
+ * reconstruction.
+ *   cucd_inter_tu_forward  TComTrQuant::transformNxN (xT / xTransformSkip, TComTrQuant.cpp:860-919, 1376-1440, 1857-1978):
+ *                          coef = m_plTempCoeff, what xRateDistOptQuant reads; dist_zero (may be NULL) = nonCoeffDist /
+ *                          puiZeroDist of xEstimateResidualQT = getDistPart(0, resi), the distortion of the TU with CBF 0.
+ *   cucd_inter_tu_recon    for levels chosen by the caller (the host's RDOQ): invTransformNxN (xDeQuant + xIT /
+ *                          xITransformSkip, TComTrQuant.cpp:927-985, 1242-1352, 1462-1586); rresi (may be NULL) = the
+ *                          inverse-transformed residual as Pel (clipped to int16, not a reconstruction), dist =
+ *                          getDistPart(rresi, resi) (TComRdCost.cpp:433-455) = sum of ((resi - rresi)^2 >> 2(bit_depth - 8))
+ *                          accumulated in uint32 with wrap-around as HM's Distortion (UInt).  A TU whose levels are all
+ *                          zero gets rresi = 0 and dist == dist_zero.
+ *   cucd_inter_tu_code     the whole chain with HM's plain quantiser (--RDOQ=0): xQuant with flat scaling lists
+ *                          (TComTrQuant.cpp:1126-1240) and, with CUCD_TU_SIGN_HIDING, signBitHidingHDQ (:991-1123);
+ *                          level = pcCoeff, abs_sum (may be NULL) = uiAbsSum (the CBF), rresi, dist, dist_zero (may be NULL) as above.
+ * Chroma distortions are returned before m_distortionWeight (TComRdCost.cpp:447-450).  Limits as for the intra calls; no
+ * cross-component prediction, RDPCM, transquant bypass or weighted prediction.  nTU == 0 is a no-op.
+ * ---------------------------------------------------------------------------------------------- */
+int cucd_inter_tu_forward(cucd_handle* h, int nTU, const cucd_tu_desc* desc, const int16_t* resi,
+                          int32_t* coef, uint32_t* dist_zero);
+int cucd_inter_tu_recon(cucd_handle* h, int nTU, const cucd_tu_desc* desc, const int16_t* resi,
+                        const int32_t* level, int16_t* rresi, uint32_t* dist);
+int cucd_inter_tu_code(cucd_handle* h, int nTU, const cucd_tu_desc* desc, const int16_t* resi, int flags,
+                       int32_t* level, int16_t* rresi, uint32_t* dist, uint32_t* dist_zero, int32_t* abs_sum);
+
+/* ------------------------------------------------------------------------------------------------
  * CU texture features and AQ activity of the picture given to cucd_set_cur_picture.
  * cucd_tmv_features  replaces getTMVFeature(rpcBestCU) (tools_YS.cpp:1682-1839, call site TEncCu.cpp:1558-1570):
  *                    feat[i*130 + f*26 + k] = m_adFeature[f][k] of CU i - five 3x3 directional planes (original,
@@ -368,7 +404,7 @@ int cucd_set_rmd_path(cucd_handle* h, int path);
  * the number of calls averaged, or a negative status; *avg_ms = mean duration of one launch. */
 int cucd_rmd_kernel_time(cucd_handle* h, int nCalls, float* avg_ms);
 /* Device time between the first and the last kernel of the most recent batch call on this handle (cucd_intra_rmd_batch,
- * cucd_me_sad_surface, cucd_me_subpel_cost, cucd_me_mc_cost, cucd_intra_tu_*, cucd_tmv_features, cucd_aq_activity): CUDA events on
+ * cucd_me_sad_surface, cucd_me_subpel_cost, cucd_me_mc_cost, cucd_intra_tu_*, cucd_inter_tu_*, cucd_tmv_features, cucd_aq_activity): CUDA events on
  * the library's stream, host<->device
  * copies outside.  What bench_rows.py reports as the kernel-only figure of those paths. */
 int cucd_last_kernel_time(cucd_handle* h, float* ms);
