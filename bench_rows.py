@@ -13,8 +13,9 @@ each on a 1080p-sized workload, and prints ONE JSON line per row:
            bounded sample, on `cores` host threads
 Rows: s2 (cucd_intra_rmd_batch), f1 (cucd_queue_*: K concurrent instances), s3 (cucd_me_sad_surface), f3 (cucd_me_subpel_cost),
 a12 (cucd_tmv_features), a13 (cucd_aq_activity), f2 (cucd_intra_tu_code / _forward / _recon).  Usage: python bench_rows.py [--iters 5] > gpurun_out/rows.jsonl
-Last rows: f5 (cucd_me_mc_cost, motion compensation + distortion of inter candidates; row_f5 runs it on its own) and f6
-(cucd_inter_tu_forward / _code / _recon, the TUs of inter residual quadtrees; row_f6).  --only f5 / f6 runs one of them alone.
+Last rows: f5 (cucd_me_mc_cost, motion compensation + distortion of inter candidates; row_f5 runs it on its own), f6
+(cucd_inter_tu_forward / _code / _recon, the TUs of inter residual quadtrees; row_f6) and f7 (cucd_me_mc_chroma, the 4:2:0 chroma of
+f5's candidates; row_f7).  --only f5 / f6 / f7 runs one of them alone.
 """
 import argparse
 import ctypes as C
@@ -92,11 +93,11 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--iters", type=int, default=5)
     ap.add_argument("--cpu-threads", type=int, default=min(16, os.cpu_count() or 1))
-    ap.add_argument("--only", choices=["f5", "f6"], default=None, help="run one of the last rows alone")
+    ap.add_argument("--only", choices=["f5", "f6", "f7"], default=None, help="run one of the last rows alone")
     a = ap.parse_args()
     cucd = importlib.import_module("fast-cu-decision-hevc_b200")
     if a.only:
-        (row_f5 if a.only == "f5" else row_f6)(cucd, a.iters, a.cpu_threads)
+        {"f5": row_f5, "f6": row_f6, "f7": row_f7}[a.only](cucd, a.iters, a.cpu_threads)
         return
     oracle = _util.load_oracle()
     ref = _util.load_hmref()
@@ -260,6 +261,7 @@ def main():
     eng.close()
     row_f5(cucd, a.iters, T)
     row_f6(cucd, a.iters, T)
+    row_f7(cucd, a.iters, T)
 
 
 def gpu_identity():
@@ -270,6 +272,21 @@ def gpu_identity():
         return r.stdout.strip().splitlines()[0]
     except (OSError, IndexError, subprocess.SubprocessError):
         return "unknown"
+
+
+def f5_candidates(rng):
+    """the candidates of row_f5: every whole 32x32, 16x16 and 8x8 PU of a 1920x1080 picture carries five (quarter-pel MVs within
+    +-64 samples; a third uni L0, a third uni L1, a third bi; Hadamard)"""
+    descs = []
+    for n in (32, 16, 8):
+        for y in range(0, H - n + 1, n):
+            for x in range(0, W - n + 1, n):
+                for c in range(5):
+                    mv = [int(v) for v in rng.integers(-256, 257, 4)]
+                    kind = (len(descs)) % 3
+                    ref = ((0, -1), (-1, 1), (0, 1))[kind]
+                    descs.append(dict(x=x, y=y, w=n, h=n, ref_idx=ref, mvx=(mv[0], mv[1]), mvy=(mv[2], mv[3]), use_hadamard=1))
+    return descs
 
 
 def row_f5(cucd, iters=5, threads=8):
@@ -285,15 +302,7 @@ def row_f5(cucd, iters=5, threads=8):
     eng.set_cur_picture(org)
     for k, r in enumerate(refs):
         eng.set_ref_picture(k, r, pad, pad)
-    descs = []
-    for n in (32, 16, 8):
-        for y in range(0, H - n + 1, n):
-            for x in range(0, W - n + 1, n):
-                for c in range(5):
-                    mv = [int(v) for v in rng.integers(-256, 257, 4)]
-                    kind = (len(descs)) % 3
-                    ref = ((0, -1), (-1, 1), (0, 1))[kind]
-                    descs.append(dict(x=x, y=y, w=n, h=n, ref_idx=ref, mvx=(mv[0], mv[1]), mvy=(mv[2], mv[3]), use_hadamard=1))
+    descs = f5_candidates(rng)
     arr, n_c, samples = cucd.Engine.mc_descs(descs)
     dist = np.zeros(n_c, np.uint32)
     pred = np.zeros(samples, np.int16)
@@ -335,6 +344,63 @@ def row_f5(cucd, iters=5, threads=8):
           "single_candidate_latency_us": {"median": float(np.median(lat)) * 1e6, "p10": float(np.percentile(lat, 10)) * 1e6,
                                           "p90": float(np.percentile(lat, 90)) * 1e6, "calls": len(lat), "candidate": "16x16 bi, Hadamard"}},
          p_s=p_s, h2d=int(n_c * 44), d2h=int(dist.nbytes))
+
+
+def row_f7(cucd, iters=5, threads=8):
+    """f7: 4:2:0 chroma motion compensation + SSE (cucd_me_mc_chroma) of exactly the f5 workload: the same 1920x1080 10-bit picture
+    size, two references, the same candidate array (five per whole 32/16/8 PU), one call; chroma planes 960x540 with an 80 / 2 margin.
+    Latency: one request of one 16x16 bi candidate (its 8x8 Cb and Cr blocks)."""
+    bd, pad = 10, 40
+    Wc, Hc = W // 2, H // 2
+    org_c = [_util.textured_plane(Wc, Hc, bd, seed=71 + c) for c in range(2)]
+    refs_c = [[np.pad(_util.pseudo_recon(_util.textured_plane(Wc, Hc, bd, seed=71 + c, t=k + 1), bd), pad, mode="edge") for c in range(2)] for k in range(2)]
+    eng = cucd.Engine(W, H, bit_depth=bd)
+    eng.set_cur_picture_chroma(*org_c)
+    for k in range(2):
+        eng.set_ref_picture_chroma(k, *refs_c[k], pad, pad)
+    descs = f5_candidates(np.random.default_rng(5))
+    arr, n_c, samples = cucd.Engine.mc_descs(descs)
+    sse = np.zeros(2 * n_c, np.uint32)
+    pred = np.zeros(samples // 2, np.int16)
+    k_s, w_s, p_s = timed(lambda: eng.me_mc_chroma_raw(arr, n_c, sse), eng, iters, pin=(sse,))
+    kp_s, wp_s, _ = timed(lambda: eng.me_mc_chroma_raw(arr, n_c, sse, pred), eng, iters, pin=(sse, pred))
+    n_lists = sum(2 if d["ref_idx"][0] >= 0 and d["ref_idx"][1] >= 0 else 1 for d in descs)
+    # per candidate: the two source blocks, 44 descriptor bytes, two sse words, and per used list two (w/2 + 3)(h/2 + 3) windows
+    algo = sum(d["w"] * d["h"] // 2 * 2 + 44 + 8 for d in descs) + sum(2 * (d["w"] // 2 + 3) * (d["h"] // 2 + 3) * 2 for d in descs for r in d["ref_idx"] if r >= 0)
+    import mc_chroma_util
+    mco = mc_chroma_util.load_mc_chroma_oracle()
+    samp = descs[::97]
+    Wp = Wc + 2 * pad
+
+    def work(i):
+        d = samp[i]
+        cx, cy, cw, ch = d["x"] // 2, d["y"] // 2, d["w"] // 2, d["h"] // 2
+        for c in range(2):
+            blk = np.ascontiguousarray(org_c[c][cy:cy + ch, cx:cx + cw])
+            a = [(C.c_void_p(refs_c[r][c].ctypes.data + 2 * ((cy + (d["mvy"][l] >> 3) + pad) * Wp + cx + (d["mvx"][l] >> 3) + pad)), d["mvx"][l] & 7, d["mvy"][l] & 7)
+                 for l, r in enumerate(d["ref_idx"]) if r >= 0]
+            b = a[1] if len(a) == 2 else (None, 0, 0)
+            mco.oracle_mc_chroma_cost(bd, P(blk, i16p), cw, len(a), a[0][0], Wp, a[0][1], a[0][2], b[0], Wp, b[1], b[2], cw, ch, None)
+    sec = cpu_parallel(work, len(samp), threads)
+    one = [dict(x=960, y=528, w=16, h=16, ref_idx=(0, 1), mvx=(37, -90), mvy=(-13, 58), use_hadamard=1)]
+    one_arr, _, _ = cucd.Engine.mc_descs(one)
+    one_sse = np.zeros(2, np.uint32)
+    for _ in range(50):
+        eng.me_mc_chroma_raw(one_arr, 1, one_sse)
+    lat = []
+    for _ in range(2000):
+        t0 = time.perf_counter()
+        eng.me_mc_chroma_raw(one_arr, 1, one_sse)
+        lat.append(time.perf_counter() - t0)
+    eng.close()
+    emit("f7_me_mc_chroma", "candidate/s", n_c, k_s, w_s, algo,
+         {"value": len(samp) / sec, "unit": "candidate/s", "cores": threads, "kind": "port",
+          "sample": f"every 97th candidate ({len(samp)}, Cb and Cr) through tests/mc_chroma_oracle.c in {sec:.2f} s"},
+         {"gpu": gpu_identity(), "bit_depth": bd, "chroma_format": "4:2:0", "pus": n_c // 5, "candidates_per_call": n_c, "lists_per_call": n_lists,
+          "with_pred": {"kernel_ms": kp_s * 1e3, "e2e_ms": wp_s * 1e3, "d2h_bytes": int(sse.nbytes + pred.nbytes)},
+          "single_candidate_latency_us": {"median": float(np.median(lat)) * 1e6, "p10": float(np.percentile(lat, 10)) * 1e6,
+                                          "p90": float(np.percentile(lat, 90)) * 1e6, "calls": len(lat), "candidate": "16x16 bi (8x8 Cb + Cr)"}},
+         p_s=p_s, h2d=int(n_c * 44), d2h=int(sse.nbytes))
 
 
 def row_f6(cucd, iters=5, threads=8):

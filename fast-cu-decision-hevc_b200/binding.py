@@ -155,6 +155,9 @@ def load_library():
     lib.cucd_me_sad_surface_src.argtypes = [C.c_void_p, C.c_int, C.POINTER(_MeDesc), C.c_void_p, C.c_void_p]
     lib.cucd_me_subpel_cost_src.argtypes = [C.c_void_p, C.c_int, C.POINTER(_SubpelDesc), C.c_void_p, C.c_void_p]
     lib.cucd_me_mc_cost.argtypes = [C.c_void_p, C.c_int, C.POINTER(_McDesc), C.c_void_p, C.c_void_p]
+    lib.cucd_set_ref_picture_chroma.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int]
+    lib.cucd_set_cur_picture_chroma.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]
+    lib.cucd_me_mc_chroma.argtypes = [C.c_void_p, C.c_int, C.POINTER(_McDesc), C.c_void_p, C.c_void_p]
     lib.cucd_intra_tu_forward.argtypes = [C.c_void_p, C.c_int, C.POINTER(_TuDesc), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.cucd_intra_tu_recon.argtypes = [C.c_void_p, C.c_int, C.POINTER(_TuDesc), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.cucd_intra_tu_code.argtypes = [C.c_void_p, C.c_int, C.POINTER(_TuDesc), C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
@@ -523,6 +526,43 @@ class Engine:
             res.append(pred[off:off + w * h].reshape(h, w))
             off += w * h
         return dist, res
+
+    # ---- 4:2:0 chroma of inter candidates (cucd_me_mc_chroma) ------------------------------------------------
+    def set_ref_picture_chroma(self, ref_idx, cb_padded, cr_padded, margin_x, margin_y):
+        """cb_padded, cr_padded: (H/2 + 2my, W/2 + 2mx) int16 planes including the replicated margins (chroma samples), one stride.
+        Call after set_ref_picture(ref_idx, ...): that call marks the slot's chroma unset."""
+        (cb, stride), (cr, stride_r) = _plane(cb_padded), _plane(cr_padded)
+        assert cb.shape == cr.shape == (self.height // 2 + 2 * margin_y, self.width // 2 + 2 * margin_x) and stride == stride_r
+        off = 2 * (margin_y * stride + margin_x)
+        self._check(self.lib.cucd_set_ref_picture_chroma(self.h, int(ref_idx), cb.ctypes.data + off, cr.ctypes.data + off, stride, int(margin_x),
+                                                         int(margin_y)), "cucd_set_ref_picture_chroma")
+
+    def set_cur_picture_chroma(self, cb, cr):
+        """cb, cr: (H/2, W/2) int16 planes of the current picture, one stride.  Call after set_cur_picture."""
+        (cb, stride), (cr, stride_r) = _plane(cb), _plane(cr)
+        assert cb.shape == cr.shape == (self.height // 2, self.width // 2) and stride == stride_r
+        self._check(self.lib.cucd_set_cur_picture_chroma(self.h, cb.ctypes.data, cr.ctypes.data, stride), "cucd_set_cur_picture_chroma")
+
+    def me_mc_chroma_raw(self, arr, n, sse, pred=None):
+        """cucd_me_mc_chroma with a prebuilt descriptor array (mc_descs); sse: uint32 host array of 2 n, pred: int16 host array of
+        n_samples / 2 (the luma sample count of mc_descs) or None"""
+        self._check(self.lib.cucd_me_mc_chroma(self.h, n, arr, sse.ctypes.data, None if pred is None else pred.ctypes.data), "cucd_me_mc_chroma")
+
+    def me_mc_chroma(self, descs, want_pred=False):
+        """4:2:0 chroma motion compensation + SSE of inter candidates (cucd_me_mc_chroma) on the descriptors of me_mc_cost.  Returns sse,
+        (n, 2) uint32 (Cb, Cr), and with want_pred=True also the list of (Cb, Cr) pairs of (h/2, w/2) int16 predictions: (sse, preds)."""
+        arr, n, samples = self.mc_descs(descs)
+        sse = np.zeros((n, 2), np.uint32)
+        pred = np.zeros(max(samples // 2, 1), np.int16) if want_pred else None
+        self.me_mc_chroma_raw(arr, n, sse, pred)
+        if not want_pred:
+            return sse
+        res, off = [], 0
+        for d in descs:
+            cw, ch = int(d["w"]) // 2, int(d["h"]) // 2
+            res.append((pred[off:off + cw * ch].reshape(ch, cw), pred[off + cw * ch:off + 2 * cw * ch].reshape(ch, cw)))
+            off += 2 * cw * ch
+        return sse, res
 
     # ---- intra luma TU coding (xIntraCodingTUBlock) ------------------------------------------------
     @staticmethod

@@ -241,6 +241,9 @@ int cucd_destroy(cucd_handle* h) {
   h->bOut.release(); h->bStage.release(); h->hStage.release(); h->hStageOut.release(); h->hScratch.release();
   for (auto& r : h->refs) r.buf.release();
   h->dCur.release(); h->dRefPtr.release(); h->dRefStride.release();
+  for (auto& r : h->refCb) r.buf.release();
+  for (auto& r : h->refCr) r.buf.release();
+  h->dCurC.release(); h->dRefPtrC.release(); h->dRefStrideC.release();
   for (int i = 0; i < cucd_handle::kTimeRing; i++) { if (h->evRmd0[i]) cudaEventDestroy(h->evRmd0[i]); if (h->evRmd1[i]) cudaEventDestroy(h->evRmd1[i]); }
   for (int i = 0; i < cucd_handle::kGroups; i++) { if (h->evUpG[i]) cudaEventDestroy(h->evUpG[i]); if (h->evRmdG[i]) cudaEventDestroy(h->evRmdG[i]); }
   h->hDevScratch.release(); h->dDevStage.release();

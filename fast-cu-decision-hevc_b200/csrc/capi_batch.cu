@@ -347,6 +347,8 @@ int cucd_set_ref_picture(cucd_handle* h, int ref_idx, const int16_t* recY, int s
   if (!h || ref_idx < 0 || ref_idx >= 64 || !recY || marginX < 0 || marginY < 0 || stride < h->cfg.width + 2 * marginX)
     return fail(h, CUCD_ERR_INVALID, "cucd_set_ref_picture: bad argument");
   LOCK(h);
+  // the slot's chroma belongs to the picture being replaced: unset it before anything can fail
+  if ((int)h->refCb.size() > ref_idx) h->refCb[ref_idx].set = false;
   CK(cudaSetDevice(h->cfg.device));
   if ((int)h->refs.size() <= ref_idx) h->refs.resize(ref_idx + 1);
   RefPlane& r = h->refs[ref_idx];
@@ -365,6 +367,7 @@ int cucd_set_ref_picture(cucd_handle* h, int ref_idx, const int16_t* recY, int s
 int cucd_set_cur_picture(cucd_handle* h, const int16_t* orgY, int stride) {
   if (!h || !orgY || stride < h->cfg.width) return fail(h, CUCD_ERR_INVALID, "cucd_set_cur_picture: bad argument");
   LOCK(h);
+  h->curCSet = false;                              // likewise the current chroma
   CK(cudaSetDevice(h->cfg.device));
   CK(h->dCur.reserve(h->planeSamples));
   if (h->cfg.auto_pin_host) pin_host_range(h, orgY, ((size_t)(h->cfg.height - 1) * stride + h->cfg.width) * 2);
@@ -649,6 +652,120 @@ int cucd_me_mc_cost(cucd_handle* h, int nPU, const cucd_mc_desc* desc, uint32_t*
   if (!io.direct) CK(cudaEventRecord(h->evK0, h->sMain));
   CK(launch_me_mc(mp, reinterpret_cast<const McJob*>(dAll), reinterpret_cast<const int32_t*>(dAll + jobBytes), nCta, io.dout<uint32_t>(oDist),
                   pred ? io.dout<int16_t>(oPred) : nullptr, h->sMain, &h->launches));
+  if (!io.direct) { CK(cudaEventRecord(h->evK1, h->sMain)); h->kTimed = true; } else h->kTimed = false;
+  if (io.download(h->sMain) != CUCD_OK) return CUCD_ERR_CUDA;
+  flush_launches(h);
+  return CUCD_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
+// 4:2:0 chroma motion compensation and SSE of inter candidates, me_core.cuh me_mcc_*
+// ------------------------------------------------------------------------------------------------
+// one (W / 2) x (H / 2) plane whose first padded sample is `first` (stride in samples) into dst (pitch samples), pw x ph samples
+static int upload_chroma_plane(cucd_handle* h, int16_t* dst, int pitch, const int16_t* first, int stride, int pw, int ph) {
+  if (h->cfg.auto_pin_host) pin_host_range(h, first, ((size_t)(ph - 1) * stride + pw) * 2);
+  CK(cudaMemcpy2DAsync(dst, (size_t)pitch * 2, first, (size_t)stride * 2, (size_t)pw * 2, ph, cudaMemcpyHostToDevice, h->sMain));
+  return CUCD_OK;
+}
+
+int cucd_set_ref_picture_chroma(cucd_handle* h, int ref_idx, const int16_t* recCb, const int16_t* recCr, int strideC, int marginX, int marginY) {
+  if (!h || ref_idx < 0 || ref_idx >= 64 || !recCb || !recCr || marginX < 0 || marginY < 0 || strideC < (h->cfg.width >> 1) + 2 * marginX)
+    return fail(h, CUCD_ERR_INVALID, "cucd_set_ref_picture_chroma: bad argument");
+  LOCK(h);
+  CK(cudaSetDevice(h->cfg.device));
+  if ((int)h->refCb.size() <= ref_idx) { h->refCb.resize(ref_idx + 1); h->refCr.resize(ref_idx + 1); }
+  RefPlane* r[2] = {&h->refCb[ref_idx], &h->refCr[ref_idx]};
+  const int16_t* src[2] = {recCb, recCr};
+  const int pw = (h->cfg.width >> 1) + 2 * marginX, ph = (h->cfg.height >> 1) + 2 * marginY;
+  const int pitch = (pw + 7) & ~7;
+  r[0]->set = false;
+  h->refTableCDirty = true;
+  for (int c = 0; c < 2; c++) {
+    CK(r[c]->buf.reserve((size_t)pitch * ph));
+    if (upload_chroma_plane(h, r[c]->buf.p, pitch, src[c] - (ptrdiff_t)marginY * strideC - marginX, strideC, pw, ph) != CUCD_OK) return CUCD_ERR_CUDA;
+  }
+  CK(cudaStreamSynchronize(h->sMain));
+  for (int c = 0; c < 2; c++) { r[c]->stride = pitch; r[c]->marginX = marginX; r[c]->marginY = marginY; r[c]->set = true; }
+  return CUCD_OK;
+}
+
+int cucd_set_cur_picture_chroma(cucd_handle* h, const int16_t* orgCb, const int16_t* orgCr, int strideC) {
+  if (!h || !orgCb || !orgCr || strideC < (h->cfg.width >> 1)) return fail(h, CUCD_ERR_INVALID, "cucd_set_cur_picture_chroma: bad argument");
+  LOCK(h);
+  CK(cudaSetDevice(h->cfg.device));
+  const int wc = h->cfg.width >> 1, hc = h->cfg.height >> 1, pitch = (wc + 7) & ~7;
+  h->curCSet = false;
+  CK(h->dCurC.reserve((size_t)2 * pitch * hc));
+  if (upload_chroma_plane(h, h->dCurC.p, pitch, orgCb, strideC, wc, hc) != CUCD_OK ||
+      upload_chroma_plane(h, h->dCurC.p + (size_t)pitch * hc, pitch, orgCr, strideC, wc, hc) != CUCD_OK)
+    return CUCD_ERR_CUDA;
+  CK(cudaStreamSynchronize(h->sMain));
+  h->curStrideC = pitch; h->curCSet = true;
+  return CUCD_OK;
+}
+
+// the chroma twin of sync_ref_table: [2 slot + plane] plane pointers, [slot] strides
+static int sync_ref_table_chroma(cucd_handle* h) {
+  if (!h->refTableCDirty) return CUCD_OK;
+  const size_t n = h->refCb.size();
+  std::vector<const int16_t*> refPtr(2 * n, nullptr);
+  std::vector<int32_t> refStride(n, 0);
+  for (size_t i = 0; i < n; i++) { refPtr[2 * i] = h->refCb[i].buf.p; refPtr[2 * i + 1] = h->refCr[i].buf.p; refStride[i] = h->refCb[i].stride; }
+  CK(h->dRefPtrC.reserve(std::max<size_t>(128, refPtr.size()))); CK(h->dRefStrideC.reserve(std::max<size_t>(64, refStride.size())));
+  CK(cudaMemcpyAsync(h->dRefPtrC.p, refPtr.data(), refPtr.size() * sizeof(void*), cudaMemcpyHostToDevice, h->sMain));
+  CK(cudaMemcpyAsync(h->dRefStrideC.p, refStride.data(), refStride.size() * 4, cudaMemcpyHostToDevice, h->sMain));
+  CK(cudaStreamSynchronize(h->sMain));                 // the vectors above are about to go away
+  h->refTableCDirty = false;
+  return CUCD_OK;
+}
+
+int cucd_me_mc_chroma(cucd_handle* h, int nPU, const cucd_mc_desc* desc, uint32_t* sse, int16_t* pred) {
+  if (!h || nPU < 0 || (nPU > 0 && (!desc || !sse))) return fail(h, CUCD_ERR_INVALID, "cucd_me_mc_chroma: bad argument");
+  if (nPU == 0) return CUCD_OK;
+  LOCK(h);
+  if (!h->curCSet) return fail(h, CUCD_ERR_INVALID, "cucd_me_mc_chroma: cucd_set_cur_picture_chroma not called since the last cucd_set_cur_picture");
+  CK(cudaSetDevice(h->cfg.device));
+  const int W = h->cfg.width, H = h->cfg.height, Wc = W >> 1, Hc = H >> 1;
+  std::vector<McJob> jobs(nPU);
+  long long predOff = 0;
+  for (int i = 0; i < nPU; i++) {
+    const cucd_mc_desc& d = desc[i];
+    if (d.w < 4 || d.h < 4 || d.w > 64 || d.h > 64 || (d.w & 3) || (d.h & 3) || d.x < 0 || d.y < 0 || d.x + d.w > W || d.y + d.h > H)
+      return fail(h, CUCD_ERR_INVALID, "cucd_me_mc_chroma: bad PU (w, h multiples of 4 in 4..64, inside the picture)");
+    const int cx = d.x >> 1, cy = d.y >> 1, cw = d.w >> 1, ch = d.h >> 1;
+    int nl = 0, slot[2], mvx[2], mvy[2], stride[2], mX[2], mY[2];
+    for (int l = 0; l < 2; l++) {
+      if (d.ref_idx[l] < 0) continue;
+      if (d.ref_idx[l] >= (int)h->refCb.size() || !h->refCb[d.ref_idx[l]].set)
+        return fail(h, CUCD_ERR_INVALID, "cucd_me_mc_chroma: chroma of the reference picture not set (cucd_set_ref_picture_chroma after cucd_set_ref_picture)");
+      const RefPlane& r = h->refCb[d.ref_idx[l]];
+      const int ix = cx + (d.mvx[l] >> 3), iy = cy + (d.mvy[l] >> 3);
+      if (ix - 1 < -r.marginX || iy - 1 < -r.marginY || ix + cw + 1 > Wc - 1 + r.marginX || iy + ch + 1 > Hc - 1 + r.marginY)
+        return fail(h, CUCD_ERR_INVALID, "cucd_me_mc_chroma: the interpolation support leaves the padded chroma plane");
+      slot[nl] = d.ref_idx[l]; mvx[nl] = d.mvx[l]; mvy[nl] = d.mvy[l]; stride[nl] = r.stride; mX[nl] = r.marginX; mY[nl] = r.marginY; nl++;
+    }
+    if (nl == 0) return fail(h, CUCD_ERR_INVALID, "cucd_me_mc_chroma: a candidate uses neither list (ref_idx both < 0)");
+    jobs[i] = me_mcc_job(cy * h->curStrideC + cx, cx, cy, cw, ch, nl, slot, mvx, mvy, stride, mX, mY, i, predOff);
+    predOff += 2LL * cw * ch;
+  }
+  const size_t jobBytes = up16((size_t)nPU * sizeof(McJob)), ctaBytes = up16((size_t)(nPU + 1) * sizeof(int32_t));
+  CK(h->hScratch.reserve(jobBytes + ctaBytes));
+  McJob* sorted = reinterpret_cast<McJob*>(h->hScratch.p);
+  int32_t* ctaFirst = reinterpret_cast<int32_t*>(h->hScratch.p + jobBytes);
+  const int nCta = me_mcc_plan(nPU, jobs.data(), sorted, ctaFirst);
+  if (sync_ref_table_chroma(h) != CUCD_OK) return CUCD_ERR_CUDA;
+  BatchIo io(h);
+  const int iAll = io.add_in(h->hScratch.p, jobBytes + ctaBytes, true);
+  const int oSse = io.add_out(sse, (size_t)nPU * 2 * sizeof(uint32_t));
+  const int oPred = io.add_out(pred, (size_t)predOff * sizeof(int16_t));
+  if (io.reserve() != CUCD_OK || io.upload(h->sMain) != CUCD_OK) return CUCD_ERR_CUDA;
+  McChromaPlanes cp;
+  cp.cur[0] = h->dCurC.p; cp.cur[1] = h->dCurC.p + (size_t)h->curStrideC * Hc; cp.curStride = h->curStrideC;
+  cp.ref = h->dRefPtrC.p; cp.refStride = h->dRefStrideC.p; cp.bitDepth = h->cfg.bit_depth;
+  const uint8_t* dAll = io.din<uint8_t>(iAll);
+  if (!io.direct) CK(cudaEventRecord(h->evK0, h->sMain));
+  CK(launch_me_mc_chroma(cp, reinterpret_cast<const McJob*>(dAll), reinterpret_cast<const int32_t*>(dAll + jobBytes), nCta, io.dout<uint32_t>(oSse),
+                         pred ? io.dout<int16_t>(oPred) : nullptr, h->sMain, &h->launches));
   if (!io.direct) { CK(cudaEventRecord(h->evK1, h->sMain)); h->kTimed = true; } else h->kTimed = false;
   if (io.download(h->sMain) != CUCD_OK) return CUCD_ERR_CUDA;
   flush_launches(h);

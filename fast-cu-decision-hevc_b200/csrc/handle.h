@@ -160,6 +160,12 @@ struct cucd_handle {
   bool refTableDirty = true;
   cucd::DevBuf<int16_t> dCur; int curStride = 0; bool curSet = false;
   cucd::DevBuf<const int16_t*> dRefPtr; cucd::DevBuf<int32_t> dRefStride;
+  // 4:2:0 chroma of the same slots and of the current picture (cucd_set_ref/cur_picture_chroma); setting a slot's or the current
+  // luma clears its chroma flag, so a slot never pairs the luma of one picture with the chroma of another
+  std::vector<cucd::RefPlane> refCb, refCr;       // per slot, set together: refCb's flag, stride and margins stand for both
+  bool refTableCDirty = true;
+  cucd::DevBuf<const int16_t*> dRefPtrC; cucd::DevBuf<int32_t> dRefStrideC;   // [2 slot + plane], [slot]
+  cucd::DevBuf<int16_t> dCurC; int curStrideC = 0; bool curCSet = false;      // Cb plane, then Cr at curStrideC * (height / 2)
   // job records of the device-resident ME calls (cucd_dev_me_*): their own pinned / device blocks, guarded by events
   cucd::PinBuf<uint8_t> hDevScratch; cucd::DevBuf<uint8_t> dDevStage;
   cudaEvent_t evDevUp = nullptr, evDevDone = nullptr; bool devBusy = false;

@@ -122,6 +122,16 @@ cudaError_t launch_me_subpel(const MePlanes& mp, const SubpelJob* jobs, int nJob
 // dist[outIndex] per candidate, pred (may be null) the w x h predictions at predOff
 struct McJob;
 cudaError_t launch_me_mc(const MePlanes& mp, const McJob* jobs, const int32_t* ctaFirst, int nCta, uint32_t* dist, int16_t* pred, cudaStream_t st, int* launches);
+// 4:2:0 chroma of the same candidates (me_core.cuh me_mcc_*, McJob in chroma samples): sse[2 outIndex + plane], pred (may be null) the
+// Cb then Cr (w / 2) x (h / 2) blocks at predOff
+struct McChromaPlanes {
+  const int16_t* cur[2]; int curStride;   // the current picture's Cb, Cr planes
+  const int16_t* const* ref;              // device array: [2 slot + plane] the first sample of slot's padded Cb / Cr plane
+  const int32_t* refStride;               // device array: per slot, both planes
+  int bitDepth;
+};
+cudaError_t launch_me_mc_chroma(const McChromaPlanes& cp, const McJob* jobs, const int32_t* ctaFirst, int nCta, uint32_t* sse, int16_t* pred, cudaStream_t st,
+                                int* launches);
 cudaError_t launch_me_sad(const MePlanes& mp, const MeJob* jobs, int nJobs, const int32_t* tileJob, const int32_t* tileIdx, int nTilesDy, int nTilesO,
                           uint32_t* out, cudaStream_t st, int* launches);
 

@@ -419,26 +419,31 @@ inline McJob me_mc_job(int curOff, int x, int y, int w, int h, int nl, const int
   j.outIndex = outIndex; j.predOff = predOff;
   return j;
 }
-// host: the jobs sorted by class into `sorted`, every class cut into CTAs of me_mc_per_cta candidates; CTA b takes
+// host: the jobs sorted by class (cls(job) < NC) into `sorted`, every class cut into CTAs of per(job) jobs; CTA b takes
 // sorted[ctaFirst[b] .. ctaFirst[b + 1]).  ctaFirst has room for n + 1 entries; returns the number of CTAs.
-inline int me_mc_plan(int n, const McJob* jobs, McJob* sorted, int32_t* ctaFirst) {
-  int start[kMcClasses + 1] = {0};
-  for (int i = 0; i < n; i++) start[me_mc_class(jobs[i].w, jobs[i].h, jobs[i].nl, jobs[i].had) + 1]++;
-  for (int c = 0; c < kMcClasses; c++) start[c + 1] += start[c];
+template <int NC, class Cls, class Per>
+inline int me_plan_classes(int n, const McJob* jobs, McJob* sorted, int32_t* ctaFirst, Cls cls, Per per) {
+  int start[NC + 1] = {0};
+  for (int i = 0; i < n; i++) start[cls(jobs[i]) + 1]++;
+  for (int c = 0; c < NC; c++) start[c + 1] += start[c];
   // stable scatter: start[c] advances to the end of class c
-  for (int i = 0; i < n; i++) sorted[start[me_mc_class(jobs[i].w, jobs[i].h, jobs[i].nl, jobs[i].had)]++] = jobs[i];
+  for (int i = 0; i < n; i++) sorted[start[cls(jobs[i])]++] = jobs[i];
   int nCta = 0;
   for (int b = 0; b < n;) {
     const McJob& j = sorted[b];
-    const int c = me_mc_class(j.w, j.h, j.nl, j.had), per = me_mc_per_cta(j.w, j.h, j.nl), e = start[c];
-    for (; b < e; b += per) ctaFirst[nCta++] = b;
+    const int e = start[cls(j)], k = per(j);
+    for (; b < e; b += k) ctaFirst[nCta++] = b;
     b = e;
   }
   ctaFirst[nCta] = n;
   return nCta;
 }
+inline int me_mc_plan(int n, const McJob* jobs, McJob* sorted, int32_t* ctaFirst) {
+  return me_plan_classes<kMcClasses>(n, jobs, sorted, ctaFirst, [](const McJob& j) { return me_mc_class(j.w, j.h, j.nl, j.had); },
+                                     [](const McJob& j) { return me_mc_per_cta(j.w, j.h, j.nl); });
+}
 struct McGeo {
-  int w, h, bd, head, nl, n, wh, pw /* w + 7 */, win /* (w + 7)(h + 7) */, tmp /* (h + 7) w */;
+  int w, h, bd, head, nl, n, wh, pw /* w + 7 (chroma: w + 3) */, win /* pw (h + 7 | h + 3) */, tmp /* (h + 7 | h + 3) w */;
   uint32_t invW, invPw, invWh, invWin, invTmp;
 };
 CUCD_HD McGeo me_mc_geo(int w, int h, int nl, int n, int bd) {
@@ -504,6 +509,125 @@ CUCD_HD void me_mc_ver(int tid, const McGeo& g, const McJob* jobs, const int16_t
     v = v < 0 ? 0 : (v > maxVal ? maxVal : v);
     sPred[i] = (int16_t)v;
     if (pred) pred[j.predOff + rem] = (int16_t)v;
+  }
+}
+
+// =============================================================================================================================
+// 4:2:0 chroma motion compensation and SSE of inter candidates (cucd_me_mc_chroma): the chroma branch of xPredInterBlk
+// (TComInterpolationFilter::m_chromaFilter, filterHor / filterVer with 4 taps at p - 1 .. p + 2), TComYuv::addAvg for bi, and the
+// getDistPart SSE of encodeResAndCalcRdInterCU, before the chroma weight.  Same layout as the luma kernel: McJob records (w, h, x, y
+// in chroma samples, eighth-pel fractions 0..7, had = 0) sorted into classes of equal chroma shape and list count, a CTA takes
+// me_mcc_per_cta() candidates of one class, and both planes of a candidate go to the same CTA as plane-candidates p = 2 k + plane.
+//   stage  the Cb / Cr source blocks and, per plane-candidate and list, the (w + 3) x (h + 3) window at (-1, -1) from the integer MV
+//   hor    rows -> 14-bit intermediates, h + 3 rows per list
+//   ver    columns, uni: rounded and clipped; bi: sum >> 6 per list, then addAvg.  The predictions overwrite the dead windows.
+//   sse    sum ((org - pred)^2 >> 2 (bd - 8)) per plane-candidate
+// Both passes run the 4-tap filter at every fraction: m_chromaFilter[0] = {0, 64, 0, 0} turns it into the copy.  The two-stage form
+// equals the four xPredInterBlk branches by the argument beside me_mc_ver, which only needs taps that sum to 64: stage 1 is
+// (sum c s - (8192 << (6 - head))) >> (6 - head) ((s << head) - 8192 at fraction 0, filterCopy isFirst); stage 2 is filterVer
+// (!isFirst) on it, and for fy = 0 (and fx = 0) the sum over taps {0, 64, 0, 0} leaves the single-stage results of filterHor
+// (isFirst, isLast) and filterVer (isFirst, !bi) unchanged, because 2^head divides every term that is dropped.
+// Intermediate bounds (exact over the eight filters, head = 14 - bd): stage 1 in [-10 750, 10 733] and the bi stage 2 in
+// [-14 107, 14 089] at 10 bits, less at 8 and 9 bits: both int16; the sums are int32.  SSE of a 32 x 32 plane < 2^27: an int counter.
+// =============================================================================================================================
+// every class: chroma w, h in 2, 4, .., 32 and 1 or 2 lists
+constexpr int kMccClasses = 16 * 16 * 2;
+inline int me_mcc_class(int w, int h, int nl) { return (((w >> 1) - 1) * 16 + (h >> 1) - 1) * 2 + nl - 1; }
+// the caps of the luma kernel, two plane-candidates per candidate
+CUCD_HD int me_mcc_per_cta(int w, int h, int nl) {
+  int k = kMcCurCap / (2 * w * h);
+  const int kw = kMcWinCap / (2 * nl * (w + 3) * (h + 3)), kt = kMcTmpCap / (2 * nl * (h + 3) * w);
+  k = k < kw ? k : kw; k = k < kt ? k : kt;
+  return k < kMcMaxCand ? k : kMcMaxCand;
+}
+// host: the job of a candidate's chroma block (x, y, w, h: the luma PU >> 1), luma quarter-pel = chroma eighth-pel MVs; slot, mvx, mvy,
+// stride, mX, mY per used list as for me_mc_job, the strides and margins those of the slot's chroma planes
+inline McJob me_mcc_job(int curOff, int x, int y, int w, int h, int nl, const int* slot, const int* mvx, const int* mvy, const int* stride, const int* mX,
+                        const int* mY, int outIndex, long long predOff) {
+  McJob j;
+  j.curOff = curOff;
+  for (int l = 0; l < 2; l++) {
+    const int u = l < nl ? l : 0;
+    j.refOff[l] = (y + (mvy[u] >> 3) - 1 + mY[u]) * stride[u] + x + (mvx[u] >> 3) - 1 + mX[u];
+    j.refSlot[l] = (int16_t)slot[u]; j.fx[l] = (int8_t)(mvx[u] & 7); j.fy[l] = (int8_t)(mvy[u] & 7);
+  }
+  j.w = (int16_t)w; j.h = (int16_t)h; j.nl = (int8_t)nl; j.had = 0; j.pad = 0;
+  j.outIndex = outIndex; j.predOff = predOff;
+  return j;
+}
+inline int me_mcc_plan(int n, const McJob* jobs, McJob* sorted, int32_t* ctaFirst) {
+  return me_plan_classes<kMccClasses>(n, jobs, sorted, ctaFirst, [](const McJob& j) { return me_mcc_class(j.w, j.h, j.nl); },
+                                      [](const McJob& j) { return me_mcc_per_cta(j.w, j.h, j.nl); });
+}
+CUCD_HD McGeo me_mcc_geo(int w, int h, int nl, int n, int bd) {
+  McGeo g;
+  g.w = w; g.h = h; g.bd = bd; g.head = 14 - bd; g.nl = nl; g.n = n; g.wh = w * h; g.pw = w + 3; g.win = (w + 3) * (h + 3); g.tmp = (h + 3) * w;
+  g.invW = me_inv((uint32_t)w); g.invPw = me_inv((uint32_t)g.pw); g.invWh = me_inv((uint32_t)g.wh); g.invWin = me_inv((uint32_t)g.win); g.invTmp = me_inv((uint32_t)g.tmp);
+  return g;
+}
+// sum s[(k - 1) * stride] * m_chromaFilter[frac][k], frac = 0..7:
+//   {0, 64, 0, 0} {-2, 58, 10, -2} {-4, 54, 16, -2} {-6, 46, 28, -4} {-4, 36, 36, -4} {-4, 28, 46, -6} {-2, 16, 54, -4} {-2, 10, 58, -2}
+// held as byte lanes of three constants (|c0|, c1, |c3|; c2 = 64 - c1 + |c0| + |c3|), so a warp whose lanes see different fractions
+// does not branch
+CUCD_HD int chroma_filter4(const int16_t* s, int stride, int frac) {
+  const int sh = 8 * frac;
+  const int n0 = (int)((0x0202040406040200ull >> sh) & 0xff), c1 = (int)((0x0a101c242e363a40ull >> sh) & 0xff), n3 = (int)((0x0204060404020200ull >> sh) & 0xff);
+  return -n0 * s[-stride] + c1 * s[0] + (64 - c1 + n0 + n3) * s[stride] - n3 * s[2 * stride];
+}
+// every index below is < 10240 and every divisor <= 35 * 35: the multiply-high divisions are exact.  cur[plane]: the current
+// picture's Cb / Cr plane; ref[2 slot + plane]: the first sample of slot's padded Cb / Cr plane, refStride[slot] of both
+CUCD_HD void me_mcc_stage(int tid, const McGeo& g, const McJob* jobs, const int16_t* const* cur, int curStride, const int16_t* const* ref, const int32_t* refStride,
+                          int16_t* sCur, int16_t* sWin) {
+  for (int i = tid; i < 2 * g.n * g.wh; i += 256) {
+    const int p = (int)me_mulhi((uint32_t)i, g.invWh), rem = i - p * g.wh;
+    const int y = (int)me_mulhi((uint32_t)rem, g.invW), x = rem - y * g.w;
+    const int16_t* c = (p & 1) ? cur[1] : cur[0];                                      // a select, not an indexed (local-memory) copy of the array
+    sCur[i] = c[jobs[p >> 1].curOff + (long long)y * curStride + x];
+  }
+  for (int i = tid; i < 2 * g.n * g.nl * g.win; i += 256) {
+    const int pl = (int)me_mulhi((uint32_t)i, g.invWin), rem = i - pl * g.win;          // pl = (2 k + plane) nl + l
+    const int y = (int)me_mulhi((uint32_t)rem, g.invPw), x = rem - y * g.pw;
+    const int p = pl >> (g.nl - 1), l = pl & (g.nl - 1);
+    const McJob& j = jobs[p >> 1];
+    const int slot = j.refSlot[l];
+    sWin[i] = ref[2 * slot + (p & 1)][j.refOff[l] + (long long)y * refStride[slot] + x];
+  }
+}
+// rows of every window -> sTmp[pl][r][c], r = 0 .. h + 2 (filterHor, isFirst, !isLast)
+CUCD_HD void me_mcc_hor(int tid, const McGeo& g, const McJob* jobs, const int16_t* sWin, int16_t* sTmp) {
+  for (int i = tid; i < 2 * g.n * g.nl * g.tmp; i += 256) {
+    const int pl = (int)me_mulhi((uint32_t)i, g.invTmp), rem = i - pl * g.tmp;
+    const int r = (int)me_mulhi((uint32_t)rem, g.invW), c = rem - r * g.w;
+    const int fx = jobs[pl >> g.nl].fx[pl & (g.nl - 1)];
+    sTmp[i] = (int16_t)((chroma_filter4(&sWin[pl * g.win + r * g.pw + c + 1], 1, fx) - (8192 << (6 - g.head))) >> (6 - g.head));
+  }
+}
+// columns -> the clipped prediction sPred[p][r][c]; pred (may be null) holds a candidate's Cb block, then its Cr block, at predOff
+CUCD_HD void me_mcc_ver(int tid, const McGeo& g, const McJob* jobs, const int16_t* sTmp, int16_t* sPred, int16_t* pred) {
+  const int maxVal = (1 << g.bd) - 1;
+  for (int i = tid; i < 2 * g.n * g.wh; i += 256) {
+    const int p = (int)me_mulhi((uint32_t)i, g.invWh), rem = i - p * g.wh;
+    const int r = (int)me_mulhi((uint32_t)rem, g.invW), c = rem - r * g.w;
+    const McJob& j = jobs[p >> 1];
+    int v;
+    if (g.nl == 1) {
+      v = (chroma_filter4(&sTmp[p * g.tmp + (r + 1) * g.w + c], g.w, j.fy[0]) + (1 << (5 + g.head)) + (8192 << 6)) >> (6 + g.head);
+    } else {
+      const int p0 = chroma_filter4(&sTmp[2 * p * g.tmp + (r + 1) * g.w + c], g.w, j.fy[0]) >> 6;
+      const int p1 = chroma_filter4(&sTmp[(2 * p + 1) * g.tmp + (r + 1) * g.w + c], g.w, j.fy[1]) >> 6;
+      v = (p0 + p1 + (1 << g.head) + 16384) >> (g.head + 1);
+    }
+    v = v < 0 ? 0 : (v > maxVal ? maxVal : v);
+    sPred[i] = (int16_t)v;
+    if (pred) pred[j.predOff + (long long)(p & 1) * g.wh + rem] = (int16_t)v;
+  }
+}
+// getDistPart (TComRdCost::xGetSSE): sSum[p] += (org - pred)^2 >> 2 (bd - 8)
+CUCD_HD void me_mcc_sse(int tid, const McGeo& g, const int16_t* sCur, const int16_t* sPred, int* sSum) {
+  const int shift = 2 * (g.bd - 8);
+  for (int i = tid; i < 2 * g.n * g.wh; i += 256) {
+    const int d = (int)sCur[i] - (int)sPred[i], v = (d * d) >> shift;
+    if (v) me_smem_add(&sSum[me_mulhi((uint32_t)i, g.invWh)], v);
   }
 }
 

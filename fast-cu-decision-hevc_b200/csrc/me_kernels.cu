@@ -386,6 +386,39 @@ me_mc_kernel(const MePlanes mp, const McJob* __restrict__ jobs, const int32_t* _
   if (tid < g.n) dist[J[tid].outIndex] = (uint32_t)sSum[tid] >> (g.bd - 8);
 }
 
+// 4:2:0 chroma motion compensation + SSE (me_core.cuh, me_mcc_*): a CTA takes the candidates jobs[ctaFirst[b] .. ctaFirst[b + 1]) of
+// one class, both planes of each; the predictions reuse the shared memory of the dead reference windows.
+__global__ void __launch_bounds__(256)
+me_mc_chroma_kernel(const McChromaPlanes cp, const McJob* __restrict__ jobs, const int32_t* __restrict__ ctaFirst, uint32_t* __restrict__ sse,
+                    int16_t* __restrict__ pred) {
+  __shared__ __align__(16) int16_t sCur[kMcCurCap];
+  __shared__ __align__(16) int16_t sWin[kMcWinCap];
+  __shared__ __align__(16) int16_t sTmp[kMcTmpCap];
+  __shared__ int sSum[2 * kMcMaxCand];
+  const int tid = threadIdx.x;
+  const int first = ctaFirst[blockIdx.x];
+  const McJob* J = jobs + first;
+  const McGeo g = me_mcc_geo(J[0].w, J[0].h, J[0].nl, ctaFirst[blockIdx.x + 1] - first, cp.bitDepth);
+  if (tid < 2 * g.n) sSum[tid] = 0;
+  me_mcc_stage(tid, g, J, cp.cur, cp.curStride, cp.ref, cp.refStride, sCur, sWin);
+  __syncthreads();
+  me_mcc_hor(tid, g, J, sWin, sTmp);
+  __syncthreads();
+  me_mcc_ver(tid, g, J, sTmp, sWin, pred);
+  __syncthreads();
+  me_mcc_sse(tid, g, sCur, sWin, sSum);
+  __syncthreads();
+  if (tid < 2 * g.n) sse[2 * J[tid >> 1].outIndex + (tid & 1)] = (uint32_t)sSum[tid];
+}
+
+cudaError_t launch_me_mc_chroma(const McChromaPlanes& cp, const McJob* jobs, const int32_t* ctaFirst, int nCta, uint32_t* sse, int16_t* pred, cudaStream_t st,
+                                int* launches) {
+  if (nCta <= 0) return cudaSuccess;
+  me_mc_chroma_kernel<<<nCta, 256, 0, st>>>(cp, jobs, ctaFirst, sse, pred);
+  if (launches) *launches += 1;
+  return cudaGetLastError();
+}
+
 cudaError_t launch_me_mc(const MePlanes& mp, const McJob* jobs, const int32_t* ctaFirst, int nCta, uint32_t* dist, int16_t* pred, cudaStream_t st, int* launches) {
   if (nCta <= 0) return cudaSuccess;
   me_mc_kernel<<<nCta, 256, 0, st>>>(mp, jobs, ctaFirst, dist, pred);

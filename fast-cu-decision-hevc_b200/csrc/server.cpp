@@ -178,6 +178,46 @@ int main(int argc, char** argv) {
           reply(s, rc, rc == CUCD_OK ? nullptr : cucd_last_error(k.h));
           break;
         }
+        case CUCD_IPC_SET_REF_CHROMA: {
+          // margins come from the client: bound them by the arena and size the planes in 64 bits, so that a huge margin fails the
+          // size check instead of overflowing
+          const int mx = s.args[1], my = s.args[2];
+          const long long pw64 = k.W / 2 + 2LL * mx, ph64 = k.H / 2 + 2LL * my;
+          if (mx < 0 || my < 0 || (unsigned long long)mx > hdr->arena_bytes || (unsigned long long)my > hdr->arena_bytes ||
+              s.in_bytes > hdr->arena_bytes || (unsigned long long)(pw64 * ph64) * 4 > s.in_bytes) {
+            reply(s, CUCD_ERR_INVALID, "cucd_set_ref_picture_chroma: request size disagrees");
+            break;
+          }
+          const int pw = (int)pw64, ph = (int)ph64;                  // both planes fit the arena: far below 2^31
+          const int16_t* cb = reinterpret_cast<const int16_t*>(in) + (size_t)my * pw + mx;
+          const int rc = k.h ? cucd_set_ref_picture_chroma(k.h, s.args[0], cb, cb + (size_t)pw * ph, pw, mx, my) : CUCD_ERR_INVALID;
+          reply(s, rc, rc == CUCD_OK ? nullptr : cucd_last_error(k.h));
+          break;
+        }
+        case CUCD_IPC_SET_CUR_CHROMA: {
+          const size_t plane = (size_t)(k.W / 2) * (k.H / 2);
+          if (2 * plane * 2 > s.in_bytes) { reply(s, CUCD_ERR_INVALID, "cucd_set_cur_picture_chroma: request size disagrees"); break; }
+          const int16_t* cb = reinterpret_cast<const int16_t*>(in);
+          const int rc = k.h ? cucd_set_cur_picture_chroma(k.h, cb, cb + plane, k.W / 2) : CUCD_ERR_INVALID;
+          reply(s, rc, rc == CUCD_OK ? nullptr : cucd_last_error(k.h));
+          break;
+        }
+        case CUCD_IPC_MC_CHROMA: {
+          // the reply must fit what the client reserved: sse, then (args[0]) the Cb and Cr predictions
+          const size_t nC = (size_t)(s.n > 0 ? s.n : 0), sseBytes = (nC * 8 + 15) & ~(size_t)15;
+          const cucd_mc_desc* desc = reinterpret_cast<const cucd_mc_desc*>(in);
+          size_t need = sseBytes;
+          if (nC * sizeof(cucd_mc_desc) <= s.in_bytes && s.args[0])
+            for (size_t i = 0; i < nC; i++) need += 2 * (size_t)(desc[i].w > 0 ? desc[i].w / 2 : 0) * (size_t)(desc[i].h > 0 ? desc[i].h / 2 : 0) * 2;
+          if (nC * sizeof(cucd_mc_desc) > s.in_bytes || need > s.out_bytes || s.out_off + s.out_bytes > hdr->arena_bytes) {
+            reply(s, CUCD_ERR_INVALID, "cucd_me_mc_chroma: request and reply sizes disagree");
+            break;
+          }
+          int16_t* pred = s.args[0] ? reinterpret_cast<int16_t*>(out + sseBytes) : nullptr;
+          const int rc = k.h ? cucd_me_mc_chroma(k.h, s.n, desc, reinterpret_cast<uint32_t*>(out), pred) : CUCD_ERR_INVALID;
+          reply(s, rc, rc == CUCD_OK ? nullptr : cucd_last_error(k.h));
+          break;
+        }
         default:
           reply(s, CUCD_ERR_INVALID, "unknown request");
       }
@@ -239,10 +279,10 @@ int main(int argc, char** argv) {
   if (segPinned) cudaHostUnregister(mem);
   printf("{\"clients\": %d, \"closed\": %d, \"seconds\": %.3f, \"rmd_requests\": %lld, \"rmd_pus\": %lld, \"rmd_batches\": %lld, \"pus_per_batch\": %.1f, "
          "\"requests_per_batch\": %.2f, \"max_batch_pus\": %lld, \"rmd_busy_seconds\": %.3f, \"frames\": %lld, \"me_surfaces\": %lld, \"subpel\": %lld, "
-         "\"mc\": %lld, \"set_ref\": %lld, \"window_us\": %.1f, \"segment_pinned\": %s}\n",
+         "\"mc\": %lld, \"mc_chroma\": %lld, \"set_ref\": %lld, \"window_us\": %.1f, \"segment_pinned\": %s}\n",
          nSeen, nClosed, (now_us() - t0) * 1e-6, rmdReqs, rmdPus, rmdBatches, rmdBatches ? (double)rmdPus / rmdBatches : 0.0,
          rmdBatches ? (double)rmdReqs / rmdBatches : 0.0, maxBatchPus, rmdBusyUs * 1e-6, nReq[CUCD_IPC_FRAME], nReq[CUCD_IPC_ME_SURFACE], nReq[CUCD_IPC_SUBPEL],
-         nReq[CUCD_IPC_MC], nReq[CUCD_IPC_SET_REF], windowUs, segPinned ? "true" : "false");
+         nReq[CUCD_IPC_MC], nReq[CUCD_IPC_MC_CHROMA], nReq[CUCD_IPC_SET_REF], windowUs, segPinned ? "true" : "false");
   munmap(mem, total);
   shm_unlink(name.c_str());
   return 0;

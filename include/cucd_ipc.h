@@ -9,7 +9,7 @@
  * own slot + arena and sleeps on a futex; the server turns everything that is pending into one batch per request kind.
  *   S2  (cucd_intra_rmd_batch)   stateless: requests of ALL instances with the same bit depth are coalesced into one batch
  *   S1  (cuCUDecide_frame), S3 (cucd_set_cur/ref_picture, cucd_me_sad_surface), sub-pel (cucd_me_subpel_cost), inter candidates
- *        (cucd_me_mc_cost): served on the instance's own handle inside the server (they depend on that instance's pictures), in
+ *        (cucd_me_mc_cost, cucd_set_ref/cur_picture_chroma, cucd_me_mc_chroma): served on the instance's own handle inside the server (they depend on that instance's pictures), in
  *        arrival order.  A server that predates an op answers it with CUCD_ERR_INVALID, "unknown request".
  * The client side below is header-only C++ (what the reference's shim includes); the entry points mirror the C ABI of
  * include/cucudecide.h one to one, so an integration switches between in-process and server mode without other changes.
@@ -37,7 +37,7 @@
 #define CUCD_IPC_ARENA_BYTES ((size_t)96 << 20)      /* request + reply payload of one instance (a padded 2160p plane is 34 MB) */
 
 enum cucd_ipc_op { CUCD_IPC_OPEN = 1, CUCD_IPC_CLOSE, CUCD_IPC_FRAME, CUCD_IPC_RMD, CUCD_IPC_SET_CUR, CUCD_IPC_SET_REF, CUCD_IPC_ME_SURFACE, CUCD_IPC_SUBPEL,
-                   CUCD_IPC_MC };
+                   CUCD_IPC_MC, CUCD_IPC_SET_REF_CHROMA, CUCD_IPC_SET_CUR_CHROMA, CUCD_IPC_MC_CHROMA };
 enum cucd_ipc_state { CUCD_IPC_FREE = 0, CUCD_IPC_IDLE = 1, CUCD_IPC_READY = 2, CUCD_IPC_DONE = 3, CUCD_IPC_CLOSED = 4 };
 
 struct alignas(128) cucd_ipc_slot {
@@ -172,6 +172,44 @@ struct cucd_ipc_client {
     s->args[0] = pred ? 1 : 0;
     const int rc = call(CUCD_IPC_MC, nPU, inBytes, outBytes);
     if (rc == CUCD_OK) { memcpy(dist, reply(), (size_t)nPU * 4); if (pred) memcpy(pred, reply() + distBytes, samples * 2); }
+    return rc;
+  }
+  /* cucd_set_ref_picture_chroma: request = [padded Cb | padded Cr], (W/2 + 2 marginX) x (H/2 + 2 marginY) each, tight */
+  int set_ref_picture_chroma(int W, int H, int ref_idx, const int16_t* recCb, const int16_t* recCr, int strideC, int marginX, int marginY) {
+    const int pw = W / 2 + 2 * marginX, ph = H / 2 + 2 * marginY;
+    const size_t plane = (size_t)pw * ph;
+    const int16_t* src[2] = {recCb, recCr};
+    for (int c = 0; c < 2; c++) {
+      const int16_t* first = src[c] - (ptrdiff_t)marginY * strideC - marginX;
+      for (int r = 0; r < ph; r++) memcpy(arena + (c * plane + (size_t)r * pw) * 2, first + (size_t)r * strideC, (size_t)pw * 2);
+    }
+    s->args[0] = ref_idx; s->args[1] = marginX; s->args[2] = marginY;
+    return call(CUCD_IPC_SET_REF_CHROMA, 1, 2 * plane * 2, 0);
+  }
+  /* cucd_set_cur_picture_chroma: request = [Cb | Cr], (W/2) x (H/2) each, tight */
+  int set_cur_picture_chroma(int W, int H, const int16_t* orgCb, const int16_t* orgCr, int strideC) {
+    const size_t plane = (size_t)(W / 2) * (H / 2);
+    const int16_t* src[2] = {orgCb, orgCr};
+    for (int c = 0; c < 2; c++)
+      for (int r = 0; r < H / 2; r++) memcpy(arena + (c * plane + (size_t)r * (W / 2)) * 2, src[c] + (size_t)r * strideC, (size_t)(W / 2) * 2);
+    return call(CUCD_IPC_SET_CUR_CHROMA, 1, 2 * plane * 2, 0);
+  }
+  /* cucd_me_mc_chroma: reply = [sse (2 per candidate) | pad | pred (Cb, Cr blocks)]; pred may be NULL (args[0] tells the server) */
+  int me_mc_chroma(int nPU, const cucd_mc_desc* desc, uint32_t* sse, int16_t* pred) {
+    if (nPU < 0 || (nPU > 0 && (!desc || !sse))) { snprintf(err, sizeof err, "me_mc_chroma: bad argument"); return CUCD_ERR_INVALID; }
+    size_t samples = 0;
+    for (int i = 0; i < nPU; i++) samples += 2 * (size_t)(desc[i].w > 0 ? desc[i].w / 2 : 0) * (size_t)(desc[i].h > 0 ? desc[i].h / 2 : 0);
+    const size_t inBytes = (size_t)nPU * sizeof(cucd_mc_desc), sseBytes = ((size_t)nPU * 8 + 15) & ~(size_t)15;
+    const size_t outBytes = sseBytes + (pred ? samples * 2 : 0);
+    if (((inBytes + 255) & ~(size_t)255) + outBytes > hdr->arena_bytes) {
+      snprintf(err, sizeof err, "me_mc_chroma: %d candidates need %llu bytes, more than the %llu-byte arena", nPU,
+               (unsigned long long)(((inBytes + 255) & ~(size_t)255) + outBytes), (unsigned long long)hdr->arena_bytes);
+      return CUCD_ERR_NOMEM;
+    }
+    memcpy(arena, desc, inBytes);
+    s->args[0] = pred ? 1 : 0;
+    const int rc = call(CUCD_IPC_MC_CHROMA, nPU, inBytes, outBytes);
+    if (rc == CUCD_OK) { memcpy(sse, reply(), (size_t)nPU * 8); if (pred) memcpy(pred, reply() + sseBytes, samples * 2); }
     return rc;
   }
 };

@@ -242,6 +242,26 @@ typedef struct {
 int cucd_me_mc_cost(cucd_handle* h, int nPU, const cucd_mc_desc* desc, uint32_t* dist, int16_t* pred);
 
 /* ------------------------------------------------------------------------------------------------
+ * Chroma motion compensation and SSE of the same inter candidates: the chroma half of TComPrediction::motionCompensation and the
+ * distortion encodeResAndCalcRdInterCU takes of it.  4:2:0 only; chroma samples use the handle's bit_depth.
+ * Prediction: the chroma branch of xPredInterBlk with TComInterpolationFilter::m_chromaFilter (4 taps at p - 1 .. p + 2, filterHor /
+ * filterVer), for bi the two 14-bit list predictions averaged by TComYuv::addAvg before the clip.  Weighted prediction is not covered.
+ * The planes of a reference slot / of the current picture are (W / 2) x (H / 2) samples; margins and stride in chroma samples (HM:
+ * the luma margin >> 1).  Set chroma after luma: cucd_set_ref_picture(slot) marks that slot's chroma unset and cucd_set_cur_picture
+ * marks the current chroma unset, so that a slot never pairs the luma of one picture with the chroma of another. */
+int cucd_set_ref_picture_chroma(cucd_handle* h, int ref_idx, const int16_t* recCb, const int16_t* recCr, int strideC, int marginX, int marginY);
+int cucd_set_cur_picture_chroma(cucd_handle* h, const int16_t* orgCb, const int16_t* orgCr, int strideC);
+/* desc: the cucd_mc_desc array of cucd_me_mc_cost, unchanged (x, y, w, h the LUMA PU; the chroma block is (x/2, y/2, w/2, h/2), 2..32
+ * on a side; mvx / mvy the luma quarter-pel MVs, i.e. eighth-pel chroma MVs: integer part mv >> 3, fraction mv & 7; use_hadamard is
+ * ignored).  The 4-tap support of every used list must stay inside the padded chroma plane:
+ *   x/2 + (mvx >> 3) - 1 >= -marginX, x/2 + (mvx >> 3) + w/2 + 1 <= W/2 - 1 + marginX, and the same vertically.
+ * sse[2 i] / sse[2 i + 1]: the Cb / Cr getDistPart of candidate i, sum ((org - pred)^2 >> 2 (bitDepth - 8)) in uint32, before
+ * m_distortionWeight (the convention of the chroma TU calls).  pred (may be NULL): per candidate the clipped Cb block, then the Cr
+ * block, (w/2) x (h/2) each, row-major.  Rejects what cucd_me_mc_cost rejects, a slot whose chroma is not set, and a call before
+ * cucd_set_cur_picture_chroma.  nPU == 0 is a no-op. */
+int cucd_me_mc_chroma(cucd_handle* h, int nPU, const cucd_mc_desc* desc, uint32_t* sse, int16_t* pred);
+
+/* ------------------------------------------------------------------------------------------------
  * The same two searches for a caller-supplied source block ("pattern key") instead of the block of the current picture:
  * what the bi-predictive refinement of xMotionEstimation needs (if (bBi), TEncSearch.cpp:3787-3797, 3826-3849: the key is
  * m_cYuvPredTemp = 2 * org - prediction of the other list, TComYuv::removeHighFreq, so its samples may be negative or exceed
@@ -298,8 +318,8 @@ int cucd_intra_tu_code(cucd_handle* h, int nTU, const cucd_tu_desc* desc, const 
  * Inter TU coding: the arithmetic of TEncSearch::xEstimateResidualQT (TEncSearch.cpp, called by
  * encodeResAndCalcRdInterCU for every inter candidate) for the TUs of inter residual quadtrees.  An inter residual does not depend on the
  * reconstruction of the TU before it, so every TU of every RQT depth of a CU, luma and chroma, and the TUs of all merge
- * candidates of a PU can go in one call.  resi holds the residual blocks org - pred (cut by the caller from pcResi; chroma from
- * the caller's own chroma motion compensation), N*N per TU back to back in descriptor order; coef / level / rresi use the same
+ * candidates of a PU can go in one call.  resi holds the residual blocks org - pred (cut by the caller from pcResi; the luma
+ * prediction from cucd_me_mc_cost, the chroma one from cucd_me_mc_chroma), N*N per TU back to back in descriptor order; coef / level / rresi use the same
  * layout, dist / dist_zero / abs_sum hold one value per TU.  Descriptors as above with mode = 0; flags CUCD_TU_TRANSFORM_SKIP
  * (4x4 only) and / or CUCD_TU_CHROMA.
  * Precondition: |resi| <= 2^bit_depth - 1, which the difference of two in-range planes satisfies (the forward stages keep
@@ -404,7 +424,7 @@ int cucd_set_rmd_path(cucd_handle* h, int path);
  * the number of calls averaged, or a negative status; *avg_ms = mean duration of one launch. */
 int cucd_rmd_kernel_time(cucd_handle* h, int nCalls, float* avg_ms);
 /* Device time between the first and the last kernel of the most recent batch call on this handle (cucd_intra_rmd_batch,
- * cucd_me_sad_surface, cucd_me_subpel_cost, cucd_me_mc_cost, cucd_intra_tu_*, cucd_inter_tu_*, cucd_tmv_features, cucd_aq_activity): CUDA events on
+ * cucd_me_sad_surface, cucd_me_subpel_cost, cucd_me_mc_cost, cucd_me_mc_chroma, cucd_intra_tu_*, cucd_inter_tu_*, cucd_tmv_features, cucd_aq_activity): CUDA events on
  * the library's stream, host<->device
  * copies outside.  What bench_rows.py reports as the kernel-only figure of those paths. */
 int cucd_last_kernel_time(cucd_handle* h, float* ms);
