@@ -15,7 +15,8 @@ Rows: s2 (cucd_intra_rmd_batch), f1 (cucd_queue_*: K concurrent instances), s3 (
 a12 (cucd_tmv_features), a13 (cucd_aq_activity), f2 (cucd_intra_tu_code / _forward / _recon).  Usage: python bench_rows.py [--iters 5] > gpurun_out/rows.jsonl
 Last rows: f5 (cucd_me_mc_cost, motion compensation + distortion of inter candidates; row_f5 runs it on its own), f6
 (cucd_inter_tu_forward / _code / _recon, the TUs of inter residual quadtrees; row_f6) and f7 (cucd_me_mc_chroma, the 4:2:0 chroma of
-f5's candidates; row_f7).  --only f5 / f6 / f7 runs one of them alone.
+f5's candidates; row_f7) and f8 (cucd_me_search / _src, the motion search of bench.py's inter workloads against the surface route it
+replaces; row_f8).  --only f5 / f6 / f7 / f8 runs one of them alone.
 """
 import argparse
 import ctypes as C
@@ -93,11 +94,11 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--iters", type=int, default=5)
     ap.add_argument("--cpu-threads", type=int, default=min(16, os.cpu_count() or 1))
-    ap.add_argument("--only", choices=["f5", "f6", "f7"], default=None, help="run one of the last rows alone")
+    ap.add_argument("--only", choices=["f5", "f6", "f7", "f8"], default=None, help="run one of the last rows alone")
     a = ap.parse_args()
     cucd = importlib.import_module("fast-cu-decision-hevc_b200")
     if a.only:
-        {"f5": row_f5, "f6": row_f6, "f7": row_f7}[a.only](cucd, a.iters, a.cpu_threads)
+        {"f5": row_f5, "f6": row_f6, "f7": row_f7, "f8": row_f8}[a.only](cucd, a.iters, a.cpu_threads)
         return
     oracle = _util.load_oracle()
     ref = _util.load_hmref()
@@ -262,6 +263,7 @@ def main():
     row_f5(cucd, a.iters, T)
     row_f6(cucd, a.iters, T)
     row_f7(cucd, a.iters, T)
+    row_f8(cucd, a.iters, T)
 
 
 def gpu_identity():
@@ -454,6 +456,116 @@ def row_f6(cucd, iters=5, threads=8):
               "qp": "32 luma / 31 chroma", "sign_hiding": True},
              p_s=p_s, h2d=int(in_bytes + n_tu * 16), d2h=int(out_bytes))
     eng.close()
+
+
+
+def row_f8(cucd, iters=5, threads=8):
+    """f8: motion search (cucd_me_search) on the ME part of bench.py's inter workloads: the 42 900 square PUs of a 1920x1080 picture
+    (bench.inter_pus), +-64 windows, FEN sub_shift (1 above 8x8), FRAC with Hadamard, lambda = floor(65536 sqrt(0.57 2^((32 - 12) / 3)))
+    (QP 32), predictors drawn in +-64 samples.  ldp1080p: 8-bit, one reference; ra1080p10: 10-bit, two references (one call for both).
+    Baseline in the same run: the surface route to the same answer (cucd_me_sad_surface + host argmin, cucd_me_subpel_cost + host walk),
+    whose results must equal the search's.  f8_me_search_src: +-4 windows with signed keys (cucd_me_search_src) on the same PUs."""
+    import bench
+    import me_search_util as msu
+    R, M = bench.ME_RANGE, bench.ME_MARGIN
+    pus = bench.inter_pus(W, H)
+    lam = msu.lambda_cost(32)
+    mso = msu.load_me_search_oracle()
+    gpu = gpu_identity()
+    for cfg, bd, nref in (("ldp1080p", 8, 1), ("ra1080p10", 10, 2)):
+        org = _util.textured_plane(W, H, bd, seed=81)
+        refs = [np.ascontiguousarray(np.pad(_util.pseudo_recon(_util.textured_plane(W, H, bd, seed=82 + k), bd), M, mode="edge")) for k in range(nref)]
+        rng = np.random.default_rng(83)
+        eng = cucd.Engine(W, H, bit_depth=bd)
+        eng.set_cur_picture(org)
+        for k, r in enumerate(refs):
+            eng.set_ref_picture(k, r, M, M)
+        for row, rad, signed in (("f8_me_search", R, False), ("f8_me_search_src", 4, True)):
+            descs = []
+            for k in range(nref):
+                preds = rng.integers(-4 * R, 4 * R + 1, (len(pus), 2))
+                descs += [dict(x=x, y=y, w=s, h=s, ref_idx=k, left=-rad, right=rad, top=-rad, bottom=rad, sub_shift=1 if s > 8 else 0, pred_x=int(p[0]),
+                               pred_y=int(p[1]), flags=msu.FRAC | msu.HAD, **{"lambda": lam}) for (x, y, s), p in zip(pus, preds)]
+            arr, n = cucd.Engine.search_descs(descs)
+            res = np.zeros(n, cucd.SEARCH_RESULT)
+            src = None
+            if signed:
+                src = rng.integers(-(1 << bd), 2 << bd, sum(d["w"] * d["h"] for d in descs)).astype(np.int16)
+            k_s, w_s, p_s = timed(lambda: eng.me_search_raw(arr, n, res, src), eng, iters, pin=(res,) + ((src,) if signed else ()))
+            h2d = n * 56 + (0 if src is None else src.nbytes)
+            d2h = n * 24
+            # algorithmic bytes: per PU its source block, its (w + 2 rad)^2 reference window, the (w + 9)^2 window of the sub-pel stage,
+            # the descriptor and the result
+            algo = sum(d["w"] * d["h"] * 2 + (d["w"] + 2 * rad) * (d["h"] + 2 * rad) * 2 + (d["w"] + 9) * (d["h"] + 9) * 2 + 56 + 24 for d in descs)
+            # the checker on host threads, every 97th PU
+            samp = descs[::97]
+            blocks = msu.src_blocks(dict(org=org), samp)
+            sc = dict(bd=bd, M=M, refs={k: r for k, r in enumerate(refs)})
+
+            def work(i):
+                d = samp[i]
+                blk, r = blocks[i], np.zeros(6, np.int32)
+                mso.oracle_me_search(bd, P(blk, i16p), d["w"], d["w"], d["h"], msu.ref_base(sc, d), refs[d["ref_idx"]].shape[1], d["left"], d["right"], d["top"],
+                                     d["bottom"], d["sub_shift"], d["pred_x"], d["pred_y"], lam, d["flags"], P(r, i32p))
+            cpu = None
+            if src is None:                 # the signed-key row: the same checker, not timed twice
+                sec = cpu_parallel(work, len(samp), threads)
+                cpu = {"value": len(samp) / sec, "unit": "PU/s", "cores": threads, "kind": "port",
+                       "sample": f"every 97th PU ({len(samp)}) through tests/me_search_oracle.c in {sec:.2f} s"}
+            extra = {"gpu": gpu, "config": cfg, "bit_depth": bd, "refs": nref, "pus_per_call": n, "window": f"+-{rad}", "flags": "FRAC|HADAMARD",
+                     "lambda": lam, "lambda_note": "floor(65536 sqrt(0.57 2^((QP - 12) / 3))) at QP 32", "signed_keys": signed}
+            if not signed:
+                extra["surface_route"] = surface_route(cucd, eng, descs, res, R, lam)
+            emit(row, "PU/s", n, k_s, w_s, algo, cpu, extra, p_s=p_s, h2d=int(h2d), d2h=int(d2h))
+        eng.close()
+
+
+def surface_route(cucd, eng, descs, res, R, lam):
+    """today's route to cucd_me_search's answer, timed once on the wall clock: cucd_me_sad_surface in chunks + numpy argmin of
+    sad + cost_2, cucd_me_subpel_cost at the argmin + numpy walk.  Checks that it gives the search's results."""
+    import me_search_util as msu
+    n = len(descs)
+    side = 2 * R + 1
+    xs = np.arange(-R, R + 1)
+    mv = np.zeros((n, 2), np.int64)
+    sad = np.zeros(n, np.int64)
+    preds = np.array([(d["pred_x"], d["pred_y"]) for d in descs], np.int64)
+    chunk = 4096
+    surf = np.zeros(chunk * side * side, np.uint32)
+    eng.pin_host_buffer(surf)
+    t_gpu = t_host = 0.0
+    t0 = time.perf_counter()
+    for c0 in range(0, n, chunk):
+        part = descs[c0:c0 + chunk]
+        arr, m, total = cucd.Engine.me_descs(part)
+        ta = time.perf_counter()
+        eng.me_sad_surface_raw(arr, m, surf[:total])
+        tb = time.perf_counter()
+        s = surf[:total].reshape(m, side, side).astype(np.uint64)
+        p = preds[c0:c0 + m]
+        bits = msu.np_bits(4 * xs[None, :] - p[:, :1])[:, None, :] + msu.np_bits(4 * xs[None, :] - p[:, 1:])[:, :, None]
+        cost = ((np.uint64(lam) * bits.astype(np.uint64)) & np.uint64(0xFFFFFFFF)) >> np.uint64(16)
+        k = np.argmin((s + cost).reshape(m, -1), axis=1)
+        mv[c0:c0 + m, 0] = k % side - R
+        mv[c0:c0 + m, 1] = k // side - R
+        sad[c0:c0 + m] = s.reshape(m, -1)[np.arange(m), k].astype(np.int64)
+        t_gpu += tb - ta
+        t_host += time.perf_counter() - tb
+    eng.unpin_host_buffer(surf)
+    sp = [dict(x=d["x"], y=d["y"], w=d["w"], h=d["h"], ref_idx=d["ref_idx"], mvx=int(m_[0]), mvy=int(m_[1]), use_hadamard=1) for d, m_ in zip(descs, mv)]
+    ta = time.perf_counter()
+    arr, m = cucd.Engine.subpel_descs(sp)
+    T = np.zeros((m, 49), np.uint32)
+    eng.me_subpel_cost_raw(arr, m, T)
+    tb = time.perf_counter()
+    qmv, fc = msu.walk_batch(T, mv, preds, lam)
+    t1 = time.perf_counter()
+    t_gpu += tb - ta
+    t_host += t1 - tb
+    want = np.concatenate([mv, sad[:, None], qmv, fc[:, None]], axis=1)
+    same = bool(np.array_equal(msu.as_rows(res), want))
+    return {"wall_ms": (t1 - t0) * 1e3, "gpu_calls_ms": t_gpu * 1e3, "host_argmin_walk_ms": t_host * 1e3, "d2h_bytes": int(n * side * side * 4 + n * 49 * 4),
+            "h2d_bytes": int(n * 40 + n * 32), "round_trips": 2, "results_equal": same}
 
 
 if __name__ == "__main__":

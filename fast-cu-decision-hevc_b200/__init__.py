@@ -20,6 +20,9 @@ from .binding import (  # noqa: F401
     PACKED_CTU_BYTES,
     PUS_PER_CTU,
     RmdQueue,
+    SEARCH_FRAC,
+    SEARCH_HADAMARD,
+    SEARCH_RESULT,
     TU_INTRA_SLICE,
     TU_SIGN_HIDING,
     declared_symbols,

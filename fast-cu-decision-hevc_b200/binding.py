@@ -91,6 +91,16 @@ class _SubpelDesc(C.Structure):
     _fields_ = [(n, C.c_int) for n in ("x", "y", "w", "h", "ref_idx", "mvx", "mvy", "use_hadamard")]
 
 
+class _SearchDesc(C.Structure):
+    _fields_ = [(n, C.c_int) for n in ("x", "y", "w", "h", "ref_idx", "left", "right", "top", "bottom", "sub_shift", "pred_x", "pred_y")] + \
+               [("lambda_", C.c_uint32), ("flags", C.c_int)]
+
+
+SEARCH_FRAC, SEARCH_HADAMARD = 1, 2       # cucd_search_desc.flags
+# cucd_search_result: integer MV and its SAD, final quarter-pel MV and the cost of the quarter stage's best
+SEARCH_RESULT = np.dtype([("mvx", np.int32), ("mvy", np.int32), ("sad", np.uint32), ("qmvx", np.int32), ("qmvy", np.int32), ("frac_cost", np.uint32)])
+
+
 class _McDesc(C.Structure):
     _fields_ = [("x", C.c_int), ("y", C.c_int), ("w", C.c_int), ("h", C.c_int), ("ref_idx", C.c_int * 2), ("mvx", C.c_int * 2), ("mvy", C.c_int * 2),
                 ("use_hadamard", C.c_int)]
@@ -154,6 +164,8 @@ def load_library():
     lib.cucd_me_subpel_cost.argtypes = [C.c_void_p, C.c_int, C.POINTER(_SubpelDesc), C.c_void_p]
     lib.cucd_me_sad_surface_src.argtypes = [C.c_void_p, C.c_int, C.POINTER(_MeDesc), C.c_void_p, C.c_void_p]
     lib.cucd_me_subpel_cost_src.argtypes = [C.c_void_p, C.c_int, C.POINTER(_SubpelDesc), C.c_void_p, C.c_void_p]
+    lib.cucd_me_search.argtypes = [C.c_void_p, C.c_int, C.POINTER(_SearchDesc), C.c_void_p]
+    lib.cucd_me_search_src.argtypes = [C.c_void_p, C.c_int, C.POINTER(_SearchDesc), C.c_void_p, C.c_void_p]
     lib.cucd_me_mc_cost.argtypes = [C.c_void_p, C.c_int, C.POINTER(_McDesc), C.c_void_p, C.c_void_p]
     lib.cucd_set_ref_picture_chroma.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int]
     lib.cucd_set_cur_picture_chroma.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]
@@ -489,6 +501,35 @@ class Engine:
             src = np.ascontiguousarray(src, np.int16)
             assert src.size == sum(int(d["w"]) * int(d["h"]) for d in descs)
             self._check(self.lib.cucd_me_subpel_cost_src(self.h, n, arr, src.ctypes.data, out.ctypes.data), "cucd_me_subpel_cost_src")
+        return out
+
+    @staticmethod
+    def search_descs(descs):
+        """list of dicts(x,y,w,h,ref_idx,left,right,top,bottom,sub_shift,pred_x,pred_y,lambda,flags) -> (ctypes array, n): build once, reuse"""
+        arr = (_SearchDesc * max(len(descs), 1))()
+        for i, d in enumerate(descs):
+            for k in ("x", "y", "w", "h", "ref_idx", "left", "right", "top", "bottom", "sub_shift", "pred_x", "pred_y", "flags"):
+                setattr(arr[i], k, int(d[k]))
+            arr[i].lambda_ = int(d["lambda"]) & 0xFFFFFFFF
+        return arr, len(descs)
+
+    def me_search_raw(self, arr, n, out, src=None):
+        """cucd_me_search (cucd_me_search_src when src is given) with a prebuilt descriptor array; out: SEARCH_RESULT host array of n"""
+        if src is None:
+            self._check(self.lib.cucd_me_search(self.h, n, arr, out.ctypes.data), "cucd_me_search")
+        else:
+            self._check(self.lib.cucd_me_search_src(self.h, n, arr, src.ctypes.data, out.ctypes.data), "cucd_me_search_src")
+
+    def me_search(self, descs, src=None):
+        """descs: list of dicts(x,y,w,h,ref_idx,left,right,top,bottom,sub_shift,pred_x,pred_y,lambda,flags). Returns a SEARCH_RESULT
+        structured array (mvx, mvy, sad, qmvx, qmvy, frac_cost) with one record per PU.
+        src: optional int16 array with the PUs' own w x h source blocks back to back (cucd_me_search_src: bi-predictive search)."""
+        arr, n = self.search_descs(descs)
+        out = np.zeros(n, SEARCH_RESULT)
+        if src is not None:
+            src = np.ascontiguousarray(src, np.int16)
+            assert src.size == sum(int(d["w"]) * int(d["h"]) for d in descs)
+        self.me_search_raw(arr, n, out, src)
         return out
 
     @staticmethod

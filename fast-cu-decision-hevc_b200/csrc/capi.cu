@@ -247,6 +247,7 @@ int cucd_destroy(cucd_handle* h) {
   for (int i = 0; i < cucd_handle::kTimeRing; i++) { if (h->evRmd0[i]) cudaEventDestroy(h->evRmd0[i]); if (h->evRmd1[i]) cudaEventDestroy(h->evRmd1[i]); }
   for (int i = 0; i < cucd_handle::kGroups; i++) { if (h->evUpG[i]) cudaEventDestroy(h->evUpG[i]); if (h->evRmdG[i]) cudaEventDestroy(h->evRmdG[i]); }
   h->hDevScratch.release(); h->dDevStage.release();
+  h->hSearch.release(); h->dSearch.release();
   if (h->evDevUp) cudaEventDestroy(h->evDevUp);
   if (h->evDevDone) cudaEventDestroy(h->evDevDone);
   h->dNeeded.release();

@@ -605,6 +605,89 @@ int cucd_dev_me_subpel_cost(cucd_handle* h, void* stream, int nPU, const cucd_su
 }
 
 // ------------------------------------------------------------------------------------------------
+// Motion search: xPatternSearch without a surface (the Argmin form of the SAD kernels), then the refinement walk of the FRAC PUs
+// over sub-pel tables that stay on the device (me_core.cuh, me_search_*)
+// ------------------------------------------------------------------------------------------------
+static_assert(sizeof(cucd_search_result) == sizeof(MeSearchOut), "cucd_search_result is MeSearchOut");
+static int me_search_impl(cucd_handle* h, int nPU, const cucd_search_desc* desc, const int16_t* src, cucd_search_result* out) {
+  const bool own = src != nullptr;
+  if (!own && !h->curSet) return fail(h, CUCD_ERR_INVALID, "cucd_me_search: cucd_set_cur_picture not called");
+  CK(cudaSetDevice(h->cfg.device));
+  std::vector<cucd_me_desc> md(nPU);
+  int nFrac = 0;
+  for (int i = 0; i < nPU; i++) {
+    const cucd_search_desc& d = desc[i];
+    if (d.flags & ~(CUCD_SEARCH_FRAC | CUCD_SEARCH_HADAMARD)) return fail(h, CUCD_ERR_INVALID, "cucd_me_search: unknown flags");
+    if (d.pred_x < -32768 || d.pred_x > 32767 || d.pred_y < -32768 || d.pred_y > 32767) return fail(h, CUCD_ERR_INVALID, "cucd_me_search: predictor outside the int16 range");
+    md[i] = cucd_me_desc{d.x, d.y, d.w, d.h, d.ref_idx, d.left, d.right, d.top, d.bottom, d.sub_shift};
+    nFrac += (d.flags & CUCD_SEARCH_FRAC) ? 1 : 0;
+  }
+  size_t jobBytes, tileBytes, srcSamples = 0; long long total, nTilesDy, nTilesO;
+  const int rc = me_build_jobs(h, nPU, md.data(), h->hScratch, jobBytes, tileBytes, total, nTilesDy, nTilesO, own, &srcSamples);
+  if (rc != CUCD_OK) return rc;
+  const int W = h->cfg.width, H = h->cfg.height;
+  for (int i = 0; i < nPU; i++) {
+    const cucd_search_desc& d = desc[i];
+    if (!(d.flags & CUCD_SEARCH_FRAC)) continue;
+    const RefPlane& r = h->refs[d.ref_idx];
+    if (d.h & 3) return fail(h, CUCD_ERR_INVALID, "cucd_me_search: CUCD_SEARCH_FRAC needs h % 4 == 0");
+    if (d.x + d.left - 4 < -r.marginX || d.y + d.top - 4 < -r.marginY || d.x + d.right + d.w + 4 > W - 1 + r.marginX || d.y + d.bottom + d.h + 4 > H - 1 + r.marginY)
+      return fail(h, CUCD_ERR_INVALID, "cucd_me_search: the 8-tap support of the window leaves the padded reference picture");
+  }
+  // pinned records: [cost records | sub-pel jobs | FRAC list]; device scratch: [keys | completed sub-pel jobs | tables]
+  const size_t costBytes = up16((size_t)nPU * sizeof(MeSearchCost)), subBytes = up16((size_t)nFrac * sizeof(SubpelJob)), fracBytes = up16((size_t)nFrac * 4);
+  CK(h->hSearch.reserve(costBytes + subBytes + fracBytes));
+  MeSearchCost* cost = reinterpret_cast<MeSearchCost*>(h->hSearch.p);
+  SubpelJob* sub = reinterpret_cast<SubpelJob*>(h->hSearch.p + costBytes);
+  int32_t* fracJob = reinterpret_cast<int32_t*>(h->hSearch.p + costBytes + subBytes);
+  const MeJob* jobs = reinterpret_cast<const MeJob*>(h->hScratch.p);
+  for (int i = 0, f = 0; i < nPU; i++) {
+    const cucd_search_desc& d = desc[i];
+    const bool frac = (d.flags & CUCD_SEARCH_FRAC) != 0;
+    cost[i] = MeSearchCost{d.lambda, d.pred_x, d.pred_y, frac ? f : -1};
+    if (!frac) continue;
+    sub[f] = SubpelJob{jobs[i].curOff, jobs[i].refOff, d.ref_idx, (int16_t)d.w, (int16_t)d.h, (d.flags & CUCD_SEARCH_HADAMARD) ? 1 : 0};
+    fracJob[f++] = i;
+  }
+  const size_t keyBytes = up16((size_t)nPU * 8), tabBytes = up16((size_t)nFrac * CUCD_SUBPEL_POINTS * 4);
+  CK(h->dSearch.reserve(keyBytes + subBytes + tabBytes));
+  if (sync_ref_table(h) != CUCD_OK) return CUCD_ERR_CUDA;
+  BatchIo io(h);
+  const int iAll = io.add_in(h->hScratch.p, jobBytes + 2 * tileBytes, true);
+  const int iRec = io.add_in(h->hSearch.p, costBytes + subBytes + fracBytes, true);
+  const int iSrc = own ? io.add_in(src, srcSamples * sizeof(int16_t)) : -1;
+  const int oRes = io.add_out(out, (size_t)nPU * sizeof(cucd_search_result));
+  if (io.reserve() != CUCD_OK || io.upload(h->sMain) != CUCD_OK) return CUCD_ERR_CUDA;
+  MePlanes mp;
+  mp.cur = own ? io.din<int16_t>(iSrc) : h->dCur.p; mp.curStride = own ? 0 : h->curStride;
+  mp.ref = h->dRefPtr.p; mp.refStride = h->dRefStride.p; mp.bitDepth = h->cfg.bit_depth;
+  const uint8_t* dAll = io.din<uint8_t>(iAll);
+  const uint8_t* dRec = io.din<uint8_t>(iRec);
+  uint8_t* dS = h->dSearch.p;
+  if (!io.direct) CK(cudaEventRecord(h->evK0, h->sMain));
+  CK(launch_me_search(mp, reinterpret_cast<const MeJob*>(dAll), nPU, reinterpret_cast<const int32_t*>(dAll + jobBytes), reinterpret_cast<const int32_t*>(dAll + jobBytes + tileBytes),
+                      (int)nTilesDy, (int)nTilesO, reinterpret_cast<const MeSearchCost*>(dRec), reinterpret_cast<unsigned long long*>(dS),
+                      reinterpret_cast<const SubpelJob*>(dRec + costBytes), reinterpret_cast<SubpelJob*>(dS + keyBytes), reinterpret_cast<const int32_t*>(dRec + costBytes + subBytes),
+                      nFrac, reinterpret_cast<uint32_t*>(dS + keyBytes + subBytes), io.dout<MeSearchOut>(oRes), h->sMain, &h->launches));
+  if (!io.direct) { CK(cudaEventRecord(h->evK1, h->sMain)); h->kTimed = true; } else h->kTimed = false;
+  if (io.download(h->sMain) != CUCD_OK) return CUCD_ERR_CUDA;
+  flush_launches(h);
+  return CUCD_OK;
+}
+int cucd_me_search(cucd_handle* h, int nPU, const cucd_search_desc* desc, cucd_search_result* out) {
+  if (!h || nPU < 0 || (nPU > 0 && (!desc || !out))) return fail(h, CUCD_ERR_INVALID, "cucd_me_search: bad argument");
+  if (nPU == 0) return CUCD_OK;
+  LOCK(h);
+  return me_search_impl(h, nPU, desc, nullptr, out);
+}
+int cucd_me_search_src(cucd_handle* h, int nPU, const cucd_search_desc* desc, const int16_t* src, cucd_search_result* out) {
+  if (!h || nPU < 0 || (nPU > 0 && (!desc || !src || !out))) return fail(h, CUCD_ERR_INVALID, "cucd_me_search_src: bad argument");
+  if (nPU == 0) return CUCD_OK;
+  LOCK(h);
+  return me_search_impl(h, nPU, desc, src, out);
+}
+
+// ------------------------------------------------------------------------------------------------
 // Motion compensation and distortion of inter candidates (uni- and bi-predictive), me_core.cuh me_mc_*
 // ------------------------------------------------------------------------------------------------
 int cucd_me_mc_cost(cucd_handle* h, int nPU, const cucd_mc_desc* desc, uint32_t* dist, int16_t* pred) {

@@ -168,6 +168,9 @@ struct cucd_handle {
   cucd::DevBuf<int16_t> dCurC; int curStrideC = 0; bool curCSet = false;      // Cb plane, then Cr at curStrideC * (height / 2)
   // job records of the device-resident ME calls (cucd_dev_me_*): their own pinned / device blocks, guarded by events
   cucd::PinBuf<uint8_t> hDevScratch; cucd::DevBuf<uint8_t> dDevStage;
+  // cucd_me_search: pinned records (cost records, sub-pel jobs, FRAC list) beside hScratch's ME jobs / tiles, and device scratch
+  // (keys, completed sub-pel jobs, 49-entry tables)
+  cucd::PinBuf<uint8_t> hSearch; cucd::DevBuf<uint8_t> dSearch;
   cudaEvent_t evDevUp = nullptr, evDevDone = nullptr; bool devBusy = false;
 };
 

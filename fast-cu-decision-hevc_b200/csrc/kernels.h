@@ -134,5 +134,13 @@ cudaError_t launch_me_mc_chroma(const McChromaPlanes& cp, const McJob* jobs, con
                                 int* launches);
 cudaError_t launch_me_sad(const MePlanes& mp, const MeJob* jobs, int nJobs, const int32_t* tileJob, const int32_t* tileIdx, int nTilesDy, int nTilesO,
                           uint32_t* out, cudaStream_t st, int* launches);
+// motion search (me_core.cuh, MeSearchCost / MeSearchOut): the job and tile records of launch_me_sad plus a cost record per job; keys[nJobs]
+// device scratch; subIn the host-filled sub-pel jobs of the FRAC PUs (refOff at the PU origin), completed into subDev (device scratch);
+// fracJob[f] the job of sub-pel job f; tables[nFrac][49] device scratch; out[nJobs] the results
+struct MeSearchCost;
+struct MeSearchOut;
+cudaError_t launch_me_search(const MePlanes& mp, const MeJob* jobs, int nJobs, const int32_t* tileJob, const int32_t* tileIdx, int nTilesDy, int nTilesO,
+                             const MeSearchCost* cost, unsigned long long* keys, const SubpelJob* subIn, SubpelJob* subDev, const int32_t* fracJob, int nFrac,
+                             uint32_t* tables, MeSearchOut* out, cudaStream_t st, int* launches);
 
 }  // namespace cucd

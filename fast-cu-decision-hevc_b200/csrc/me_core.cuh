@@ -631,4 +631,112 @@ CUCD_HD void me_mcc_sse(int tid, const McGeo& g, const int16_t* sCur, const int1
   }
 }
 
+// =============================================================================================================================
+// Motion search (cucd_me_search): HM's full search xPatternSearch (TEncSearch.cpp:3886-3943) and the refinement walk of
+// xPatternSearchFracDIF / xPatternRefinement (:4340-4376, :808-865) on top of the SAD surface and sub-pel table arithmetic.
+//   integer  the SAD kernels in their Argmin form: a candidate becomes the key ((sad + cost_2(mv)) << 32) | (dy * cols + dx), a
+//            warp keeps the least key of its lanes (64-bit shuffles) and one atomicMin per warp folds it into keys[job].  The least
+//            key is HM's first strict minimum in raster order (mvy outer, mvx inner); sad + cost < 2^23 + 2^16 never wraps.
+//   prep     one thread per PU: decodes the key, writes (mv, sad) and completes the PU's sub-pel job (FRAC).
+//   walk     one thread per FRAC PU: HM's 9-point half stage, then the 9-point quarter stage, over the 49-entry table.
+// B(v) = xGetComponentBits, cost_s(x, y) = (uint32)(lambda * (B((x << s) - predX) + B((y << s) - predY))) >> 16: the 32-bit product
+// wraps, as m_uiCost * getBits(x, y) >> 16 does in TComRdCost.
+// =============================================================================================================================
+constexpr unsigned long long kMeNoKey = ~0ull;
+struct MeSearchCost {
+  uint32_t lambda;     // m_uiCost = floor(65536 sqrt(lambda))
+  int32_t predX, predY;  // m_mvPredictor in quarter pels
+  int32_t frac;        // index of the PU's sub-pel job, -1 without CUCD_SEARCH_FRAC
+};
+struct MeArgmin { const MeSearchCost* cost; unsigned long long* keys; };   // the Argmin epilogue's inputs (null in the Surface form)
+struct MeSearchOut { int32_t mvx, mvy; uint32_t sad; int32_t qmvx, qmvy; uint32_t fracCost; };   // = cucd_search_result
+enum class MeOut { Surface, Argmin };
+
+CUCD_HD int me_clz(uint32_t v) {
+#if defined(__CUDA_ARCH__)
+  return __clz(v);
+#else
+  return __builtin_clz(v);
+#endif
+}
+CUCD_HD uint32_t me_mv_bits(int v) {                     // xGetComponentBits: 1 + 2 floor(log2 t), t = v <= 0 ? -2v + 1 : 2v
+  const uint32_t t = v <= 0 ? ((uint32_t)-v << 1) + 1u : (uint32_t)v << 1;
+  return 1u + 2u * (uint32_t)(31 - me_clz(t));
+}
+CUCD_HD uint32_t me_mv_cost(const MeSearchCost& c, int x, int y, int s) {
+  return (c.lambda * (me_mv_bits(x * (1 << s) - c.predX) + me_mv_bits(y * (1 << s) - c.predY))) >> 16;
+}
+// the key of candidate (dx, dy) of a cols-wide window whose top-left MV is (left, top)
+CUCD_HD unsigned long long me_search_key(uint32_t sad, int dx, int dy, int cols, int left, int top, const MeSearchCost& c) {
+  return ((unsigned long long)(sad + me_mv_cost(c, left + dx, top + dy, 2)) << 32) | (uint32_t)(dy * cols + dx);
+}
+CUCD_HD unsigned long long me_key_min(unsigned long long a, unsigned long long b) { return b < a ? b : a; }
+// least key of a dy-lane thread's K candidates dx = dx0 + SPW k, dy (sad[] as the dy-lane SAD runs leave them, before the output shifts)
+template <int K, int SPW>
+CUCD_HD unsigned long long me_dy_lane_key(const uint32_t* sad, int subShift, int shiftOut, bool valid, int dx0, int dy, int cols, int left, int top,
+                                          const MeSearchCost& c) {
+  if (!valid) return kMeNoKey;
+  // dx grows with i: the first strict minimum of sad + cost is the least key (32-bit compares keep the M tile's registers free)
+  const uint32_t costY = me_mv_bits((top + dy) * 4 - c.predY);
+  uint32_t best = 0xffffffffu;
+  int bi = 0;
+#pragma unroll
+  for (int i = 0; i < K; i++) {
+    const uint32_t v = ((sad[i] << subShift) >> shiftOut) + ((c.lambda * (me_mv_bits((left + dx0 + SPW * i) * 4 - c.predX) + costY)) >> 16);
+    if (i == 0 || v < best) { best = v; bi = i; }
+  }
+  return ((unsigned long long)best << 32) | (uint32_t)(dy * cols + dx0 + SPW * bi);
+}
+#if defined(__CUDACC__)
+// every lane of the warp takes part (lanes without a candidate bring kMeNoKey); lane 0 folds the warp's least key into *key
+__device__ __forceinline__ void me_key_warp_commit(unsigned long long k, int lane, unsigned long long* key) {
+#pragma unroll
+  for (int m = 16; m > 0; m >>= 1) k = me_key_min(k, __shfl_xor_sync(0xffffffffu, k, m));
+  if (lane == 0 && k != kMeNoKey) atomicMin(key, k);
+}
+#endif
+
+// prep, thread i < nPU: the integer result of PU i from its key; a FRAC PU's sub-pel job (pre-filled by the host with the PU origin
+// in refOff) moves to the integer MV.  Job = MeJob, Sub = SubpelJob (kernels.h)
+template <class Job, class Sub>
+CUCD_HD void me_search_prep(int i, const unsigned long long* keys, const Job* jobs, const MeSearchCost* costs, const int32_t* refStride,
+                            const Sub* subIn, Sub* subOut, MeSearchOut* out) {
+  const Job& j = jobs[i];
+  const MeSearchCost& c = costs[i];
+  const unsigned long long k = keys[i];
+  const int cols = j.right - j.left + 1;
+  const uint32_t idx = (uint32_t)k, dy = idx / (uint32_t)cols, dx = idx - dy * (uint32_t)cols;
+  const int mvx = j.left + (int)dx, mvy = j.top + (int)dy;
+  MeSearchOut o;
+  o.mvx = mvx; o.mvy = mvy; o.sad = (uint32_t)(k >> 32) - me_mv_cost(c, mvx, mvy, 2);
+  o.qmvx = 4 * mvx; o.qmvy = 4 * mvy; o.fracCost = 0;
+  out[i] = o;
+  if (c.frac >= 0) {
+    Sub sj = subIn[c.frac];
+    sj.refOff += mvy * refStride[sj.refSlot] + mvx;
+    subOut[c.frac] = sj;
+  }
+}
+
+// walk: HM's orders of the half stage (s_acMvRefineH) and of the quarter stage (s_acMvRefineQ); each stage starts from the largest
+// distortion and keeps the first strict minimum
+CUCD_HD void me_search_walk(const uint32_t* T /*49*/, const MeSearchCost& c, MeSearchOut& o) {
+  const int hx[9] = {0, 0, 0, -1, 1, -1, 1, -1, 1}, hy[9] = {0, -1, 1, 0, 0, -1, -1, 1, 1};
+  const int qx[9] = {0, 0, 0, -1, 1, -1, 1, -1, 1}, qy[9] = {0, -1, 1, -1, -1, 0, 0, 1, 1};
+  const int mvx = o.mvx, mvy = o.mvy;
+  uint32_t best = 0xffffffffu;
+  int bx = 0, by = 0;
+  for (int i = 0; i < 9; i++) {
+    const uint32_t d = T[(2 * hy[i] + 3) * 7 + 2 * hx[i] + 3] + me_mv_cost(c, 2 * mvx + hx[i], 2 * mvy + hy[i], 1);
+    if (d < best) { best = d; bx = hx[i]; by = hy[i]; }
+  }
+  best = 0xffffffffu;
+  int qbx = 0, qby = 0;
+  for (int i = 0; i < 9; i++) {
+    const uint32_t d = T[(2 * by + qy[i] + 3) * 7 + 2 * bx + qx[i] + 3] + me_mv_cost(c, 4 * mvx + 2 * bx + qx[i], 4 * mvy + 2 * by + qy[i], 0);
+    if (d < best) { best = d; qbx = qx[i]; qby = qy[i]; }
+  }
+  o.qmvx = 4 * mvx + 2 * bx + qbx; o.qmvy = 4 * mvy + 2 * by + qby; o.fracCost = best;
+}
+
 }  // namespace cucd

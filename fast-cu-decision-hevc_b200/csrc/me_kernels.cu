@@ -25,10 +25,12 @@ constexpr int kMeRefRows = 64 + kMeTileY;
 // SIGNED: the source blocks are caller-supplied and may hold any int16 (the bi-predictive search compares 2 * org - other prediction,
 // TEncSearch.cpp:3787-3797): |a - b| per half through the signed SIMD intrinsic instead of max - min of packed words, whose 32-bit
 // subtraction would borrow across the halves for negative samples.
-template <bool SIGNED>
+// OUT (all three SAD kernels): Surface stores every candidate's SAD at out[outOff + dy * cols + dx]; Argmin folds the candidates
+// of a warp into the least search key (me_core.cuh, me_search_key) and commits it to am.keys[job] instead.
+template <bool SIGNED, MeOut OUT = MeOut::Surface>
 __global__ void __launch_bounds__(256)
 me_sad_kernel(const MePlanes mp, const MeJob* __restrict__ jobs, const int32_t* __restrict__ tileJob, const int32_t* __restrict__ tileIdx,
-              uint32_t* __restrict__ out) {
+              uint32_t* __restrict__ out, const MeArgmin am) {
   __shared__ __align__(16) int16_t sCur[64 * 64];
   __shared__ __align__(16) int16_t sRef[kMeRefRows * kMeRefPitch];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -52,7 +54,7 @@ me_sad_kernel(const MePlanes mp, const MeJob* __restrict__ jobs, const int32_t* 
   __syncthreads();
 
   const int dx = dx0 + lane, dy = dy0 + warp;
-  if (dx >= cols || dy >= rows) return;
+  if (OUT == MeOut::Surface && (dx >= cols || dy >= rows)) return;   // Argmin: every lane joins the warp's key reduction
   const int step = 1 << job.subShift;
   const uint32_t* cw = reinterpret_cast<const uint32_t*>(sCur);
   const uint32_t* rw = reinterpret_cast<const uint32_t*>(sRef);
@@ -72,7 +74,12 @@ me_sad_kernel(const MePlanes mp, const MeJob* __restrict__ jobs, const int32_t* 
       prev = next;
     }
   }
-  out[job.outOff + (long long)dy * cols + dx] = ((uint32_t)acc << job.subShift) >> (mp.bitDepth - 8);
+  const uint32_t sad = ((uint32_t)acc << job.subShift) >> (mp.bitDepth - 8);
+  if constexpr (OUT == MeOut::Surface) out[job.outOff + (long long)dy * cols + dx] = sad;
+  else {
+    const int ji = tileJob[blockIdx.x];
+    me_key_warp_commit(dx < cols && dy < rows ? me_search_key(sad, dx, dy, cols, job.left, job.top, am.cost[ji]) : kMeNoKey, lane, am.keys + ji);
+  }
 }
 
 // 8-bit content: the same tile of candidates with samples staged as BYTES - four absolute differences and their accumulation are one
@@ -82,9 +89,10 @@ constexpr int kMe8Pitch = 64 + kMeTileX + 8;         // bytes per staged referen
 constexpr int kMe8TileY = 16;                        // candidate rows per CTA: a thread owns dy = warp and warp + 8 (they share the source loads)
 constexpr int kMe8RefRows = 64 + kMe8TileY;
 
+template <MeOut OUT = MeOut::Surface>
 __global__ void __launch_bounds__(256)
 me_sad_u8_kernel(const MePlanes mp, const MeJob* __restrict__ jobs, const int32_t* __restrict__ tileJob, const int32_t* __restrict__ tileIdx,
-                 uint32_t* __restrict__ out) {
+                 uint32_t* __restrict__ out, const MeArgmin am) {
   __shared__ __align__(16) uint8_t sCur[64 * 64];
   __shared__ __align__(16) uint8_t sRef[kMe8RefRows * kMe8Pitch];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -108,7 +116,7 @@ me_sad_u8_kernel(const MePlanes mp, const MeJob* __restrict__ jobs, const int32_
   __syncthreads();
 
   const int dx = dx0 + lane, dyA = dy0 + warp, dyB = dyA + 8;
-  if (dx >= cols || dyA >= rows) return;
+  if (OUT == MeOut::Surface && (dx >= cols || dyA >= rows)) return;
   const bool hasB = dyB < rows;
   const uint32_t* cw = reinterpret_cast<const uint32_t*>(sCur);
   const uint32_t* rw = reinterpret_cast<const uint32_t*>(sRef);
@@ -128,8 +136,16 @@ me_sad_u8_kernel(const MePlanes mp, const MeJob* __restrict__ jobs, const int32_
       pa = na; pb = nb;
     }
   }
-  out[job.outOff + (long long)dyA * cols + dx] = accA << job.subShift;               // bitDepth 8: no final shift
-  if (hasB) out[job.outOff + (long long)dyB * cols + dx] = accB << job.subShift;
+  if constexpr (OUT == MeOut::Surface) {
+    out[job.outOff + (long long)dyA * cols + dx] = accA << job.subShift;               // bitDepth 8: no final shift
+    if (hasB) out[job.outOff + (long long)dyB * cols + dx] = accB << job.subShift;
+  } else {
+    const int ji = tileJob[blockIdx.x];
+    const MeSearchCost& c = am.cost[ji];
+    const bool okA = dx < cols && dyA < rows, okB = okA && hasB;
+    const unsigned long long kA = okA ? me_search_key(accA << job.subShift, dx, dyA, cols, job.left, job.top, c) : kMeNoKey;
+    me_key_warp_commit(me_key_min(kA, okB ? me_search_key(accB << job.subShift, dx, dyB, cols, job.left, job.top, c) : kMeNoKey), lane, am.keys + ji);
+  }
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -139,10 +155,10 @@ me_sad_u8_kernel(const MePlanes mp, const MeJob* __restrict__ jobs, const int32_
 // candidate: 1 VABSDIFF4.U8.ACC + 3/8 of a load / permute instead of 3.5 instructions; per two 16-bit samples: VIMNMX.S16x2 + two
 // packed additions (sum c + sum r - 2 sum min) instead of 7.  Results leave through shared memory as 128-byte rows of the surface.
 // ---------------------------------------------------------------------------------------------------------------------
-template <bool U8>
+template <bool U8, MeOut OUT = MeOut::Surface>
 __global__ void __launch_bounds__(256)
 me_sad_dy_kernel(const MePlanes mp, const MeJob* __restrict__ jobs, const int32_t* __restrict__ tileJob, const int32_t* __restrict__ tileIdx,
-                 uint32_t* __restrict__ out) {
+                 uint32_t* __restrict__ out, const MeArgmin am) {
   constexpr int P = U8 ? kMeDyPitch8 : kMeDyPitch16, SPW = U8 ? 4 : 2;
   __shared__ __align__(16) uint32_t sCur[64 * 64 / SPW];
   __shared__ __align__(16) uint32_t sRef[kMeDyRows * P];
@@ -169,6 +185,14 @@ me_sad_dy_kernel(const MePlanes mp, const MeJob* __restrict__ jobs, const int32_
       if (U8) me_dy_sad_u8<kMeDyK>(sCur, sRef, w >> 2, h, step, lam, q.wbase, q.s, sad);
       else me_dy_sad_s16<kMeDyK>(sCur, sRef, w >> 1, h, step, lam, q.wbase, q.s, me_fold_rows(mp.bitDepth, w >> 1), sad);
     }
+    if constexpr (OUT == MeOut::Argmin) {                              // `work` is warp uniform
+      // the tile origin is read again here, not kept live across the SAD runs (no spill at 64 registers)
+      int k2, xr, yr;
+      me_tile_unpack(*(const volatile int32_t*)&tileIdx[blockIdx.x], k2, xr, yr);
+      if (work) me_key_warp_commit(me_dy_lane_key<kMeDyK, SPW>(sad, job.subShift, shiftOut, lam < tl.nLam, xr + q.delta0, yr + lam, cols, job.left, job.top,
+                                                              am.cost[tileJob[blockIdx.x]]), lane, am.keys + tileJob[blockIdx.x]);
+      return;
+    }
     __syncthreads();                                                   // the staged window is dead: its space carries the tile out
     if (work) {
 #pragma unroll
@@ -184,7 +208,12 @@ me_sad_dy_kernel(const MePlanes mp, const MeJob* __restrict__ jobs, const int32_
     uint32_t sad[1];
     if (U8) me_dy_sad_u8<1>(sCur, sRef, w >> 2, h, step, lam, q.wbase, q.s, sad);
     else me_dy_sad_s16<1>(sCur, sRef, w >> 1, h, step, lam, q.wbase, q.s, me_fold_rows(mp.bitDepth, w >> 1), sad);
-    if (lam < tl.nLam) out[job.outOff + (long long)(y0 + lam) * cols + x0 + q.delta0] = (sad[0] << job.subShift) >> shiftOut;
+    if constexpr (OUT == MeOut::Argmin) {
+      int k2, xr, yr;
+      me_tile_unpack(*(const volatile int32_t*)&tileIdx[blockIdx.x], k2, xr, yr);
+      me_key_warp_commit(me_dy_lane_key<1, SPW>(sad, job.subShift, shiftOut, lam < tl.nLam, xr + q.delta0, yr + lam, cols, job.left, job.top, am.cost[tileJob[blockIdx.x]]),
+                         lane, am.keys + tileJob[blockIdx.x]);
+    } else if (lam < tl.nLam) out[job.outOff + (long long)(y0 + lam) * cols + x0 + q.delta0] = (sad[0] << job.subShift) >> shiftOut;
   }
 }
 
@@ -438,22 +467,62 @@ cudaError_t launch_me_subpel(const MePlanes& mp, const SubpelJob* jobs, int nJob
 }
 
 // tile records: [0, nTilesDy) the dy-lane tiles (M, E), [nTilesDy, nTilesDy + nTilesO) the dx-lane tiles (O); the two launches write disjoint candidates
-cudaError_t launch_me_sad(const MePlanes& mp, const MeJob* jobs, int nJobs, const int32_t* tileJob, const int32_t* tileIdx, int nTilesDy, int nTilesO,
-                          uint32_t* out, cudaStream_t st, int* launches) {
-  (void)nJobs;
+template <MeOut OUT>
+static cudaError_t launch_sad_tiles(const MePlanes& mp, const MeJob* jobs, const int32_t* tileJob, const int32_t* tileIdx, int nTilesDy, int nTilesO, uint32_t* out,
+                                    const MeArgmin& am, cudaStream_t st, int* launches) {
   if (nTilesDy > 0) {
     if (mp.curStride == 0) return cudaErrorInvalidValue;                // dy-lane tiles need the picture-resident (unsigned) source
-    if (mp.bitDepth == 8) me_sad_dy_kernel<true><<<nTilesDy, 256, 0, st>>>(mp, jobs, tileJob, tileIdx, out);
-    else me_sad_dy_kernel<false><<<nTilesDy, 256, 0, st>>>(mp, jobs, tileJob, tileIdx, out);
+    if (mp.bitDepth == 8) me_sad_dy_kernel<true, OUT><<<nTilesDy, 256, 0, st>>>(mp, jobs, tileJob, tileIdx, out, am);
+    else me_sad_dy_kernel<false, OUT><<<nTilesDy, 256, 0, st>>>(mp, jobs, tileJob, tileIdx, out, am);
     if (launches) *launches += 1;
     const cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return e;
   }
   if (nTilesO <= 0) return cudaSuccess;
   tileJob += nTilesDy; tileIdx += nTilesDy;
-  if (mp.curStride == 0) me_sad_kernel<true><<<nTilesO, 256, 0, st>>>(mp, jobs, tileJob, tileIdx, out);     // caller-supplied (possibly signed) source blocks
-  else if (mp.bitDepth == 8) me_sad_u8_kernel<<<nTilesO, 256, 0, st>>>(mp, jobs, tileJob, tileIdx, out);
-  else me_sad_kernel<false><<<nTilesO, 256, 0, st>>>(mp, jobs, tileJob, tileIdx, out);
+  if (mp.curStride == 0) me_sad_kernel<true, OUT><<<nTilesO, 256, 0, st>>>(mp, jobs, tileJob, tileIdx, out, am);     // caller-supplied (possibly signed) source blocks
+  else if (mp.bitDepth == 8) me_sad_u8_kernel<OUT><<<nTilesO, 256, 0, st>>>(mp, jobs, tileJob, tileIdx, out, am);
+  else me_sad_kernel<false, OUT><<<nTilesO, 256, 0, st>>>(mp, jobs, tileJob, tileIdx, out, am);
+  if (launches) *launches += 1;
+  return cudaGetLastError();
+}
+cudaError_t launch_me_sad(const MePlanes& mp, const MeJob* jobs, int nJobs, const int32_t* tileJob, const int32_t* tileIdx, int nTilesDy, int nTilesO,
+                          uint32_t* out, cudaStream_t st, int* launches) {
+  (void)nJobs;
+  return launch_sad_tiles<MeOut::Surface>(mp, jobs, tileJob, tileIdx, nTilesDy, nTilesO, out, MeArgmin{nullptr, nullptr}, st, launches);
+}
+
+// cucd_me_search: keys (~0, then the Argmin SAD kernels) -> prep -> sub-pel tables of the FRAC PUs -> walk
+__global__ void __launch_bounds__(128)
+me_search_prep_kernel(const MePlanes mp, const MeJob* __restrict__ jobs, int nJobs, const MeSearchCost* __restrict__ cost, const unsigned long long* __restrict__ keys,
+                      const SubpelJob* __restrict__ subIn, SubpelJob* __restrict__ subOut, MeSearchOut* __restrict__ out) {
+  const int i = blockIdx.x * 128 + threadIdx.x;
+  if (i < nJobs) me_search_prep(i, keys, jobs, cost, mp.refStride, subIn, subOut, out);
+}
+__global__ void __launch_bounds__(128)
+me_search_walk_kernel(const int32_t* __restrict__ fracJob, int nFrac, const MeSearchCost* __restrict__ cost, const uint32_t* __restrict__ tables,
+                      MeSearchOut* __restrict__ out) {
+  const int f = blockIdx.x * 128 + threadIdx.x;
+  if (f >= nFrac) return;
+  const int i = fracJob[f];
+  MeSearchOut o = out[i];
+  me_search_walk(tables + (size_t)f * 49, cost[i], o);
+  out[i] = o;
+}
+
+cudaError_t launch_me_search(const MePlanes& mp, const MeJob* jobs, int nJobs, const int32_t* tileJob, const int32_t* tileIdx, int nTilesDy, int nTilesO,
+                             const MeSearchCost* cost, unsigned long long* keys, const SubpelJob* subIn, SubpelJob* subDev, const int32_t* fracJob, int nFrac,
+                             uint32_t* tables, MeSearchOut* out, cudaStream_t st, int* launches) {
+  if (nJobs <= 0) return cudaSuccess;
+  cudaError_t e = cudaMemsetAsync(keys, 0xff, (size_t)nJobs * sizeof(unsigned long long), st);
+  if (e != cudaSuccess) return e;
+  e = launch_sad_tiles<MeOut::Argmin>(mp, jobs, tileJob, tileIdx, nTilesDy, nTilesO, nullptr, MeArgmin{cost, keys}, st, launches);
+  if (e != cudaSuccess) return e;
+  me_search_prep_kernel<<<(nJobs + 127) / 128, 128, 0, st>>>(mp, jobs, nJobs, cost, keys, subIn, subDev, out);
+  if (launches) *launches += 1;
+  if ((e = cudaGetLastError()) != cudaSuccess || nFrac <= 0) return e;
+  if ((e = launch_me_subpel(mp, subDev, nFrac, tables, st, launches)) != cudaSuccess) return e;
+  me_search_walk_kernel<<<(nFrac + 127) / 128, 128, 0, st>>>(fracJob, nFrac, cost, tables, out);
   if (launches) *launches += 1;
   return cudaGetLastError();
 }

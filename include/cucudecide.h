@@ -273,6 +273,49 @@ int cucd_me_sad_surface_src(cucd_handle* h, int nPU, const cucd_me_desc* desc, c
 int cucd_me_subpel_cost_src(cucd_handle* h, int nPU, const cucd_subpel_desc* desc, const int16_t* src, uint32_t* cost);
 
 /* ------------------------------------------------------------------------------------------------
+ * Motion search: HM's full integer search xPatternSearch (TEncSearch.cpp:3886-3943) and, with CUCD_SEARCH_FRAC, the refinement
+ * walk of xPatternSearchFracDIF / xPatternRefinement (:4340-4376, :808-865) around its result, one motion vector per PU and
+ * reference in one call: what xMotionEstimation runs when !m_iFastSearch || bBi.  Nothing but the result leaves the GPU.
+ *   B(v) = xGetComponentBits(v): t = v <= 0 ? (-v << 1) + 1 : v << 1, B = 1 + 2 floor(log2 t).
+ *   cost_s(x, y) = (uint32_t)(lambda * (B((x << s) - pred_x) + B((y << s) - pred_y))) >> 16, the product a wrapping 32-bit
+ *     unsigned product, as m_uiCost * getBits(x, y) >> 16.
+ *   Integer stage: mvy = top..bottom (outer), mvx = left..right (inner), c = SAD(mv) + cost_2(mv) with SAD the cucd_me_sad_surface
+ *     entry; the first strict minimum gives (mvx, mvy) and sad = its SAD.
+ *   FRAC: T = the 49-entry cucd_me_subpel_cost table at (mvx, mvy), use_hadamard = CUCD_SEARCH_HADAMARD.
+ *     H = (0,0),(0,-1),(0,1),(-1,0),(1,0),(-1,-1),(1,-1),(-1,1),(1,1)   (s_acMvRefineH)
+ *     Q = (0,0),(0,-1),(0,1),(-1,-1),(1,-1),(-1,0),(1,0),(-1,1),(1,1)   (s_acMvRefineQ)
+ *     half stage:    d_i = T[(2 H_i.y + 3) * 7 + 2 H_i.x + 3] + cost_1(2 mv + H_i); the first strict minimum gives hb
+ *     quarter stage: d_i = T[(2 hb.y + Q_i.y + 3) * 7 + 2 hb.x + Q_i.x + 3] + cost_0(4 mv + 2 hb + Q_i); the first strict minimum
+ *                    gives qb and frac_cost; qmv = 4 mv + 2 hb + qb.
+ * These orders and formulas restate HM-16.3; they could not be checked against the HM sources in this repository (the encoder
+ * proof checks them where the reference build exists).
+ * Rejected with CUCD_ERR_INVALID (the handle stays usable): whatever cucd_me_sad_surface rejects, unknown flags, a pred component
+ * outside [-2^15, 2^15 - 1], nPU < 0, NULL pointers; with CUCD_SEARCH_FRAC also h % 4 != 0 and a window whose 8-tap support can
+ * leave the padded plane: x + left - 4 < -marginX, x + right + w + 4 > W - 1 + marginX, and the same vertically (HM's clipMv keeps
+ * every legal window inside).  A 1x1 window refines a given integer MV.  nPU == 0 is a no-op.
+ * cucd_me_search_src takes the PUs' own w x h source blocks back to back (any int16), as cucd_me_sad_surface_src.
+ * ---------------------------------------------------------------------------------------------- */
+typedef struct {
+  int x, y, w, h;                /* PU, as cucd_me_desc */
+  int ref_idx;                   /* cucd_set_ref_picture slot */
+  int left, right, top, bottom;  /* inclusive integer window = cMvSrchRngLT / RB after xSetSearchRange (already clipped, >> 2) */
+  int sub_shift;                 /* integer stage iSubShift, as cucd_me_desc */
+  int pred_x, pred_y;            /* m_mvPredictor in quarter pels (TComRdCost::setPredictor), each in [-2^15, 2^15 - 1] */
+  uint32_t lambda;               /* m_uiCost after getMotionCost(true, 0, ..) = (UInt)floor(65536.0 * sqrtLambda) */
+  int flags;                     /* CUCD_SEARCH_FRAC | CUCD_SEARCH_HADAMARD */
+} cucd_search_desc;
+#define CUCD_SEARCH_FRAC     1     /* run xPatternSearchFracDIF's walk around the integer result */
+#define CUCD_SEARCH_HADAMARD 2     /* sub-pel DistFunc = xGetHADs (getUseHADME() && !lossless), else xGetSAD */
+typedef struct {
+  int32_t mvx, mvy;              /* integer result of xPatternSearch (integer pels) */
+  uint32_t sad;                  /* ruiSAD = the DistFunc value at (mvx, mvy) */
+  int32_t qmvx, qmvy;            /* final MV in quarter pels: 4 mv + 2 half + quarter (FRAC), else 4 mv */
+  uint32_t frac_cost;            /* FRAC: ruiCost of xPatternSearchFracDIF (distortion + mv cost of the quarter stage's best), else 0 */
+} cucd_search_result;
+int cucd_me_search(cucd_handle* h, int nPU, const cucd_search_desc* desc, cucd_search_result* out);
+int cucd_me_search_src(cucd_handle* h, int nPU, const cucd_search_desc* desc, const int16_t* src, cucd_search_result* out);
+
+/* ------------------------------------------------------------------------------------------------
  * Intra luma TU coding (SURVEY.md 8f.2): the arithmetic of TEncSearch::xIntraCodingTUBlock (TEncSearch.cpp:1092-1387) for a
  * batch of luma TUs with caller-supplied borders, packed like S2: org holds the N*N source blocks back to back, border
  * the 4N+1 unfiltered reference arrays; coef / level / pred / reco use the layout of org (N*N per TU, row-major; coefficient
@@ -424,7 +467,7 @@ int cucd_set_rmd_path(cucd_handle* h, int path);
  * the number of calls averaged, or a negative status; *avg_ms = mean duration of one launch. */
 int cucd_rmd_kernel_time(cucd_handle* h, int nCalls, float* avg_ms);
 /* Device time between the first and the last kernel of the most recent batch call on this handle (cucd_intra_rmd_batch,
- * cucd_me_sad_surface, cucd_me_subpel_cost, cucd_me_mc_cost, cucd_me_mc_chroma, cucd_intra_tu_*, cucd_inter_tu_*, cucd_tmv_features, cucd_aq_activity): CUDA events on
+ * cucd_me_sad_surface, cucd_me_subpel_cost, cucd_me_search, cucd_me_mc_cost, cucd_me_mc_chroma, cucd_intra_tu_*, cucd_inter_tu_*, cucd_tmv_features, cucd_aq_activity): CUDA events on
  * the library's stream, host<->device
  * copies outside.  What bench_rows.py reports as the kernel-only figure of those paths. */
 int cucd_last_kernel_time(cucd_handle* h, float* ms);
