@@ -343,6 +343,14 @@ int cucd_queue_stats(cucd_queue* q, long long* requests, long long* pus, long lo
 // ------------------------------------------------------------------------------------------------
 // S3: integer ME SAD surfaces
 // ------------------------------------------------------------------------------------------------
+// The kernels of the device-resident ME calls (cucd_dev_me_*) may still be queued on the caller's stream; they read dCur, the
+// reference planes and the reference table.  Each such call makes its stream wait for the previous one (dev_records_begin), so
+// the last evDevDone covers all of them: sMain waits for it before it overwrites any of the three.
+static int wait_dev_me(cucd_handle* h) {
+  if (h->devBusy) CK(cudaStreamWaitEvent(h->sMain, h->evDevDone, 0));
+  return CUCD_OK;
+}
+
 int cucd_set_ref_picture(cucd_handle* h, int ref_idx, const int16_t* recY, int stride, int marginX, int marginY) {
   if (!h || ref_idx < 0 || ref_idx >= 64 || !recY || marginX < 0 || marginY < 0 || stride < h->cfg.width + 2 * marginX)
     return fail(h, CUCD_ERR_INVALID, "cucd_set_ref_picture: bad argument");
@@ -350,6 +358,7 @@ int cucd_set_ref_picture(cucd_handle* h, int ref_idx, const int16_t* recY, int s
   // the slot's chroma belongs to the picture being replaced: unset it before anything can fail
   if ((int)h->refCb.size() > ref_idx) h->refCb[ref_idx].set = false;
   CK(cudaSetDevice(h->cfg.device));
+  if (wait_dev_me(h) != CUCD_OK) return CUCD_ERR_CUDA;
   if ((int)h->refs.size() <= ref_idx) h->refs.resize(ref_idx + 1);
   RefPlane& r = h->refs[ref_idx];
   const int pw = h->cfg.width + 2 * marginX, ph = h->cfg.height + 2 * marginY;
@@ -359,6 +368,7 @@ int cucd_set_ref_picture(cucd_handle* h, int ref_idx, const int16_t* recY, int s
   if (h->cfg.auto_pin_host) pin_host_range(h, first, ((size_t)(ph - 1) * stride + pw) * 2);
   CK(cudaMemcpy2DAsync(r.buf.p, (size_t)pitch * 2, first, (size_t)stride * 2, (size_t)pw * 2, ph, cudaMemcpyHostToDevice, h->sMain));
   CK(cudaStreamSynchronize(h->sMain));
+  h->devBusy = false;                              // sMain waited for the queued device-resident ME work: it has finished
   r.stride = pitch; r.marginX = marginX; r.marginY = marginY; r.set = true;
   h->refTableDirty = true;
   return CUCD_OK;
@@ -369,10 +379,12 @@ int cucd_set_cur_picture(cucd_handle* h, const int16_t* orgY, int stride) {
   LOCK(h);
   h->curCSet = false;                              // likewise the current chroma
   CK(cudaSetDevice(h->cfg.device));
+  if (wait_dev_me(h) != CUCD_OK) return CUCD_ERR_CUDA;
   CK(h->dCur.reserve(h->planeSamples));
   if (h->cfg.auto_pin_host) pin_host_range(h, orgY, ((size_t)(h->cfg.height - 1) * stride + h->cfg.width) * 2);
   CK(cudaMemcpy2DAsync(h->dCur.p, (size_t)h->pitch * 2, orgY, (size_t)stride * 2, (size_t)h->cfg.width * 2, h->cfg.height, cudaMemcpyHostToDevice, h->sMain));
   CK(cudaStreamSynchronize(h->sMain));
+  h->devBusy = false;
   h->curStride = h->pitch; h->curSet = true;
   return CUCD_OK;
 }
@@ -380,6 +392,7 @@ int cucd_set_cur_picture(cucd_handle* h, const int16_t* orgY, int stride) {
 // the device-side table of resident reference planes changes only when a plane is (re)allocated: upload it then, not per call
 static int sync_ref_table(cucd_handle* h) {
   if (!h->refTableDirty) return CUCD_OK;
+  if (wait_dev_me(h) != CUCD_OK) return CUCD_ERR_CUDA;
   std::vector<const int16_t*> refPtr(h->refs.size(), nullptr);
   std::vector<int32_t> refStride(h->refs.size(), 0);
   for (size_t i = 0; i < h->refs.size(); i++) { refPtr[i] = h->refs[i].buf.p; refStride[i] = h->refs[i].stride; }
@@ -489,8 +502,9 @@ int cucd_me_sad_surface_src(cucd_handle* h, int nPU, const cucd_me_desc* desc, c
 // Device-resident variants: the surfaces / cost tables stay in HBM (d_out), everything is enqueued on `stream` and the call does
 // not wait for the GPU.  The job records travel through buffers of their own, guarded by an event, so that back-to-back calls on
 // one stream pipeline and a host-buffer call in between cannot overwrite records a queued kernel still has to read.
+// devBusy stays set: should this call be rejected, the work of the previous one may still be queued (wait_dev_me).
 static int dev_records_begin(cucd_handle* h, cudaStream_t st) {
-  if (h->devBusy) { CK(cudaEventSynchronize(h->evDevUp)); CK(cudaStreamWaitEvent(st, h->evDevDone, 0)); h->devBusy = false; }
+  if (h->devBusy) { CK(cudaEventSynchronize(h->evDevUp)); CK(cudaStreamWaitEvent(st, h->evDevDone, 0)); }
   return CUCD_OK;
 }
 int cucd_dev_me_sad_surface(cucd_handle* h, void* stream, int nPU, const cucd_me_desc* desc, uint32_t* d_sad) {

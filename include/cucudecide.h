@@ -445,7 +445,9 @@ int cucd_dev_frames(cucd_handle* h, void* stream, int nPics, const int16_t* d_or
                     const int16_t* d_rec, long long recPicStride, int recStride, const cucd_dev_out* out, double* yc_host);
 /* S3 and the fractional-pel refinement with the results left in HBM: d_sad / d_cost are device pointers laid out like sadOut /
  * cost of cucd_me_sad_surface / cucd_me_subpel_cost (pictures through cucd_set_cur_picture / cucd_set_ref_picture as there); the
- * descriptors are host memory and are consumed before the call returns.  Enqueued on `stream`, no wait for the GPU. */
+ * descriptors are host memory and are consumed before the call returns.  Enqueued on `stream`, no wait for the GPU.
+ * cucd_set_cur_picture / cucd_set_ref_picture wait for the device-resident ME work still queued before they replace a plane, so a
+ * caller may upload the next picture right after enqueueing these calls: the queued work sees the pictures it was enqueued with. */
 int cucd_dev_me_sad_surface(cucd_handle* h, void* stream, int nPU, const cucd_me_desc* desc, uint32_t* d_sad);
 int cucd_dev_me_subpel_cost(cucd_handle* h, void* stream, int nPU, const cucd_subpel_desc* desc, uint32_t* d_cost);
 /* The host fit sits between the two feature passes; the split form lets a caller overlap it with GPU work of its own
