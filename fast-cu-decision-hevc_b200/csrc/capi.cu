@@ -321,7 +321,7 @@ int cucd_rmd_kernel_time(cucd_handle* h, int nCalls, float* avg_ms) {
 int cucd_last_kernel_time(cucd_handle* h, float* ms) {
   if (!h || !ms) return fail(h, CUCD_ERR_INVALID, "cucd_last_kernel_time: bad argument");
   LOCK(h);
-  if (!h->kTimed) return fail(h, CUCD_ERR_INVALID, "cucd_last_kernel_time: no batch call yet");
+  if (!h->kTimed) return fail(h, CUCD_ERR_INVALID, "cucd_last_kernel_time: the last batch call was not timed (there was none, or it was small enough for the zero-copy path)");
   CK(cudaEventElapsedTime(ms, h->evK0, h->evK1));
   return CUCD_OK;
 }

@@ -37,12 +37,14 @@ bool host_pinned(cucd_handle* h, const void* p, size_t bytes) {
 // Requests of a live encoder are tiny (one PU: ~1 KB in, 140 B out; one 128 x 128 SAD tile: 64 KB out) and latency bound: two DMA
 // copies, two timing events and a blocking stream wait cost several times the kernel.  Below `directLimit` bytes the kernels read
 // their inputs from and write their results to page-locked HOST memory directly (zero copy over PCIe, unified addressing) and the
-// call polls one event: a host memcpy each way, the launches, one cudaEventRecord.  CUCD_DIRECT_LIMIT=<bytes> (0 = off).
+// call polls one event: a host memcpy each way, the launches, one cudaEventRecord.  Such calls are therefore not timed
+// (cucd_last_kernel_time).  CUCD_DIRECT_LIMIT=<bytes> (0 = off).
 inline size_t direct_limit() {
   static const size_t v = [] { const char* e = getenv("CUCD_DIRECT_LIMIT"); return e ? (size_t)strtoull(e, nullptr, 10) : (size_t)96 << 10; }();
   return v;
 }
 
+// A host-buffer call: add its arrays, begin(), launch its kernels on the same stream, finish().
 struct BatchIo {
   struct Part { const void* src; void* dst; size_t bytes, off; bool pinned; };
   cucd_handle* h;
@@ -55,64 +57,61 @@ struct BatchIo {
   int add_out(void* dst, size_t bytes) { out[nOut] = Part{nullptr, dst, dst ? bytes : 0, outBytes, false}; outBytes += up16(dst ? bytes : 0); return nOut++; }
   // device-side room for an array the kernels produce but the caller did not ask for
   int add_scratch_out(size_t bytes) { out[nOut] = Part{nullptr, nullptr, 0, outBytes, false}; outBytes += up16(bytes); return nOut++; }
-  int reserve() {
+  template <class T> T* din(int i) const { return reinterpret_cast<T*>((direct ? h->hStage.p : h->bStage.p) + in[i].off); }
+  template <class T> T* dout(int i) const { return reinterpret_cast<T*>((direct ? h->hStageOut.p : reinterpret_cast<uint8_t*>(h->bOut.p)) + out[i].off); }
+  // choose the direct or the staged path and put the inputs where din() points; a staged call then records evK0
+  int begin(cudaStream_t st) {
     direct = inBytes + outBytes <= direct_limit() && inBytes + 256 <= kStageLimit && outBytes + 256 <= kStageLimit;
     if (direct) {
       CK(h->hStage.reserve(kStageLimit)); CK(h->hStageOut.reserve(kStageLimit));
       if (!h->evDirect) CK(cudaEventCreateWithFlags(&h->evDirect, cudaEventDisableTiming));
+      for (int i = 0; i < nIn; i++) if (in[i].bytes) memcpy(h->hStage.p + in[i].off, in[i].src, in[i].bytes);
       return CUCD_OK;
     }
     CK(h->bStage.reserve(inBytes + 256));
     CK(h->bOut.reserve(outBytes / 4 + 64));
-    return CUCD_OK;
-  }
-  template <class T> T* din(int i) const { return reinterpret_cast<T*>((direct ? h->hStage.p : h->bStage.p) + in[i].off); }
-  template <class T> T* dout(int i) const { return reinterpret_cast<T*>((direct ? h->hStageOut.p : reinterpret_cast<uint8_t*>(h->bOut.p)) + out[i].off); }
-  int upload(cudaStream_t st) {
-    if (direct) {
-      for (int i = 0; i < nIn; i++) if (in[i].bytes) memcpy(h->hStage.p + in[i].off, in[i].src, in[i].bytes);
-      return CUCD_OK;
-    }
     bool allPinned = true;
     for (int i = 0; i < nIn; i++) allPinned = allPinned && in[i].pinned;
     if (inBytes <= kStageLimit && !allPinned) {
       CK(h->hStage.reserve(kStageLimit));
       for (int i = 0; i < nIn; i++) if (in[i].bytes) memcpy(h->hStage.p + in[i].off, in[i].src, in[i].bytes);
       CK(cudaMemcpyAsync(h->bStage.p, h->hStage.p, inBytes, cudaMemcpyHostToDevice, st));
-      return CUCD_OK;
+    } else {
+      for (int i = 0; i < nIn; i++) {
+        if (!in[i].bytes) continue;
+        if (!in[i].pinned && in[i].bytes >= (64u << 10)) host_pinned(h, in[i].src, in[i].bytes);    // registers the range when auto_pin_host is set
+        CK(cudaMemcpyAsync(h->bStage.p + in[i].off, in[i].src, in[i].bytes, cudaMemcpyHostToDevice, st));
+      }
     }
-    for (int i = 0; i < nIn; i++) {
-      if (!in[i].bytes) continue;
-      if (!in[i].pinned && in[i].bytes >= (64u << 10)) host_pinned(h, in[i].src, in[i].bytes);    // registers the range when auto_pin_host is set
-      CK(cudaMemcpyAsync(h->bStage.p + in[i].off, in[i].src, in[i].bytes, cudaMemcpyHostToDevice, st));
-    }
+    CK(cudaEventRecord(h->evK0, st));
     return CUCD_OK;
   }
-  // enqueue the copies back, wait for the stream, hand the results to the caller
-  int download(cudaStream_t st) {
+  // after the launches: record evK1 (staged calls only), wait for the stream, hand the results to the caller
+  int finish(cudaStream_t st) {
+    if (!direct) CK(cudaEventRecord(h->evK1, st));
+    h->kTimed = !direct;
     if (direct) {
       CK(cudaEventRecord(h->evDirect, st));
       cudaError_t e;
       while ((e = cudaEventQuery(h->evDirect)) == cudaErrorNotReady) { }
       CK(e);
       for (int i = 0; i < nOut; i++) if (out[i].bytes) memcpy(out[i].dst, h->hStageOut.p + out[i].off, out[i].bytes);
-      return CUCD_OK;
-    }
-    size_t wanted = 0;
-    for (int i = 0; i < nOut; i++) wanted += out[i].bytes;
-    if (outBytes <= kStageLimit) {
+    } else if (outBytes <= kStageLimit) {
+      size_t wanted = 0;
+      for (int i = 0; i < nOut; i++) wanted += out[i].bytes;
       CK(h->hStageOut.reserve(kStageLimit));
       if (wanted) CK(cudaMemcpyAsync(h->hStageOut.p, h->bOut.p, outBytes, cudaMemcpyDeviceToHost, st));
       CK(cudaStreamSynchronize(st));
       for (int i = 0; i < nOut; i++) if (out[i].bytes) memcpy(out[i].dst, h->hStageOut.p + out[i].off, out[i].bytes);
-      return CUCD_OK;
+    } else {
+      for (int i = 0; i < nOut; i++) {
+        if (!out[i].bytes) continue;
+        if (out[i].bytes >= (64u << 10)) host_pinned(h, out[i].dst, out[i].bytes);
+        CK(cudaMemcpyAsync(out[i].dst, reinterpret_cast<uint8_t*>(h->bOut.p) + out[i].off, out[i].bytes, cudaMemcpyDeviceToHost, st));
+      }
+      CK(cudaStreamSynchronize(st));
     }
-    for (int i = 0; i < nOut; i++) {
-      if (!out[i].bytes) continue;
-      if (out[i].bytes >= (64u << 10)) host_pinned(h, out[i].dst, out[i].bytes);
-      CK(cudaMemcpyAsync(out[i].dst, reinterpret_cast<uint8_t*>(h->bOut.p) + out[i].off, out[i].bytes, cudaMemcpyDeviceToHost, st));
-    }
-    CK(cudaStreamSynchronize(st));
+    flush_launches(h);
     return CUCD_OK;
   }
 };
@@ -140,9 +139,7 @@ int rmd_batch_core(cucd_handle* h, int nPU, const cucd_pu_desc* desc, const int3
   const int iPus = io.add_in(pus, (size_t)nPU * sizeof(BatchPu), true);
   io.inBytes += 256;                                  // the kernels read whole 16-byte words past the last block
   const int oSad = io.add_out(sad, (size_t)nPU * kNumModes * sizeof(uint32_t));
-  if (io.reserve() != CUCD_OK) return CUCD_ERR_CUDA;
-  if (io.upload(h->sMain) != CUCD_OK) return CUCD_ERR_CUDA;
-  if (!io.direct) CK(cudaEventRecord(h->evK0, h->sMain));
+  if (io.begin(h->sMain) != CUCD_OK) return CUCD_ERR_CUDA;
   for (int l = 6; l >= 2; l--) {
     if (!count[l]) continue;
     BatchSource bs;
@@ -156,10 +153,7 @@ int rmd_batch_core(cucd_handle* h, int nPU, const cucd_pu_desc* desc, const int3
     else
       CK(launch_rmd_batch(l, bs, h->cfg.bit_depth, h->cfg.strong_intra_smoothing, h->sMain, &h->launches));
   }
-  if (!io.direct) { CK(cudaEventRecord(h->evK1, h->sMain)); h->kTimed = true; } else h->kTimed = false;
-  if (io.download(h->sMain) != CUCD_OK) return CUCD_ERR_CUDA;
-  flush_launches(h);
-  return CUCD_OK;
+  return io.finish(h->sMain);
 }
 
 // offsets of back-to-back packed PUs (the layout of the public batch calls); false on a bad size or an overflowing batch
@@ -175,6 +169,42 @@ bool packed_offsets(int n, const uint8_t* log2s, int stride, int lo, int hi, std
   }
   return true;
 }
+
+// the reference plane of slot `idx` of `v`, or null when there is no such slot or it has not been set
+const RefPlane* ref_slot(const std::vector<RefPlane>& v, int idx) {
+  return idx >= 0 && idx < (int)v.size() && v[idx].set ? &v[idx] : nullptr;
+}
+
+// samples [x0, x1] x [y0, y1] of a W x H picture lie inside r's padded plane
+bool inside_padded(const RefPlane& r, int W, int H, int x0, int y0, int x1, int y1) {
+  return x0 >= -r.marginX && y0 >= -r.marginY && x1 <= W - 1 + r.marginX && y1 <= H - 1 + r.marginY;
+}
+
+// HM's PU shapes (AMP 12 / 24 / 48 included): w and h multiples of 4 in 4..64, inside the W x H picture
+template <class D> bool pu_shape_ok(const D& d, int W, int H) {
+  return d.w >= 4 && d.h >= 4 && d.w <= 64 && d.h <= 64 && !(d.w & 3) && !(d.h & 3) && d.x >= 0 && d.y >= 0 && d.x + d.w <= W && d.y + d.h <= H;
+}
+
+// the planes the ME kernels read: the caller's packed source blocks (stride 0) or, when ownSrc is null, the resident current picture
+MePlanes me_planes(const cucd_handle* h, const int16_t* ownSrc) {
+  MePlanes mp;
+  mp.cur = ownSrc ? ownSrc : h->dCur.p; mp.curStride = ownSrc ? 0 : h->curStride;
+  mp.ref = h->dRefPtr.p; mp.refStride = h->dRefStride.p; mp.bitDepth = h->cfg.bit_depth;
+  return mp;
+}
+
+// The record block of an ME batch, as me_build_jobs lays it out in pinned scratch and the calls copy it to the device:
+// [MeJob per PU | tileJob | tileIdx], each part 16-byte aligned.  Tile records (me_core.cuh): the dy-lane tiles of every PU
+// first, then the dx-lane tiles; nTilesDy / nTilesO count them.
+struct MeRecords {
+  size_t jobBytes = 0, tileBytes = 0;
+  long long total = 0, nTilesDy = 0, nTilesO = 0;   // total: SAD surface entries of the batch
+  size_t srcSamples = 0;                             // samples of the caller's packed source blocks (cucd_me_*_src)
+  size_t bytes() const { return jobBytes + 2 * tileBytes; }
+  MeJob* jobs(uint8_t* base) const { return reinterpret_cast<MeJob*>(base); }
+  int32_t* tileJob(uint8_t* base) const { return reinterpret_cast<int32_t*>(base + jobBytes); }
+  int32_t* tileIdx(uint8_t* base) const { return reinterpret_cast<int32_t*>(base + jobBytes + tileBytes); }
+};
 
 }  // namespace
 
@@ -404,38 +434,36 @@ static int sync_ref_table(cucd_handle* h) {
   return CUCD_OK;
 }
 
-// validate the PUs, build job + tile records into `scratch` (pinned); returns the sizes through the references
+// validate the PUs, build job + tile records into `scratch` (pinned) and describe them in `rec`
 // ownBlocks: the source blocks are the caller's (cucd_me_sad_surface_src): offsets run through the packed block array
-// Tile records (me_core.cuh): the dy-lane tiles of every PU first, then the dx-lane tiles; nTilesDy / nTilesO count them.
-static int me_build_jobs(cucd_handle* h, int nPU, const cucd_me_desc* desc, PinBuf<uint8_t>& scratch, size_t& jobBytes, size_t& tileBytes, long long& total, long long& nTilesDy,
-                         long long& nTilesO, bool ownBlocks = false, size_t* srcSamples = nullptr) {
+static int me_build_jobs(cucd_handle* h, int nPU, const cucd_me_desc* desc, PinBuf<uint8_t>& scratch, MeRecords& rec, bool ownBlocks = false) {
   const int W = h->cfg.width, H = h->cfg.height;
   const int tileRows = (h->cfg.bit_depth == 8 && !ownBlocks) ? 16 : 8;     // me_sad_u8_kernel covers 32 x 16 candidates per CTA, me_sad_kernel 32 x 8
   const bool fast = !ownBlocks;                                            // caller-supplied blocks may hold signed samples: dx-lane kernel only
-  total = 0; nTilesDy = 0; nTilesO = 0;
+  rec = MeRecords();
   for (int i = 0; i < nPU; i++) {
     const cucd_me_desc& d = desc[i];
     // HM's PU widths are multiples of 4 (4..64, AMP 12 / 24 / 48 included); the 8-bit kernel reads the source as 32-bit words
     if (d.w < 4 || d.h < 4 || d.w > 64 || d.h > 64 || (d.w & 3) || d.x < 0 || d.y < 0 || d.x + d.w > W || d.y + d.h > H || d.left > d.right || d.top > d.bottom ||
         d.sub_shift < 0 || d.sub_shift > 4)
       return fail(h, CUCD_ERR_INVALID, "cucd_me_sad_surface: bad PU / window (width must be a multiple of 4)");
-    if (d.ref_idx < 0 || d.ref_idx >= (int)h->refs.size() || !h->refs[d.ref_idx].set) return fail(h, CUCD_ERR_INVALID, "cucd_me_sad_surface: reference picture not set");
-    const RefPlane& r = h->refs[d.ref_idx];
-    if (d.x + d.left < -r.marginX || d.y + d.top < -r.marginY || d.x + d.w - 1 + d.right > W - 1 + r.marginX || d.y + d.h - 1 + d.bottom > H - 1 + r.marginY)
+    const RefPlane* r = ref_slot(h->refs, d.ref_idx);
+    if (!r) return fail(h, CUCD_ERR_INVALID, "cucd_me_sad_surface: reference picture not set");
+    if (!inside_padded(*r, W, H, d.x + d.left, d.y + d.top, d.x + d.w - 1 + d.right, d.y + d.h - 1 + d.bottom))
       return fail(h, CUCD_ERR_INVALID, "cucd_me_sad_surface: window leaves the padded reference picture");
     const int cols = d.right - d.left + 1, rows = d.bottom - d.top + 1;
     if (cols > kMeMaxWindow || rows > kMeMaxWindow) return fail(h, CUCD_ERR_INVALID, "cucd_me_sad_surface: window too large");
-    me_enum_tiles(cols, rows, fast && me_width_is_hm(d.w), tileRows, [&](int kind, int, int) { if (kind == kMeKindO) nTilesO++; else nTilesDy++; });
-    total += (long long)cols * rows;
+    me_enum_tiles(cols, rows, fast && me_width_is_hm(d.w), tileRows, [&](int kind, int, int) { if (kind == kMeKindO) rec.nTilesO++; else rec.nTilesDy++; });
+    rec.total += (long long)cols * rows;
   }
-  const long long nTiles = nTilesDy + nTilesO;
+  const long long nTiles = rec.nTilesDy + rec.nTilesO;
   if (nTiles > 0x7fffffffll) return fail(h, CUCD_ERR_INVALID, "cucd_me_sad_surface: batch too large");
-  jobBytes = up16((size_t)nPU * sizeof(MeJob)); tileBytes = up16((size_t)nTiles * 4);
-  CK(scratch.reserve(jobBytes + 2 * tileBytes));
-  MeJob* jobs = reinterpret_cast<MeJob*>(scratch.p);
-  int32_t* tileJob = reinterpret_cast<int32_t*>(scratch.p + jobBytes);
-  int32_t* tileIdx = reinterpret_cast<int32_t*>(scratch.p + jobBytes + tileBytes);
-  long long off = 0; size_t ntDy = 0, ntO = (size_t)nTilesDy, blockOff = 0;
+  rec.jobBytes = up16((size_t)nPU * sizeof(MeJob)); rec.tileBytes = up16((size_t)nTiles * 4);
+  CK(scratch.reserve(rec.bytes()));
+  MeJob* jobs = rec.jobs(scratch.p);
+  int32_t* tileJob = rec.tileJob(scratch.p);
+  int32_t* tileIdx = rec.tileIdx(scratch.p);
+  long long off = 0; size_t ntDy = 0, ntO = (size_t)rec.nTilesDy, blockOff = 0;
   for (int i = 0; i < nPU; i++) {
     const cucd_me_desc& d = desc[i];
     const RefPlane& r = h->refs[d.ref_idx];
@@ -457,7 +485,7 @@ static int me_build_jobs(cucd_handle* h, int nPU, const cucd_me_desc* desc, PinB
     off += (long long)cols * rows;
   }
   if (blockOff > 0x7fffffffull) return fail(h, CUCD_ERR_INVALID, "cucd_me_sad_surface_src: batch too large");
-  if (srcSamples) *srcSamples = blockOff;
+  rec.srcSamples = blockOff;
   return CUCD_OK;
 }
 
@@ -465,26 +493,19 @@ static int me_sad_surface_impl(cucd_handle* h, int nPU, const cucd_me_desc* desc
   const bool own = src != nullptr;
   if (!own && !h->curSet) return fail(h, CUCD_ERR_INVALID, "cucd_me_sad_surface: cucd_set_cur_picture not called");
   CK(cudaSetDevice(h->cfg.device));
-  size_t jobBytes, tileBytes, srcSamples = 0; long long total, nTilesDy, nTilesO;
-  const int rc = me_build_jobs(h, nPU, desc, h->hScratch, jobBytes, tileBytes, total, nTilesDy, nTilesO, own, &srcSamples);
+  MeRecords rec;
+  const int rc = me_build_jobs(h, nPU, desc, h->hScratch, rec, own);
   if (rc != CUCD_OK) return rc;
   if (sync_ref_table(h) != CUCD_OK) return CUCD_ERR_CUDA;
   BatchIo io(h);
-  const int iAll = io.add_in(h->hScratch.p, jobBytes + 2 * tileBytes, true);
-  const int iSrc = own ? io.add_in(src, srcSamples * sizeof(int16_t)) : -1;
-  const int oSad = io.add_out(sadOut, (size_t)total * sizeof(uint32_t));
-  if (io.reserve() != CUCD_OK || io.upload(h->sMain) != CUCD_OK) return CUCD_ERR_CUDA;
-  MePlanes mp;
-  mp.cur = own ? io.din<int16_t>(iSrc) : h->dCur.p; mp.curStride = own ? 0 : h->curStride;
-  mp.ref = h->dRefPtr.p; mp.refStride = h->dRefStride.p; mp.bitDepth = h->cfg.bit_depth;
-  const uint8_t* dAll = io.din<uint8_t>(iAll);
-  if (!io.direct) CK(cudaEventRecord(h->evK0, h->sMain));
-  CK(launch_me_sad(mp, reinterpret_cast<const MeJob*>(dAll), nPU, reinterpret_cast<const int32_t*>(dAll + jobBytes), reinterpret_cast<const int32_t*>(dAll + jobBytes + tileBytes),
-                   (int)nTilesDy, (int)nTilesO, io.dout<uint32_t>(oSad), h->sMain, &h->launches));
-  if (!io.direct) { CK(cudaEventRecord(h->evK1, h->sMain)); h->kTimed = true; } else h->kTimed = false;
-  if (io.download(h->sMain) != CUCD_OK) return CUCD_ERR_CUDA;
-  flush_launches(h);
-  return CUCD_OK;
+  const int iAll = io.add_in(h->hScratch.p, rec.bytes(), true);
+  const int iSrc = own ? io.add_in(src, rec.srcSamples * sizeof(int16_t)) : -1;
+  const int oSad = io.add_out(sadOut, (size_t)rec.total * sizeof(uint32_t));
+  if (io.begin(h->sMain) != CUCD_OK) return CUCD_ERR_CUDA;
+  uint8_t* dAll = io.din<uint8_t>(iAll);
+  CK(launch_me_sad(me_planes(h, own ? io.din<int16_t>(iSrc) : nullptr), rec.jobs(dAll), nPU, rec.tileJob(dAll), rec.tileIdx(dAll), (int)rec.nTilesDy, (int)rec.nTilesO,
+                   io.dout<uint32_t>(oSad), h->sMain, &h->launches));
+  return io.finish(h->sMain);
 }
 int cucd_me_sad_surface(cucd_handle* h, int nPU, const cucd_me_desc* desc, uint32_t* sadOut) {
   if (!h || nPU < 0 || (nPU > 0 && (!desc || !sadOut))) return fail(h, CUCD_ERR_INVALID, "cucd_me_sad_surface: bad argument");
@@ -515,18 +536,15 @@ int cucd_dev_me_sad_surface(cucd_handle* h, void* stream, int nPU, const cucd_me
   CK(cudaSetDevice(h->cfg.device));
   cudaStream_t st = (cudaStream_t)stream;
   if (dev_records_begin(h, st) != CUCD_OK) return CUCD_ERR_CUDA;
-  size_t jobBytes, tileBytes; long long total, nTilesDy, nTilesO;
-  const int rc = me_build_jobs(h, nPU, desc, h->hDevScratch, jobBytes, tileBytes, total, nTilesDy, nTilesO);
+  MeRecords rec;
+  const int rc = me_build_jobs(h, nPU, desc, h->hDevScratch, rec);
   if (rc != CUCD_OK) return rc;
   if (sync_ref_table(h) != CUCD_OK) return CUCD_ERR_CUDA;
-  CK(h->dDevStage.reserve(jobBytes + 2 * tileBytes));
-  CK(cudaMemcpyAsync(h->dDevStage.p, h->hDevScratch.p, jobBytes + 2 * tileBytes, cudaMemcpyHostToDevice, st));
+  CK(h->dDevStage.reserve(rec.bytes()));
+  CK(cudaMemcpyAsync(h->dDevStage.p, h->hDevScratch.p, rec.bytes(), cudaMemcpyHostToDevice, st));
   CK(cudaEventRecord(h->evDevUp, st));
-  MePlanes mp;
-  mp.cur = h->dCur.p; mp.curStride = h->curStride; mp.ref = h->dRefPtr.p; mp.refStride = h->dRefStride.p; mp.bitDepth = h->cfg.bit_depth;
-  const uint8_t* dAll = h->dDevStage.p;
-  CK(launch_me_sad(mp, reinterpret_cast<const MeJob*>(dAll), nPU, reinterpret_cast<const int32_t*>(dAll + jobBytes), reinterpret_cast<const int32_t*>(dAll + jobBytes + tileBytes),
-                   (int)nTilesDy, (int)nTilesO, d_sad, st, &h->launches));
+  uint8_t* dAll = h->dDevStage.p;
+  CK(launch_me_sad(me_planes(h, nullptr), rec.jobs(dAll), nPU, rec.tileJob(dAll), rec.tileIdx(dAll), (int)rec.nTilesDy, (int)rec.nTilesO, d_sad, st, &h->launches));
   CK(cudaEventRecord(h->evDevDone, st)); h->devBusy = true;
   flush_launches(h);
   return CUCD_OK;
@@ -542,16 +560,15 @@ static int subpel_build_jobs(cucd_handle* h, int nPU, const cucd_subpel_desc* de
   SubpelJob* jobs = reinterpret_cast<SubpelJob*>(scratch.p);
   for (int i = 0; i < nPU; i++) {
     const cucd_subpel_desc& d = desc[i];
-    if (d.w < 4 || d.h < 4 || d.w > 64 || d.h > 64 || (d.w & 3) || (d.h & 3) || d.x < 0 || d.y < 0 || d.x + d.w > W || d.y + d.h > H)
-      return fail(h, CUCD_ERR_INVALID, "cucd_me_subpel_cost: bad PU");
-    if (d.ref_idx < 0 || d.ref_idx >= (int)h->refs.size() || !h->refs[d.ref_idx].set) return fail(h, CUCD_ERR_INVALID, "cucd_me_subpel_cost: reference picture not set");
-    const RefPlane& r = h->refs[d.ref_idx];
-    if (d.x + d.mvx - 4 < -r.marginX || d.y + d.mvy - 4 < -r.marginY || d.x + d.mvx + d.w + 4 > W - 1 + r.marginX || d.y + d.mvy + d.h + 4 > H - 1 + r.marginY)
+    if (!pu_shape_ok(d, W, H)) return fail(h, CUCD_ERR_INVALID, "cucd_me_subpel_cost: bad PU");
+    const RefPlane* r = ref_slot(h->refs, d.ref_idx);
+    if (!r) return fail(h, CUCD_ERR_INVALID, "cucd_me_subpel_cost: reference picture not set");
+    if (!inside_padded(*r, W, H, d.x + d.mvx - 4, d.y + d.mvy - 4, d.x + d.mvx + d.w + 4, d.y + d.mvy + d.h + 4))
       return fail(h, CUCD_ERR_INVALID, "cucd_me_subpel_cost: the interpolation support leaves the padded reference picture");
     SubpelJob& j = jobs[i];
     j.curOff = ownBlocks ? (int32_t)blockOff : d.y * h->curStride + d.x;
     blockOff += (size_t)d.w * d.h;
-    j.refOff = (d.y + d.mvy + r.marginY) * r.stride + d.x + d.mvx + r.marginX;
+    j.refOff = (d.y + d.mvy + r->marginY) * r->stride + d.x + d.mvx + r->marginX;
     j.refSlot = d.ref_idx; j.w = (int16_t)d.w; j.h = (int16_t)d.h; j.useHadamard = d.use_hadamard ? 1 : 0;
   }
   if (blockOff > 0x7fffffffull) return fail(h, CUCD_ERR_INVALID, "cucd_me_subpel_cost_src: batch too large");
@@ -571,16 +588,9 @@ static int me_subpel_cost_impl(cucd_handle* h, int nPU, const cucd_subpel_desc* 
   const int iJobs = io.add_in(h->hScratch.p, (size_t)nPU * sizeof(SubpelJob), true);
   const int iSrc = own ? io.add_in(src, srcSamples * sizeof(int16_t)) : -1;
   const int oCost = io.add_out(cost, (size_t)nPU * CUCD_SUBPEL_POINTS * sizeof(uint32_t));
-  if (io.reserve() != CUCD_OK || io.upload(h->sMain) != CUCD_OK) return CUCD_ERR_CUDA;
-  MePlanes mp;
-  mp.cur = own ? io.din<int16_t>(iSrc) : h->dCur.p; mp.curStride = own ? 0 : h->curStride;
-  mp.ref = h->dRefPtr.p; mp.refStride = h->dRefStride.p; mp.bitDepth = h->cfg.bit_depth;
-  if (!io.direct) CK(cudaEventRecord(h->evK0, h->sMain));
-  CK(launch_me_subpel(mp, io.din<SubpelJob>(iJobs), nPU, io.dout<uint32_t>(oCost), h->sMain, &h->launches));
-  if (!io.direct) { CK(cudaEventRecord(h->evK1, h->sMain)); h->kTimed = true; } else h->kTimed = false;
-  if (io.download(h->sMain) != CUCD_OK) return CUCD_ERR_CUDA;
-  flush_launches(h);
-  return CUCD_OK;
+  if (io.begin(h->sMain) != CUCD_OK) return CUCD_ERR_CUDA;
+  CK(launch_me_subpel(me_planes(h, own ? io.din<int16_t>(iSrc) : nullptr), io.din<SubpelJob>(iJobs), nPU, io.dout<uint32_t>(oCost), h->sMain, &h->launches));
+  return io.finish(h->sMain);
 }
 int cucd_me_subpel_cost(cucd_handle* h, int nPU, const cucd_subpel_desc* desc, uint32_t* cost) {
   if (!h || nPU < 0 || (nPU > 0 && (!desc || !cost))) return fail(h, CUCD_ERR_INVALID, "cucd_me_subpel_cost: bad argument");
@@ -610,9 +620,7 @@ int cucd_dev_me_subpel_cost(cucd_handle* h, void* stream, int nPU, const cucd_su
   CK(h->dDevStage.reserve(bytes));
   CK(cudaMemcpyAsync(h->dDevStage.p, h->hDevScratch.p, bytes, cudaMemcpyHostToDevice, st));
   CK(cudaEventRecord(h->evDevUp, st));
-  MePlanes mp;
-  mp.cur = h->dCur.p; mp.curStride = h->curStride; mp.ref = h->dRefPtr.p; mp.refStride = h->dRefStride.p; mp.bitDepth = h->cfg.bit_depth;
-  CK(launch_me_subpel(mp, reinterpret_cast<const SubpelJob*>(h->dDevStage.p), nPU, d_cost, st, &h->launches));
+  CK(launch_me_subpel(me_planes(h, nullptr), reinterpret_cast<const SubpelJob*>(h->dDevStage.p), nPU, d_cost, st, &h->launches));
   CK(cudaEventRecord(h->evDevDone, st)); h->devBusy = true;
   flush_launches(h);
   return CUCD_OK;
@@ -636,16 +644,15 @@ static int me_search_impl(cucd_handle* h, int nPU, const cucd_search_desc* desc,
     md[i] = cucd_me_desc{d.x, d.y, d.w, d.h, d.ref_idx, d.left, d.right, d.top, d.bottom, d.sub_shift};
     nFrac += (d.flags & CUCD_SEARCH_FRAC) ? 1 : 0;
   }
-  size_t jobBytes, tileBytes, srcSamples = 0; long long total, nTilesDy, nTilesO;
-  const int rc = me_build_jobs(h, nPU, md.data(), h->hScratch, jobBytes, tileBytes, total, nTilesDy, nTilesO, own, &srcSamples);
+  MeRecords rec;
+  const int rc = me_build_jobs(h, nPU, md.data(), h->hScratch, rec, own);
   if (rc != CUCD_OK) return rc;
   const int W = h->cfg.width, H = h->cfg.height;
   for (int i = 0; i < nPU; i++) {
     const cucd_search_desc& d = desc[i];
     if (!(d.flags & CUCD_SEARCH_FRAC)) continue;
-    const RefPlane& r = h->refs[d.ref_idx];
     if (d.h & 3) return fail(h, CUCD_ERR_INVALID, "cucd_me_search: CUCD_SEARCH_FRAC needs h % 4 == 0");
-    if (d.x + d.left - 4 < -r.marginX || d.y + d.top - 4 < -r.marginY || d.x + d.right + d.w + 4 > W - 1 + r.marginX || d.y + d.bottom + d.h + 4 > H - 1 + r.marginY)
+    if (!inside_padded(h->refs[d.ref_idx], W, H, d.x + d.left - 4, d.y + d.top - 4, d.x + d.right + d.w + 4, d.y + d.bottom + d.h + 4))
       return fail(h, CUCD_ERR_INVALID, "cucd_me_search: the 8-tap support of the window leaves the padded reference picture");
   }
   // pinned records: [cost records | sub-pel jobs | FRAC list]; device scratch: [keys | completed sub-pel jobs | tables]
@@ -654,7 +661,7 @@ static int me_search_impl(cucd_handle* h, int nPU, const cucd_search_desc* desc,
   MeSearchCost* cost = reinterpret_cast<MeSearchCost*>(h->hSearch.p);
   SubpelJob* sub = reinterpret_cast<SubpelJob*>(h->hSearch.p + costBytes);
   int32_t* fracJob = reinterpret_cast<int32_t*>(h->hSearch.p + costBytes + subBytes);
-  const MeJob* jobs = reinterpret_cast<const MeJob*>(h->hScratch.p);
+  const MeJob* jobs = rec.jobs(h->hScratch.p);
   for (int i = 0, f = 0; i < nPU; i++) {
     const cucd_search_desc& d = desc[i];
     const bool frac = (d.flags & CUCD_SEARCH_FRAC) != 0;
@@ -667,26 +674,19 @@ static int me_search_impl(cucd_handle* h, int nPU, const cucd_search_desc* desc,
   CK(h->dSearch.reserve(keyBytes + subBytes + tabBytes));
   if (sync_ref_table(h) != CUCD_OK) return CUCD_ERR_CUDA;
   BatchIo io(h);
-  const int iAll = io.add_in(h->hScratch.p, jobBytes + 2 * tileBytes, true);
+  const int iAll = io.add_in(h->hScratch.p, rec.bytes(), true);
   const int iRec = io.add_in(h->hSearch.p, costBytes + subBytes + fracBytes, true);
-  const int iSrc = own ? io.add_in(src, srcSamples * sizeof(int16_t)) : -1;
+  const int iSrc = own ? io.add_in(src, rec.srcSamples * sizeof(int16_t)) : -1;
   const int oRes = io.add_out(out, (size_t)nPU * sizeof(cucd_search_result));
-  if (io.reserve() != CUCD_OK || io.upload(h->sMain) != CUCD_OK) return CUCD_ERR_CUDA;
-  MePlanes mp;
-  mp.cur = own ? io.din<int16_t>(iSrc) : h->dCur.p; mp.curStride = own ? 0 : h->curStride;
-  mp.ref = h->dRefPtr.p; mp.refStride = h->dRefStride.p; mp.bitDepth = h->cfg.bit_depth;
-  const uint8_t* dAll = io.din<uint8_t>(iAll);
+  if (io.begin(h->sMain) != CUCD_OK) return CUCD_ERR_CUDA;
+  uint8_t* dAll = io.din<uint8_t>(iAll);
   const uint8_t* dRec = io.din<uint8_t>(iRec);
   uint8_t* dS = h->dSearch.p;
-  if (!io.direct) CK(cudaEventRecord(h->evK0, h->sMain));
-  CK(launch_me_search(mp, reinterpret_cast<const MeJob*>(dAll), nPU, reinterpret_cast<const int32_t*>(dAll + jobBytes), reinterpret_cast<const int32_t*>(dAll + jobBytes + tileBytes),
-                      (int)nTilesDy, (int)nTilesO, reinterpret_cast<const MeSearchCost*>(dRec), reinterpret_cast<unsigned long long*>(dS),
+  CK(launch_me_search(me_planes(h, own ? io.din<int16_t>(iSrc) : nullptr), rec.jobs(dAll), nPU, rec.tileJob(dAll), rec.tileIdx(dAll), (int)rec.nTilesDy, (int)rec.nTilesO,
+                      reinterpret_cast<const MeSearchCost*>(dRec), reinterpret_cast<unsigned long long*>(dS),
                       reinterpret_cast<const SubpelJob*>(dRec + costBytes), reinterpret_cast<SubpelJob*>(dS + keyBytes), reinterpret_cast<const int32_t*>(dRec + costBytes + subBytes),
                       nFrac, reinterpret_cast<uint32_t*>(dS + keyBytes + subBytes), io.dout<MeSearchOut>(oRes), h->sMain, &h->launches));
-  if (!io.direct) { CK(cudaEventRecord(h->evK1, h->sMain)); h->kTimed = true; } else h->kTimed = false;
-  if (io.download(h->sMain) != CUCD_OK) return CUCD_ERR_CUDA;
-  flush_launches(h);
-  return CUCD_OK;
+  return io.finish(h->sMain);
 }
 int cucd_me_search(cucd_handle* h, int nPU, const cucd_search_desc* desc, cucd_search_result* out) {
   if (!h || nPU < 0 || (nPU > 0 && (!desc || !out))) return fail(h, CUCD_ERR_INVALID, "cucd_me_search: bad argument");
@@ -716,17 +716,16 @@ int cucd_me_mc_cost(cucd_handle* h, int nPU, const cucd_mc_desc* desc, uint32_t*
   long long predOff = 0;
   for (int i = 0; i < nPU; i++) {
     const cucd_mc_desc& d = desc[i];
-    if (d.w < 4 || d.h < 4 || d.w > 64 || d.h > 64 || (d.w & 3) || (d.h & 3) || d.x < 0 || d.y < 0 || d.x + d.w > W || d.y + d.h > H)
-      return fail(h, CUCD_ERR_INVALID, "cucd_me_mc_cost: bad PU (w, h multiples of 4 in 4..64, inside the picture)");
+    if (!pu_shape_ok(d, W, H)) return fail(h, CUCD_ERR_INVALID, "cucd_me_mc_cost: bad PU (w, h multiples of 4 in 4..64, inside the picture)");
     int nl = 0, slot[2], mvx[2], mvy[2], stride[2], mX[2], mY[2];
     for (int l = 0; l < 2; l++) {
       if (d.ref_idx[l] < 0) continue;
-      if (d.ref_idx[l] >= (int)h->refs.size() || !h->refs[d.ref_idx[l]].set) return fail(h, CUCD_ERR_INVALID, "cucd_me_mc_cost: reference picture not set");
-      const RefPlane& r = h->refs[d.ref_idx[l]];
+      const RefPlane* r = ref_slot(h->refs, d.ref_idx[l]);
+      if (!r) return fail(h, CUCD_ERR_INVALID, "cucd_me_mc_cost: reference picture not set");
       const int ix = d.x + (d.mvx[l] >> 2), iy = d.y + (d.mvy[l] >> 2);
-      if (ix - 3 < -r.marginX || iy - 3 < -r.marginY || ix + d.w + 3 > W - 1 + r.marginX || iy + d.h + 3 > H - 1 + r.marginY)
+      if (!inside_padded(*r, W, H, ix - 3, iy - 3, ix + d.w + 3, iy + d.h + 3))
         return fail(h, CUCD_ERR_INVALID, "cucd_me_mc_cost: the interpolation support leaves the padded reference picture");
-      slot[nl] = d.ref_idx[l]; mvx[nl] = d.mvx[l]; mvy[nl] = d.mvy[l]; stride[nl] = r.stride; mX[nl] = r.marginX; mY[nl] = r.marginY; nl++;
+      slot[nl] = d.ref_idx[l]; mvx[nl] = d.mvx[l]; mvy[nl] = d.mvy[l]; stride[nl] = r->stride; mX[nl] = r->marginX; mY[nl] = r->marginY; nl++;
     }
     if (nl == 0) return fail(h, CUCD_ERR_INVALID, "cucd_me_mc_cost: a candidate uses neither list (ref_idx both < 0)");
     jobs[i] = me_mc_job(d.y * h->curStride + d.x, d.x, d.y, d.w, d.h, nl, slot, mvx, mvy, stride, mX, mY, d.use_hadamard, i, predOff);
@@ -742,17 +741,11 @@ int cucd_me_mc_cost(cucd_handle* h, int nPU, const cucd_mc_desc* desc, uint32_t*
   const int iAll = io.add_in(h->hScratch.p, jobBytes + ctaBytes, true);
   const int oDist = io.add_out(dist, (size_t)nPU * sizeof(uint32_t));
   const int oPred = io.add_out(pred, (size_t)predOff * sizeof(int16_t));
-  if (io.reserve() != CUCD_OK || io.upload(h->sMain) != CUCD_OK) return CUCD_ERR_CUDA;
-  MePlanes mp;
-  mp.cur = h->dCur.p; mp.curStride = h->curStride; mp.ref = h->dRefPtr.p; mp.refStride = h->dRefStride.p; mp.bitDepth = h->cfg.bit_depth;
+  if (io.begin(h->sMain) != CUCD_OK) return CUCD_ERR_CUDA;
   const uint8_t* dAll = io.din<uint8_t>(iAll);
-  if (!io.direct) CK(cudaEventRecord(h->evK0, h->sMain));
-  CK(launch_me_mc(mp, reinterpret_cast<const McJob*>(dAll), reinterpret_cast<const int32_t*>(dAll + jobBytes), nCta, io.dout<uint32_t>(oDist),
+  CK(launch_me_mc(me_planes(h, nullptr), reinterpret_cast<const McJob*>(dAll), reinterpret_cast<const int32_t*>(dAll + jobBytes), nCta, io.dout<uint32_t>(oDist),
                   pred ? io.dout<int16_t>(oPred) : nullptr, h->sMain, &h->launches));
-  if (!io.direct) { CK(cudaEventRecord(h->evK1, h->sMain)); h->kTimed = true; } else h->kTimed = false;
-  if (io.download(h->sMain) != CUCD_OK) return CUCD_ERR_CUDA;
-  flush_launches(h);
-  return CUCD_OK;
+  return io.finish(h->sMain);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -827,19 +820,17 @@ int cucd_me_mc_chroma(cucd_handle* h, int nPU, const cucd_mc_desc* desc, uint32_
   long long predOff = 0;
   for (int i = 0; i < nPU; i++) {
     const cucd_mc_desc& d = desc[i];
-    if (d.w < 4 || d.h < 4 || d.w > 64 || d.h > 64 || (d.w & 3) || (d.h & 3) || d.x < 0 || d.y < 0 || d.x + d.w > W || d.y + d.h > H)
-      return fail(h, CUCD_ERR_INVALID, "cucd_me_mc_chroma: bad PU (w, h multiples of 4 in 4..64, inside the picture)");
+    if (!pu_shape_ok(d, W, H)) return fail(h, CUCD_ERR_INVALID, "cucd_me_mc_chroma: bad PU (w, h multiples of 4 in 4..64, inside the picture)");
     const int cx = d.x >> 1, cy = d.y >> 1, cw = d.w >> 1, ch = d.h >> 1;
     int nl = 0, slot[2], mvx[2], mvy[2], stride[2], mX[2], mY[2];
     for (int l = 0; l < 2; l++) {
       if (d.ref_idx[l] < 0) continue;
-      if (d.ref_idx[l] >= (int)h->refCb.size() || !h->refCb[d.ref_idx[l]].set)
-        return fail(h, CUCD_ERR_INVALID, "cucd_me_mc_chroma: chroma of the reference picture not set (cucd_set_ref_picture_chroma after cucd_set_ref_picture)");
-      const RefPlane& r = h->refCb[d.ref_idx[l]];
+      const RefPlane* r = ref_slot(h->refCb, d.ref_idx[l]);
+      if (!r) return fail(h, CUCD_ERR_INVALID, "cucd_me_mc_chroma: chroma of the reference picture not set (cucd_set_ref_picture_chroma after cucd_set_ref_picture)");
       const int ix = cx + (d.mvx[l] >> 3), iy = cy + (d.mvy[l] >> 3);
-      if (ix - 1 < -r.marginX || iy - 1 < -r.marginY || ix + cw + 1 > Wc - 1 + r.marginX || iy + ch + 1 > Hc - 1 + r.marginY)
+      if (!inside_padded(*r, Wc, Hc, ix - 1, iy - 1, ix + cw + 1, iy + ch + 1))
         return fail(h, CUCD_ERR_INVALID, "cucd_me_mc_chroma: the interpolation support leaves the padded chroma plane");
-      slot[nl] = d.ref_idx[l]; mvx[nl] = d.mvx[l]; mvy[nl] = d.mvy[l]; stride[nl] = r.stride; mX[nl] = r.marginX; mY[nl] = r.marginY; nl++;
+      slot[nl] = d.ref_idx[l]; mvx[nl] = d.mvx[l]; mvy[nl] = d.mvy[l]; stride[nl] = r->stride; mX[nl] = r->marginX; mY[nl] = r->marginY; nl++;
     }
     if (nl == 0) return fail(h, CUCD_ERR_INVALID, "cucd_me_mc_chroma: a candidate uses neither list (ref_idx both < 0)");
     jobs[i] = me_mcc_job(cy * h->curStrideC + cx, cx, cy, cw, ch, nl, slot, mvx, mvy, stride, mX, mY, i, predOff);
@@ -855,18 +846,14 @@ int cucd_me_mc_chroma(cucd_handle* h, int nPU, const cucd_mc_desc* desc, uint32_
   const int iAll = io.add_in(h->hScratch.p, jobBytes + ctaBytes, true);
   const int oSse = io.add_out(sse, (size_t)nPU * 2 * sizeof(uint32_t));
   const int oPred = io.add_out(pred, (size_t)predOff * sizeof(int16_t));
-  if (io.reserve() != CUCD_OK || io.upload(h->sMain) != CUCD_OK) return CUCD_ERR_CUDA;
+  if (io.begin(h->sMain) != CUCD_OK) return CUCD_ERR_CUDA;
   McChromaPlanes cp;
   cp.cur[0] = h->dCurC.p; cp.cur[1] = h->dCurC.p + (size_t)h->curStrideC * Hc; cp.curStride = h->curStrideC;
   cp.ref = h->dRefPtrC.p; cp.refStride = h->dRefStrideC.p; cp.bitDepth = h->cfg.bit_depth;
   const uint8_t* dAll = io.din<uint8_t>(iAll);
-  if (!io.direct) CK(cudaEventRecord(h->evK0, h->sMain));
   CK(launch_me_mc_chroma(cp, reinterpret_cast<const McJob*>(dAll), reinterpret_cast<const int32_t*>(dAll + jobBytes), nCta, io.dout<uint32_t>(oSse),
                          pred ? io.dout<int16_t>(oPred) : nullptr, h->sMain, &h->launches));
-  if (!io.direct) { CK(cudaEventRecord(h->evK1, h->sMain)); h->kTimed = true; } else h->kTimed = false;
-  if (io.download(h->sMain) != CUCD_OK) return CUCD_ERR_CUDA;
-  flush_launches(h);
-  return CUCD_OK;
+  return io.finish(h->sMain);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -922,8 +909,7 @@ static int tu_batch(cucd_handle* h, const char* who, int stage, int flags, int n
   const int oDist = dist ? io.add_out(dist, (size_t)nTU * sizeof(uint32_t)) : io.add_scratch_out((size_t)nTU * sizeof(uint32_t));
   const int oAbs = absSum ? io.add_out(absSum, (size_t)nTU * sizeof(int32_t)) : io.add_scratch_out((size_t)nTU * sizeof(int32_t));
   const int oZero = distZero ? io.add_out(distZero, (size_t)nTU * sizeof(uint32_t)) : -1;
-  if (io.reserve() != CUCD_OK || io.upload(h->sMain) != CUCD_OK) return CUCD_ERR_CUDA;
-  CK(cudaEventRecord(h->evK0, h->sMain));
+  if (io.begin(h->sMain) != CUCD_OK) return CUCD_ERR_CUDA;
   for (int l = 5; l >= 2; l--) {
     if (!count[l]) continue;
     TuBatch tb;
@@ -937,10 +923,7 @@ static int tu_batch(cucd_handle* h, const char* who, int stage, int flags, int n
     tb.dist = io.dout<uint32_t>(oDist); tb.absSum = io.dout<int32_t>(oAbs);
     CK(launch_tu(l, tb, h->sMain, &h->launches));
   }
-  CK(cudaEventRecord(h->evK1, h->sMain)); h->kTimed = true;
-  if (io.download(h->sMain) != CUCD_OK) return CUCD_ERR_CUDA;
-  flush_launches(h);
-  return CUCD_OK;
+  return io.finish(h->sMain);
 }
 
 int cucd_intra_tu_forward(cucd_handle* h, int nTU, const cucd_tu_desc* desc, const int16_t* org, const int16_t* border, int32_t* coef, int16_t* pred) {
@@ -993,13 +976,9 @@ int cucd_tmv_features(cucd_handle* h, int nCU, const cucd_cu_desc* cus, double* 
   BatchIo io(h);
   const int iCus = io.add_in(v, (size_t)nCU * sizeof(TmvCu), true);
   const int oFeat = io.add_out(feat, (size_t)nCU * CUCD_TMV_FEATURES * sizeof(double));
-  if (io.reserve() != CUCD_OK || io.upload(h->sMain) != CUCD_OK) return CUCD_ERR_CUDA;
-  CK(cudaEventRecord(h->evK0, h->sMain));
+  if (io.begin(h->sMain) != CUCD_OK) return CUCD_ERR_CUDA;
   CK(launch_tmv_features(h->dCur.p, h->curStride, io.din<TmvCu>(iCus), nCU, io.dout<double>(oFeat), h->sMain, &h->launches));
-  CK(cudaEventRecord(h->evK1, h->sMain)); h->kTimed = true;
-  if (io.download(h->sMain) != CUCD_OK) return CUCD_ERR_CUDA;
-  flush_launches(h);
-  return CUCD_OK;
+  return io.finish(h->sMain);
 }
 
 int cucd_aq_activity(cucd_handle* h, int max_aq_depth, double* const* activity, double* avg_activity) {

@@ -471,7 +471,9 @@ int cucd_rmd_kernel_time(cucd_handle* h, int nCalls, float* avg_ms);
 /* Device time between the first and the last kernel of the most recent batch call on this handle (cucd_intra_rmd_batch,
  * cucd_me_sad_surface, cucd_me_subpel_cost, cucd_me_search, cucd_me_mc_cost, cucd_me_mc_chroma, cucd_intra_tu_*, cucd_inter_tu_*, cucd_tmv_features, cucd_aq_activity): CUDA events on
  * the library's stream, host<->device
- * copies outside.  What bench_rows.py reports as the kernel-only figure of those paths. */
+ * copies outside.  What bench_rows.py reports as the kernel-only figure of those paths.  A call small enough for the
+ * zero-copy path (its kernels read and write page-locked host memory; CUCD_DIRECT_LIMIT bytes, 96 KB by default) is not
+ * timed: after one, this call fails with CUCD_ERR_INVALID. */
 int cucd_last_kernel_time(cucd_handle* h, float* ms);
 /* the host-side fit that sits between the two passes (TEncSlice.cpp:291-392): hist = 16*4096 counts
  * of ONE picture, nBlocks = (W/4)*(H/4); writes yc[16] and thr[16] */
