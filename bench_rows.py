@@ -16,7 +16,8 @@ a12 (cucd_tmv_features), a13 (cucd_aq_activity), f2 (cucd_intra_tu_code / _forwa
 Last rows: f5 (cucd_me_mc_cost, motion compensation + distortion of inter candidates; row_f5 runs it on its own), f6
 (cucd_inter_tu_forward / _code / _recon, the TUs of inter residual quadtrees; row_f6) and f7 (cucd_me_mc_chroma, the 4:2:0 chroma of
 f5's candidates; row_f7) and f8 (cucd_me_search / _src, the motion search of bench.py's inter workloads against the surface route it
-replaces; row_f8).  --only f5 / f6 / f7 / f8 runs one of them alone.
+replaces; row_f8) and f9 (cucd_me_tz_search, the TZ search of the same workloads, depth by depth; row_f9).  --only f5 / f6 / f7 / f8 / f9
+runs one of them alone.
 """
 import argparse
 import ctypes as C
@@ -94,11 +95,11 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--iters", type=int, default=5)
     ap.add_argument("--cpu-threads", type=int, default=min(16, os.cpu_count() or 1))
-    ap.add_argument("--only", choices=["f5", "f6", "f7", "f8"], default=None, help="run one of the last rows alone")
+    ap.add_argument("--only", choices=["f5", "f6", "f7", "f8", "f9"], default=None, help="run one of the last rows alone")
     a = ap.parse_args()
     cucd = importlib.import_module("fast-cu-decision-hevc_b200")
     if a.only:
-        {"f5": row_f5, "f6": row_f6, "f7": row_f7, "f8": row_f8}[a.only](cucd, a.iters, a.cpu_threads)
+        {"f5": row_f5, "f6": row_f6, "f7": row_f7, "f8": row_f8, "f9": row_f9}[a.only](cucd, a.iters, a.cpu_threads)
         return
     oracle = _util.load_oracle()
     ref = _util.load_hmref()
@@ -264,6 +265,7 @@ def main():
     row_f6(cucd, a.iters, T)
     row_f7(cucd, a.iters, T)
     row_f8(cucd, a.iters, T)
+    row_f9(cucd, a.iters, T)
 
 
 def gpu_identity():
@@ -566,6 +568,176 @@ def surface_route(cucd, eng, descs, res, R, lam):
     same = bool(np.array_equal(msu.as_rows(res), want))
     return {"wall_ms": (t1 - t0) * 1e3, "gpu_calls_ms": t_gpu * 1e3, "host_argmin_walk_ms": t_host * 1e3, "d2h_bytes": int(n * side * side * 4 + n * 49 * 4),
             "h2d_bytes": int(n * 40 + n * 32), "round_trips": 2, "results_equal": same}
+
+
+def row_f9(cucd, iters=5, threads=8):
+    """f9: TZ search (cucd_me_tz_search) on the ME part of bench.py's inter workloads: the 42 900 square PUs of a 1920x1080 picture
+    (bench.inter_pus), source textured_plane(t=1), references pseudo_recon of t=0 (real (2, 1) motion); ldp1080p 8-bit with one
+    reference, ra1080p10 10-bit with two (one call per depth for both).  +-64, FEN sub_shift, FRAC with Hadamard, lambda of QP 32; the
+    calls go depth by depth (64, 32, 16, 8): a PU's predictor is its parent's quarter-pel result and its TZ_2NX2N start its parent's
+    integer result (depth 0: predictor (0, 0), no 2Nx2N start).  Box = the legal area of the 80-sample margin, window = xSetSearchRange
+    around the predictor.  Times are summed over the four calls.  In the same run: HM's probes per PU and the kernel's evaluated points
+    (checker and CPU replay on every 97th PU), the checker's rate on host threads, the surface route to the same answers (cucd_me_sad_surface
+    over the bounding box of each PU's probes, the checker's walk on it, cucd_me_subpel_cost + host walk; must be equal) and
+    cucd_me_search +-64 on the same PUs and windows, for scale."""
+    import bench
+    import me_search_util as msu
+    import me_tz_util as mtu
+    R, M = bench.ME_RANGE, bench.ME_MARGIN
+    pus = bench.inter_pus(W, H)
+    lam = msu.lambda_cost(32)
+    tz = mtu.load_me_tz_oracle()
+    emul = mtu.load_me_tz_emul()
+    gpu = gpu_identity()
+    for cfg, bd, nref in (("ldp1080p", 8, 1), ("ra1080p10", 10, 2)):
+        org = _util.textured_plane(W, H, bd, seed=91, t=1)
+        refs = [np.ascontiguousarray(np.pad(_util.pseudo_recon(_util.textured_plane(W, H, bd, seed=91, t=0), bd, seed=92 + k), M, mode="edge"))
+                for k in range(nref)]
+        sc = dict(bd=bd, W=W, H=H, M=M, org=org, refs={k: r for k, r in enumerate(refs)})
+        eng = cucd.Engine(W, H, bit_depth=bd)
+        eng.set_cur_picture(org)
+        for k, r in enumerate(refs):
+            eng.set_ref_picture(k, r, M, M)
+        # one pass depth by depth builds every depth's descriptors from its parents' results
+        parent = {}
+        depths = []
+        for size in (64, 32, 16, 8):
+            descs = []
+            for k in range(nref):
+                for x, y, s in pus:
+                    if s != size:
+                        continue
+                    p = parent.get((k, x & ~(2 * s - 1), y & ~(2 * s - 1), 2 * s))
+                    pred = (0, 0) if p is None else (p[3], p[4])
+                    fl = msu.FRAC | msu.HAD | (0 if p is None else mtu.TZ2N)
+                    descs.append(mtu.tz_desc(sc, x, y, s, s, k, pred, R, sub_shift=1 if s > 8 else 0, lam=lam, flags=fl,
+                                             mv2n=(0, 0) if p is None else (p[0], p[1])))
+            arr = cucd.Engine.tz_descs(descs)
+            res = np.zeros(len(arr), cucd.SEARCH_RESULT)
+            eng.me_tz_search_raw(arr, res)
+            for d, r in zip(descs, res):
+                parent[(d["ref_idx"], d["x"], d["y"], d["w"])] = tuple(int(r[f]) for f in ("mvx", "mvy", "sad", "qmvx", "qmvy"))
+            depths.append((descs, arr, res))
+        n = sum(len(a) for _, a, _ in depths)
+        k_s = w_s = p_s = 0.0
+        direct = []
+        for _, arr, res in depths:
+            try:
+                k1, w1, p1 = timed(lambda: eng.me_tz_search_raw(arr, res), eng, iters, pin=(res,))
+            except cucd.CucdError:            # a call small enough for the zero-copy path is not timed: its call time stands for the kernel
+                direct.append(len(arr))
+                ws = []
+                for _ in range(iters):
+                    t0 = time.perf_counter()
+                    eng.me_tz_search_raw(arr, res)
+                    ws.append(time.perf_counter() - t0)
+                k1 = w1 = p1 = float(np.median(ws))
+            k_s, w_s, p_s = k_s + k1, w_s + w1, p_s + p1
+        descs = [d for ds, _, _ in depths for d in ds]
+        got = np.concatenate([msu.as_rows(r) for _, _, r in depths])
+        # cucd_me_search over the same windows, for scale
+        sarr, sn = cucd.Engine.search_descs([dict(d, flags=msu.FRAC | msu.HAD) for d in descs])
+        sres = np.zeros(sn, cucd.SEARCH_RESULT)
+        fk, fw, _ = timed(lambda: eng.me_search_raw(sarr, sn, sres), eng, iters, pin=(sres,))
+        # HM's probes (checker) and the kernel's evaluated points (CPU replay) on a sample; the checker's rate on host threads
+        samp = descs[::97]
+        probes, raster, evals, first_hm, first_all = [], [], [], [], []
+        for d in samp:
+            _, tr, cnt = mtu.oracle_tz(tz, sc, d, trace_cap=20000)
+            probes.append(cnt)
+            raster.append(int((tr[:, 4] == 3).sum()))
+            first_hm.append(int((tr[:, 4] == 1).sum()))
+            first_all.append(first_search_points(mtu, d, tr))
+            res6 = np.zeros(6, np.int32)
+            tr2 = np.zeros((20000, 6), np.int32)
+            ev, g = np.zeros(1, np.int32), np.zeros(1, np.int32)
+            blk = mtu.src_block(sc, d)
+            emul.emul_me_tz_search(bd, P(blk, i16p), d["w"], mtu.ref_base(sc, d), refs[d["ref_idx"]].shape[1], P(mtu.desc_row(d), i32p), P(res6, i32p),
+                                   tr2.ctypes.data, 20000, ev.ctypes.data, g.ctypes.data)
+            evals.append(int(ev[0]))
+
+        def work(i):
+            mtu.oracle_tz(tz, sc, samp[i])
+        sec = cpu_parallel(work, len(samp), threads)
+        cpu = {"value": len(samp) / sec, "unit": "PU/s", "cores": threads, "kind": "port",
+               "sample": f"every 97th PU ({len(samp)}) through tests/me_tz_oracle.c in {sec:.2f} s"}
+        h2d = n * (16 + 20 + 4 + 48) + sum(4 * (len(a) // 4 + 2) for _, a, _ in depths)
+        d2h = n * 24
+        # algorithmic bytes: per PU its source block, the reference block of every HM probe (sample mean), the sub-pel window, the records
+        mean_probes = float(np.mean(probes))
+        algo = int(sum(d["w"] * d["h"] * 2 * (1 + mean_probes) + (d["w"] + 9) * (d["h"] + 9) * 2 + 88 + 24 for d in descs))
+        extra = {"gpu": gpu, "config": cfg, "bit_depth": bd, "refs": nref, "pus_per_call": n, "calls": 4, "window": f"+-{R}", "flags": "FRAC|HADAMARD (+TZ_2NX2N below depth 0)",
+                 "lambda": lam, "lambda_note": "floor(65536 sqrt(0.57 2^((QP - 12) / 3))) at QP 32",
+                 "hm_probes_per_pu": {"mean": mean_probes, "max": int(max(probes)), "raster_share": float(sum(raster) / max(1, sum(probes))),
+                                      "sample": len(samp)},
+                 "kernel_points_per_pu": {"mean": float(np.mean(evals)), "over_hm": float(sum(evals) / max(1, sum(probes))),
+                                          "first_search_hm_mean": float(np.mean(first_hm)), "first_search_all_distances_mean": float(np.mean(first_all))},
+                 "zero_copy_calls_pus": direct, "zero_copy_note": "calls on the zero-copy path are not timed: their call time is counted as kernel time",
+                 "me_search_same_pus": {"kernel_ms": fk * 1e3, "e2e_ms": fw * 1e3},
+                 "surface_route": tz_surface_route(cucd, eng, tz, mtu, msu, sc, descs, got, threads)}
+        emit("f9_me_tz_search", "PU/s", n, k_s, w_s, algo, cpu, extra, p_s=p_s, h2d=int(h2d), d2h=int(d2h))
+        eng.close()
+
+
+def first_search_points(mtu, d, tr):
+    """points the first search would probe if all its distances were evaluated at once (guards applied, no three-round stop)"""
+    st0 = tr[tr[:, 4] == 0]
+    cx, cy = (int(v) for v in st0[int(np.argmin(st0[:, 5])), :2])      # argmin: the first of equal values, as the strict '<'
+    cnt, D = 0, 1
+    while D <= d["search_range"]:
+        for dx, dy, _, _ in mtu._diamond_points(D):
+            x, y = cx + dx, cy + dy
+            cnt += (dx >= 0 or x >= d["left"]) and (dx <= 0 or x <= d["right"]) and (dy >= 0 or y >= d["top"]) and (dy <= 0 or y <= d["bottom"])
+        D *= 2
+    return cnt
+
+
+def tz_surface_route(cucd, eng, tz, mtu, msu, sc, descs, got, threads):
+    """the surface route to cucd_me_tz_search's answer: cucd_me_sad_surface over the bounding box of each PU's probes (from the
+    checker's trace), the checker's walk on that surface on host threads, cucd_me_subpel_cost at its result and the host walk"""
+    n = len(descs)
+    boxes = [None] * n
+
+    def trace(i):
+        tr = mtu.oracle_tz(tz, sc, descs[i], trace_cap=20000)[1]
+        boxes[i] = (int(tr[:, 0].min()), int(tr[:, 0].max()), int(tr[:, 1].min()), int(tr[:, 1].max()))
+    cpu_parallel(trace, n, threads)
+    ints = np.zeros((n, 3), np.int64)
+    t_gpu = t_host = 0.0
+    t0 = time.perf_counter()
+    chunk = 2048
+    for c0 in range(0, n, chunk):
+        part = [dict(d, left=b[0], right=b[1], top=b[2], bottom=b[3]) for d, b in zip(descs[c0:c0 + chunk], boxes[c0:c0 + chunk])]
+        arr, m, total = cucd.Engine.me_descs(part)
+        surf = np.zeros(total, np.uint32)
+        ta = time.perf_counter()
+        eng.me_sad_surface_raw(arr, m, surf)
+        tb = time.perf_counter()
+        offs = np.cumsum([0] + [(d["right"] - d["left"] + 1) * (d["bottom"] - d["top"] + 1) for d in part])
+
+        def walk(i):
+            d = part[i]
+            s = surf[offs[i]:offs[i + 1]].reshape(d["bottom"] - d["top"] + 1, d["right"] - d["left"] + 1)
+            r = mtu.oracle_tz(tz, {"bd": sc["bd"]}, dict(descs[c0 + i], flags=descs[c0 + i]["flags"] & mtu.TZ2N), surface=(s, d["left"], d["top"]))[0]
+            ints[c0 + i] = r[:3]
+        cpu_parallel(walk, m, threads)
+        t_gpu += tb - ta
+        t_host += time.perf_counter() - tb
+    sp = [dict(x=d["x"], y=d["y"], w=d["w"], h=d["h"], ref_idx=d["ref_idx"], mvx=int(r[0]), mvy=int(r[1]), use_hadamard=1) for d, r in zip(descs, ints)]
+    ta = time.perf_counter()
+    arr, m = cucd.Engine.subpel_descs(sp)
+    T = np.zeros((m, 49), np.uint32)
+    eng.me_subpel_cost_raw(arr, m, T)
+    tb = time.perf_counter()
+    preds = np.array([(d["pred_x"], d["pred_y"]) for d in descs], np.int64)
+    qmv, fc = msu.walk_batch(T, ints[:, :2], preds, descs[0]["lambda"])
+    t1 = time.perf_counter()
+    t_gpu += tb - ta
+    t_host += t1 - tb
+    want = np.concatenate([ints, qmv, fc[:, None]], axis=1)
+    return {"wall_ms": (t1 - t0) * 1e3, "gpu_calls_ms": t_gpu * 1e3, "host_walks_ms": t_host * 1e3,
+            "d2h_bytes": int(sum((b[1] - b[0] + 1) * (b[3] - b[2] + 1) for b in boxes) * 4 + n * 49 * 4), "results_equal": bool(np.array_equal(got, want)),
+            "pus_equal": int((got == want).all(axis=1).sum()), "pus": n}
 
 
 if __name__ == "__main__":

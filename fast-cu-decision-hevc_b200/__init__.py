@@ -23,8 +23,10 @@ from .binding import (  # noqa: F401
     SEARCH_FRAC,
     SEARCH_HADAMARD,
     SEARCH_RESULT,
+    SEARCH_TZ_2NX2N,
     TU_INTRA_SLICE,
     TU_SIGN_HIDING,
+    TZ_DESC,
     declared_symbols,
     load_library,
     tcm_fit,

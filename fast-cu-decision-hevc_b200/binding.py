@@ -99,6 +99,11 @@ class _SearchDesc(C.Structure):
 SEARCH_FRAC, SEARCH_HADAMARD = 1, 2       # cucd_search_desc.flags
 # cucd_search_result: integer MV and its SAD, final quarter-pel MV and the cost of the quarter stage's best
 SEARCH_RESULT = np.dtype([("mvx", np.int32), ("mvy", np.int32), ("sad", np.uint32), ("qmvx", np.int32), ("qmvy", np.int32), ("frac_cost", np.uint32)])
+SEARCH_TZ_2NX2N = 4                       # cucd_tz_desc.flags: start at mv2n, raster window around the best start
+# cucd_tz_desc, field for field
+TZ_DESC = np.dtype([(n, np.int32) for n in ("x", "y", "w", "h", "ref_idx", "left", "right", "top", "bottom", "sub_shift", "pred_x", "pred_y")]
+                   + [("lambda", np.uint32), ("flags", np.int32), ("search_range", np.int32)]
+                   + [(n, np.int32) for n in ("clip_left", "clip_right", "clip_top", "clip_bottom", "mv2n_x", "mv2n_y")])
 
 
 class _McDesc(C.Structure):
@@ -166,6 +171,7 @@ def load_library():
     lib.cucd_me_subpel_cost_src.argtypes = [C.c_void_p, C.c_int, C.POINTER(_SubpelDesc), C.c_void_p, C.c_void_p]
     lib.cucd_me_search.argtypes = [C.c_void_p, C.c_int, C.POINTER(_SearchDesc), C.c_void_p]
     lib.cucd_me_search_src.argtypes = [C.c_void_p, C.c_int, C.POINTER(_SearchDesc), C.c_void_p, C.c_void_p]
+    lib.cucd_me_tz_search.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]
     lib.cucd_me_mc_cost.argtypes = [C.c_void_p, C.c_int, C.POINTER(_McDesc), C.c_void_p, C.c_void_p]
     lib.cucd_set_ref_picture_chroma.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int]
     lib.cucd_set_cur_picture_chroma.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]
@@ -530,6 +536,32 @@ class Engine:
             src = np.ascontiguousarray(src, np.int16)
             assert src.size == sum(int(d["w"]) * int(d["h"]) for d in descs)
         self.me_search_raw(arr, n, out, src)
+        return out
+
+    @staticmethod
+    def tz_descs(descs):
+        """list of dicts with the TZ_DESC fields (mv2n_x / mv2n_y may be left out: 0) -> TZ_DESC array: build once, reuse"""
+        arr = np.zeros(len(descs), TZ_DESC)
+        for i, d in enumerate(descs):
+            for k in TZ_DESC.names:
+                v = int(d.get(k, 0) if k in ("mv2n_x", "mv2n_y") else d[k])
+                arr[k][i] = v & 0xFFFFFFFF if k == "lambda" else v
+        return arr
+
+    def me_tz_search_raw(self, arr, out):
+        """cucd_me_tz_search with a prebuilt TZ_DESC array; out: SEARCH_RESULT host array of len(arr)"""
+        assert arr.dtype == TZ_DESC and arr.flags.c_contiguous and out.dtype == SEARCH_RESULT and len(out) == len(arr)
+        self._check(self.lib.cucd_me_tz_search(self.h, len(arr), arr.ctypes.data if len(arr) else None, out.ctypes.data if len(out) else None),
+                    "cucd_me_tz_search")
+
+    def me_tz_search(self, descs):
+        """descs: list of dicts with the TZ_DESC fields (x,y,w,h,ref_idx,left,right,top,bottom,sub_shift,pred_x,pred_y,lambda,flags,
+        search_range,clip_left,clip_right,clip_top,clip_bottom[,mv2n_x,mv2n_y]) or a TZ_DESC array.  Returns a SEARCH_RESULT structured
+        array (mvx, mvy, sad, qmvx, qmvy, frac_cost) with one record per PU."""
+        arr = descs if isinstance(descs, np.ndarray) else self.tz_descs(descs)
+        arr = np.ascontiguousarray(arr, TZ_DESC)
+        out = np.zeros(len(arr), SEARCH_RESULT)
+        self.me_tz_search_raw(arr, out)
         return out
 
     @staticmethod

@@ -702,6 +702,90 @@ int cucd_me_search_src(cucd_handle* h, int nPU, const cucd_search_desc* desc, co
 }
 
 // ------------------------------------------------------------------------------------------------
+// TZ search: xTZSearch's integer walk, one warp per PU and reference (me_core.cuh, me_tz_*), then the refinement walk of the FRAC
+// PUs as in cucd_me_search.  No SAD tiles: the walk reads the reference plane itself, inside the clip box.
+// ------------------------------------------------------------------------------------------------
+static_assert(kTz2Nx2N == CUCD_SEARCH_TZ_2NX2N, "MeTzJob flags are cucd_tz_desc flags");
+int cucd_me_tz_search(cucd_handle* h, int nPU, const cucd_tz_desc* desc, cucd_search_result* out) {
+  if (!h || nPU < 0 || (nPU > 0 && (!desc || !out))) return fail(h, CUCD_ERR_INVALID, "cucd_me_tz_search: bad argument");
+  if (nPU == 0) return CUCD_OK;
+  LOCK(h);
+  if (!h->curSet) return fail(h, CUCD_ERR_INVALID, "cucd_me_tz_search: cucd_set_cur_picture not called");
+  CK(cudaSetDevice(h->cfg.device));
+  const int W = h->cfg.width, H = h->cfg.height;
+  int nFrac = 0, maxSamples = 16;
+  for (int i = 0; i < nPU; i++) {
+    const cucd_tz_desc& d = desc[i];
+    if (d.w < 4 || d.h < 4 || d.w > 64 || d.h > 64 || (d.w & 3) || d.x < 0 || d.y < 0 || d.x + d.w > W || d.y + d.h > H || d.sub_shift < 0 || d.sub_shift > 4)
+      return fail(h, CUCD_ERR_INVALID, "cucd_me_tz_search: bad PU (4..64, width a multiple of 4, inside the picture) or sub_shift");
+    const RefPlane* r = ref_slot(h->refs, d.ref_idx);
+    if (!r) return fail(h, CUCD_ERR_INVALID, "cucd_me_tz_search: reference picture not set");
+    if (d.flags & ~(CUCD_SEARCH_FRAC | CUCD_SEARCH_HADAMARD | CUCD_SEARCH_TZ_2NX2N)) return fail(h, CUCD_ERR_INVALID, "cucd_me_tz_search: unknown flags");
+    if (d.pred_x < -32768 || d.pred_x > 32767 || d.pred_y < -32768 || d.pred_y > 32767) return fail(h, CUCD_ERR_INVALID, "cucd_me_tz_search: predictor outside the int16 range");
+    if (d.mv2n_x < -32768 || d.mv2n_x > 32767 || d.mv2n_y < -32768 || d.mv2n_y > 32767) return fail(h, CUCD_ERR_INVALID, "cucd_me_tz_search: mv2n outside the int16 range");
+    if (d.search_range < 0 || d.search_range > 4095) return fail(h, CUCD_ERR_INVALID, "cucd_me_tz_search: search_range outside [0, 4095]");
+    if (d.clip_left > 0 || d.clip_right < 0 || d.clip_top > 0 || d.clip_bottom < 0 || d.clip_left < -32768 || d.clip_right > 32767 || d.clip_top < -32768 ||
+        d.clip_bottom > 32767)
+      return fail(h, CUCD_ERR_INVALID, "cucd_me_tz_search: the clip box must contain (0, 0) and fit int16");
+    if (d.left > d.right || d.top > d.bottom || d.left < d.clip_left || d.right > d.clip_right || d.top < d.clip_top || d.bottom > d.clip_bottom)
+      return fail(h, CUCD_ERR_INVALID, "cucd_me_tz_search: the window must be non-empty and inside the clip box");
+    const bool frac = (d.flags & CUCD_SEARCH_FRAC) != 0;
+    if (frac && (d.h & 3)) return fail(h, CUCD_ERR_INVALID, "cucd_me_tz_search: CUCD_SEARCH_FRAC needs h % 4 == 0");
+    // every probe lies in the box: the box's blocks (and their 8-tap support with FRAC) bound every read
+    const int e = frac ? 4 : 0;
+    if (!inside_padded(*r, W, H, d.x + d.clip_left - e, d.y + d.clip_top - e, d.x + d.clip_right + d.w - 1 + (frac ? 5 : 0), d.y + d.clip_bottom + d.h - 1 + (frac ? 5 : 0)))
+      return fail(h, CUCD_ERR_INVALID, "cucd_me_tz_search: the clip box leaves the padded reference picture");
+    nFrac += frac ? 1 : 0;
+    maxSamples = std::max(maxSamples, d.w * d.h);
+  }
+  // pinned records: [cost records | sub-pel jobs | FRAC list | TZ jobs in class order | CTA starts]; device scratch: [completed
+  // sub-pel jobs | tables]
+  const size_t costBytes = up16((size_t)nPU * sizeof(MeSearchCost)), subBytes = up16((size_t)nFrac * sizeof(SubpelJob)), fracBytes = up16((size_t)nFrac * 4);
+  const size_t jobBytes = up16((size_t)nPU * sizeof(MeTzJob)), ctaBytes = up16((size_t)(nPU + 1) * 4);
+  std::vector<MeTzJob> jobs(nPU);
+  CK(h->hSearch.reserve(costBytes + subBytes + fracBytes + jobBytes + ctaBytes));
+  uint8_t* base = h->hSearch.p;
+  MeSearchCost* cost = reinterpret_cast<MeSearchCost*>(base);
+  SubpelJob* sub = reinterpret_cast<SubpelJob*>(base + costBytes);
+  int32_t* fracJob = reinterpret_cast<int32_t*>(base + costBytes + subBytes);
+  for (int i = 0, f = 0; i < nPU; i++) {
+    const cucd_tz_desc& d = desc[i];
+    const RefPlane& r = h->refs[d.ref_idx];
+    const bool frac = (d.flags & CUCD_SEARCH_FRAC) != 0;
+    MeTzJob& j = jobs[i];
+    j.curOff = d.y * h->curStride + d.x;
+    j.refOff = (d.y + r.marginY) * r.stride + d.x + r.marginX;
+    j.refSlot = d.ref_idx; j.w = (int16_t)d.w; j.h = (int16_t)d.h;
+    j.subShift = (int16_t)(me_width_is_hm(d.w) ? d.sub_shift : 0);       // the generic xGetSAD ignores iSubShift
+    j.flags = (int16_t)d.flags;
+    j.left = (int16_t)d.left; j.right = (int16_t)d.right; j.top = (int16_t)d.top; j.bottom = (int16_t)d.bottom;
+    j.clipL = (int16_t)d.clip_left; j.clipR = (int16_t)d.clip_right; j.clipT = (int16_t)d.clip_top; j.clipB = (int16_t)d.clip_bottom;
+    j.mv2nX = (int16_t)d.mv2n_x; j.mv2nY = (int16_t)d.mv2n_y; j.range = (int16_t)d.search_range; j.pad = 0;
+    j.outIndex = i;
+    cost[i] = MeSearchCost{d.lambda, d.pred_x, d.pred_y, frac ? f : -1};
+    if (!frac) continue;
+    sub[f] = SubpelJob{j.curOff, j.refOff, d.ref_idx, (int16_t)d.w, (int16_t)d.h, (d.flags & CUCD_SEARCH_HADAMARD) ? 1 : 0};
+    fracJob[f++] = i;
+  }
+  const size_t jobsAt = costBytes + subBytes + fracBytes;
+  const int nCta = me_tz_plan(nPU, jobs.data(), reinterpret_cast<MeTzJob*>(base + jobsAt), reinterpret_cast<int32_t*>(base + jobsAt + jobBytes));
+  const size_t tabBytes = up16((size_t)nFrac * CUCD_SUBPEL_POINTS * 4);
+  CK(h->dSearch.reserve(subBytes + tabBytes));
+  if (sync_ref_table(h) != CUCD_OK) return CUCD_ERR_CUDA;
+  BatchIo io(h);
+  const int iRec = io.add_in(base, jobsAt + jobBytes + ctaBytes, true);
+  const int oRes = io.add_out(out, (size_t)nPU * sizeof(cucd_search_result));
+  if (io.begin(h->sMain) != CUCD_OK) return CUCD_ERR_CUDA;
+  const uint8_t* dRec = io.din<uint8_t>(iRec);
+  uint8_t* dS = h->dSearch.p;
+  CK(launch_me_tz_search(me_planes(h, nullptr), reinterpret_cast<const MeTzJob*>(dRec + jobsAt), reinterpret_cast<const int32_t*>(dRec + jobsAt + jobBytes), nCta,
+                         maxSamples, reinterpret_cast<const MeSearchCost*>(dRec), reinterpret_cast<const SubpelJob*>(dRec + costBytes), reinterpret_cast<SubpelJob*>(dS),
+                         reinterpret_cast<const int32_t*>(dRec + costBytes + subBytes), nFrac, reinterpret_cast<uint32_t*>(dS + subBytes), io.dout<MeSearchOut>(oRes),
+                         h->sMain, &h->launches));
+  return io.finish(h->sMain);
+}
+
+// ------------------------------------------------------------------------------------------------
 // Motion compensation and distortion of inter candidates (uni- and bi-predictive), me_core.cuh me_mc_*
 // ------------------------------------------------------------------------------------------------
 int cucd_me_mc_cost(cucd_handle* h, int nPU, const cucd_mc_desc* desc, uint32_t* dist, int16_t* pred) {

@@ -142,5 +142,11 @@ struct MeSearchOut;
 cudaError_t launch_me_search(const MePlanes& mp, const MeJob* jobs, int nJobs, const int32_t* tileJob, const int32_t* tileIdx, int nTilesDy, int nTilesO,
                              const MeSearchCost* cost, unsigned long long* keys, const SubpelJob* subIn, SubpelJob* subDev, const int32_t* fracJob, int nFrac,
                              uint32_t* tables, MeSearchOut* out, cudaStream_t st, int* launches);
+// TZ search (me_core.cuh, me_tz_*): CTA b walks jobs[ctaFirst[b] .. ctaFirst[b + 1]) (me_tz_plan), maxSamples >= w * h of every job;
+// cost[outIndex] per PU in the caller's order; then the sub-pel tables and the walk of the FRAC PUs as in launch_me_search
+struct MeTzJob;
+cudaError_t launch_me_tz_search(const MePlanes& mp, const MeTzJob* jobs, const int32_t* ctaFirst, int nCta, int maxSamples, const MeSearchCost* cost,
+                                const SubpelJob* subIn, SubpelJob* subDev, const int32_t* fracJob, int nFrac, uint32_t* tables, MeSearchOut* out, cudaStream_t st,
+                                int* launches);
 
 }  // namespace cucd

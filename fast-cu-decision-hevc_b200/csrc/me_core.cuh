@@ -421,8 +421,8 @@ inline McJob me_mc_job(int curOff, int x, int y, int w, int h, int nl, const int
 }
 // host: the jobs sorted by class (cls(job) < NC) into `sorted`, every class cut into CTAs of per(job) jobs; CTA b takes
 // sorted[ctaFirst[b] .. ctaFirst[b + 1]).  ctaFirst has room for n + 1 entries; returns the number of CTAs.
-template <int NC, class Cls, class Per>
-inline int me_plan_classes(int n, const McJob* jobs, McJob* sorted, int32_t* ctaFirst, Cls cls, Per per) {
+template <int NC, class Job, class Cls, class Per>
+inline int me_plan_classes(int n, const Job* jobs, Job* sorted, int32_t* ctaFirst, Cls cls, Per per) {
   int start[NC + 1] = {0};
   for (int i = 0; i < n; i++) start[cls(jobs[i]) + 1]++;
   for (int c = 0; c < NC; c++) start[c + 1] += start[c];
@@ -430,7 +430,7 @@ inline int me_plan_classes(int n, const McJob* jobs, McJob* sorted, int32_t* cta
   for (int i = 0; i < n; i++) sorted[start[cls(jobs[i])]++] = jobs[i];
   int nCta = 0;
   for (int b = 0; b < n;) {
-    const McJob& j = sorted[b];
+    const Job& j = sorted[b];
     const int e = start[cls(j)], k = per(j);
     for (; b < e; b += k) ctaFirst[nCta++] = b;
     b = e;
@@ -737,6 +737,198 @@ CUCD_HD void me_search_walk(const uint32_t* T /*49*/, const MeSearchCost& c, MeS
     if (d < best) { best = d; qbx = qx[i]; qby = qy[i]; }
   }
   o.qmvx = 4 * mvx + 2 * bx + qbx; o.qmvy = 4 * mvy + 2 * by + qby; o.fracCost = best;
+}
+
+// =============================================================================================================================
+// TZ search (cucd_me_tz_search): the integer walk of xTZSearch with TZ_SEARCH_CONFIGURATION (TEncSearch.cpp: xTZSearch,
+// xTZSearchHelp, xTZ8PointDiamondSearch, xTZ2PointSearch; include/cucudecide.h states the rules), then the refinement walk of
+// cucd_me_search.  One warp per (PU, reference) job; a CTA takes up to kTzWarps jobs of one PU shape.
+// The walk is a chain of STAGES whose centre is fixed while they run: the start points, the first search (the diamonds
+// D = 1, 2, 4, .. <= search_range, stopped after three rounds without a better point), the two-point search, the raster and every
+// star-refinement iteration.  A stage is a list of points in HM's order, cut into SEGMENTS (a diamond each; one segment for the
+// two-point search and the raster; one per start point).  A segment's outcome is its least key (cost << 32 | point index), folded
+// into the walk's state with one strict '<' (me_tz_fold): the same as HM's sequence of probes, because a point of a segment never
+// sees the update of another point of the same segment (fixed centre) and a point visited again cannot beat the best.
+//   lanes   G lanes (a power of two, me_tz_lanes) share one probe's samples, so a chunk of 32 / G consecutive points of the stage runs
+//           at once; a group's partial sums meet through xor shuffles inside the group, a segment's keys through xor shuffles
+//           across the groups.  Chunks run in order and stop once the first search's stop has been decided.
+// =============================================================================================================================
+constexpr int kTzWarps = 4;                    // jobs of a CTA
+constexpr int kTz2Nx2N = 4;                    // CUCD_SEARCH_TZ_2NX2N
+struct MeTzJob {
+  int32_t curOff;                              // PU origin inside the current picture plane
+  int32_t refOff;                              // co-located sample (mv 0) inside the padded plane of refSlot
+  int32_t refSlot;
+  int16_t w, h, subShift, flags;               // subShift: 0 for the generic widths (me_width_is_hm)
+  int16_t left, right, top, bottom;            // the descriptor window `win`
+  int16_t clipL, clipR, clipT, clipB;          // the clip box: every probe lies inside it
+  int16_t mv2nX, mv2nY, range, pad;
+  int32_t outIndex;                            // PU index in the caller's order (costs, results)
+};
+inline int me_tz_class(int w, int h) { return ((w >> 2) - 1) * 16 + (h >> 2) - 1; }
+constexpr int kTzClasses = 16 * 16;
+inline int me_tz_plan(int n, const MeTzJob* jobs, MeTzJob* sorted, int32_t* ctaFirst) {
+  return me_plan_classes<kTzClasses>(n, jobs, sorted, ctaFirst, [](const MeTzJob& j) { return me_tz_class(j.w, j.h); }, [](const MeTzJob&) { return kTzWarps; });
+}
+// lanes per probe: about 16 samples per lane (an 8x8 PU: 4 lanes, 8 probes at once; 32x32 and up: one probe per warp)
+CUCD_HD int me_tz_lanes(int samples) { int g = 1; while (g < 32 && 16 * g < samples) g <<= 1; return g; }
+
+struct MeTzWin { int left, right, top, bottom; };
+struct MeTzState { int bx, by; uint32_t best; int dist, round, pt; };
+struct MeTzPoint { int x, y, p, d; bool ok; };
+enum { kTzStart = 0, kTzDiamonds = 1, kTzTwo = 2, kTzRaster = 3 };
+struct MeTzStage {
+  int kind, cx, cy, n, stop;                   // n points; stop: the first search's three-round stop
+  MeTzWin win;                                 // the guard window; the raster window for kTzRaster
+  int pt, cols;                                // kTzTwo: the case; kTzRaster: points per row
+  int sx0, sy0, sx2, sy2;                      // kTzStart: the predictor and the 2Nx2N start (point 1 is (0, 0))
+};
+CUCD_HD int me_tz_clamp(int v, int lo, int hi) { return v < lo ? lo : (v > hi ? hi : v); }
+// first point of segment k (k = segment count: the stage's n)
+CUCD_HD int me_tz_seg_first(const MeTzStage& s, int k) {
+  if (s.kind == kTzStart) return k;
+  if (s.kind != kTzDiamonds) return k ? s.n : 0;
+  return k == 0 ? 0 : (k <= 4 ? 4 + 8 * (k - 1) : 28 + 16 * (k - 4));
+}
+CUCD_HD int me_tz_seg_of(const MeTzStage& s, int i) {
+  if (s.kind == kTzStart) return i;
+  if (s.kind != kTzDiamonds) return 0;
+  return i < 4 ? 0 : (i < 28 ? 1 + ((i - 4) >> 3) : 4 + ((i - 28) >> 4));
+}
+// the diamonds D = 1, 2, 4, .. <= range around (cx, cy)
+CUCD_HD MeTzStage me_tz_diamonds(int cx, int cy, const MeTzWin& win, int range, int stop) {
+  MeTzStage s{};
+  s.kind = kTzDiamonds; s.cx = cx; s.cy = cy; s.win = win; s.stop = stop;
+  int k = 0;
+  for (int D = 1; D <= range; D <<= 1) k++;
+  s.n = me_tz_seg_first(s, k);
+  return s;
+}
+CUCD_HD MeTzStage me_tz_two(int cx, int cy, const MeTzWin& win, int pt) {
+  MeTzStage s{};
+  s.kind = kTzTwo; s.cx = cx; s.cy = cy; s.win = win; s.pt = pt; s.n = pt >= 1 && pt <= 8 ? 2 : 0;
+  return s;
+}
+CUCD_HD MeTzStage me_tz_raster(const MeTzWin& r) {
+  MeTzStage s{};
+  s.kind = kTzRaster; s.win = r; s.cols = (r.right - r.left) / 5 + 1; s.n = s.cols * ((r.bottom - r.top) / 5 + 1);
+  return s;
+}
+// point i of a stage.  Guards: a point that moves left / right / up / down from the centre must not cross win's left / right / top /
+// bottom border - xTZ8PointDiamondSearch's and xTZ2PointSearch's tests, which the all-inside branches pass anyway.
+// Offsets are packed tables (no indexed local arrays in the kernel): a direction nibble is (sx + 1) | (sy + 1) << 2, sx, sy in -1..1.
+CUCD_HD int me_tz_dir_x(uint32_t e) { return (int)(e & 3u) - 1; }
+CUCD_HD int me_tz_dir_y(uint32_t e) { return (int)((e >> 2) & 3u) - 1; }
+CUCD_HD MeTzPoint me_tz_point(const MeTzStage& s, int i) {
+  MeTzPoint q;
+  int dx = 0, dy = 0;
+  q.p = 0;
+  if (s.kind == kTzStart) {
+    q.x = i == 0 ? s.sx0 : (i == 1 ? 0 : s.sx2); q.y = i == 0 ? s.sy0 : (i == 1 ? 0 : s.sy2); q.d = 0; q.ok = true;
+    return q;
+  }
+  if (s.kind == kTzRaster) {
+    const int r = i / s.cols;
+    q.x = s.win.left + 5 * (i - r * s.cols); q.y = s.win.top + 5 * r; q.d = 5; q.ok = true;
+    return q;
+  }
+  if (s.kind == kTzTwo) {
+    // xTZ2PointSearch, cases 1..8: byte pt - 1 holds the first point's direction in its low nibble, the second's in its high nibble
+    const uint32_t e = (uint32_t)(0x96A894A208612014ull >> (8 * (s.pt - 1) + 4 * i)) & 15u;
+    dx = me_tz_dir_x(e); dy = me_tz_dir_y(e); q.d = 2;
+  } else {
+    const int k = me_tz_seg_of(s, i), D = 1 << k, j = i - me_tz_seg_first(s, k);
+    q.d = D;
+    if (D <= 8) {
+      // D = 1: up, left, right, down (points 2, 4, 5, 7); D = 2..8: up, the two upper diagonals, left, right, the two lower diagonals,
+      // down (points 2, 1, 3, 4, 5, 6, 8, 7), the diagonals at D / 2
+      const uint32_t e = D == 1 ? (0x9641u >> (4 * j)) & 15u : (0x9A864201u >> (4 * j)) & 15u;
+      q.p = (int)(((D == 1 ? 0x7542u : 0x78654312u) >> (4 * j)) & 15u);
+      const int sx = me_tz_dir_x(e), sy = me_tz_dir_y(e), a = (sx != 0 && sy != 0) ? D >> 1 : D;
+      dx = sx * a; dy = sy * a;
+      if (sx != 0 && sy != 0) q.d = D >> 1;
+    } else if (j < 4) {
+      const uint32_t e = (0x9641u >> (4 * j)) & 15u;                  // up, left, right, down
+      dx = me_tz_dir_x(e) * D; dy = me_tz_dir_y(e) * D;
+    } else {
+      const int qk = (D >> 2) * (((j - 4) >> 2) + 1), m = (j - 4) & 3;  // k = 1..3: upper left, upper right, lower left, lower right
+      dx = (m & 1) ? qk : -qk; dy = (m & 2) ? D - qk : qk - D;
+    }
+  }
+  q.x = s.cx + dx; q.y = s.cy + dy;
+  q.ok = (dx >= 0 || q.x >= s.win.left) && (dx <= 0 || q.x <= s.win.right) && (dy >= 0 || q.y >= s.win.top) && (dy <= 0 || q.y <= s.win.bottom);
+  return q;
+}
+// segment k's least key has been found: HM's round count, then one strict '<'.  Returns true when the stage stops here.
+CUCD_HD bool me_tz_fold(MeTzState& st, const MeTzStage& s, unsigned long long key) {
+  if (s.kind == kTzDiamonds) st.round++;
+  if (key != kMeNoKey && (uint32_t)(key >> 32) < st.best) {
+    const MeTzPoint q = me_tz_point(s, (int)(uint32_t)key);
+    st.best = (uint32_t)(key >> 32); st.bx = q.x; st.by = q.y; st.dist = q.d; st.round = 0; st.pt = q.p;
+  }
+  return s.stop && st.round >= 3;
+}
+// xTZSearch's sequence of stages.  run(stage, state) evaluates a stage and folds its segments into the state (the kernel: a warp,
+// the CPU replay: 32 emulated lanes); the clip box bounds the start points, win guards the diamonds and the two-point search.
+template <class Run>
+CUCD_HD MeTzState me_tz_walk(const MeTzJob& j, const MeSearchCost& c, Run&& run) {
+  MeTzState st;
+  st.bx = 0; st.by = 0; st.best = 0xffffffffu; st.dist = 0; st.round = 0; st.pt = 0;
+  const MeTzWin win{j.left, j.right, j.top, j.bottom};
+  MeTzStage s{};
+  s.kind = kTzStart; s.n = (j.flags & kTz2Nx2N) ? 3 : 2;
+  s.sx0 = me_tz_clamp(c.predX, 4 * j.clipL, 4 * j.clipR) >> 2; s.sy0 = me_tz_clamp(c.predY, 4 * j.clipT, 4 * j.clipB) >> 2;
+  s.sx2 = me_tz_clamp(j.mv2nX, j.clipL, j.clipR); s.sy2 = me_tz_clamp(j.mv2nY, j.clipT, j.clipB);
+  run(s, st);
+  MeTzWin rwin = win;                                                   // xSetSearchRange around the best start (TZ_2NX2N)
+  if (j.flags & kTz2Nx2N)
+    rwin = MeTzWin{me_tz_clamp(st.bx - j.range, j.clipL, j.clipR), me_tz_clamp(st.bx + j.range, j.clipL, j.clipR),
+                   me_tz_clamp(st.by - j.range, j.clipT, j.clipB), me_tz_clamp(st.by + j.range, j.clipT, j.clipB)};
+  run(me_tz_diamonds(st.bx, st.by, win, j.range, 1), st);
+  if (st.dist == 1) { st.dist = 0; run(me_tz_two(st.bx, st.by, win, st.pt), st); }
+  if (st.dist > 5) { st.dist = 5; run(me_tz_raster(rwin), st); }
+  while (st.dist > 0) {                                                 // ends: every iteration that goes on lowered best
+    const int cx = st.bx, cy = st.by;
+    st.dist = 0; st.pt = 0;
+    run(me_tz_diamonds(cx, cy, win, j.range, 0), st);
+    if (st.dist == 1) { st.dist = 0; if (st.pt != 0) run(me_tz_two(st.bx, st.by, win, st.pt), st); }
+  }
+  return st;
+}
+CUCD_HD int16_t me_ld16(const int16_t* p) {
+#if defined(__CUDA_ARCH__)
+  return __ldg(p);
+#else
+  return *p;
+#endif
+}
+// lane g of the G lanes that probe the reference block at ref: its part of sum |cur - ref| over the staged rows (nr rows of w samples,
+// row r of the PU at r << subShift); sample index s = r w + col, s / w as one multiply-high (s w < 2^32)
+CUCD_HD uint32_t me_tz_sad_part(const int16_t* sCur, const int16_t* ref, int refStride, int w, int nr, int subShift, int g, int G) {
+  const uint32_t invW = me_inv((uint32_t)w);
+  uint32_t acc = 0;
+  for (int s = g; s < nr * w; s += G) {
+    const int r = (int)me_mulhi((uint32_t)s, invW), col = s - r * w;
+    acc += (uint32_t)iabs32((int)sCur[s] - (int)me_ld16(ref + (long long)(r << subShift) * refStride + col));
+  }
+  return acc;
+}
+// the probe's value c = SAD + cost_2 from the group's total (xGetSAD*: << iSubShift, then >> (bitDepth - 8))
+CUCD_HD uint32_t me_tz_probe_cost(uint32_t total, int subShift, int bitDepth, const MeSearchCost& c, int x, int y) {
+  return ((total << subShift) >> (bitDepth - 8)) + me_mv_cost(c, x, y, 2);
+}
+// the integer result of a finished walk, and the PU's sub-pel job (FRAC) moved to it; Sub = SubpelJob (kernels.h)
+template <class Sub>
+CUCD_HD void me_tz_finish(const MeTzState& st, const MeTzJob& j, const MeSearchCost& c, int refStride, const Sub* subIn, Sub* subOut, MeSearchOut* out) {
+  MeSearchOut o;
+  o.mvx = st.bx; o.mvy = st.by; o.sad = st.best - me_mv_cost(c, st.bx, st.by, 2);
+  o.qmvx = 4 * st.bx; o.qmvy = 4 * st.by; o.fracCost = 0;
+  out[j.outIndex] = o;
+  if (c.frac >= 0) {
+    Sub sj = subIn[c.frac];
+    sj.refOff += st.by * refStride + st.bx;
+    subOut[c.frac] = sj;
+  }
 }
 
 }  // namespace cucd

@@ -527,4 +527,67 @@ cudaError_t launch_me_search(const MePlanes& mp, const MeJob* jobs, int nJobs, c
   return cudaGetLastError();
 }
 
+// cucd_me_tz_search (me_core.cuh, me_tz_*): warp `warp` of CTA b walks job ctaFirst[b] + warp.  Its source block (the rows the
+// sub-sampled SAD reads) sits in shared memory, the reference samples come from the padded plane through the read-only path.
+__global__ void __launch_bounds__(32 * kTzWarps)
+me_tz_kernel(const MePlanes mp, const MeTzJob* __restrict__ jobs, const int32_t* __restrict__ ctaFirst, int maxSamples, const MeSearchCost* __restrict__ cost,
+             const SubpelJob* __restrict__ subIn, SubpelJob* __restrict__ subOut, MeSearchOut* __restrict__ out) {
+  extern __shared__ __align__(16) int16_t sTz[];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int ji = ctaFirst[blockIdx.x] + warp;
+  if (ji >= ctaFirst[blockIdx.x + 1]) return;                          // warp uniform
+  const MeTzJob j = jobs[ji];
+  const MeSearchCost c = cost[j.outIndex];
+  const int w = j.w, nr = (j.h + (1 << j.subShift) - 1) >> j.subShift;
+  int16_t* sCur = sTz + warp * maxSamples;
+  const int16_t* cur = mp.cur + j.curOff;
+  const uint32_t invW = me_inv((uint32_t)w);
+  for (int s = lane; s < nr * w; s += 32) {
+    const int r = (int)__umulhi((uint32_t)s, invW);
+    sCur[s] = cur[(size_t)(r << j.subShift) * mp.curStride + s - r * w];
+  }
+  __syncwarp();
+  const int refStride = mp.refStride[j.refSlot];
+  const int16_t* ref0 = mp.ref[j.refSlot] + j.refOff;
+  const int G = me_tz_lanes(nr * w), g = lane & (G - 1), slot = lane / G, P = 32 / G;
+  const MeTzState st = me_tz_walk(j, c, [&](const MeTzStage& s, MeTzState& state) {
+    unsigned long long pend = kMeNoKey;
+    for (int base = 0; base < s.n; base += P) {
+      const int i = base + slot, end = min(base + P, s.n);
+      MeTzPoint q;
+      q.ok = false;
+      if (i < s.n) q = me_tz_point(s, i);
+      uint32_t part = q.ok ? me_tz_sad_part(sCur, ref0 + (long long)q.y * refStride + q.x, refStride, w, nr, j.subShift, g, G) : 0u;
+      for (int m = 1; m < G; m <<= 1) part += __shfl_xor_sync(0xffffffffu, part, m);
+      const unsigned long long key = q.ok ? ((unsigned long long)me_tz_probe_cost(part, j.subShift, mp.bitDepth, c, q.x, q.y) << 32) | (uint32_t)i : kMeNoKey;
+      const int k1 = me_tz_seg_of(s, end - 1);
+      for (int k = me_tz_seg_of(s, base); k <= k1; k++) {               // the segments of the chunk, in order
+        unsigned long long kk = i < end && me_tz_seg_of(s, i) == k ? key : kMeNoKey;
+        for (int m = G; m < 32; m <<= 1) kk = me_key_min(kk, __shfl_xor_sync(0xffffffffu, kk, m));
+        pend = me_key_min(pend, kk);
+        if (me_tz_seg_first(s, k + 1) <= end) {                          // segment k is complete
+          const bool stop = me_tz_fold(state, s, pend);
+          pend = kMeNoKey;
+          if (stop) return;
+        }
+      }
+    }
+  });
+  if (lane == 0) me_tz_finish(st, j, c, refStride, subIn, subOut, out);
+}
+
+cudaError_t launch_me_tz_search(const MePlanes& mp, const MeTzJob* jobs, const int32_t* ctaFirst, int nCta, int maxSamples, const MeSearchCost* cost,
+                                const SubpelJob* subIn, SubpelJob* subDev, const int32_t* fracJob, int nFrac, uint32_t* tables, MeSearchOut* out, cudaStream_t st,
+                                int* launches) {
+  if (nCta <= 0) return cudaSuccess;
+  me_tz_kernel<<<nCta, 32 * kTzWarps, (size_t)kTzWarps * maxSamples * sizeof(int16_t), st>>>(mp, jobs, ctaFirst, maxSamples, cost, subIn, subDev, out);
+  if (launches) *launches += 1;
+  cudaError_t e = cudaGetLastError();
+  if (e != cudaSuccess || nFrac <= 0) return e;
+  if ((e = launch_me_subpel(mp, subDev, nFrac, tables, st, launches)) != cudaSuccess) return e;
+  me_search_walk_kernel<<<(nFrac + 127) / 128, 128, 0, st>>>(fracJob, nFrac, cost, tables, out);
+  if (launches) *launches += 1;
+  return cudaGetLastError();
+}
+
 }  // namespace cucd

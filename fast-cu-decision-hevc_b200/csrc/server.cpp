@@ -228,6 +228,16 @@ int main(int argc, char** argv) {
           reply(s, rc, rc == CUCD_OK ? nullptr : cucd_last_error(k.h));
           break;
         }
+        case CUCD_IPC_ME_TZ_SEARCH: {
+          const size_t nP = (size_t)(s.n > 0 ? s.n : 0);
+          if (nP * sizeof(cucd_tz_desc) > s.in_bytes || nP * sizeof(cucd_search_result) > s.out_bytes || s.out_off + s.out_bytes > hdr->arena_bytes) {
+            reply(s, CUCD_ERR_INVALID, "cucd_me_tz_search: request and reply sizes disagree");
+            break;
+          }
+          const int rc = k.h ? cucd_me_tz_search(k.h, s.n, reinterpret_cast<const cucd_tz_desc*>(in), reinterpret_cast<cucd_search_result*>(out)) : CUCD_ERR_INVALID;
+          reply(s, rc, rc == CUCD_OK ? nullptr : cucd_last_error(k.h));
+          break;
+        }
         default:
           reply(s, CUCD_ERR_INVALID, "unknown request");
       }
@@ -289,10 +299,10 @@ int main(int argc, char** argv) {
   if (segPinned) cudaHostUnregister(mem);
   printf("{\"clients\": %d, \"closed\": %d, \"seconds\": %.3f, \"rmd_requests\": %lld, \"rmd_pus\": %lld, \"rmd_batches\": %lld, \"pus_per_batch\": %.1f, "
          "\"requests_per_batch\": %.2f, \"max_batch_pus\": %lld, \"rmd_busy_seconds\": %.3f, \"frames\": %lld, \"me_surfaces\": %lld, \"subpel\": %lld, "
-         "\"mc\": %lld, \"mc_chroma\": %lld, \"search\": %lld, \"set_ref\": %lld, \"window_us\": %.1f, \"segment_pinned\": %s}\n",
+         "\"mc\": %lld, \"mc_chroma\": %lld, \"search\": %lld, \"tz\": %lld, \"set_ref\": %lld, \"window_us\": %.1f, \"segment_pinned\": %s}\n",
          nSeen, nClosed, (now_us() - t0) * 1e-6, rmdReqs, rmdPus, rmdBatches, rmdBatches ? (double)rmdPus / rmdBatches : 0.0,
          rmdBatches ? (double)rmdReqs / rmdBatches : 0.0, maxBatchPus, rmdBusyUs * 1e-6, nReq[CUCD_IPC_FRAME], nReq[CUCD_IPC_ME_SURFACE], nReq[CUCD_IPC_SUBPEL],
-         nReq[CUCD_IPC_MC], nReq[CUCD_IPC_MC_CHROMA], nReq[CUCD_IPC_ME_SEARCH], nReq[CUCD_IPC_SET_REF], windowUs, segPinned ? "true" : "false");
+         nReq[CUCD_IPC_MC], nReq[CUCD_IPC_MC_CHROMA], nReq[CUCD_IPC_ME_SEARCH], nReq[CUCD_IPC_ME_TZ_SEARCH], nReq[CUCD_IPC_SET_REF], windowUs, segPinned ? "true" : "false");
   munmap(mem, total);
   shm_unlink(name.c_str());
   return 0;

@@ -9,7 +9,7 @@
  * own slot + arena and sleeps on a futex; the server turns everything that is pending into one batch per request kind.
  *   S2  (cucd_intra_rmd_batch)   stateless: requests of ALL instances with the same bit depth are coalesced into one batch
  *   S1  (cuCUDecide_frame), S3 (cucd_set_cur/ref_picture, cucd_me_sad_surface), sub-pel (cucd_me_subpel_cost), inter candidates
- *        (cucd_me_mc_cost, cucd_set_ref/cur_picture_chroma, cucd_me_mc_chroma), motion search (cucd_me_search; the _src form stays
+ *        (cucd_me_mc_cost, cucd_set_ref/cur_picture_chroma, cucd_me_mc_chroma), motion search (cucd_me_search, cucd_me_tz_search; the _src form stays
  *        in process): served on the instance's own handle inside the server (they depend on that instance's pictures), in
  *        arrival order.  A server that predates an op answers it with CUCD_ERR_INVALID, "unknown request".
  * The client side below is header-only C++ (what the reference's shim includes); the entry points mirror the C ABI of
@@ -38,7 +38,8 @@
 #define CUCD_IPC_ARENA_BYTES ((size_t)96 << 20)      /* request + reply payload of one instance (a padded 2160p plane is 34 MB) */
 
 enum cucd_ipc_op { CUCD_IPC_OPEN = 1, CUCD_IPC_CLOSE, CUCD_IPC_FRAME, CUCD_IPC_RMD, CUCD_IPC_SET_CUR, CUCD_IPC_SET_REF, CUCD_IPC_ME_SURFACE, CUCD_IPC_SUBPEL,
-                   CUCD_IPC_MC, CUCD_IPC_SET_REF_CHROMA, CUCD_IPC_SET_CUR_CHROMA, CUCD_IPC_MC_CHROMA, CUCD_IPC_ME_SEARCH };
+                   CUCD_IPC_MC, CUCD_IPC_SET_REF_CHROMA, CUCD_IPC_SET_CUR_CHROMA, CUCD_IPC_MC_CHROMA, CUCD_IPC_ME_SEARCH,
+                   CUCD_IPC_ME_TZ_SEARCH };
 enum cucd_ipc_state { CUCD_IPC_FREE = 0, CUCD_IPC_IDLE = 1, CUCD_IPC_READY = 2, CUCD_IPC_DONE = 3, CUCD_IPC_CLOSED = 4 };
 
 struct alignas(128) cucd_ipc_slot {
@@ -224,6 +225,20 @@ struct cucd_ipc_client {
     }
     memcpy(arena, desc, inBytes);
     const int rc = call(CUCD_IPC_ME_SEARCH, nPU, inBytes, outBytes);
+    if (rc == CUCD_OK) memcpy(out, reply(), outBytes);
+    return rc;
+  }
+  /* cucd_me_tz_search: reply = one cucd_search_result per PU */
+  int me_tz_search(int nPU, const cucd_tz_desc* desc, cucd_search_result* out) {
+    if (nPU < 0 || (nPU > 0 && (!desc || !out))) { snprintf(err, sizeof err, "me_tz_search: bad argument"); return CUCD_ERR_INVALID; }
+    const size_t inBytes = (size_t)nPU * sizeof(cucd_tz_desc), outBytes = (size_t)nPU * sizeof(cucd_search_result);
+    if (((inBytes + 255) & ~(size_t)255) + outBytes > hdr->arena_bytes) {
+      snprintf(err, sizeof err, "me_tz_search: %d PUs need %llu bytes, more than the %llu-byte arena", nPU,
+               (unsigned long long)(((inBytes + 255) & ~(size_t)255) + outBytes), (unsigned long long)hdr->arena_bytes);
+      return CUCD_ERR_NOMEM;
+    }
+    memcpy(arena, desc, inBytes);
+    const int rc = call(CUCD_IPC_ME_TZ_SEARCH, nPU, inBytes, outBytes);
     if (rc == CUCD_OK) memcpy(out, reply(), outBytes);
     return rc;
   }

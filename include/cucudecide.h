@@ -316,6 +316,55 @@ int cucd_me_search(cucd_handle* h, int nPU, const cucd_search_desc* desc, cucd_s
 int cucd_me_search_src(cucd_handle* h, int nPU, const cucd_search_desc* desc, const int16_t* src, cucd_search_result* out);
 
 /* ------------------------------------------------------------------------------------------------
+ * TZ search: HM's xTZSearch integer walk and, with CUCD_SEARCH_FRAC, the refinement walk of cucd_me_search around its result, one
+ * motion vector per PU and reference in one call: what xMotionEstimation runs when m_iFastSearch && !bBi (--FastSearch=1).
+ * Nothing but the result leaves the GPU.  TZ_SEARCH_CONFIGURATION: iRaster 5, zero-vector test on, first search diamond with
+ * stop after 3 rounds, raster on (not always), raster refinement off, star refinement diamond with no stop.
+ *   probe(x, y, p, d): c = SAD(x, y) + cost_2(x, y) (SAD and cost_2 as cucd_me_search, including the generic widths' iSubShift 0);
+ *     if c < best: best = c, b = (x, y), dist = d, round = 0, pt = p.  win = [left, right] x [top, bottom]; box = the clip box.
+ *   1. best = ~0; probe(clamp(pred_x, 4 clip_left, 4 clip_right) >> 2, (the same for y), 0, 0) (arithmetic shift); probe(0, 0, 0, 0);
+ *      with CUCD_SEARCH_TZ_2NX2N probe(clamp(mv2n into box), 0, 0) and rwin = (b +- search_range) clamped into box, else rwin = win.
+ *   2. first search, c = b: for D = 1, 2, 4, .. <= search_range: Diamond(c, D); break when round >= 3.
+ *   3. if dist == 1: dist = 0, TwoPoint.   4. if dist > 5: dist = 5, probe(x, y, 0, 5) for y = rwin.top, +5, .. <= rwin.bottom (outer),
+ *      x = rwin.left, +5, .. <= rwin.right (inner).
+ *   5. while dist > 0: c = b, dist = 0, pt = 0; Diamond(c, D) for every D = 1, 2, .. <= search_range; if dist == 1: dist = 0 and
+ *      TwoPoint when pt != 0.
+ *   6. mvx, mvy = b, sad = SAD(b); FRAC: qmv and frac_cost from cucd_me_search's walk at b, else qmv = 4 b, frac_cost = 0.
+ *   Diamond(c, D): round += 1, then the points below in this order (p, d), each skipped when it fails its guard: a point left /
+ *   right / above / below the centre must satisfy x >= left / x <= right / y >= top / y <= bottom of win.
+ *     D = 1:     (cx, cy-1) 2, (cx-1, cy) 4, (cx+1, cy) 5, (cx, cy+1) 7; d = 1.
+ *     D = 2..8:  h = D/2: (cx, cy-D) 2 D, (cx-h, cy-h) 1 h, (cx+h, cy-h) 3 h, (cx-D, cy) 4 D, (cx+D, cy) 5 D, (cx-h, cy+h) 6 h,
+ *                (cx+h, cy+h) 8 h, (cx, cy+D) 7 D.
+ *     D > 8:     q = D/4, p 0, d D: (cx, cy-D), (cx-D, cy), (cx+D, cy), (cx, cy+D), then for k = 1, 2, 3: (cx-qk, cy-D+qk),
+ *                (cx+qk, cy-D+qk), (cx-qk, cy+D-qk), (cx+qk, cy+D-qk).
+ *   TwoPoint: c = b; the two points of case pt, p 0, d 2, guarded as above: 1 (-1,0) (0,-1); 2 (-1,-1) (1,-1); 3 (0,-1) (1,0);
+ *     4 (-1,1) (-1,-1); 5 (1,-1) (1,1); 6 (-1,0) (0,1); 7 (-1,1) (1,1); 8 (1,0) (0,1), offsets from c.
+ * These rules restate HM-16.3 (xTZSearch, xTZSearchHelp, xTZ8PointDiamondSearch, xTZ2PointSearch); they are not pinned against the
+ * HM sources in this repository.
+ * Rejected with CUCD_ERR_INVALID (the handle stays usable): what cucd_me_search rejects about PU, slot, sub_shift, flags (here
+ * CUCD_SEARCH_FRAC | CUCD_SEARCH_HADAMARD | CUCD_SEARCH_TZ_2NX2N), predictor and pointers; win empty or not inside box; a box
+ * that does not contain (0, 0) or does not fit int16; a box whose blocks leave the padded plane (x + clip_left < -marginX,
+ * x + clip_right + w - 1 > W - 1 + marginX, the same vertically; with FRAC the 8-tap support: 4 samples more on each side and one
+ * more on the right / bottom, as cucd_me_search); search_range outside [0, 4095]; mv2n outside int16; with FRAC h % 4 != 0.
+ * Every probe lies in box, so the box check bounds every read (HM's clipMv area meets it with an 80-sample margin).  nPU == 0 is
+ * a no-op.
+ * ---------------------------------------------------------------------------------------------- */
+typedef struct {
+  int x, y, w, h;                /* PU, as cucd_me_desc */
+  int ref_idx;                   /* cucd_set_ref_picture slot */
+  int left, right, top, bottom;  /* cMvSrchRngLT / RB of xMotionEstimation (xSetSearchRange around the predictor), integer pels */
+  int sub_shift;                 /* iSubShift of xTZSearchHelp (FEN and rows > 8), as cucd_me_desc */
+  int pred_x, pred_y;            /* m_mvPredictor, quarter pels, each in [-2^15, 2^15 - 1] */
+  uint32_t lambda;               /* m_uiCost, as cucd_search_desc */
+  int flags;                     /* CUCD_SEARCH_FRAC | CUCD_SEARCH_HADAMARD | CUCD_SEARCH_TZ_2NX2N */
+  int search_range;              /* m_iSearchRange: diamond distances 1, 2, 4, .. <= search_range; raster re-centring range */
+  int clip_left, clip_right, clip_top, clip_bottom;  /* TComDataCU::clipMv of the PU's CU, integer pels (HM's quarter-pel bounds >> 2) */
+  int mv2n_x, mv2n_y;            /* m_integerMv2Nx2N[list][ref], integer pels; a start point when CUCD_SEARCH_TZ_2NX2N */
+} cucd_tz_desc;
+#define CUCD_SEARCH_TZ_2NX2N 4     /* xTZSearch's pIntegerMv2Nx2NPred: start at mv2n and re-centre the raster window on the best start */
+int cucd_me_tz_search(cucd_handle* h, int nPU, const cucd_tz_desc* desc, cucd_search_result* out);
+
+/* ------------------------------------------------------------------------------------------------
  * Intra luma TU coding (SURVEY.md 8f.2): the arithmetic of TEncSearch::xIntraCodingTUBlock (TEncSearch.cpp:1092-1387) for a
  * batch of luma TUs with caller-supplied borders, packed like S2: org holds the N*N source blocks back to back, border
  * the 4N+1 unfiltered reference arrays; coef / level / pred / reco use the layout of org (N*N per TU, row-major; coefficient
@@ -469,7 +518,7 @@ int cucd_set_rmd_path(cucd_handle* h, int path);
  * the number of calls averaged, or a negative status; *avg_ms = mean duration of one launch. */
 int cucd_rmd_kernel_time(cucd_handle* h, int nCalls, float* avg_ms);
 /* Device time between the first and the last kernel of the most recent batch call on this handle (cucd_intra_rmd_batch,
- * cucd_me_sad_surface, cucd_me_subpel_cost, cucd_me_search, cucd_me_mc_cost, cucd_me_mc_chroma, cucd_intra_tu_*, cucd_inter_tu_*, cucd_tmv_features, cucd_aq_activity): CUDA events on
+ * cucd_me_sad_surface, cucd_me_subpel_cost, cucd_me_search, cucd_me_tz_search, cucd_me_mc_cost, cucd_me_mc_chroma, cucd_intra_tu_*, cucd_inter_tu_*, cucd_tmv_features, cucd_aq_activity): CUDA events on
  * the library's stream, host<->device
  * copies outside.  What bench_rows.py reports as the kernel-only figure of those paths.  A call small enough for the
  * zero-copy path (its kernels read and write page-locked host memory; CUCD_DIRECT_LIMIT bytes, 96 KB by default) is not
