@@ -24,7 +24,8 @@ constexpr int kMeRefRows = 64 + kMeTileY;
 
 // SIGNED: the source blocks are caller-supplied and may hold any int16 (the bi-predictive search compares 2 * org - other prediction,
 // TEncSearch.cpp:3787-3797): |a - b| per half through the signed SIMD intrinsic instead of max - min of packed words, whose 32-bit
-// subtraction would borrow across the halves for negative samples.
+// subtraction would borrow across the halves for negative samples.  A half of that difference reaches 65535 (key -32768 against a
+// reference sample of 32767), so the halves are summed as unsigned (IDP.2A.U16): the signed form would read 32768 .. 65535 as negative.
 // OUT (all three SAD kernels): Surface stores every candidate's SAD at out[outOff + dy * cols + dx]; Argmin folds the candidates
 // of a warp into the least search key (me_core.cuh, me_search_key) and commits it to am.keys[job] instead.
 template <bool SIGNED, MeOut OUT = MeOut::Surface>
@@ -69,8 +70,8 @@ me_sad_kernel(const MePlanes mp, const MeJob* __restrict__ jobs, const int32_t* 
       const uint32_t next = rw[rbase + j + 1];
       const uint32_t r = funnel_r(prev, next, e16);
       const uint32_t c = cw[cbase + j];
-      const uint32_t d = SIGNED ? __vabsdiffs2(c, r) : __vmaxs2(c, r) - __vmins2(c, r);
-      acc = __dp2a_lo((int)d, 0x0101, acc);
+      if constexpr (SIGNED) acc = (int)__dp2a_lo(__vabsdiffs2(c, r), 0x0101u, (uint32_t)acc);
+      else acc = __dp2a_lo((int)(__vmaxs2(c, r) - __vmins2(c, r)), 0x0101, acc);
       prev = next;
     }
   }

@@ -97,6 +97,17 @@ def textured_plane(W, H, bit_depth=8, seed=20261018, t=0):
     return Y.astype(np.int16)
 
 
+def full_range_keys(rng, shape):
+    """caller-supplied source keys from all of int16 (the `_src` calls accept any value): uniform samples with runs of -32768 and of
+    32767 along the last axis.  Against a reference sample r, a key k gives |k - r| up to 65535, beyond the int16 range of a half-word"""
+    k = rng.integers(-32768, 32768, shape)
+    flat = k.reshape(-1)
+    for v in (-32768, 32767):
+        for s in rng.integers(0, flat.size, max(1, flat.size // 64)):
+            flat[s:s + int(rng.integers(4, 40))] = v
+    return k.astype(np.int16)
+
+
 def pseudo_recon(org, bit_depth=8, seed=7):
     """A stand-in reconstruction: the source low-passed a little plus small noise (what a codec's
     reconstruction looks like statistically), so that borders differ from the source."""

@@ -114,6 +114,24 @@ def oracle_tz_rows(lib, sc, descs):
     return np.stack([oracle_tz(lib, sc, d)[0] for d in descs]) if descs else np.zeros((0, 6), np.int64)
 
 
+def emul_tz(emul, sc, d, cap=200000):
+    """(res (6,) int64, trace (n, 6) int64, points evaluated, lanes per probe) of the CPU replay of me_tz_kernel for one PU: the integer
+    result and the points of every folded segment"""
+    res = np.zeros(6, np.int32)
+    tr = np.zeros((cap, 6), np.int32)
+    ev, lanes = np.zeros(1, np.int32), np.zeros(1, np.int32)
+    blk = src_block(sc, d)
+    row = desc_row(d)
+    n = emul.emul_me_tz_search(sc["bd"], P(blk, i16p), d["w"], ref_base(sc, d), sc["refs"][d["ref_idx"]].shape[1], P(row, i32p), P(res, i32p), tr.ctypes.data,
+                               cap, ev.ctypes.data, lanes.ctypes.data)
+    assert 0 <= n <= cap
+    out = res.astype(np.int64)
+    out[2] = int(res[2]) & 0xFFFFFFFF
+    t = tr[:n].astype(np.int64)
+    t[:, 5] &= 0xFFFFFFFF
+    return out, t, int(ev[0]), int(lanes[0])
+
+
 # ---- an independent statement of the walk --------------------------------------------------------------------------------------
 def py_bits(v):
     t = -2 * v + 1 if v <= 0 else 2 * v

@@ -247,7 +247,7 @@ def test_me_dy_lane_kernel_code_extreme_values(emul, oracle, bd):
             _emul_me_surface(emul, oracle, bd, cur, refp, M, x, y, w, h, -32, 32, -40, 31, sub)
 
 
-@pytest.mark.parametrize("bd", [8, 10])
+@pytest.mark.parametrize("bd", [8, 9, 10])
 def test_subpel_small_pu_kernel_code_vs_oracle(emul, oracle, bd):
     """me_subpel_small_kernel (one CTA per PU, all 49 quarter-pel positions; csrc/me_core.cuh) against the oracle's restatement of
     xPatternSearchFracDIF (TEncSearch.cpp:4340-4376): every PU shape with w * h <= 256 HM has, Hadamard and SAD, textured and

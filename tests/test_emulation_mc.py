@@ -28,7 +28,7 @@ def check(emul, mco, sc, descs):
     return n_cta
 
 
-@pytest.mark.parametrize("bd", [8, 10])
+@pytest.mark.parametrize("bd", [8, 9, 10])
 def test_emul_mc_matches_oracle_in_one_mixed_batch(emul, mco, bd):
     sc = mc_scene(bd, seed=bd)
     rng = np.random.default_rng(bd + 1)
@@ -38,7 +38,7 @@ def test_emul_mc_matches_oracle_in_one_mixed_batch(emul, mco, bd):
     assert n_cta < len(descs)                                # small candidates share CTAs
 
 
-@pytest.mark.parametrize("bd", [8, 10])
+@pytest.mark.parametrize("bd", [8, 9, 10])
 def test_emul_mc_packs_many_small_candidates(emul, mco, bd):
     """one class per shape with more candidates than a CTA holds: the last CTA of a class is partial"""
     sc = mc_scene(bd, seed=20 + bd)
@@ -49,7 +49,7 @@ def test_emul_mc_packs_many_small_candidates(emul, mco, bd):
     check(emul, mco, sc, descs)
 
 
-@pytest.mark.parametrize("bd", [8, 10])
+@pytest.mark.parametrize("bd", [8, 9, 10])
 def test_emul_mc_every_fraction_pair(emul, mco, bd):
     sc = mc_scene(bd, seed=30 + bd)
     descs = []

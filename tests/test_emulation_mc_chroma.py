@@ -30,7 +30,7 @@ def check(emul, mco, sc, descs):
     return n_cta
 
 
-@pytest.mark.parametrize("bd", [8, 10])
+@pytest.mark.parametrize("bd", [8, 9, 10])
 def test_emul_mc_chroma_matches_oracle_in_one_mixed_batch(emul, mco, bd):
     sc = mcc_scene(bd, seed=bd)
     rng = np.random.default_rng(bd + 1)
@@ -40,7 +40,7 @@ def test_emul_mc_chroma_matches_oracle_in_one_mixed_batch(emul, mco, bd):
     assert n_cta < len(descs)                                # small candidates share CTAs
 
 
-@pytest.mark.parametrize("bd", [8, 10])
+@pytest.mark.parametrize("bd", [8, 9, 10])
 def test_emul_mc_chroma_packs_many_small_candidates(emul, mco, bd):
     """more candidates of one class than a CTA holds (64 of a 2x4 chroma block): the last CTA of a class is partial"""
     sc = mcc_scene(bd, seed=20 + bd)
@@ -52,7 +52,7 @@ def test_emul_mc_chroma_packs_many_small_candidates(emul, mco, bd):
     assert n_cta > 6                                         # six classes; 70 uni 2x4 blocks take two CTAs
 
 
-@pytest.mark.parametrize("bd", [8, 10])
+@pytest.mark.parametrize("bd", [8, 9, 10])
 def test_emul_mc_chroma_every_fraction_pair(emul, mco, bd):
     sc = mcc_scene(bd, seed=30 + bd)
     descs = []

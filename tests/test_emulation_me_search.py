@@ -53,7 +53,7 @@ def want_keys(mso, sc, descs, src=None):
     return out
 
 
-@pytest.mark.parametrize("bd", [8, 10])
+@pytest.mark.parametrize("bd", [8, 9, 10])
 def test_argmin_epilogue_matches_checker(emul, mso, oracle, bd):
     sc = mc_scene(bd, seed=50 + bd)
     rng = np.random.default_rng(bd + 7)

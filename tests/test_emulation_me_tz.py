@@ -1,11 +1,10 @@
 """CPU replay of me_tz_kernel (tests/emul/me_tz_emul.cpp: the me_tz_* phases of csrc/me_core.cuh with the kernel's lane mapping and its
 two xor butterflies) against the checker tests/me_tz_oracle.c: the points of every stage with their values, in HM's order, and the
-final integer result, at 8 and 10 bit, with extreme sample values."""
+final integer result, at 8, 9 and 10 bit, with extreme sample values."""
 import numpy as np
 import pytest
 
-from _util import P, i16p, i32p
-from me_tz_util import FRAC, HAD, MC_SHAPES, TZ2N, desc_row, lambda_cost, load_me_tz_emul, load_me_tz_oracle, mc_scene, oracle_tz, ref_base, src_block, tz_desc
+from me_tz_util import FRAC, HAD, MC_SHAPES, TZ2N, emul_tz, lambda_cost, load_me_tz_emul, load_me_tz_oracle, mc_scene, oracle_tz, tz_desc
 
 
 @pytest.fixture(scope="module")
@@ -18,27 +17,11 @@ def emul():
     return load_me_tz_emul()
 
 
-def replay(emul, sc, d, cap=200000):
-    res = np.zeros(6, np.int32)
-    tr = np.zeros((cap, 6), np.int32)
-    ev, lanes = np.zeros(1, np.int32), np.zeros(1, np.int32)
-    blk = src_block(sc, d)
-    row = desc_row(d)
-    n = emul.emul_me_tz_search(sc["bd"], P(blk, i16p), d["w"], ref_base(sc, d), sc["refs"][d["ref_idx"]].shape[1], P(row, i32p), P(res, i32p), tr.ctypes.data,
-                               cap, ev.ctypes.data, lanes.ctypes.data)
-    assert 0 <= n <= cap
-    out = res.astype(np.int64)
-    out[2] = int(res[2]) & 0xFFFFFFFF
-    t = tr[:n].astype(np.int64)
-    t[:, 5] &= 0xFFFFFFFF
-    return out, t, int(ev[0]), int(lanes[0])
-
-
 def check(tz, emul, sc, descs):
     lanes, extra = set(), 0
     for d in descs:
         want, wtrace, nprobe = oracle_tz(tz, sc, dict(d, flags=d["flags"] & ~(FRAC | HAD)), trace_cap=200000)
-        got, gtrace, ev, g = replay(emul, sc, d)
+        got, gtrace, ev, g = emul_tz(emul, sc, d)
         assert np.array_equal(got[:3], want[:3]), d
         assert np.array_equal(gtrace, wtrace), d                       # every stage's points, values and order
         assert ev >= nprobe
@@ -62,7 +45,7 @@ def descs_for(sc, rng, shapes=MC_SHAPES):
     return out
 
 
-@pytest.mark.parametrize("bd", [8, 10])
+@pytest.mark.parametrize("bd", [8, 9, 10])
 def test_replay_matches_checker_on_pictures(tz, emul, bd):
     sc = mc_scene(bd, seed=bd + 90)
     lanes, extra = check(tz, emul, sc, descs_for(sc, np.random.default_rng(bd + 90)))
@@ -70,7 +53,7 @@ def test_replay_matches_checker_on_pictures(tz, emul, bd):
     assert extra > 0                                                   # chunks past the first search's stop were evaluated and dropped
 
 
-@pytest.mark.parametrize("bd", [8, 10])
+@pytest.mark.parametrize("bd", [8, 9, 10])
 def test_replay_matches_checker_on_extreme_samples(tz, emul, bd):
     """source at 2^bd - 1, references of 0 and 2^bd - 1: the largest SADs and sums the kernel forms"""
     sc = mc_scene(bd, seed=bd + 95)

@@ -182,7 +182,7 @@ def test_bench_me_workload_device_resident(cucd, oracle, name):
                 assert np.array_equal(_u32(d_sub[i]), _oracle_subpel(oracle, bd, cur, refs[k], M, sp[k][i])), (name, k, sp[k][i])
 
 
-@pytest.mark.parametrize("bd,n_refs", [(8, 1), (10, 2)])
+@pytest.mark.parametrize("bd,n_refs", [(8, 1), (9, 2), (10, 2)])
 def test_small_picture_me_device_resident_vs_oracle(cucd, oracle, bd, n_refs):
     """416x240 (partial CTUs on the bottom edge): every square PU, every candidate and every sub-pel table against the oracle"""
     torch, _ = _torch()

@@ -46,7 +46,7 @@ def check_all_calls(eng, ito, bd, tus, res):
             assert np.array_equal(rresi[sl], w["rresi"]) and dist[i] == w["dist"], key
 
 
-@pytest.mark.parametrize("bd", [8, 10])
+@pytest.mark.parametrize("bd", [8, 9, 10])
 def test_random_batches_vs_checker(cucd, ito, bd):
     """shuffled sizes (size bucketing and the scatter back to caller order), in a small batch and in one of 6000 TUs that spans
     several waves of CTAs"""
@@ -80,7 +80,7 @@ def test_encoder_tu_records_through_the_inter_calls(cucd, ito, clip):
         assert np.array_equal(rresi[sl], w["rresi"]) and dist[i] == w["dist"] and dz[i] == w["dist_zero"]
 
 
-@pytest.mark.parametrize("bd", [8, 10])
+@pytest.mark.parametrize("bd", [8, 9, 10])
 def test_extreme_residuals(cucd, ito, bd):
     """+-(2^bd - 1) constant and checkerboard blocks at every size (luma, chroma, transform skip), low and high QP; an all-zero
     residual gives abs_sum 0 and dist 0"""

@@ -33,7 +33,7 @@ def assert_equal(descs, got_d, got_p, want_d, want_p):
         assert got_d[i] == want_d[i], d
 
 
-@pytest.mark.parametrize("bd", [8, 10])
+@pytest.mark.parametrize("bd", [8, 9, 10])
 def test_mc_vs_oracle_mixed_batch_and_single_candidates(cucd, mco, bd):
     """the coverage of test_emulation_mc.py: 22 shapes x (uni L0, uni L1, bi, bi with identical motion) x (Hadamard, SAD), random and
     extreme fractions, supports at the margin's corners; in one mixed batch and as batches of one candidate"""

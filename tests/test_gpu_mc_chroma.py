@@ -37,7 +37,7 @@ def assert_equal(descs, got_s, got_p, want_s, want_p):
         assert np.array_equal(got_s[i], want_s[i]), d
 
 
-@pytest.mark.parametrize("bd", [8, 10])
+@pytest.mark.parametrize("bd", [8, 9, 10])
 def test_mc_chroma_vs_oracle_mixed_batch_and_single_candidates(cucd, mco, bd):
     """the coverage of test_emulation_mc_chroma.py: the chroma blocks of 22 PU shapes x (uni L0, uni L1, bi, bi with identical
     motion), random and extreme eighth-pel fractions, supports at the chroma margin's corners; in one mixed batch and one per call"""

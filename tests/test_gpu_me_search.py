@@ -9,7 +9,7 @@ import time
 import numpy as np
 import pytest
 
-from _util import ROOT, pseudo_recon, textured_plane
+from _util import ROOT, full_range_keys, pseudo_recon, textured_plane
 from me_search_util import (FRAC, HAD, LAMBDAS, MC_SHAPES, as_rows, lambda_cost, load_me_search_oracle, mc_scene, np_bits, np_walk, oracle_search,
                             search_desc, search_descs, walk_batch)
 
@@ -34,7 +34,7 @@ def assert_rows(descs, got, want):
         assert np.array_equal(got[i], want[i]), (d, got[i], want[i])
 
 
-@pytest.mark.parametrize("bd", [8, 10])
+@pytest.mark.parametrize("bd", [8, 9, 10])
 def test_search_vs_checker_mixed_batch_and_single_pus(cucd, mso, bd):
     """22 shapes x (+-64, +-4, 1x1) x (FRAC + Hadamard, FRAC + SAD, integer only), lambdas {0, QP 22, QP 37, 2^32 - 1}, predictors
     anywhere in int16, windows clipped at the corners, sub_shift 0 and 1: one shuffled batch, then batches of one PU"""
@@ -50,14 +50,26 @@ def test_search_vs_checker_mixed_batch_and_single_pus(cucd, mso, bd):
             assert np.array_equal(as_rows(eng.me_search([descs[i]]))[0], want[i]), descs[i]
 
 
-@pytest.mark.parametrize("bd", [8, 10])
-def test_search_src_signed_keys(cucd, mso, bd):
-    """caller-supplied keys outside [0, 2^bd), as the bi-predictive refinement sends them"""
+@pytest.mark.parametrize("bd,keys", [pytest.param(bd, k, id=str(bd) if k == "hm" else f"{bd}-{k}") for k in ("hm", "int16") for bd in (8, 9, 10)])
+def test_search_src_signed_keys(cucd, mso, bd, keys):
+    """caller-supplied keys outside [0, 2^bd), as the bi-predictive refinement sends them.  keys "int16": samples from all of int16 with
+    runs of both ends and whole blocks of -32768 against the scene's reference runs of 0 and 2^bd - 1, in +-40 windows (several dx-lane
+    tiles a row)"""
     sc = mc_scene(bd, seed=bd + 200)
     rng = np.random.default_rng(bd + 200)
-    descs = search_descs(sc, rng, radii=(8, 4, 0))
+    descs = search_descs(sc, rng, radii=(8, 4, 0) if keys == "hm" else (40, 8, 0))
     hi = 1 << bd
-    src = rng.integers(-hi, 2 * hi, sum(d["w"] * d["h"] for d in descs)).astype(np.int16)
+    n = sum(d["w"] * d["h"] for d in descs)
+    if keys == "hm":
+        src = rng.integers(-hi, 2 * hi, n).astype(np.int16)
+    else:
+        src = full_range_keys(rng, n)
+        off = 0
+        for i, d in enumerate(descs):
+            if i % 4 == 0:
+                src[off:off + d["w"] * d["h"]] = -32768
+            off += d["w"] * d["h"]
+        assert max(d["right"] - d["left"] + 1 for d in descs) > 64
     want = oracle_search(mso, sc, descs, src)
     with cucd.Engine(sc["W"], sc["H"], bit_depth=bd) as eng:                 # no current picture needed
         for s, p in sc["refs"].items():

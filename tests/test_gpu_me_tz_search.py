@@ -71,7 +71,7 @@ def assert_rows(descs, got, want):
         assert np.array_equal(got[i], want[i]), (d, got[i], want[i])
 
 
-@pytest.mark.parametrize("bd", [8, 10])
+@pytest.mark.parametrize("bd", [8, 9, 10])
 @pytest.mark.parametrize("kind", ["moving", "unrelated", "constant"])
 def test_tz_search_vs_checker(cucd, tz, bd, kind):
     """22 shapes x (FRAC + Hadamard, FRAC + SAD, integer only) x (with and without TZ_2NX2N), lambdas {0, QP 22, QP 37, 2^32 - 1}: one

@@ -64,7 +64,7 @@ def test_rmd_batch_edge_cases(eng8, oracle):
             assert np.array_equal(got[k], want), (n, k)
 
 
-@pytest.mark.parametrize("bd", [8, 10])
+@pytest.mark.parametrize("bd", [8, 9, 10])
 def test_rmd_batch_extreme_values(cucd, oracle, bd):
     hi = (1 << bd) - 1
     with cucd.Engine(64, 64, bit_depth=bd) as eng:
@@ -192,7 +192,7 @@ def test_me_probes_vs_reference_encoder_dump(cucd):
             assert s.shape == (1, 1) and int(s[0, 0]) == int(sad), (cols, rows, sub)
 
 
-@pytest.mark.parametrize("bd", [8, 10])
+@pytest.mark.parametrize("bd", [8, 9, 10])
 def test_me_surfaces_vs_oracle(cucd, oracle, bd):
     W, H, M = 192, 128, 80
     cur = textured_plane(W, H, bd, seed=21, t=1)
@@ -295,7 +295,7 @@ def test_half_precision_tensor_core_path_extreme_values(cucd, oracle):
 
 
 # ---- packed cost tables (cucd_frame_out.rmd_cost_packed) carry the same numbers -------------------------------
-@pytest.mark.parametrize("bd,W,H", [(8, 200, 136), (10, 136, 72)])
+@pytest.mark.parametrize("bd,W,H", [(8, 200, 136), (9, 104, 88), (10, 136, 72)])
 def test_packed_cost_tables_equal_wide_tables(cucd, oracle, bd, W, H):
     org = textured_plane(W, H, bd, seed=11)
     rec = pseudo_recon(org, bd)
@@ -504,7 +504,7 @@ def test_texture_features_vs_reference_golden(cucd, tag):
             eng.aq_activity(5)
 
 
-@pytest.mark.parametrize("bd", [8, 10])
+@pytest.mark.parametrize("bd", [8, 9, 10])
 def test_texture_features_vs_oracle_1080p_rows(cucd, oracle, bd):
     from _util import all_cus, oracle_aq_activity, oracle_tmv_features
     W, H = 1920, 1080

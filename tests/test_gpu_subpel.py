@@ -6,7 +6,7 @@ import ctypes as C
 import numpy as np
 import pytest
 
-from _util import P, frac_records, golden, i16p, u32p, pseudo_recon, textured_plane
+from _util import P, frac_records, full_range_keys, golden, i16p, u32p, pseudo_recon, textured_plane
 
 pytestmark = pytest.mark.gpu
 
@@ -37,7 +37,7 @@ def test_subpel_vs_reference_encoder_dump(cucd, clip):
     assert done == len(recs)
 
 
-@pytest.mark.parametrize("bd", [8, 10])
+@pytest.mark.parametrize("bd", [8, 9, 10])
 def test_subpel_vs_oracle(cucd, oracle, bd):
     W, H, M = 416, 240, 80
     org = textured_plane(W, H, bd, seed=21)
@@ -70,29 +70,42 @@ def test_subpel_vs_oracle(cucd, oracle, bd):
         assert np.array_equal(got[i].ravel(), want), d
 
 
-@pytest.mark.parametrize("bd", [8, 10])
-def test_bipred_key_blocks_vs_oracle(cucd, oracle, bd):
+@pytest.mark.parametrize("bd,keys", [pytest.param(bd, k, id=str(bd) if k == "hm" else f"{bd}-{k}") for k in ("hm", "int16") for bd in (8, 9, 10)])
+def test_bipred_key_blocks_vs_oracle(cucd, oracle, bd, keys):
     """cucd_me_sad_surface_src / cucd_me_subpel_cost_src: the bi-predictive refinement of xMotionEstimation (TEncSearch.cpp:3787-3849)
     searches with the key 2 * org - prediction of the other list (TComYuv::removeHighFreq): samples below 0 and above the bit depth's
-    range, caller-supplied blocks instead of the current picture.  Integer search (+-4, xPatternSearch) and the 49 sub-pel positions."""
+    range, caller-supplied blocks instead of the current picture.  Integer search (+-4, xPatternSearch) and the 49 sub-pel positions.
+    keys "int16": what the header allows beyond HM's keys - samples from all of int16 with runs of both ends, whole blocks of -32768
+    against reference runs of 0 and 2^bd - 1 (|key - ref| up to 32768 + 2^bd - 1), and +-40 windows (several dx-lane tiles a row)."""
     W, H, M = 256, 128, 80
     hi = (1 << bd) - 1
-    org = textured_plane(W, H, bd, seed=33).astype(np.int32)
-    other = pseudo_recon(textured_plane(W, H, bd, seed=34, t=2), bd).astype(np.int32)
-    other[:, ::3] = hi; other[::5, :] = 0                      # push 2 * org - other to both ends of [-hi, 2 * hi]
-    key = (2 * org - other).astype(np.int16)
-    assert key.min() < 0 and key.max() > hi
     rec = pseudo_recon(textured_plane(W, H, bd, seed=33, t=1), bd)
+    if keys == "hm":
+        org = textured_plane(W, H, bd, seed=33).astype(np.int32)
+        other = pseudo_recon(textured_plane(W, H, bd, seed=34, t=2), bd).astype(np.int32)
+        other[:, ::3] = hi; other[::5, :] = 0                  # push 2 * org - other to both ends of [-hi, 2 * hi]
+        key = (2 * org - other).astype(np.int16)
+        assert key.min() < 0 and key.max() > hi
+        R = 4
+    else:
+        key = full_range_keys(np.random.default_rng(bd + 60), (H, W))
+        rec[3::7, :] = hi; rec[:, 5::11] = 0
+        R = 40
     refp = np.pad(rec, M, mode="edge")
     rng = np.random.default_rng(8)
     shapes = [(64, 64), (32, 32), (16, 16), (8, 8), (64, 32), (16, 64), (32, 24), (12, 16), (8, 4), (4, 8)]
     me, sp, blocks = [], [], []
-    for w, h in shapes:
+    for k, (w, h) in enumerate(shapes):
         x = int(rng.integers(0, (W - w) // 4 + 1)) * 4; y = int(rng.integers(0, (H - h) // 4 + 1)) * 4
         cx, cy = int(rng.integers(-20, 21)), int(rng.integers(-20, 21))
-        me.append(dict(x=x, y=y, w=w, h=h, ref_idx=0, left=cx - 4, right=cx + 4, top=cy - 4, bottom=cy + 4, sub_shift=1 if h > 8 else 0))
+        me.append(dict(x=x, y=y, w=w, h=h, ref_idx=0, left=cx - R, right=cx + R, top=cy - R, bottom=cy + R, sub_shift=1 if h > 8 else 0))
         sp.append(dict(x=x, y=y, w=w, h=h, ref_idx=0, mvx=cx, mvy=cy, use_hadamard=int(rng.integers(0, 2))))
-        blocks.append(np.ascontiguousarray(key[y:y + h, x:x + w]))
+        blk = np.array(key[y:y + h, x:x + w])
+        if keys == "int16" and k % 3 == 0:
+            blk[:] = -32768 if k % 2 == 0 else 32767
+        blocks.append(blk)
+    if keys == "int16":
+        assert sum(b.min() == b.max() == -32768 for b in blocks) >= 2 and sum(b.min() == b.max() == 32767 for b in blocks) >= 1
     src = np.concatenate([b.ravel() for b in blocks])
     with cucd.Engine(W, H, bit_depth=bd) as eng:
         eng.set_ref_picture(0, refp, M, M)                     # no cucd_set_cur_picture: the source blocks are the caller's

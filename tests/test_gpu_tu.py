@@ -40,7 +40,7 @@ def test_tu_kernels_vs_reference_encoder_dump(cucd, clip):
             assert np.array_equal(reco2, reco) and np.array_equal(dist2, dist)
 
 
-@pytest.mark.parametrize("bd", [8, 10])
+@pytest.mark.parametrize("bd", [8, 9, 10])
 def test_tu_kernels_vs_oracle_random(cucd, oracle, bd):
     """every size x every mode, low and high QP, extreme samples, transform skip, sign hiding on/off, P-slice rounding"""
     rng = np.random.default_rng(40 + bd)
